@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — DataChunk -> Arrow materialisation throughput (BASELINE.json metric) on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--rows R]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--rows R] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload of `value` (config.workload): BASELINE.json configs[1], the synthetic lineitem-shaped table
@@ -25,6 +25,9 @@ the per-GPU string byte totals (the host exclusive scan that rebases offsets acr
   roofline     the dominant kernel family of the C2 step: algorithmic bytes / its CUDA-event time
   cpu_baseline the oracle port of the reference's getters + decoders, 1 core, <= 1 M-row sample;
   cpu_columnar an -O3 -march=native OpenMP columnar conversion on all host cores (oracle/columnar.c)
+
+`--dump-outputs DIR` writes, after the timed steps, what the last timed step of `value` computed on rank 0 (a fixed, seeded
+sample of its rows; see dump_step_outputs) as DIR/<name>.npy, so that two builds can be compared output for output.
 
 `--impl reference` times the reference's own CPU path (oracle port: the reference cannot be built
 here, SURVEY.md §8c) on the host cores.  Nothing here reads /root/reference.
@@ -51,6 +54,8 @@ CPU_SAMPLE_ROWS = 1_000_000  # the reference's decoders return [] above this (sr
 WINDOW_CHUNKS = 489          # parity windows: ~1 M rows of whole chunks
 GETTER_CHUNKS = 488          # e2e_getters results: 999 424 rows, just under the reference decoders' 1 000 000-row cap
 VS = 2048
+DUMP_ROWS = 1 << 16          # --dump-outputs: sampled rows of the C2 step (~28 MB of .npy at the default table)
+DUMP_MAX_BYTES = 64 << 20
 
 
 def env_int(name, default):
@@ -249,6 +254,59 @@ class DeviceStep:
             if self.db.string_error(so) != 0:
                 from duckdb_mbt_b200 import native as nat
                 raise RuntimeError("string kernel flagged an error: " + nat.last_error())
+
+
+def dump_step_outputs(step: DeviceStep, out_dir: str, seed: int = 0) -> dict:
+    """Write the Arrow buffers a DeviceStep's last run produced, at a fixed, seeded sample of DUMP_ROWS rows (always the
+    first and the last), as out_dir/<name>.npy:
+      rows.npy                  the sampled row indices (float64, ascending)
+      <column>.values.npy       fixed-width values (float64; decimal128 / hugeint as the unscaled integer, exact up to 2^53)
+      <column>.validity.npy     the validity bit of every sampled row (float32 0 / 1), every column
+      <column>.offsets.npy      utf8 offsets (start, end) of every sampled row (float64, shape (rows, 2))
+      <column>.data.npy         the sampled rows' utf8 bytes, concatenated in row order (float32)
+    The sample depends only on the row count and the seed, so runs with the same arguments write comparable files.
+    Returns {file name: shape}."""
+    import numpy as np
+    import torch
+    from duckdb_mbt_b200 import chunks as ch
+    db = step.db
+    n = db.nrows
+    rng = np.random.default_rng(seed)
+    rows = np.unique(np.concatenate([[0, n - 1], rng.integers(0, n, max(DUMP_ROWS - 2, 0))]))
+    idx = torch.from_numpy(rows).to(db.device)
+    out = {"rows": rows.astype(np.float64)}
+    for o in step.plan[0]:
+        name = db.batch.columns[o.col].name
+        bits = o.bitmap[: (n + 7) // 8][idx // 8].to(torch.int32) >> (idx % 8).to(torch.int32)
+        out[name + ".validity"] = (bits & 1).cpu().numpy().astype(np.float32)
+        if o.op == ch.OP_VALIDITY_ONLY:
+            continue
+        w = o.width
+        v = o.values[: n * w].view(n, w)[idx].cpu().numpy()
+        if w == 16:
+            lo, hi = v.view(np.int64)[:, 0], v.view(np.int64)[:, 1]
+            out[name + ".values"] = np.where(hi == lo >> 63, lo.astype(np.float64),
+                                             hi.astype(np.float64) * 2.0 ** 64 + lo.view(np.uint64).astype(np.float64))
+        else:
+            float_type = {4: ch.T_FLOAT, 8: ch.T_DOUBLE}.get(w)
+            dt = np.dtype(("f" if db.batch.columns[o.col].type_id == float_type else "i") + str(w))
+            out[name + ".values"] = v.view(dt).reshape(-1).astype(np.float64)
+    for so in step.strings:
+        name = db.batch.columns[so.col].name
+        offs = so.offsets[: (n + 1) * (8 if so.mode == 1 else 4)].view(torch.int64 if so.mode == 1 else torch.int32)
+        start, end = offs[idx].to(torch.int64), offs[idx + 1].to(torch.int64)
+        lens = end - start
+        first = torch.cumsum(lens, 0) - lens
+        pos = torch.repeat_interleave(start - first, lens) + torch.arange(int(lens.sum().item()), device=db.device)
+        out[name + ".offsets"] = torch.stack([start, end], dim=1).cpu().numpy().astype(np.float64)
+        out[name + ".data"] = so.data[pos].cpu().numpy().astype(np.float32)
+    total = sum(a.nbytes for a in out.values())
+    if total > DUMP_MAX_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {DUMP_MAX_BYTES}-byte cap")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    return {name: list(a.shape) for name, a in out.items()}
 
 
 # ----------------------------------------------------------------------------- parity before timing (oracle = checker)
@@ -666,6 +724,9 @@ def run_ours(args, rank, local_rank, world):
     barrier()
     dev_ms = ev_a.elapsed_time(ev_b)
     step.check()
+    if args.dump_outputs and rank == 0:
+        files = dump_step_outputs(step, args.dump_outputs)
+        print(f"bench.py: {len(files)} arrays of the last timed step written to {args.dump_outputs}", file=sys.stderr, flush=True)
     fixed_ms = sum(sp[0].elapsed_time(sp[1]) for sp in spans) / steps
     string_ms = sum(sp[1].elapsed_time(sp[2]) for sp in spans) / steps
     string_cols = [db.batch.columns[so.col].name for so in step.strings]
@@ -1110,7 +1171,13 @@ def main():
     ap.add_argument("--no-parity", action="store_true", help="skip the oracle comparison before timing")
     ap.add_argument("--no-configs", action="store_true", help="skip C1 / C3 / C4 / C5")
     ap.add_argument("--no-layout-leg", action="store_true", help="skip e2e_duckdb_layout / e2e_getters")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write a seeded row sample of what the last one "
+                                                          "computed (rank 0) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what the GPU path computed: it needs --impl ours")
     rank = env_int("RANK", 0)
     local_rank = env_int("LOCAL_RANK", 0)
     world = env_int("WORLD_SIZE", 1)

@@ -6,6 +6,7 @@ import ctypes as C
 import hashlib
 import os
 import subprocess
+import tempfile
 import time
 from typing import List, Optional
 
@@ -32,9 +33,13 @@ def lib_path() -> str:
     return os.path.join(_HERE, f"libcolumnar.{_cpu_tag()}.so")
 
 
-def build(force: bool = False) -> str:
-    src, out = os.path.join(_HERE, "columnar.c"), lib_path()
-    if force or not os.path.exists(out) or os.path.getmtime(out) < os.path.getmtime(src):
+def _stale(out: str) -> bool:
+    return not os.path.exists(out) or os.path.getmtime(out) < os.path.getmtime(os.path.join(_HERE, "columnar.c"))
+
+
+def build(force: bool = False, out: Optional[str] = None) -> str:
+    src, out = os.path.join(_HERE, "columnar.c"), out or lib_path()
+    if force or _stale(out):
         err = None
         for cc in ("/usr/bin/gcc", "gcc", os.environ.get("CC", "cc")):  # (a wrapper gcc without libgomp.spec exists in this image)
             try:
@@ -52,7 +57,12 @@ def build(force: bool = False) -> str:
 def lib():
     global _lib
     if _lib is None:
-        L = C.CDLL(build())
+        if _stale(lib_path()):
+            # not built in the tree for this CPU (the tree may be read-only): compile into a temporary directory, load, remove
+            with tempfile.TemporaryDirectory(prefix="dmb_columnar_") as tmp:
+                L = C.CDLL(build(out=os.path.join(tmp, os.path.basename(lib_path()))))
+        else:
+            L = C.CDLL(lib_path())
         L.col_fixed.restype = C.c_int64
         L.col_fixed.argtypes = [C.POINTER(OraBatch), C.c_int32, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]
         L.col_string.restype = C.c_int64

@@ -219,7 +219,7 @@ __device__ __forceinline__ uint64_t ld_status(const unsigned long long *p) {
 }
 __device__ __forceinline__ unsigned long long global_ns() { unsigned long long t; asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t)); return t; }
 
-// Two-level decoupled look-back (string_pack_kernel, string_short_kernel, list_emit_kernel).  With ~450 persistent CTAs that claim tiles two iterations ahead, the nearest
+// Two-level decoupled look-back (string_pack_kernel, enum_pack_kernel, list_emit_kernel).  With ~450 persistent CTAs that claim tiles two iterations ahead, the nearest
 // predecessor whose PREFIX is out is typically 150-300 tiles back; a tile-by-tile look-back of 256 words per round then sits
 // on the edge between one L2 round trip and two, and the launch is bistable (late prefixes make every look-back longer,
 // which makes the prefixes later: 0.82 vs 1.15-1.47 ms per 60 M rows on all-pointer columns).  So tiles also add their
@@ -240,7 +240,7 @@ __device__ __forceinline__ uint64_t lookback_groups(const unsigned long long *st
   uint64_t st0 = 0, st1 = 0, ga = 0, gb = 0;
   uint64_t prefix = 0;
   unsigned long long t0 = 0;
-  // a needed word is not out yet: poll again at once (an eager look-back -- string_short_kernel, list_emit_kernel -- starts
+  // a needed word is not out yet: poll again at once (an eager look-back -- enum_pack_kernel, list_emit_kernel -- starts
   // when its neighbours are about to publish), back off after a few tries, look at the clock every 64th.  Warp-uniform:
   // true when the wait limit has passed (flagged; the host discards the outputs).
   unsigned spins = 0;

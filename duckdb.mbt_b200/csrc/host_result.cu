@@ -555,8 +555,8 @@ int32_t string_source(Result *r, Scope &sc, int j, bool arrow_mode, bool as_text
       if (!d.data.empty() && check_cuda(cudaMemcpyAsync(d.d_data, hp + ob, d.data.size(), cudaMemcpyHostToDevice, c.s_compute), "enum dictionary data H2D")) return -1;
       r->bytes_h2d += d.offsets.size() * sizeof(uint32_t) + d.data.size();
     }
-    static const bool no_fused = getenv("DMB_ENUM_TWO_STEP") != nullptr;  // A/B: keep the string_t intermediate
-    const bool fused = arrow_mode && !no_fused && d.size() <= DMB_ENUM_FUSED_MAX_LABELS && d.max_len <= 12;
+    // one fused launch (indices -> utf8) when the dictionary fits its label table; otherwise the string_t intermediate
+    const bool fused = arrow_mode && d.size() <= DMB_ENUM_FUSED_MAX_LABELS && d.max_len <= 12;
     dmb_string_t *d_str = fused ? nullptr : (dmb_string_t *)sc.dalloc(nslots * sizeof(dmb_string_t));
     unsigned long long *d_bad = (unsigned long long *)sc.dalloc(8);
     std::vector<dmb_vec_desc> vecs((size_t)(nch > 0 ? nch : 1));
@@ -1854,16 +1854,6 @@ int32_t materialise_arrow(Result *r) {
         if (ga) return w_in[(size_t)a] < w_in[(size_t)b];              // ... by increasing copy-in
         return w_out[(size_t)a] > w_out[(size_t)b];                    // the others by decreasing copy-out
       });
-      static const bool pyramid = getenv("DMB_ORDER_PYRAMID") != nullptr;  // A/B knob: round 1's order
-      if (pyramid) {
-        std::vector<int> sorted((size_t)ncols);
-        for (int j = 0; j < ncols; ++j) sorted[(size_t)j] = j;
-        std::stable_sort(sorted.begin(), sorted.end(), [&](int a, int b) { return w_in[(size_t)a] < w_in[(size_t)b]; });
-        int front = 0, back = ncols - 1;
-        for (int k = 0; k < ncols; ++k) {
-          if (k % 2 == 0) order[(size_t)front++] = sorted[(size_t)k]; else order[(size_t)back--] = sorted[(size_t)k];
-        }
-      }
     }
     for (int k = 0; k < ncols; ++k) {
       const int j = order[(size_t)k];

@@ -15,11 +15,9 @@
 
 #include "dmb_common.cuh"
 
-#ifndef DMB_GROUP_U
-#define DMB_GROUP_U 4  // 16-byte vectors in flight per thread in the narrow-type group path
-#endif
-
 namespace dmb {
+
+constexpr int kGroupU = 4;  // 16-byte vectors in flight per thread in the narrow-type group path
 
 // ------------------------------------------------------------------ value conversions
 // duckdb_value_int64 semantics (libduckdb, un-vendored; cast failure yields 0).  Only the
@@ -262,7 +260,7 @@ template <typename S, typename D, typename F>
 __device__ __forceinline__ void convert_group(const dmb_fixed_job &job, const BatchView &b, int64_t c0, int G, F f) {
   constexpr int W = sizeof(S) > sizeof(D) ? sizeof(S) : sizeof(D);
   constexpr int R = 16 / W;
-  constexpr int U = DMB_GROUP_U;
+  constexpr int U = kGroupU;
   constexpr int VPC = kVec / R;  // vectors per full chunk
   using PS = Pack<S, R>;
   using PD = Pack<D, R>;
@@ -409,7 +407,7 @@ struct GroupOf {
   static constexpr int W = sizeof(S) > sizeof(D) ? sizeof(S) : sizeof(D);
   static constexpr int R = 16 / W;
   // validity only: one tile per warp
-  static constexpr int value = KIND == kKindValidityOnly ? kThreads / 32 : ((KIND == kKindConvert && R >= 4) ? (kThreads * DMB_GROUP_U) / (kVec / R) : 1);
+  static constexpr int value = KIND == kKindValidityOnly ? kThreads / 32 : ((KIND == kKindConvert && R >= 4) ? (kThreads * kGroupU) / (kVec / R) : 1);
 };
 
 template <typename S, typename D, typename F, int KIND>
@@ -587,7 +585,7 @@ extern "C" int32_t dmb_dev_fixed_batch(const dmb_fixed_job *jobs_dev, const dmb_
     else if ((jobs_host[j0].op & 0xff) != DMB_DST_BOOL_BITS) {
       const int wi = dmb_phys_width(jobs_host[j0].op >> 8), wo = dmb_op_out_width(jobs_host[j0].op);
       const int w = wi > wo ? wi : wo;
-      if (w > 0 && w <= 4) group = (kThreads * DMB_GROUP_U) / (kVec / (16 / w));
+      if (w > 0 && w <= 4) group = (kThreads * kGroupU) / (kVec / (16 / w));
     }
     const int64_t items = (int64_t)(j1 - j0) * ((nchunks + group - 1) / group);
     const int grid = (int)(items < max_grid ? items : max_grid);

@@ -31,22 +31,14 @@
 // front(j + 1) needs nothing from other CTAs and back(j) only look-backs over aggregates published in fronts, so the
 // resident grid cannot deadlock.  Hand-offs are named barriers (F: worker warp 0 -> L, B: L -> workers), alternating pairs.
 
-#include <stdlib.h>
-
 #include "dmb_common.cuh"
 
 namespace dmb {
 
 constexpr int kListRpt = kVec / kThreads;    // rows per worker thread: 8
 constexpr int kListCta = kThreads + 32;      // 8 worker warps + L
-#ifndef DMB_LIST_CTAS
-#define DMB_LIST_CTAS 4
-#endif
-
-#ifndef DMB_LIST_COPY_UNROLL
-#define DMB_LIST_COPY_UNROLL 4  // 16-byte vectors of the contiguous copy in flight per thread
-#endif
-constexpr int kListCopyUnroll = DMB_LIST_COPY_UNROLL;
+constexpr int kListCtas = 4;                 // CTAs per SM (launch bound)
+constexpr int kListCopyUnroll = 4;           // 16-byte vectors of the contiguous copy in flight per thread
 
 struct ListEntry {
   uint64_t offset, length;
@@ -56,9 +48,6 @@ enum { kLBarWorkers = 1, kLBarF0 = 2, kLBarF1 = 3, kLBarB0 = 4, kLBarB1 = 5 };
 __device__ __forceinline__ void lbar_sync(int id, int n) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(n) : "memory"); }
 __device__ __forceinline__ void lbar_arrive(int id, int n) { asm volatile("bar.arrive %0, %1;" ::"r"(id), "r"(n) : "memory"); }
 
-#ifndef DMB_LIST_PREFETCH
-#define DMB_LIST_PREFETCH 1
-#endif
 // [p, p + bytes) -> L2, trimmed to the whole 16-byte units inside the range (a hint: nothing outside the range is touched)
 __device__ __forceinline__ void l2_prefetch(const void *p, uint32_t bytes) {
   const uintptr_t a = (reinterpret_cast<uintptr_t>(p) + 15u) & ~(uintptr_t)15, e = (reinterpret_cast<uintptr_t>(p) + bytes) & ~(uintptr_t)15;
@@ -99,7 +88,7 @@ struct ListShared {
 };
 
 template <int W, bool LARGE>
-__global__ void __launch_bounds__(kListCta, DMB_LIST_CTAS)
+__global__ void __launch_bounds__(kListCta, kListCtas)
 list_emit_kernel(dmb_list_job job, BatchView b, unsigned long long *status, unsigned long long *flags) {
   __shared__ ListShared sm;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -124,7 +113,6 @@ list_emit_kernel(dmb_list_job job, BatchView b, unsigned long long *status, unsi
       }
       __syncwarp();
       lbar_arrive(kLBarB0 + buf, kThreads + 32);
-#if DMB_LIST_PREFETCH
       // L has time to spare: pull what the workers will read next into L2 (bulk prefetches, one instruction each) -- the entries
       // (+ mask) of the chunk after next, whose front() starts an iteration from now, and the child vector (+ its mask) of the
       // next chunk, whose back() follows that.  The workers' loads then wait for L2, not for DRAM.
@@ -148,7 +136,6 @@ list_emit_kernel(dmb_list_job job, BatchView b, unsigned long long *status, unsi
           }
         }
       }
-#endif
     }
     return;
   }
@@ -464,8 +451,6 @@ extern "C" int32_t dmb_dev_list_batch(const dmb_list_job *job, const uint32_t *c
     if (check_cuda(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, kListCta, 0), "list_emit_kernel occupancy")) return -1;
     if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
     if (per_sm < 1) { set_error("list_emit_kernel does not fit an SM"); return -1; }
-    static const int cap = getenv("DMB_LIST_MAX_CTAS") ? atoi(getenv("DMB_LIST_MAX_CTAS")) : 0;  // (A/B knob)
-    if (cap > 0 && per_sm > cap) per_sm = cap;
     const int64_t resident = (int64_t)per_sm * sms;
     const int g1 = (int)(nchunks < resident ? nchunks : resident);
     kernel<<<g1, kListCta, 0, st>>>(*job, b, status, flags);

@@ -24,19 +24,12 @@
 // malloc/strlen/memcpy getters :2474-2510 and :2699-2755.  DMB_STR_REF_BLOB reproduces the
 // getter's NUL-terminated stream (strlen semantics) instead of Arrow offsets.
 
-#include <stdlib.h>
-
 #include "dmb_common.cuh"
 
 namespace dmb {
 
-#ifndef DMB_STR_TILE_ROWS
-#define DMB_STR_TILE_ROWS 512
-#endif
-#ifndef DMB_STR_MIN_CTAS
-#define DMB_STR_MIN_CTAS 7
-#endif
-constexpr int kStrTileRows = DMB_STR_TILE_ROWS;
+constexpr int kStrTileRows = 512;
+constexpr int kStrMinCtas = 7;                          // CTAs per SM of string_batch_kernel (launch bound)
 constexpr int kStrTilesPerChunk = kVec / kStrTileRows;
 constexpr int kStrPerThread = kStrTileRows / kThreads;  // 2 consecutive rows per thread in the scan
 constexpr int kMapVecs = 2048;                          // output vectors per window (32 KiB of utf8 data)
@@ -53,14 +46,6 @@ __device__ __forceinline__ int64_t claim_tile(unsigned long long *scratch, long 
   __syncthreads();
   return (int64_t)*slot;
 }
-
-#ifdef DMB_STR_TRACE
-__device__ unsigned long long g_str_trace[40000 * 8];
-__device__ __forceinline__ unsigned long long gtimer() { unsigned long long t; asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t)); return t; }
-#define DMB_TRACE(k) do { if (threadIdx.x == 0 && blockIdx.x < 40000) g_str_trace[blockIdx.x * 8 + (k)] = gtimer(); } while (0)
-#else
-#define DMB_TRACE(k) do { } while (0)
-#endif
 
 struct StrSmem {
   uint4 str[kStrTileRows];            // string_t copies
@@ -164,7 +149,6 @@ __device__ __forceinline__ void gather_runs(StrSmem &sm, int tid, int lane, int 
       }
     }
     __syncthreads();
-    DMB_TRACE(4);
     // (b) fast pass: every warp owns an equal, contiguous share of the window's vectors; vectors
     //     inside one run are finished here, the others go to the warp's own queue
     uint16_t *my_slow = sm.slow + warp * (kMapVecs / (kThreads / 32));
@@ -241,7 +225,7 @@ __device__ __forceinline__ void gather_runs(StrSmem &sm, int tid, int lane, int 
 }
 
 template <int MODE>
-__global__ void __launch_bounds__(kThreads, DMB_STR_MIN_CTAS)
+__global__ void __launch_bounds__(kThreads, kStrMinCtas)
 string_batch_kernel(dmb_string_job job, BatchView b, unsigned long long *scratch, int64_t ntiles) {
   __shared__ StrSmem sm;
   unsigned long long *status = scratch + 2;
@@ -249,7 +233,6 @@ string_batch_kernel(dmb_string_job job, BatchView b, unsigned long long *scratch
 
   const int64_t tile = claim_tile(scratch, &sm.ticket);
   if (tile >= ntiles) return;
-  DMB_TRACE(0);
   if (tid < 17) {
     const uint32_t d = (uint32_t)tid;
     auto m = [&](uint32_t w) { return d >= 4u * w + 4u ? 0xffffffffu : (d <= 4u * w ? 0u : ((1u << (8u * (d - 4u * w))) - 1u)); };
@@ -351,12 +334,10 @@ string_batch_kernel(dmb_string_job job, BatchView b, unsigned long long *scratch
   }
   if (lane == 31) { sm.warp_sum[warp] = incl; sm.warp_run[warp] = rmax; }
   const uint32_t rmax_excl_lane = __shfl_up_sync(0xffffffffu, rmax, 1);
-  DMB_TRACE(1);
   // __syncthreads_or yields a predicate, not the OR of the values: it carries the "pointer row
   // present" bit; the (rare) error bits are reported by the thread that saw them
   if (flags & 6) atomicOr(scratch + 1, (unsigned long long)(((flags & 2) ? kErrHeapRange : 0) | ((flags & 4) ? kErrTileTooBig : 0)));
   const int tile_flags = __syncthreads_or(flags & 1);
-  DMB_TRACE(2);
   uint32_t warp_excl = 0, tile_total = 0, run_excl = 0;
 #pragma unroll
   for (int w = 0; w < kThreads / 32; ++w) {
@@ -408,7 +389,6 @@ string_batch_kernel(dmb_string_job job, BatchView b, unsigned long long *scratch
   }
   __syncthreads();
   const uint64_t base = sm.base;
-  DMB_TRACE(3);
 
   // 5. offsets
   {
@@ -475,10 +455,6 @@ string_batch_kernel(dmb_string_job job, BatchView b, unsigned long long *scratch
     return;
   }
   gather_runs<MODE>(sm, tid, lane, warp, len, my_off, total, mis, gbase, nvec);
-#ifdef DMB_STR_TRACE
-  __syncthreads();
-  DMB_TRACE(6);
-#endif
 }
 
 // ------------------------------------------------------------------ TMA-staged pack kernel
@@ -489,9 +465,10 @@ string_batch_kernel(dmb_string_job job, BatchView b, unsigned long long *scratch
 // in and out of the SM is done by the copy engine (cp.async.bulk), every long-latency step of tile
 // t+1 is issued while tile t is being packed, and the SIMT part is row-centric and small.
 //
-//   CTA = 8 (or 16) worker warps + two single-purpose warps; tiles (R*256 consecutive rows of a chunk) are
+//   CTA = NW worker warps + two single-purpose warps; tiles (NW*32*R consecutive rows of a chunk) are
 //   claimed in order from a global ticket, so every predecessor of a claimed tile is owned by a
-//   running CTA (the look-back cannot starve).
+//   running CTA (the look-back cannot starve).  NW = 8 (3 CTAs per SM) for columns with a heap and
+//   16 (2 CTAs per SM) for the lean heap-less form (pack_warps()).
 //
 //   P  claims tile j+2 (ticket, chunk metadata) and bulk-loads its string_t (and validity words)
 //      into the S buffer the workers have just left; when the workers have packed a tile it
@@ -510,42 +487,17 @@ string_batch_kernel(dmb_string_job job, BatchView b, unsigned long long *scratch
 //
 // A tile whose span or output does not fit the stages (scattered pointers, a long string) is copied
 // row by row, one warp per row and one byte per lane, straight from the heap to out_data.
-#ifdef DMB_STR_TRACE
-#define DMB_PTRACE(j, ev) do { if (blockIdx.x < 32 && (j) < 64) g_str_trace[((blockIdx.x * 64 + (j)) << 4) + (ev)] = gtimer(); } while (0)
-#else
-#define DMB_PTRACE(j, ev) do { } while (0)
-#endif
+//
+// profiles/r02_string_pack_kernel_iterations.txt has what each of these measures bought: pointer rows copied four words at
+// a time, loads first; string_t read from S in a lane-rotated order (no bank conflicts); the inlined rows' last-word select
+// as two bit tests; the two-level look-back (lookback_groups); UNIFY (inlined rows through a per-thread scratch slot and
+// the pointer rows' copy loop).
 constexpr uint32_t kPackTail = 1792;  // bytes of bookkeeping in front of the stages
-constexpr int kLookWide = 8;          // status words in flight per lane in the look-back
-#ifndef DMB_LOOK_FIRST
-#define DMB_LOOK_FIRST 8
-#endif
-constexpr int kLookFirst = DMB_LOOK_FIRST;  // ... in its first round
 constexpr int kMetaRing = 8;  // tiles j-1 (being sent) .. j+3 (ticket and metadata claimed) are alive at once
-#ifndef DMB_NOHEAP_CTAS
-#define DMB_NOHEAP_CTAS 3  // 8-worker-warp form of the heap-less pipeline (DMB_STR_PACK_NW=8): 3 CTAs/SM = 64 registers, no spills (4: 48 + spills, slower)
-#endif
-#ifndef DMB_PACK_UNROLL
-#define DMB_PACK_UNROLL 2
-#endif
-[[maybe_unused]] constexpr int kPackUnroll = DMB_PACK_UNROLL;  // words in flight per thread in the pointer-row copy loop (DMB_PACK_CHUNK=0 only)
-// A/B knobs of the pack kernel (all on by default; profiles/r02_string_pack_kernel_iterations.txt has what each one bought)
-#ifndef DMB_PACK_CHUNK
-#define DMB_PACK_CHUNK 1   // pointer rows are copied four words at a time, loads first
-#endif
-#ifndef DMB_PACK_SROT
-#define DMB_PACK_SROT 1    // string_t are read from S in a lane-rotated order (no bank conflicts), rotated back in registers
-#endif
-#ifndef DMB_PACK_SEL
-#define DMB_PACK_SEL 1     // the inlined rows' last-word select as two bit tests
-#endif
-#ifndef DMB_PACK_GROUPS
-#define DMB_PACK_GROUPS 1  // two-level look-back (per-tile words for the nearest tiles, per-group sums / prefixes before them)
-#endif
-#ifndef DMB_PACK_UNIFY
-#define DMB_PACK_UNIFY 1   // inlined rows go through a per-thread scratch slot and the pointer rows' copy loop
-#endif
 constexpr uint32_t kPackScratchPerThread = 12u;  // UNIFY kernels: one 12-byte slot per worker thread behind H
+// worker warps per CTA: 8 with a heap (16 were no faster on the C2 columns), 16 for the heap-less lean form (faster than 8:
+// see dmb_dev_string_batch)
+__host__ __device__ constexpr int pack_warps(bool heap) { return heap ? 8 : 16; }
 
 struct TileMeta {
   long long tile;            // -1: no more tiles
@@ -608,9 +560,6 @@ __device__ __forceinline__ void mbar_wait(uint32_t mbar, uint32_t parity) {
     asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2, %3;\n\tselp.u32 %0, 1, 0, p;\n\t}"
                  : "=r"(done) : "r"(mbar), "r"(parity), "r"(20000u) : "memory");
     if (done) return;
-#ifdef DMB_WAIT_SLEEP
-    __nanosleep(DMB_WAIT_SLEEP);
-#endif
     if ((spins & 63u) == 0u) {
       const unsigned long long now = global_ns();
       if (t0 == 0) t0 = now;
@@ -656,71 +605,6 @@ __device__ __forceinline__ void store_bytes(uint32_t *w, uint32_t v, uint32_t b0
 // low `n` bytes set, n in 0..3
 __device__ __forceinline__ uint32_t low_bytes3(uint32_t n) { return (1u << (8u * n)) - 1u; }
 
-// exclusive prefix of tile `tile` by decoupled look-back, executed by one warp; kLookWide status
-// words are in flight per lane, so one L2 round trip inspects 32*kLookWide predecessors; when a
-// needed word is not published yet only the unpublished ones are read again
-__device__ __forceinline__ uint64_t lookback_wide(unsigned long long *status, int64_t tile, int lane, unsigned *stats = nullptr, int first_width = kLookFirst) {
-  unsigned long long *err_flags = status - 1;  // scratch[1]
-  uint64_t prefix = 0;
-  unsigned rounds = 0, retries = 0;
-  unsigned long long t0 = 0;
-  if (tile > 0) {
-    int64_t look = tile - 1;
-    int width = first_width;  // 32 * width status words in the first round (see the call in string_pack_kernel's L warp)
-    while (true) {
-      uint64_t st[kLookWide];
-#pragma unroll
-      for (int j = 0; j < kLookWide; ++j) st[j] = 0;
-      uint64_t v;
-      int state;  // 0: keep looking  1: a prefix closed the sum  2: a needed word is not published yet
-      while (true) {
-#pragma unroll
-        for (int j = 0; j < kLookWide; ++j) {
-          const int64_t idx = look - (int64_t)(32 * j + lane);
-          if (j < width && (st[j] >> 62) == 0) st[j] = idx >= 0 ? ld_status(status + idx) : kFlagPrefix;  // before tile 0: prefix 0
-        }
-        v = 0;
-        state = 0;
-#pragma unroll
-        for (int j = 0; j < kLookWide; ++j) {
-          if (state == 0 && j < width) {
-            const uint32_t ready = __ballot_sync(0xffffffffu, (st[j] >> 62) != 0);
-            const uint32_t is_p = __ballot_sync(0xffffffffu, (st[j] >> 62) == 2);
-            const int first_p = is_p ? (__ffs(is_p) - 1) : 31;
-            const uint32_t need = first_p >= 31 ? 0xffffffffu : ((2u << first_p) - 1u);
-            if ((ready & need) != need) state = 2;
-            else {
-              if (lane <= first_p) v += st[j] & kValueMask;
-              if (is_p) state = 1;
-            }
-          }
-        }
-        if (state != 2) break;
-        ++retries;
-        __nanosleep(200);  // the unpublished tiles are owned by running CTAs
-        const unsigned long long now = global_ns();
-        if (t0 == 0) t0 = now;
-        // gave up (warp-uniform): flag it and go on with what has been summed -- the launch ends, the host reports the
-        // flag and discards the outputs; the context stays usable (a trap would poison it for every other result)
-        if (__any_sync(0xffffffffu, now - t0 > g_lookback_limit_ns)) {
-          if (lane == 0) atomicOr(err_flags, (unsigned long long)kErrTimeout);
-          state = 1;
-          break;
-        }
-      }
-#pragma unroll
-      for (int d = 16; d > 0; d >>= 1) v += __shfl_xor_sync(0xffffffffu, v, d);
-      prefix += v;
-      ++rounds;
-      if (state == 1) break;
-      look -= 32 * width;
-      width = kLookWide;
-    }
-  }
-  if (stats) *stats = rounds * 1000u + retries;
-  return prefix;
-}
-
 // bytes a row contributes: 0 for NULL / past the chunk / an unusable pointer (flagged); P and the
 // workers must agree on this, it defines the tile totals
 template <bool HEAP>
@@ -747,10 +631,12 @@ struct RowState {
   uint32_t my_off;            // tile-local offset of the thread's first row
 };
 
-template <bool LARGE, int R, int NW, bool HEAP, bool UNIFY = (DMB_PACK_UNIFY != 0)>
-__global__ void __launch_bounds__(NW * 32 + 64, NW == 8 ? (HEAP ? 3 : DMB_NOHEAP_CTAS) : 2)
+template <bool LARGE, int R, bool HEAP, bool UNIFY = true>
+__global__ void __launch_bounds__(pack_warps(HEAP) * 32 + 64, HEAP ? 3 : 2)
 string_pack_kernel(dmb_string_job job, BatchView b, unsigned long long *scratch, int64_t ntiles,
                    uint32_t ostage_bytes, uint32_t hstage_bytes) {
+  static_assert(R == 2 || R == 4, "rows per worker thread");
+  constexpr int NW = pack_warps(HEAP);
   constexpr int kWT = NW * 32;             // worker threads
   constexpr int kRows = kWT * R;
   constexpr int kTilesPerChunk = kVec / kRows;
@@ -783,7 +669,6 @@ string_pack_kernel(dmb_string_job job, BatchView b, unsigned long long *scratch,
     // spent 11 % of their stall samples waiting for S
     auto claim = [&](int k) {
       TileMeta &m = pt.meta[k & (kMetaRing - 1)];
-      DMB_PTRACE(k, 14);
       long long tile = (long long)atomicAdd(scratch, 1ull);
       if (tile >= ntiles) tile = -1;
       m.tile = tile;
@@ -813,17 +698,15 @@ string_pack_kernel(dmb_string_job job, BatchView b, unsigned long long *scratch,
       mbar_expect_tx(mb, kSBytes + (m.val ? (uint32_t)kRows / 8u : 0u));
       bulk_load(smem_u32(sbuf + (uint32_t)slot * kSBytes), m.src, kSBytes, mb);
       if (m.val) bulk_load(smem_u32(&pt.vmask[slot][0]), m.val, (uint32_t)kRows / 8u, mb);
-      DMB_PTRACE(k, 6);
     };
     // ... and T: when the workers have packed a tile, send the stage to out_data with bulk stores and
     // hand the stage back.  Both jobs are triggered by the end of a worker iteration.
     // Tickets run three tiles ahead, loads two (A/B in one run, 60 M rows: heap-less columns 0.270 -> 0.254 ms, all-pointer columns
     // 0.772 -> 0.741 ms, l_comment / l_shipinstruct shapes unchanged within the box-to-box noise of +-1 %)
-    constexpr bool kEarlyTicket = true;
     if (lane == 0) {
       claim(0);
       claim(1);  // (also past the end: the workers must meet a tile that says so)
-      if (kEarlyTicket) claim(2);
+      claim(2);
       load(0);
       load(1);
     }
@@ -832,7 +715,6 @@ string_pack_kernel(dmb_string_job job, BatchView b, unsigned long long *scratch,
       bar_sync(kBarPacked, kWL);  // the workers have finished iteration j: tile j-1 packed, tile j scanned
       bool more = false;
       if (lane == 0) {
-        DMB_PTRACE(j, 10);
         if (j > 0) {
           const TileMeta &mp = pt.meta[(j - 1) & (kMetaRing - 1)];
           const uint64_t base = pt.base[(j - 1) & (kMetaRing - 1)];
@@ -856,9 +738,7 @@ string_pack_kernel(dmb_string_job job, BatchView b, unsigned long long *scratch,
             if (q1 > q0) bulk_store(gbase + q0, so + q0, q1 - q0);
             if ((end & 15u) && q1 >= q0) bulk_store_masked(gbase + q1, so + q1, 16u, (1u << (end & 15u)) - 1u);
             bulk_store_commit();
-            DMB_PTRACE(j, 11);
             bulk_store_drain();  // the stage is free again once the copy engine has read it
-            DMB_PTRACE(j, 12);
           }
         }
         more = pt.meta[j & (kMetaRing - 1)].tile >= 0;
@@ -868,13 +748,8 @@ string_pack_kernel(dmb_string_job job, BatchView b, unsigned long long *scratch,
       bar_arrive(kBarBase, kWL);  // the stage is free
       if (lane == 0) {
         // S[j&1] held tile j: the workers have scanned it (barrier above)
-        if (kEarlyTicket) {
-          load(j + 2);
-          claim(j + 3);
-        } else {
-          claim(j + 2);
-          load(j + 2);
-        }
+        load(j + 2);
+        claim(j + 3);
       }
       __syncwarp();
     }
@@ -890,24 +765,12 @@ string_pack_kernel(dmb_string_job job, BatchView b, unsigned long long *scratch,
       bar_sync(kBarF0 + (k & 1), 64);  // tile k is scanned, its aggregate is published (or there is no tile k)
       const long long tile = m.tile;
       if (tile < 0) break;
-      if (lane == 0) DMB_PTRACE(k, 8);
-#ifdef DMB_STR_TRACE
-      unsigned lb_stats = 0;
-      const uint64_t base = lookback_wide(status, tile, lane, &lb_stats);
-      if (lane == 0 && blockIdx.x < 32 && k < 64) g_str_trace[((blockIdx.x * 64 + k) << 4) + 9] = lb_stats;
-#else
-#if DMB_PACK_GROUPS
       const uint64_t base = lookback_groups(status, status + ntiles, status + ntiles + ((ntiles + 31) >> 5), tile, lane, status - 1, (unsigned long long)kErrTimeout, g_lookback_limit_ns);
-#else
-      const uint64_t base = lookback_wide(status, tile, lane);
-#endif
-#endif
       if (lane == 0) {
         if (tile > 0) atomicExch(status + tile, kFlagPrefix | ((base + m.total) & kValueMask));
         // the last tile of a group of 32 also publishes the group's inclusive prefix, in an array of its own (32 groups = 256 bytes)
-        if (DMB_PACK_GROUPS && (tile & 31) == 31) atomicExch(status + ntiles + ((ntiles + 31) >> 5) + (tile >> 5), kFlagPrefix | ((base + m.total) & kValueMask));
+        if ((tile & 31) == 31) atomicExch(status + ntiles + ((ntiles + 31) >> 5) + (tile >> 5), kFlagPrefix | ((base + m.total) & kValueMask));
         pt.base[k & (kMetaRing - 1)] = base;
-        DMB_PTRACE(k, 15);
       }
       __syncwarp();
       bar_arrive(kBarB0 + (k & 1), kWT + 32);  // the workers may place tile k
@@ -921,8 +784,8 @@ string_pack_kernel(dmb_string_job job, BatchView b, unsigned long long *scratch,
   // with conflict-free 16-byte loads, two stripes' lengths share one 32-bit scan (a stripe sums to <= 384 < 2^16), offsets
   // leave as coalesced 4-byte stores, and the bytes are placed one by one straight at their FINAL alignment in the stage (the
   // base is known by then), which P sends out with bulk stores: no copy-out pass.  Same roles, barriers and look-back as
-  // the general form.  (The one-CTA-per-tile string_short_kernel does the same work in ~2 warp-instructions per row but sits
-  // on its dependent chain: ticket -> metadata -> string_t -> scan -> look-back -> stores; here P and L hide that chain.)
+  // the general form.  (A one-CTA-per-tile kernel does the same work in ~2 warp-instructions per row but sits on its
+  // dependent chain: ticket -> metadata -> string_t -> scan -> look-back -> stores; here P and L hide that chain.)
   if constexpr (!HEAP) {
     uint32_t c_len[R], c_y[R], c_z[R], c_w[R], c_off[R], c_lmax = 0u;
     bool cur_valid = false;
@@ -990,7 +853,7 @@ string_pack_kernel(dmb_string_job job, BatchView b, unsigned long long *scratch,
           mj.hbytes = 0u;
           mj.staged = 1;
           atomicExch(status + mj.tile, (mj.tile == 0 ? kFlagPrefix : kFlagAggregate) | (uint64_t)total);
-          if (DMB_PACK_GROUPS) atomicAdd(status + ntiles + (mj.tile >> 5), kGroupOne | (unsigned long long)total);
+          atomicAdd(status + ntiles + (mj.tile >> 5), kGroupOne | (unsigned long long)total);
         }
       }
       if (warp == 0) {  // L: tile j's look-back is due (or: there is no tile j)
@@ -1047,9 +910,7 @@ string_pack_kernel(dmb_string_job job, BatchView b, unsigned long long *scratch,
     if (j > 0 && !cur_valid) break;  // tickets are monotonic: no tile j-1, no tile j
     // ---- front(tile j)
     const int slot = j & 1;
-    if (tid == 0) DMB_PTRACE(j, 0);
     mbar_wait(smem_u32(&pt.mbar_s[slot]), (uint32_t)(j >> 1) & 1u);  // P has claimed tile j (or found none)
-    if (tid == 0) DMB_PTRACE(j, 1);
     const bool nxt_valid = pt.meta[j & (kMetaRing - 1)].tile >= 0;
     if (nxt_valid) {
       const int nrows = pt.meta[j & (kMetaRing - 1)].nrows;
@@ -1059,28 +920,23 @@ string_pack_kernel(dmb_string_job job, BatchView b, unsigned long long *scratch,
       int flags = 0;  // 2: bad heap pointer  4: oversized row
       uint32_t tsum = 0u, hmin = 0xffffffffu, hmax = 0u;
       uint4 ent[R];
-      if (DMB_PACK_SROT && (R == 2 || R == 4)) {
-        // a thread's R string_t are 16 R consecutive bytes: read in row order, the eight lanes of a quarter warp would hit
-        // only 8 / R of the eight 16-byte bank groups.  Lane i starts at row (i / (8 / R)) mod R instead and the rows are
-        // rotated back in registers.
-        const int rot = R == 4 ? (lane >> 1) & 3 : (lane >> 2) & 1;
-        uint4 t[R];
+      // a thread's R string_t are 16 R consecutive bytes: read in row order, the eight lanes of a quarter warp would hit
+      // only 8 / R of the eight 16-byte bank groups.  Lane i starts at row (i / (8 / R)) mod R instead and the rows are
+      // rotated back in registers.
+      const int rot = R == 4 ? (lane >> 1) & 3 : (lane >> 2) & 1;
+      uint4 t[R];
 #pragma unroll
-        for (int k = 0; k < R; ++k) t[k] = s[(k + rot) & (R - 1)];
-        auto sel = [](bool c, const uint4 &a, const uint4 &b) { return make_uint4(c ? a.x : b.x, c ? a.y : b.y, c ? a.z : b.z, c ? a.w : b.w); };
-        if (R == 2) {
-          ent[0] = sel(rot != 0, t[1 % R], t[0]);
-          ent[1 % R] = sel(rot != 0, t[0], t[1 % R]);
-        } else {
-          uint4 u[R];
-#pragma unroll
-          for (int k = 0; k < R; ++k) u[k] = sel((rot & 1) != 0, t[(k + 3) & (R - 1)], t[k]);
-#pragma unroll
-          for (int k = 0; k < R; ++k) ent[k] = sel((rot & 2) != 0, u[(k + 2) & (R - 1)], u[k]);
-        }
+      for (int k = 0; k < R; ++k) t[k] = s[(k + rot) & (R - 1)];
+      auto sel = [](bool c, const uint4 &a, const uint4 &b) { return make_uint4(c ? a.x : b.x, c ? a.y : b.y, c ? a.z : b.z, c ? a.w : b.w); };
+      if (R == 2) {
+        ent[0] = sel(rot != 0, t[1 % R], t[0]);
+        ent[1 % R] = sel(rot != 0, t[0], t[1 % R]);
       } else {
+        uint4 u[R];
 #pragma unroll
-        for (int k = 0; k < R; ++k) ent[k] = s[k];
+        for (int k = 0; k < R; ++k) u[k] = sel((rot & 1) != 0, t[(k + 3) & (R - 1)], t[k]);
+#pragma unroll
+        for (int k = 0; k < R; ++k) ent[k] = sel((rot & 2) != 0, u[(k + 2) & (R - 1)], u[k]);
       }
 #pragma unroll
       for (int k = 0; k < R; ++k) {
@@ -1158,7 +1014,7 @@ string_pack_kernel(dmb_string_job job, BatchView b, unsigned long long *scratch,
         // iteration earlier, made the look-backs behind it a little shorter but cost 3 % of the kernel: every row was read twice)
         m.total = total;
         atomicExch(status + m.tile, (m.tile == 0 ? kFlagPrefix : kFlagAggregate) | (uint64_t)total);
-        if (DMB_PACK_GROUPS) atomicAdd(status + ntiles + (m.tile >> 5), kGroupOne | (unsigned long long)total);  // (no return value: a reduction at L2)
+        atomicAdd(status + ntiles + (m.tile >> 5), kGroupOne | (unsigned long long)total);  // (no return value: a reduction at L2)
         if (HEAP && staged && hbytes) {
           const uint32_t mb = smem_u32(&pt.mbar_h[slot]);
           mbar_expect_tx(mb, hbytes);
@@ -1170,7 +1026,6 @@ string_pack_kernel(dmb_string_job job, BatchView b, unsigned long long *scratch,
       __syncwarp();
       bar_arrive(kBarF0 + (j & 1), 64);
     }
-    if (tid == 0) DMB_PTRACE(j, 2);
 
     // ---- back(tile j-1)
     uint64_t base = 0;
@@ -1178,7 +1033,6 @@ string_pack_kernel(dmb_string_job job, BatchView b, unsigned long long *scratch,
       bar_sync(kBarB0 + ((j - 1) & 1), kWT + 32);  // L has resolved tile j-1
       base = pt.base[(j - 1) & (kMetaRing - 1)];
     }
-    if (tid == 0) DMB_PTRACE(j, 3);
     if (cur_valid) {
       const TileMeta &mc = pt.meta[(j - 1) & (kMetaRing - 1)];
       const int nrows = mc.nrows;
@@ -1240,7 +1094,6 @@ string_pack_kernel(dmb_string_job job, BatchView b, unsigned long long *scratch,
           mbar_wait(smem_u32(&pt.mbar_h[hslot]), ph);
           ph ^= 1u;
         }
-        if (tid == 0) DMB_PTRACE(j, 4);
         uint32_t *ow = reinterpret_cast<uint32_t *>(ostage);
         const uint32_t *hw = reinterpret_cast<const uint32_t *>(hbuf + (uint32_t)hslot * hstride);
         const uint32_t hbase = (mc.hmin << 4) + (uint32_t)job.heap_host_base;  // low 32 bits of the span's host address
@@ -1355,67 +1208,49 @@ string_pack_kernel(dmb_string_job job, BatchView b, unsigned long long *scratch,
             }
             if (nw >= 2u) ow[wp + 1] = x1;
             if (nw >= 3u) ow[wp + 2] = x2;
-#if DMB_PACK_SEL
             // (nw <= 3; as a chain of equality tests this became a jump table)
             acc = ((nw & 2u) ? ((nw & 1u) ? x3 : x2) : ((nw & 1u) ? x1 : x0)) & low_bytes3(n & 3u);
-#else
-            acc = (nw == 0u ? x0 : (nw == 1u ? x1 : (nw == 2u ? x2 : x3))) & low_bytes3(n & 3u);
-#endif
           } else if (HEAP) {
             // pointer: the staged span.  Output word m of the row holds source bytes qp-4+4m .. +3
             const uint32_t qp = (cur.z[k] - hbase) + 4u - fill;
             const uint32_t sq = 8u * (qp & 3u);
             const uint32_t *s = hw + (qp >> 2);
             uint32_t prev = s[-1], nx = s[0];
-            uint32_t *o;
             const uint32_t x0 = (__funnelshift_r(prev, nx, sq) & ~low_bytes3(fill)) | acc;
             if (wp == shared_wp) store_bytes(ow + wp, x0, head, 4u); else ow[wp] = x0;  // l > 12: the word always completes
             prev = nx;
-            o = ow + wp;
-#if DMB_PACK_CHUNK
-            // four words per iteration, the loads of a group before its stores (the compiler may not move a shared-memory
-            // load over a shared-memory store), pointers bumped instead of indices recomputed: 17 instructions per four
-            // words where the plain loop took 13 per two
-            {
-              const uint32_t *sp = s + 1;
-              uint32_t *op = o + 1;
-              uint32_t left = nw - 1u;  // whole words after the first one
+            // the whole words after the first one: four per iteration, the loads of a group before its stores (the compiler
+            // may not move a shared-memory load over a shared-memory store), pointers bumped instead of indices recomputed:
+            // 17 instructions per four words where a plain word-by-word loop took 13 per two
+            const uint32_t *sp = s + 1;
+            uint32_t *op = ow + wp + 1;
+            uint32_t left = nw - 1u;
 #pragma unroll 1
-              for (; left >= 4u; left -= 4u) {
-                const uint32_t a0 = sp[0], a1 = sp[1], a2 = sp[2], a3 = sp[3];
-                op[0] = __funnelshift_r(prev, a0, sq);
-                op[1] = __funnelshift_r(a0, a1, sq);
-                op[2] = __funnelshift_r(a1, a2, sq);
-                op[3] = __funnelshift_r(a2, a3, sq);
-                prev = a3;
-                sp += 4;
-                op += 4;
-              }
-              if (left & 2u) {
-                const uint32_t a0 = sp[0], a1 = sp[1];
-                op[0] = __funnelshift_r(prev, a0, sq);
-                op[1] = __funnelshift_r(a0, a1, sq);
-                prev = a1;
-                sp += 2;
-                op += 2;
-              }
-              if (left & 1u) {
-                const uint32_t a0 = sp[0];
-                op[0] = __funnelshift_r(prev, a0, sq);
-                prev = a0;
-                sp += 1;
-              }
-              acc = (n & 3u) ? (__funnelshift_r(prev, sp[0], sq) & low_bytes3(n & 3u)) : 0u;
+            for (; left >= 4u; left -= 4u) {
+              const uint32_t a0 = sp[0], a1 = sp[1], a2 = sp[2], a3 = sp[3];
+              op[0] = __funnelshift_r(prev, a0, sq);
+              op[1] = __funnelshift_r(a0, a1, sq);
+              op[2] = __funnelshift_r(a1, a2, sq);
+              op[3] = __funnelshift_r(a2, a3, sq);
+              prev = a3;
+              sp += 4;
+              op += 4;
             }
-#else
-#pragma unroll kPackUnroll
-            for (uint32_t m = 1; m < nw; ++m) {
-              nx = s[m];
-              o[m] = __funnelshift_r(prev, nx, sq);
-              prev = nx;
+            if (left & 2u) {
+              const uint32_t a0 = sp[0], a1 = sp[1];
+              op[0] = __funnelshift_r(prev, a0, sq);
+              op[1] = __funnelshift_r(a0, a1, sq);
+              prev = a1;
+              sp += 2;
+              op += 2;
             }
-            acc = (n & 3u) ? (__funnelshift_r(prev, s[nw], sq) & low_bytes3(n & 3u)) : 0u;
-#endif
+            if (left & 1u) {
+              const uint32_t a0 = sp[0];
+              op[0] = __funnelshift_r(prev, a0, sq);
+              prev = a0;
+              sp += 1;
+            }
+            acc = (n & 3u) ? (__funnelshift_r(prev, sp[0], sq) & low_bytes3(n & 3u)) : 0u;
           }
           wp += nw;
           fill = n & 3u;
@@ -1458,7 +1293,6 @@ string_pack_kernel(dmb_string_job job, BatchView b, unsigned long long *scratch,
         }
       }
     }
-    if (tid == 0) DMB_PTRACE(j, 5);
     bar_arrive(kBarPacked, kWL);
     cur = nxt;
     cur_valid = nxt_valid;
@@ -1471,7 +1305,8 @@ string_pack_kernel(dmb_string_job job, BatchView b, unsigned long long *scratch,
 // bytes out, so the per-tile latency chain (load -> scan -> look-back) dominates: this kernel takes
 // a whole 2048-row vector per CTA, 8 rows per thread, loads them striped (lane-consecutive rows:
 // 512 contiguous bytes per request), scans the lengths with one warp scan per stripe, and builds
-// the tile's output in a zeroed shared-memory image straight from registers.
+// the tile's output in a zeroed shared-memory image straight from registers.  It serves the reference
+// blob (DMB_STR_REF_BLOB); the Arrow modes take the pack kernel's lean form.
 constexpr int kInlRows = kVec;                       // rows per tile
 constexpr int kInlPerThread = kInlRows / kThreads;   // 8
 struct InlSmem {
@@ -1635,282 +1470,27 @@ string_inline_kernel(dmb_string_job job, BatchView b, unsigned long long *scratc
   }
 }
 
-// ------------------------------------------------------------------ columns without a heap, Arrow modes
-// string_short_kernel<LARGE, RPT>: flags, codes, short names (every string inlined in its string_t).
-// Rows cost 16 bytes in and 4 + len bytes out, so nothing but the per-tile dependent chain
-// (metadata -> string_t -> scan -> look-back -> stores) can keep the kernel from the HBM roofline.
-// One CTA per tile of RPT*256 rows, many CTAs per SM, no roles and no pipeline inside the CTA:
-//   * striped loads straight into registers (lane-consecutive rows: 512 contiguous bytes per request)
-//   * two stripes' lengths share one 32-bit scan (len <= 12, so a stripe sums to <= 384 < 2^16)
-//   * the tile's aggregate is published right after the block scan; warp 0 then resolves the prefix
-//     with the wide look-back (256 status words per L2 round trip) WHILE the other warps place their
-//     bytes in the stage at tile-local positions (byte stores: no zeroing, no read-modify-write)
-//   * the stage leaves as 16-byte vectors aligned to the destination; the shift between tile-local
-//     and destination alignment is a funnel shift on the way out
-#ifndef DMB_SHORT_GROUPS
-#define DMB_SHORT_GROUPS 1  // ENUM form: the two-level look-back of the pack kernel (lookback_groups).  Measured per 60 M rows, groups vs
-                            // 256-wide tile-by-tile rounds: ENUM 0.307 vs 0.331 ms, l_shipmode shape 0.329 vs 0.335, one-byte strings 0.291 vs
-                            // 0.285 (the extra atomic per tile shows): the string_t form keeps the tile-by-tile walk
-#endif
-#ifndef DMB_SHORT_CTAS8
-#define DMB_SHORT_CTAS8 4
-#endif
-// EW = 0: rows are string_t.  EW = 1 / 2 / 4 (dmb_dev_enum_utf8): rows are ENUM indices of that many bytes and a row's string_t is
-// looked up in a table of the dictionary's labels built in shared memory (<= DMB_ENUM_FUSED_MAX_LABELS labels of <= 12 bytes), so the
-// 16-byte-per-row string_t intermediate of enum_to_string_t_kernel is never written or read.
-template <int EW> struct EnumIndex { typedef uint8_t type; };
-template <> struct EnumIndex<2> { typedef uint16_t type; };
-template <> struct EnumIndex<4> { typedef uint32_t type; };
-
-// ECTAS: CTAs per SM of the ENUM form, whose rows keep an index + a length in registers instead of a string_t
-// (6: 40 registers + 56 bytes of spills; 5: 48 registers; runtime choice DMB_ENUM_CTAS for A/B)
-// NT: threads per CTA (256; 128 / 512 are measured variants: DMB_STR_SHORT_NT)
-template <bool LARGE, int RPT, int EW, int ECTAS = 6, int NT = kThreads>
-__global__ void __launch_bounds__(NT, EW ? ECTAS : (NT == 128 ? 8 : (NT == 512 ? 2 : (RPT >= 8 ? DMB_SHORT_CTAS8 : 5))))
-string_short_kernel(dmb_string_job job, BatchView b, unsigned long long *scratch, int64_t ntiles, dmb_enum_job ej) {
-  constexpr int kRows = NT * RPT;
-  constexpr int kTilesPerChunk = kVec / kRows;
-  constexpr int kWarps = NT / 32;
-  __shared__ __align__(16) uint8_t stage[kRows * 12 + 32];
-  __shared__ uint32_t warp_sum[kWarps];
-  __shared__ uint64_t base_sh;
-  __shared__ long long ticket_sh;
-  unsigned long long *status = scratch + 2;
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int64_t tile = claim_tile(scratch, &ticket_sh);  // every predecessor is owned by a CTA that is running or done
-  if (tile >= ntiles) return;
-  const int64_t c = tile / kTilesPerChunk;
-  const int r_begin = (int)(tile % kTilesPerChunk) * kRows;
-  const int count = (int)__ldg(b.counts + c) - r_begin;  // rows of this tile that exist (may be <= 0)
-  const dmb_vec_desc vd = EW ? ej.vecs[c] : job.vecs[c];
-  const uint4 *in = reinterpret_cast<const uint4 *>(reinterpret_cast<const uint8_t *>(job.in) + (EW ? 0 : vd.data_off)) + r_begin;
-  const uint64_t *mask = vd.val_off < 0 ? nullptr : (EW ? ej.in_validity : job.in_validity) + vd.val_off + (r_begin >> 6);
-  typedef typename EnumIndex<EW>::type I;
-  const I *in_idx = reinterpret_cast<const I *>(reinterpret_cast<const uint8_t *>(ej.in_data) + (EW ? vd.data_off : 0)) + r_begin;
-  __shared__ uint4 s_tab[EW ? DMB_ENUM_FUSED_MAX_LABELS : 1];
-
-  // stripe k of warp w holds tile rows w*32*RPT + k*32 + lane
-  const int row0 = warp * (32 * RPT) + lane;
-  uint4 e[EW ? 1 : RPT];
-  uint32_t idx[EW ? RPT : 1];  // ENUM: the row's index, from the scan on: index | bytes the row contributes << 16
-#pragma unroll
-  for (int k = 0; k < RPT; ++k) {
-    const int row = row0 + 32 * k;
-    if (EW) {
-      idx[k] = row < count ? (uint32_t)in_idx[row] : 0u;  // (the index under a NULL row is read and dropped)
-    } else {
-      e[EW ? 0 : k] = make_uint4(0, 0, 0, 0);
-      if (row < count) e[EW ? 0 : k] = ld_stream(in + row);
-    }
-  }
-  if (EW) {  // the labels as string_t, once per CTA (the index loads above are in flight meanwhile)
-    for (uint32_t t = tid; t < ej.dict_size; t += NT) s_tab[t] = enum_entry(ej, t);
-    __syncthreads();
-  }
-  int bad = 0;
-  unsigned long long bad_idx = 0;
-  uint32_t lmax = 0;
-#pragma unroll
-  for (int k = 0; k < RPT; ++k) {
-    const int row = row0 + 32 * k;
-    uint32_t l = 0;
-    if (row < count) {
-      const bool valid = mask ? ((__ldg(mask + (row >> 6)) >> (row & 63)) & 1ull) : true;
-      if (EW) {
-        if (valid) {
-          if (idx[k] < ej.dict_size) l = s_tab[idx[k]].x;
-          else ++bad_idx;  // an index past the dictionary: reported, rendered as the empty string
-        }
-      } else {
-        l = valid ? e[EW ? 0 : k].x : 0u;
-      }
-      if (l > 12u) { bad = 1; l = 0; }  // a pointer string, but the batch registered no heap (ENUM: a label too long for this kernel)
-    }
-    // from here on: the bytes the row contributes
-    if (EW) idx[k] = (l ? idx[k] : 0u) | (l << 16);
-    else e[EW ? 0 : k].x = l;
-    lmax = lmax > l ? lmax : l;
-  }
-  // exclusive offsets within the warp: stripes 2i and 2i+1 scanned together in 16-bit halves
-  uint32_t off[RPT];
-  uint32_t carry = 0;
-#pragma unroll
-  for (int k = 0; k < RPT; k += 2) {
-    const uint32_t both = EW ? ((idx[k] >> 16) | (idx[k + 1] & 0xffff0000u)) : (e[EW ? 0 : k].x | (e[EW ? 0 : k + 1].x << 16));
-    uint32_t incl = both;
-#pragma unroll
-    for (int d = 1; d < 32; d <<= 1) {
-      const uint32_t n = __shfl_up_sync(0xffffffffu, incl, d);
-      if (lane >= d) incl += n;
-    }
-    const uint32_t tot = __shfl_sync(0xffffffffu, incl, 31);
-    const uint32_t excl = incl - both;
-    off[k] = carry + (excl & 0xffffu);
-    carry += tot & 0xffffu;
-    off[k + 1] = carry + (excl >> 16);
-    carry += tot >> 16;
-  }
-  if (lane == 0) warp_sum[warp] = carry;
-  if (EW && bad_idx && ej.bad_index) atomicAdd(ej.bad_index, bad_idx);
-  lmax = __reduce_max_sync(0xffffffffu, lmax);
-  const int any_bad = __syncthreads_or(bad);
-  uint32_t warp_excl = 0, tile_total = 0;
-#pragma unroll
-  for (int w = 0; w < kWarps; ++w) {
-    const uint32_t s = warp_sum[w];
-    warp_excl += w < warp ? s : 0u;
-    tile_total += s;
-  }
-  if (tid == 0) {
-    atomicExch(status + tile, (tile == 0 ? kFlagPrefix : kFlagAggregate) | (uint64_t)tile_total);
-    if (DMB_SHORT_GROUPS && EW) atomicAdd(status + ntiles + (tile >> 5), kGroupOne | (unsigned long long)tile_total);
-    if (any_bad) atomicOr(scratch + 1, (unsigned long long)kErrHeapRange);
-  }
-#ifdef DMB_SHORT_LB_FIRST
-  // decoupled look-back (warp 0)
-  if (warp == 0) {
-    const uint64_t prefix = (DMB_SHORT_GROUPS && EW) ? lookback_groups(status, status + ntiles, status + ntiles + ((ntiles + 31) >> 5), tile, lane, status - 1, (unsigned long long)kErrTimeout, g_lookback_limit_ns)
-                                             : lookback_wide(status, tile, lane);
-    if (lane == 0) {
-      if (tile > 0) atomicExch(status + tile, kFlagPrefix | ((prefix + tile_total) & kValueMask));
-      if (DMB_SHORT_GROUPS && EW && (tile & 31) == 31) atomicExch(status + ntiles + ((ntiles + 31) >> 5) + (tile >> 5), kFlagPrefix | ((prefix + tile_total) & kValueMask));
-      base_sh = prefix;
-    }
-  }
-  // place the bytes at their tile-local positions (stage byte q = byte q of the tile's output)
-#pragma unroll
-  for (int k = 0; k < RPT; ++k) off[k] += warp_excl;
-  if (EW) {  // the label again from the table, one row at a time: only index + length stay live across the scan
-#pragma unroll
-    for (int k = 0; k < RPT; ++k) {
-      const uint32_t l = idx[k] >> 16;
-      const uint4 ent = s_tab[idx[k] & 0xffffu];
-#pragma unroll
-      for (int i = 0; i < 12; ++i) {
-        if ((uint32_t)i >= lmax) break;  // warp-uniform: no issue slots for bytes past the longest label of the warp's rows
-        const uint32_t wsel = i < 4 ? ent.y : (i < 8 ? ent.z : ent.w);
-        if ((uint32_t)i < l) stage[off[k] + i] = (uint8_t)(wsel >> (8 * (i & 3)));
-      }
-    }
-  } else {
-#pragma unroll
-    for (int i = 0; i < 12; ++i) {
-      if ((uint32_t)i < lmax) {  // warp-uniform
-#pragma unroll
-        for (int k = 0; k < RPT; ++k) {
-          const uint32_t wsel = i < 4 ? e[EW ? 0 : k].y : (i < 8 ? e[EW ? 0 : k].z : e[EW ? 0 : k].w);
-          if ((uint32_t)i < e[EW ? 0 : k].x) stage[off[k] + i] = (uint8_t)(wsel >> (8 * (i & 3)));
-        }
-      }
-    }
-  }
-#else
-  // place the bytes at their tile-local positions (stage byte q = byte q of the tile's output)
-#pragma unroll
-  for (int k = 0; k < RPT; ++k) off[k] += warp_excl;
-  if (EW) {  // the label again from the table, one row at a time: only index + length stay live across the scan
-#pragma unroll
-    for (int k = 0; k < RPT; ++k) {
-      const uint32_t l = idx[k] >> 16;
-      const uint4 ent = s_tab[idx[k] & 0xffffu];
-#pragma unroll
-      for (int i = 0; i < 12; ++i) {
-        if ((uint32_t)i >= lmax) break;  // warp-uniform: no issue slots for bytes past the longest label of the warp's rows
-        const uint32_t wsel = i < 4 ? ent.y : (i < 8 ? ent.z : ent.w);
-        if ((uint32_t)i < l) stage[off[k] + i] = (uint8_t)(wsel >> (8 * (i & 3)));
-      }
-    }
-  } else {
-#pragma unroll
-    for (int i = 0; i < 12; ++i) {
-      if ((uint32_t)i < lmax) {  // warp-uniform
-#pragma unroll
-        for (int k = 0; k < RPT; ++k) {
-          const uint32_t wsel = i < 4 ? e[EW ? 0 : k].y : (i < 8 ? e[EW ? 0 : k].z : e[EW ? 0 : k].w);
-          if ((uint32_t)i < e[EW ? 0 : k].x) stage[off[k] + i] = (uint8_t)(wsel >> (8 * (i & 3)));
-        }
-      }
-    }
-  }
-  // decoupled look-back (warp 0)
-  if (warp == 0) {
-    const uint64_t prefix = (DMB_SHORT_GROUPS && EW) ? lookback_groups(status, status + ntiles, status + ntiles + ((ntiles + 31) >> 5), tile, lane, status - 1, (unsigned long long)kErrTimeout, g_lookback_limit_ns)
-                                             : lookback_wide(status, tile, lane);
-    if (lane == 0) {
-      if (tile > 0) atomicExch(status + tile, kFlagPrefix | ((prefix + tile_total) & kValueMask));
-      if (DMB_SHORT_GROUPS && EW && (tile & 31) == 31) atomicExch(status + ntiles + ((ntiles + 31) >> 5) + (tile >> 5), kFlagPrefix | ((prefix + tile_total) & kValueMask));
-      base_sh = prefix;
-    }
-  }
-#endif
-  __syncthreads();
-  const uint64_t base = base_sh;
-  const int64_t out_row0 = __ldg(b.row_off + c) + r_begin;
-  if (tid == 0) {
-    if (!LARGE && base + tile_total > 0x7fffffffull) atomicOr(scratch + 1, (unsigned long long)kErrOffsetOverflow);
-    if (tile == ntiles - 1) {
-      if (LARGE) reinterpret_cast<long long *>(job.out_offsets)[b.nrows] = (long long)(base + tile_total);
-      else reinterpret_cast<int32_t *>(job.out_offsets)[b.nrows] = (int32_t)(base + tile_total);
-      if (job.total_bytes) *job.total_bytes = base + tile_total;
-    }
-  }
-#pragma unroll
-  for (int k = 0; k < RPT; ++k) {
-    const int row = row0 + 32 * k;
-    if (row < count) {
-      if (LARGE) __stcs(reinterpret_cast<long long *>(job.out_offsets) + out_row0 + row, (long long)(base + off[k]));
-      else __stcs(reinterpret_cast<int32_t *>(job.out_offsets) + out_row0 + row, (int32_t)((uint32_t)base + off[k]));
-    }
-  }
-  if (tile_total == 0) return;
-  if (job.out_data_cap && base + tile_total > job.out_data_cap) {
-    if (tid == 0) atomicOr(scratch + 1, (unsigned long long)kErrDataCap);
-    return;
-  }
-  // stage -> out_data: destination-aligned 16-byte vectors; vector v holds tile bytes [16v - mis, 16v - mis + 16)
-  uint8_t *gdst = job.out_data + base;
-  const uint32_t mis = (uint32_t)(reinterpret_cast<uintptr_t>(gdst) & 15u);
-  const uint32_t end = mis + tile_total;
-  const uint32_t nvec = (end + 15u) >> 4;
-  const uint32_t *sw = reinterpret_cast<const uint32_t *>(stage);
-  for (uint32_t v = tid; v < nvec; v += NT) {
-    const uint32_t p = 16u * v;
-    if (p >= mis && p + 16u <= end) {
-      const uint32_t q = p - mis, sh = 8u * (q & 3u);
-      const uint32_t *s = sw + (q >> 2);
-      const uint32_t a0 = s[0], a1 = s[1], a2 = s[2], a3 = s[3], a4 = s[4];  // s[4]: inside the stage's 32 bytes of slack
-      uint4 o;
-      o.x = __funnelshift_r(a0, a1, sh);
-      o.y = __funnelshift_r(a1, a2, sh);
-      o.z = __funnelshift_r(a2, a3, sh);
-      o.w = __funnelshift_r(a3, a4, sh);
-      st_stream(reinterpret_cast<uint4 *>(gdst - mis + p), o);
-    } else {  // the neighbouring tiles own the other bytes of this vector
-      const uint32_t b0 = p > mis ? p : mis, b1 = (p + 16u) < end ? (p + 16u) : end;
-      for (uint32_t q = b0; q < b1; ++q) gdst[q - mis] = stage[q - mis];
-    }
-  }
-}
-
 // ------------------------------------------------------------------ ENUM indices -> utf8, one launch (dmb_dev_enum_utf8)
-// The ENUM form of string_short_kernel above is bound by instruction issue (ncu r03b: issue 81 %, DRAM 21 %, 141 thread
-// instructions per row: a byte load per index, up to 12 predicated byte stores per row, four 2x16-bit warp scans per thread).
-// This kernel keeps its structure -- one CTA per 2048-row vector, ticketed, the label table as string_t in shared memory,
-// bytes placed at tile-local positions while warp 0 resolves the prefix -- and removes the instructions:
+// Rows are ENUM indices of EW = 1 / 2 / 4 bytes.  A row's string_t is looked up in a table of the dictionary's labels built
+// in shared memory (<= DMB_ENUM_FUSED_MAX_LABELS labels of <= 12 bytes), so the 16-byte-per-row string_t intermediate of
+// enum_to_string_t_kernel is never written or read.  One CTA per 2048-row vector, claimed from a ticket; the bytes are
+// placed at tile-local positions in a shared-memory stage, warp 0 then resolves the prefix by look-back, and the stage
+// leaves as destination-aligned 16-byte vectors.  The work is bound by instruction issue (a form of this kernel with
+// striped rows, ncu r03b: issue 81 %, DRAM 21 %, 141 thread instructions per row: a byte load per index, up to 12
+// predicated byte stores per row, four 2x16-bit warp scans per thread), so the rows are laid out to need few instructions:
 //   * a thread owns 8 CONSECUTIVE rows: its indices arrive as one 8 / 16 / 2 x 16-byte load, its validity bits as one byte of the mask
 //   * the 8 lengths stay packed in one register (4 bits each); one 32-bit warp scan of the per-thread sums
 //   * the thread's bytes are one contiguous stream: labels are appended to a running word with funnel shifts and leave as
 //     whole 32-bit words (<= 3 stores per row); only the first / last word of the stream, which the neighbouring threads
 //     share, is written byte by byte
 //   * the 8 consecutive offsets leave as two 16-byte stores
-#ifndef DMB_ENUM_PACK_CTAS
-#define DMB_ENUM_PACK_CTAS 6
-#endif
-#ifndef DMB_ENUM_LB_FIRST
-#define DMB_ENUM_LB_FIRST 0
-#endif
+constexpr int kEnumPackCtas = 6;  // CTAs per SM (launch bound)
+template <int EW> struct EnumIndex { typedef uint8_t type; };  // the index type of EW bytes
+template <> struct EnumIndex<2> { typedef uint16_t type; };
+template <> struct EnumIndex<4> { typedef uint32_t type; };
+
 template <bool LARGE, int EW>
-__global__ void __launch_bounds__(kThreads, DMB_ENUM_PACK_CTAS)
+__global__ void __launch_bounds__(kThreads, kEnumPackCtas)
 enum_pack_kernel(dmb_string_job job, BatchView b, unsigned long long *scratch, int64_t ntiles, dmb_enum_job ej) {
   constexpr int kR = kVec / kThreads;  // 8 rows per thread
   constexpr int kWarps = kThreads / 32;
@@ -2019,17 +1599,6 @@ enum_pack_kernel(dmb_string_job job, BatchView b, unsigned long long *scratch, i
     if (any_bad) atomicOr(scratch + 1, (unsigned long long)kErrHeapRange);
   }
 
-#if DMB_ENUM_LB_FIRST
-  if (warp == 0) {  // (variant: warp 0 resolves the prefix before it places its own bytes)
-    const uint64_t prefix = lookback_groups(status, status + ntiles, status + ntiles + ((ntiles + 31) >> 5), tile, lane, status - 1,
-                                            (unsigned long long)kErrTimeout, g_lookback_limit_ns);
-    if (lane == 0) {
-      if (tile > 0) atomicExch(status + tile, kFlagPrefix | ((prefix + tile_total) & kValueMask));
-      if ((tile & 31) == 31) atomicExch(status + ntiles + ((ntiles + 31) >> 5) + (tile >> 5), kFlagPrefix | ((prefix + tile_total) & kValueMask));
-      base_sh = prefix;
-    }
-  }
-#endif
   // ---- the thread's bytes: one stream from stage byte my_off on.  Whole words only in the loop: the first word of a stream
   // that starts inside a word leaves with zeros in its low `head` bytes, and after the barrier the threads before write
   // those bytes -- the unfinished tail of their own stream -- over them, byte by byte.
@@ -2060,7 +1629,7 @@ enum_pack_kernel(dmb_string_job job, BatchView b, unsigned long long *scratch, i
   // the stream's unfinished tail: bytes [0, fill) of word wp, or [head, fill) when the whole stream lies inside its first word
   if (fill) store_bytes(sw + wp, acc, wp == wp0 ? head : 0u, fill);
   // ---- decoupled look-back (warp 0), after its own bytes are placed: the later it starts, the shorter it is
-  if (!DMB_ENUM_LB_FIRST && warp == 0) {
+  if (warp == 0) {
     const uint64_t prefix = lookback_groups(status, status + ntiles, status + ntiles + ((ntiles + 31) >> 5), tile, lane, status - 1,
                                             (unsigned long long)kErrTimeout, g_lookback_limit_ns);
     if (lane == 0) {
@@ -2173,12 +1742,6 @@ make_string_t_kernel(const uint32_t *__restrict__ lengths, const uint64_t *__res
 
 using namespace dmb;
 
-#ifdef DMB_STR_TRACE
-extern "C" int32_t dmb_dev_string_trace(unsigned long long *out, int64_t n) {
-  return (int32_t)cudaMemcpyFromSymbol(out, g_str_trace, sizeof(unsigned long long) * (size_t)n);
-}
-#endif
-
 extern "C" int32_t dmb_dev_set_lookback_limit_ns(unsigned long long ns) {
   return check_cuda(cudaMemcpyToSymbol(g_lookback_limit_ns, &ns, sizeof(ns)), "set look-back limit");
 }
@@ -2206,32 +1769,12 @@ extern "C" int32_t dmb_dev_enum_utf8(const dmb_enum_job *ejob, const dmb_string_
   const bool large = job->mode == DMB_STR_ARROW_LARGE;
   auto launch = [&](auto kernel) -> int32_t {
     kernel<<<(unsigned)nchunks, kThreads, 0, st>>>(*job, b, (unsigned long long *)scratch, nchunks, *ejob);
-    return check_cuda(cudaGetLastError(), "string_short_kernel (ENUM) launch");
+    return check_cuda(cudaGetLastError(), "enum_pack_kernel launch");
   };
-  // default: enum_pack_kernel (consecutive-row ownership, word-granular placement); DMB_ENUM_SHORT=1 keeps the ENUM form of
-  // string_short_kernel for A/B
-  static const bool enum_short = getenv("DMB_ENUM_SHORT") != nullptr;
-  if (!enum_short) {
-    switch (ejob->phys) {
-      case DMB_PHYS_U8: return large ? launch(enum_pack_kernel<true, 1>) : launch(enum_pack_kernel<false, 1>);
-      case DMB_PHYS_U16: return large ? launch(enum_pack_kernel<true, 2>) : launch(enum_pack_kernel<false, 2>);
-      case DMB_PHYS_U32: return large ? launch(enum_pack_kernel<true, 4>) : launch(enum_pack_kernel<false, 4>);
-      default: set_error("dmb_dev_enum_utf8: ENUM indices are uint8/uint16/uint32, not physical type %d", ejob->phys); return -1;
-    }
-  }
-  static const int ctas = getenv("DMB_ENUM_CTAS") ? atoi(getenv("DMB_ENUM_CTAS")) : 6;
-  if (ctas == 5) {
-    switch (ejob->phys) {
-      case DMB_PHYS_U8: return large ? launch(string_short_kernel<true, 8, 1, 5>) : launch(string_short_kernel<false, 8, 1, 5>);
-      case DMB_PHYS_U16: return large ? launch(string_short_kernel<true, 8, 2, 5>) : launch(string_short_kernel<false, 8, 2, 5>);
-      case DMB_PHYS_U32: return large ? launch(string_short_kernel<true, 8, 4, 5>) : launch(string_short_kernel<false, 8, 4, 5>);
-      default: break;
-    }
-  }
   switch (ejob->phys) {
-    case DMB_PHYS_U8: return large ? launch(string_short_kernel<true, 8, 1>) : launch(string_short_kernel<false, 8, 1>);
-    case DMB_PHYS_U16: return large ? launch(string_short_kernel<true, 8, 2>) : launch(string_short_kernel<false, 8, 2>);
-    case DMB_PHYS_U32: return large ? launch(string_short_kernel<true, 8, 4>) : launch(string_short_kernel<false, 8, 4>);
+    case DMB_PHYS_U8: return large ? launch(enum_pack_kernel<true, 1>) : launch(enum_pack_kernel<false, 1>);
+    case DMB_PHYS_U16: return large ? launch(enum_pack_kernel<true, 2>) : launch(enum_pack_kernel<false, 2>);
+    case DMB_PHYS_U32: return large ? launch(enum_pack_kernel<true, 4>) : launch(enum_pack_kernel<false, 4>);
     default: set_error("dmb_dev_enum_utf8: ENUM indices are uint8/uint16/uint32, not physical type %d", ejob->phys); return -1;
   }
 }
@@ -2251,19 +1794,16 @@ extern "C" int32_t dmb_dev_string_batch(const dmb_string_job *job, const uint32_
   };
   // Arrow modes: the TMA-staged pack kernel, unless the strings are long (long runs: the run-gather is
   // the better fit) or the heap is beyond 32-bit 16-byte units
-  static const bool no_pack = getenv("DMB_STR_NO_PACK") != nullptr;
-  if (!no_pack && (job->mode == DMB_STR_ARROW_UTF8 || job->mode == DMB_STR_ARROW_LARGE) && job->heap_len < (1ull << 35)) {
+  if ((job->mode == DMB_STR_ARROW_UTF8 || job->mode == DMB_STR_ARROW_LARGE) && job->heap_len < (1ull << 35)) {
     const bool large = job->mode == DMB_STR_ARROW_LARGE;
     // persistent grid: as many CTAs as are resident at once (tiles are claimed from a ticket)
-    auto launch_pack = [&](auto kernel, int rows_per_tile, int threads, uint32_t ob, uint32_t hb, bool unify = (DMB_PACK_UNIFY != 0)) -> int32_t {
+    auto launch_pack = [&](auto kernel, int rows_per_tile, int threads, uint32_t ob, uint32_t hb, bool unify = true) -> int32_t {
       const int64_t nt = (int64_t)(kVec / rows_per_tile) * nchunks;
       const size_t smem = (size_t)kPackTail + 2u * (size_t)rows_per_tile * 16u + ob + 2u * ((size_t)hb + 16u) + (unify ? (size_t)(threads - 64) * kPackScratchPerThread : 0u) + 128u;
       if (check_cuda(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem), "string_pack_kernel smem attribute")) return -1;
       int per_sm = 0;
       if (check_cuda(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, threads, smem), "string_pack_kernel occupancy")) return -1;
       if (per_sm < 1) { set_error("string_pack_kernel does not fit an SM (%zu bytes of shared memory)", smem); return -1; }
-      static const int cap = getenv("DMB_STR_PACK_CTAS") ? atoi(getenv("DMB_STR_PACK_CTAS")) : 0;
-      if (cap > 0 && per_sm > cap) per_sm = cap;
       int dev = 0, sms = kNumSMs;
       if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
       int64_t grid = (int64_t)per_sm * sms;
@@ -2271,30 +1811,13 @@ extern "C" int32_t dmb_dev_string_batch(const dmb_string_job *job, const uint32_
       kernel<<<(unsigned)grid, threads, smem, st>>>(*job, b, (unsigned long long *)scratch, nt, ob, hb);
       return check_cuda(cudaGetLastError(), "string_pack_kernel launch");
     };
-    static const int force_nw = getenv("DMB_STR_PACK_NW") ? atoi(getenv("DMB_STR_PACK_NW")) : 0;
-    // columns without a heap: the pipeline's lean form on whole-vector tiles (16 worker warps x 4 rows) by default --
-    // 0.270 / 0.313 ms per 60 M one-byte / l_shipmode-shaped rows, against 0.287 / 0.334 for the one-CTA-per-tile
-    // string_short_kernel (DMB_STR_SHORT_RPT=8 or 4 selects that one for A/B) and 0.297 / 0.336 for 8 worker warps
-    static const int short_rpt = getenv("DMB_STR_SHORT_RPT") ? atoi(getenv("DMB_STR_SHORT_RPT")) : 0;
-    if (job->heap_len == 0 && short_rpt > 0) {  // inlined strings only: one CTA per tile, prefix by look-back
-      auto launch_short = [&](auto kernel, int rows_per_tile, int threads = kThreads) -> int32_t {
-        const int64_t nt = (int64_t)(kVec / rows_per_tile) * nchunks;
-        kernel<<<(unsigned)nt, threads, 0, st>>>(*job, b, (unsigned long long *)scratch, nt, dmb_enum_job{});
-        return check_cuda(cudaGetLastError(), "string_short_kernel launch");
-      };
-      static const int short_nt = getenv("DMB_STR_SHORT_NT") ? atoi(getenv("DMB_STR_SHORT_NT")) : 0;  // (measured variants)
-      if (short_nt == 128) return large ? launch_short(string_short_kernel<true, 8, 0, 6, 128>, 1024, 128) : launch_short(string_short_kernel<false, 8, 0, 6, 128>, 1024, 128);
-      if (short_nt == 512) return large ? launch_short(string_short_kernel<true, 4, 0, 6, 512>, 2048, 512) : launch_short(string_short_kernel<false, 4, 0, 6, 512>, 2048, 512);
-      if (short_rpt == 4) return large ? launch_short(string_short_kernel<true, 4, 0>, 1024) : launch_short(string_short_kernel<false, 4, 0>, 1024);
-      return large ? launch_short(string_short_kernel<true, 8, 0>, 2048) : launch_short(string_short_kernel<false, 8, 0>, 2048);
-    }
-    if (job->heap_len == 0) {  // the pipeline's lean form, 4 rows per thread
-      if (force_nw == 8) {
-        const uint32_t ob = ((1024u * 12u + 64u) + 127u) & ~127u;
-        return large ? launch_pack(string_pack_kernel<true, 4, 8, false>, 1024, 8 * 32 + 64, ob, 0u) : launch_pack(string_pack_kernel<false, 4, 8, false>, 1024, 8 * 32 + 64, ob, 0u);
-      }
+    // columns without a heap: the pipeline's lean form on whole-vector tiles (16 worker warps x 4 rows) --
+    // 0.270 / 0.313 ms per 60 M one-byte / l_shipmode-shaped rows, against 0.287 / 0.334 for a one-CTA-per-tile
+    // kernel and 0.297 / 0.336 for 8 worker warps
+    if (job->heap_len == 0) {
+      constexpr int threads = pack_warps(false) * 32 + 64;
       const uint32_t ob = ((2048u * 12u + 64u) + 127u) & ~127u;
-      return large ? launch_pack(string_pack_kernel<true, 4, 16, false>, 2048, 16 * 32 + 64, ob, 0u) : launch_pack(string_pack_kernel<false, 4, 16, false>, 2048, 16 * 32 + 64, ob, 0u);
+      return large ? launch_pack(string_pack_kernel<true, 4, false>, 2048, threads, ob, 0u) : launch_pack(string_pack_kernel<false, 4, false>, 2048, threads, ob, 0u);
     }
     const double heap_per_row = (double)job->heap_len / (double)nrows;
     // the pipeline needs three CTAs per SM to hide its latencies: S[2] + O + H[2] <= ~72 KiB, i.e. a heap span of
@@ -2306,47 +1829,33 @@ extern "C" int32_t dmb_dev_string_batch(const dmb_string_job *job, const uint32_
     // shrink for it (C3: 30.8 heap bytes per row) keep the two-path kernel and the larger stage
     constexpr uint32_t kHb3 = ((233472u / 3u - 1024u - kPackTail - 2u * 512u * 16u - 2048u - 32u - 128u) / 3u) & ~127u;
     constexpr uint32_t kHb3u = ((233472u / 3u - 1024u - kPackTail - 2u * 512u * 16u - 2048u - 32u - 128u - 256u * kPackScratchPerThread) / 3u) & ~127u;
-    static const double min_slack = getenv("DMB_STR_PACK_MIN_SLACK") ? atof(getenv("DMB_STR_PACK_MIN_SLACK")) : 1.04;
-    static const double hpr_limit = getenv("DMB_STR_PACK_HPR_LIMIT") ? atof(getenv("DMB_STR_PACK_HPR_LIMIT")) : ((double)kHb3 - 1024.0 - 128.0) / (512.0 * min_slack);
-    if (heap_per_row <= hpr_limit) {
-      static const double slack = getenv("DMB_STR_PACK_SLACK") ? atof(getenv("DMB_STR_PACK_SLACK")) : 1.15;
-      // 512-row tiles, 8 worker warps, 3 CTAs per SM
-      // (measured on the C2 columns: the 16-warp CTAs are no faster, so they stay an experiment: DMB_STR_PACK_NW=16)
-      const bool wide = force_nw == 16 && heap_per_row <= 20.0;
-      const int rows = wide ? 1024 : 512;
-      uint32_t hb = ((uint32_t)(heap_per_row * rows * slack) + 1024u + 127u) & ~127u;
-      if (hb < 2048u) hb = 2048u;
-      // a stage a little tighter than `slack` asks for rather than a third CTA lost (tiles that overflow the stage
-      // are copied row by row: min_slack keeps them rare)
-      if (!wide && hb > kHb3 && (double)kHb3 >= heap_per_row * rows * min_slack + 1024.0) hb = kHb3;
-      const uint32_t ob = hb + (wide ? 4096u : 2048u);  // inlined rows add at most 12 bytes each; a tile that exceeds the stage is copied row by row
-      // few heap bytes per row (codes, short names): 1024-row tiles, 4 rows per thread, halve the per-tile costs
-      static const double r4_limit = getenv("DMB_STR_PACK_R4_LIMIT") ? atof(getenv("DMB_STR_PACK_R4_LIMIT")) : 9.5;
-      if (!wide && heap_per_row <= r4_limit) {
-        uint32_t hb4 = ((uint32_t)(heap_per_row * 1024.0 * slack) + 1024u + 127u) & ~127u;
+    constexpr double kSlack = 1.15;     // heap stage of a tile: its expected span times kSlack, + 1 KiB
+    // a stage a little tighter than kSlack asks for rather than a third CTA lost (tiles that overflow the stage are copied
+    // row by row: kMinSlack keeps them rare)
+    constexpr double kMinSlack = 1.04;
+    constexpr double kHprLimit = ((double)kHb3 - 1024.0 - 128.0) / (512.0 * kMinSlack);  // heap bytes per row the pipeline takes
+    constexpr double kR4Limit = 9.5;    // few heap bytes per row (codes, short names): 1024-row tiles, 4 rows per thread, halve the per-tile costs
+    constexpr int threads = pack_warps(true) * 32 + 64;
+    if (heap_per_row <= kHprLimit) {
+      if (heap_per_row <= kR4Limit) {
+        uint32_t hb4 = ((uint32_t)(heap_per_row * 1024.0 * kSlack) + 1024u + 127u) & ~127u;
         if (hb4 < 2048u) hb4 = 2048u;
-        const uint32_t ob4 = hb4 + 4096u + (DMB_PACK_UNIFY ? 2048u : 4096u);  // inlined rows add at most 12 bytes each: room for 6 (8) bytes per row (the scratch area took the rest of what three CTAs per SM leave)
-        return large ? launch_pack(string_pack_kernel<true, 4, 8, true>, 1024, 8 * 32 + 64, ob4, hb4)
-                     : launch_pack(string_pack_kernel<false, 4, 8, true>, 1024, 8 * 32 + 64, ob4, hb4);
+        const uint32_t ob4 = hb4 + 4096u + 2048u;  // inlined rows add at most 12 bytes each: room for 6 bytes per row (the scratch area took the rest of what three CTAs per SM leave)
+        return large ? launch_pack(string_pack_kernel<true, 4, true>, 1024, threads, ob4, hb4)
+                     : launch_pack(string_pack_kernel<false, 4, true>, 1024, threads, ob4, hb4);
       }
-      if (wide) return large ? launch_pack(string_pack_kernel<true, 2, 16, true>, 1024, 16 * 32 + 64, ob, hb) : launch_pack(string_pack_kernel<false, 2, 16, true>, 1024, 16 * 32 + 64, ob, hb);
-      static const int force_unify = getenv("DMB_STR_PACK_UNIFY") ? atoi(getenv("DMB_STR_PACK_UNIFY")) : -1;
-      const bool unify = force_unify >= 0 ? force_unify != 0 : (DMB_PACK_UNIFY != 0 && hb <= kHb3u);
-      if (!unify) return large ? launch_pack(string_pack_kernel<true, 2, 8, true, false>, 512, 8 * 32 + 64, ob, hb, false) : launch_pack(string_pack_kernel<false, 2, 8, true, false>, 512, 8 * 32 + 64, ob, hb, false);
-      return large ? launch_pack(string_pack_kernel<true, 2, 8, true, true>, 512, 8 * 32 + 64, ob, hb, true) : launch_pack(string_pack_kernel<false, 2, 8, true, true>, 512, 8 * 32 + 64, ob, hb, true);
+      // 512-row tiles, 2 rows per thread
+      uint32_t hb = ((uint32_t)(heap_per_row * 512 * kSlack) + 1024u + 127u) & ~127u;
+      if (hb < 2048u) hb = 2048u;
+      if (hb > kHb3 && (double)kHb3 >= heap_per_row * 512 * kMinSlack + 1024.0) hb = kHb3;
+      const uint32_t ob = hb + 2048u;  // inlined rows add at most 12 bytes each; a tile that exceeds the stage is copied row by row
+      if (hb <= kHb3u) return large ? launch_pack(string_pack_kernel<true, 2, true, true>, 512, threads, ob, hb, true) : launch_pack(string_pack_kernel<false, 2, true, true>, 512, threads, ob, hb, true);
+      return large ? launch_pack(string_pack_kernel<true, 2, true, false>, 512, threads, ob, hb, false) : launch_pack(string_pack_kernel<false, 2, true, false>, 512, threads, ob, hb, false);
     }
   }
-  if (job->heap_len == 0 && !getenv("DMB_STR_NO_INLINE_KERNEL")) {  // no heap: inlined strings only, whole-vector tiles
-    auto launch_inl = [&](auto kernel) -> int32_t {
-      kernel<<<(unsigned)nchunks, kThreads, 0, st>>>(*job, b, (unsigned long long *)scratch, nchunks);
-      return check_cuda(cudaGetLastError(), "string_inline_kernel launch");
-    };
-    switch (job->mode) {
-      case DMB_STR_ARROW_UTF8: return launch_inl(string_inline_kernel<DMB_STR_ARROW_UTF8>);
-      case DMB_STR_ARROW_LARGE: return launch_inl(string_inline_kernel<DMB_STR_ARROW_LARGE>);
-      case DMB_STR_REF_BLOB: return launch_inl(string_inline_kernel<DMB_STR_REF_BLOB>);
-      default: set_error("dmb_dev_string_batch: bad mode %d", job->mode); return -1;
-    }
+  if (job->heap_len == 0 && job->mode == DMB_STR_REF_BLOB) {  // no heap: inlined strings only, whole-vector tiles
+    string_inline_kernel<DMB_STR_REF_BLOB><<<(unsigned)nchunks, kThreads, 0, st>>>(*job, b, (unsigned long long *)scratch, nchunks);
+    return check_cuda(cudaGetLastError(), "string_inline_kernel launch");
   }
   switch (job->mode) {
     case DMB_STR_ARROW_UTF8: return launch(string_batch_kernel<DMB_STR_ARROW_UTF8>);

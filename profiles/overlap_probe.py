@@ -61,7 +61,7 @@ def main():
         step.check()
         return a.elapsed_time(b) / k
 
-    out = {"rows": args.rows, "pack_ctas_cap": os.environ.get("DMB_STR_PACK_CTAS")}
+    out = {"rows": args.rows}
     out["sequential_ms"] = timed(sequential, args.steps)
     out["two_streams_fixed_first_ms"] = timed(lambda: two_streams(False), args.steps)
     out["two_streams_strings_first_ms"] = timed(lambda: two_streams(True), args.steps)

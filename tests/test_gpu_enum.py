@@ -165,7 +165,7 @@ def _expected_utf8(labels, idx, valid):
     (1, 1, 12, "full", 0.0), (2048, 2, 1, "full", 0.5), (2049, 256, 12, "ragged", 0.2),   # 256 labels: the largest fused dictionary
     (300_001, 7, 8, "ragged", 0.1), (1_000_000, 7, 7, "full", 0.0), (50_000, 3, 12, "ragged", 1.0)])
 def test_enum_fused_lookup_and_pack_every_offset_and_byte(ctx, n, k, max_len, pattern, null_frac):
-    """uint8 ENUM with labels of <= 12 bytes: indices -> utf8 in ONE launch (dmb_dev_enum_utf8: string_short_kernel<.., EW>),
+    """uint8 ENUM with labels of <= 12 bytes: indices -> utf8 in ONE launch (dmb_dev_enum_utf8: enum_pack_kernel<.., EW>),
     no string_t intermediate.  Every offset and every data byte against the numpy restatement and the oracle's cells."""
     from duckdb_mbt_b200 import typed_result as tr
     batch, labels, idx, valid = _enum_batch(n, k, max_len, pattern, 900 + n + k, null_frac=null_frac)

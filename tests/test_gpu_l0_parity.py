@@ -154,7 +154,8 @@ def test_string_config_c2_columns():
 @pytest.mark.parametrize("n,pattern,max_len", [(1, "full", 12), (2048, "full", 1), (2049, "full", 12), (50_000, "ragged", 12),
                                                (70_001, "ragged", 3), (30_000, "full", 0)])
 def test_string_inline_only_columns_take_the_whole_vector_kernel(n, pattern, max_len):
-    """Columns without a heap (every string inlined): string_inline_kernel, all three modes."""
+    """Columns without a heap (every string inlined), all three modes: the pack kernel's lean form (Arrow modes) and
+    string_inline_kernel (reference blob), both on whole-vector tiles."""
     dev = _device_mod()
     rng = np.random.default_rng(900 + n)
     counts = ch.chunk_counts(n, pattern, rng)

@@ -147,7 +147,7 @@ __device__ __forceinline__ void render_i128(TB &t, unsigned __int128 u, bool is_
   }
 }
 
-// ---- DOUBLE / FLOAT: shortest decimal that reads back as the same double (what DuckDB's fmt-based
+// ---- DOUBLE / FLOAT: shortest decimal that reads back as the same double / float (what DuckDB's fmt-based
 // cast prints: "3.5", "5.333333333333333", src/duckdb_fixture_cases.mbt:20-25,167-172,216-221),
 // by Ryu (Ulf Adams, PLDI 2018): one 64x128-bit multiplication by a tabulated power of 5 gives the
 // decimal images of the value and of its two rounding-interval ends, then digits are dropped
@@ -244,10 +244,100 @@ __device__ __forceinline__ uint64_t ryu_shortest(uint64_t bits, int &exp10) {
   return out;
 }
 
+// FLOAT: Ryu's float form (f2s), the same steps on a 24-bit significand with 32-bit decimal images.  Its
+// multipliers are the high words of the double tables (61 significant bits; the inverse ones + 1).
+__device__ __forceinline__ uint32_t ryu_mul_shift32(uint32_t m, uint64_t factor, int shift) {
+  const uint64_t sum = (((uint64_t)m * (uint32_t)factor) >> 32) + (uint64_t)m * (uint32_t)(factor >> 32);
+  return (uint32_t)(sum >> (shift - 32));
+}
+__device__ __forceinline__ uint32_t ryu_pow5_inv32(uint32_t m, int q, int j) { return ryu_mul_shift32(m, __ldg(&kRyuPow5InvSplit[q][1]) + 1ull, j); }
+__device__ __forceinline__ uint32_t ryu_pow5_32(uint32_t m, int i, int j) { return ryu_mul_shift32(m, __ldg(&kRyuPow5Split[i][1]), j); }
+__device__ __forceinline__ int ryu_pow5_bits(int e) { return ((e * 1217359) >> 19) + 1; }
+// bits of a finite non-zero float -> (digits, exponent): value = digits * 10^exponent, digits shortest
+__device__ __forceinline__ uint32_t ryu_shortest_f32(uint32_t bits, int &exp10) {
+  constexpr int kBits = 61;  // 125 - 64
+  const uint32_t ieee_m = bits & ((1u << 23) - 1u);
+  const int ieee_e = (int)((bits >> 23) & 0xffu);
+  int e2;
+  uint32_t m2;
+  if (ieee_e == 0) { e2 = 1 - 127 - 23 - 2; m2 = ieee_m; }
+  else { e2 = ieee_e - 127 - 23 - 2; m2 = (1u << 23) | ieee_m; }
+  const bool accept = (m2 & 1u) == 0u;
+  const uint32_t mv = 4u * m2, mp = mv + 2u;
+  const uint32_t mm = mv - 1u - ((ieee_m != 0u || ieee_e <= 1) ? 1u : 0u);
+  uint32_t vr, vp, vm, last = 0;
+  int e10;
+  bool vm_tz = false, vr_tz = false;
+  auto pow5_multiple = [](uint32_t v, int p) { int c = 0; while (v != 0u && v % 5u == 0u) { v /= 5u; ++c; } return c >= p; };
+  if (e2 >= 0) {
+    const int q = (e2 * 78913) >> 18;
+    e10 = q;
+    const int i = -e2 + q + kBits + ryu_pow5_bits(q) - 1;
+    vr = ryu_pow5_inv32(mv, q, i);
+    vp = ryu_pow5_inv32(mp, q, i);
+    vm = ryu_pow5_inv32(mm, q, i);
+    if (q != 0 && (vp - 1u) / 10u <= vm / 10u)  // the loop below may not run: one removed digit is still needed
+      last = ryu_pow5_inv32(mv, q - 1, -e2 + q - 1 + kBits + ryu_pow5_bits(q - 1) - 1) % 10u;
+    if (q <= 9) {
+      if (mv % 5u == 0u) vr_tz = pow5_multiple(mv, q);
+      else if (accept) vm_tz = pow5_multiple(mm, q);
+      else vp -= pow5_multiple(mp, q) ? 1u : 0u;
+    }
+  } else {
+    const int q = ((-e2) * 732923) >> 20;
+    e10 = q + e2;
+    const int i = -e2 - q;
+    const int j = q - (ryu_pow5_bits(i) - kBits);
+    vr = ryu_pow5_32(mv, i, j);
+    vp = ryu_pow5_32(mp, i, j);
+    vm = ryu_pow5_32(mm, i, j);
+    if (q != 0 && (vp - 1u) / 10u <= vm / 10u)
+      last = ryu_pow5_32(mv, i + 1, q - 1 - (ryu_pow5_bits(i + 1) - kBits)) % 10u;
+    if (q <= 1) {
+      vr_tz = true;
+      if (accept) vm_tz = mm == mv - 2u;
+      else --vp;
+    } else if (q < 31) {
+      vr_tz = (mv & ((1u << (q - 1)) - 1u)) == 0u;
+    }
+  }
+  int removed = 0;
+  uint32_t out;
+  if (vm_tz || vr_tz) {
+    while (vp / 10u > vm / 10u) {
+      vm_tz = vm_tz && vm % 10u == 0u;
+      vr_tz = vr_tz && last == 0u;
+      last = vr % 10u;
+      vr /= 10u; vp /= 10u; vm /= 10u;
+      ++removed;
+    }
+    if (vm_tz) {
+      while (vm % 10u == 0u) {
+        vr_tz = vr_tz && last == 0u;
+        last = vr % 10u;
+        vr /= 10u; vp /= 10u; vm /= 10u;
+        ++removed;
+      }
+    }
+    if (vr_tz && last == 5u && vr % 2u == 0u) last = 4u;  // exactly half: round to even
+    out = vr + (((vr == vm && (!accept || !vm_tz)) || last >= 5u) ? 1u : 0u);
+  } else {
+    while (vp / 10u > vm / 10u) {
+      last = vr % 10u;
+      vr /= 10u; vp /= 10u; vm /= 10u;
+      ++removed;
+    }
+    out = vr + ((vr == vm || last >= 5u) ? 1u : 0u);
+  }
+  exp10 = e10 + removed;
+  return out;
+}
+
 // fmt-style layout of the digits: fixed notation for 1e-5 <= |v| < 1e16 (always with a fraction:
-// "1.0"), else d.ddde+XX (at least two exponent digits)
+// "1.0"), else d.ddde+XX (at least two exponent digits).  DOUBLE takes the double's shortest digits,
+// FLOAT the float's own ("0.1", not the widened double's "0.10000000149011612"), as DuckDB prints them.
 template <class TB>
-__device__ __forceinline__ void render_double(TB &t, double v) {
+__device__ __forceinline__ void render_double(TB &t, double v, bool is_float) {
   const uint64_t bits = (uint64_t)__double_as_longlong(v);
   if (((bits >> 52) & 0x7ffu) == 0x7ffu) {
     if (bits & ((1ull << 52) - 1ull)) t.push_str("nan");
@@ -256,7 +346,7 @@ __device__ __forceinline__ void render_double(TB &t, double v) {
   }
   uint64_t digits = 0;
   int e = 0;
-  if (bits & ~(1ull << 63)) digits = ryu_shortest(bits, e);
+  if (bits & ~(1ull << 63)) digits = is_float ? ryu_shortest_f32(__float_as_uint((float)v), e) : ryu_shortest(bits, e);
   while (digits != 0ull && digits % 10ull == 0ull) { digits /= 10ull; ++e; }
   char m[20];  // most significant digit first
   int nd = 0;
@@ -390,7 +480,7 @@ render_text_kernel(dmb_render_job job, const uint32_t *__restrict__ counts, int6
         }
         double fv = 0.0;
         if (job.phys == DMB_PHYS_F64) fv = reinterpret_cast<const double *>(in)[i];
-        if (job.phys == DMB_PHYS_F32) fv = (double)reinterpret_cast<const float *>(in)[i];  // the oracle widens first (UNPINNED)
+        if (job.phys == DMB_PHYS_F32) fv = (double)reinterpret_cast<const float *>(in)[i];  // exact; rendered with the float's digits
         unsigned __int128 wide = 0;
         if (job.phys == DMB_PHYS_I128 || job.phys == DMB_PHYS_U128 || job.phys == DMB_PHYS_INTERVAL) {
           const uint4 q = reinterpret_cast<const uint4 *>(in)[i];
@@ -399,16 +489,21 @@ render_text_kernel(dmb_render_job job, const uint32_t *__restrict__ counts, int6
         switch (job.type_id) {
           case DMB_TYPE_BOOLEAN: t.push_str(u ? "true" : "false"); break;
           case DMB_TYPE_UBIGINT: t.push_u64(u, 1); break;
-          case DMB_TYPE_DATE: render_date(t, v); break;
-          case DMB_TYPE_TIMESTAMP: render_timestamp(t, v, 1000000, false); break;
-          case DMB_TYPE_TIMESTAMP_TZ: render_timestamp(t, v, 1000000, true); break;
+          // DuckDB's infinite DATE is +-INT32_MAX and its infinite TIMESTAMP / TIMESTAMPTZ +-INT64_MAX; they print as words
+          case DMB_TYPE_DATE:
+            if (v == 2147483647ll || v == -2147483647ll) t.push_str(v < 0 ? "-infinity" : "infinity"); else render_date(t, v);
+            break;
+          case DMB_TYPE_TIMESTAMP: case DMB_TYPE_TIMESTAMP_TZ:
+            if (v == INT64_MAX || v == -INT64_MAX) t.push_str(v < 0 ? "-infinity" : "infinity");
+            else render_timestamp(t, v, 1000000, job.type_id == DMB_TYPE_TIMESTAMP_TZ);
+            break;
           case DMB_TYPE_TIMESTAMP_S: render_timestamp(t, v, 1, false); break;
           case DMB_TYPE_TIMESTAMP_MS: render_timestamp(t, v, 1000, false); break;
           case DMB_TYPE_TIMESTAMP_NS: render_timestamp(t, v, 1000000000, false); break;
           case DMB_TYPE_DECIMAL:
             if (job.phys == DMB_PHYS_I128) render_i128(t, wide, true, job.dec_scale); else render_decimal(t, v, job.dec_scale);
             break;
-          case DMB_TYPE_FLOAT: case DMB_TYPE_DOUBLE: render_double(t, fv); break;
+          case DMB_TYPE_FLOAT: case DMB_TYPE_DOUBLE: render_double(t, fv, job.type_id == DMB_TYPE_FLOAT); break;
           case DMB_TYPE_HUGEINT: render_i128(t, wide, true, 0); break;
           case DMB_TYPE_UHUGEINT: render_i128(t, wide, false, 0); break;
           case DMB_TYPE_TIME: render_time(t, v, 1000000); break;

@@ -84,6 +84,8 @@ def lib():
         L.ora_render_decimal64.argtypes = [C.c_int64, C.c_int, C.c_char_p]
         L.ora_render_double.restype = C.c_int
         L.ora_render_double.argtypes = [C.c_double, C.c_char_p]
+        L.ora_render_float.restype = C.c_int
+        L.ora_render_float.argtypes = [C.c_float, C.c_char_p]
         for name, vt in (("int32", None), ("int64_as_int", None), ("double", None), ("bool", None)):
             f = getattr(L, f"ora_decode_{name}")
             f.restype = C.c_int64
@@ -318,6 +320,10 @@ def render_decimal64(v: int, scale: int) -> str:
 
 def render_double(v: float) -> str:
     return _render(lib().ora_render_double, v)
+
+
+def render_float(v: float) -> str:
+    return _render(lib().ora_render_float, v)
 
 
 def rev_fixed(values: np.ndarray, bitmap: Optional[np.ndarray], bit_offset: int, nrows: int, rev_op: int, w_out: int):

@@ -994,15 +994,19 @@ int ora_render_decimal64(int64_t v, int scale, char *out) {
   out[pos] = 0;
   return pos;
 }
-/* shortest round-trip double, fmt-style (UNPINNED beyond "3.5", "5.333333333333333", "nan", "inf") */
-int ora_render_double(double v, char *out) {
+/* does the decimal text read back as v: as a double, or for FLOAT as the float v holds exactly */
+static int reads_back(const char *text, double v, int is_float) { return is_float ? strtof(text, NULL) == (float)v : strtod(text, NULL) == v; }
+
+/* shortest round-trip double (FLOAT: shortest round-trip float, DuckDB prints 0.1f as "0.1"), fmt-style
+ * (UNPINNED beyond "3.5", "5.333333333333333", "nan", "inf") */
+static int render_shortest(double v, int is_float, char *out) {
   if (isnan(v)) return sprintf(out, "nan");
   if (isinf(v)) return sprintf(out, v < 0 ? "-inf" : "inf");
   char buf[40];
   int prec;
-  for (prec = 1; prec <= 17; prec++) {
+  for (prec = 1; prec <= (is_float ? 9 : 17); prec++) {
     snprintf(buf, sizeof buf, "%.*e", prec - 1, v);
-    if (strtod(buf, NULL) == v) break;
+    if (reads_back(buf, v, is_float)) break;
     /* the correctly rounded prec-digit decimal is the closest one, but below a power of two the
      * rounding interval is half as wide as above it: the next prec-digit decimal up (or down) may
      * still read back as v although the closest does not.  Shortest round trip takes it. */
@@ -1016,7 +1020,7 @@ int ora_render_double(double v, char *out) {
         unsigned long long m2 = m + (unsigned long long)(long long)step;
         char cand[48];
         snprintf(cand, sizeof cand, "%s%llue%d", ng ? "-" : "", m2, x10 - (prec - 1));
-        if (m2 != 0 && strtod(cand, NULL) == v) {
+        if (m2 != 0 && reads_back(cand, v, is_float)) {
           /* renormalise: m2 may have gained a digit (99 -> 100) */
           char digits[24];
           int nd2 = snprintf(digits, sizeof digits, "%llu", m2);
@@ -1060,6 +1064,8 @@ int ora_render_double(double v, char *out) {
   pos += sprintf(out + pos, "e%c%02d", exp10 < 0 ? '-' : '+', exp10 < 0 ? -exp10 : exp10);
   return pos;
 }
+int ora_render_double(double v, char *out) { return render_shortest(v, 0, out); }
+int ora_render_float(float v, char *out) { return render_shortest((double)v, 1, out); }
 
 /* one fixed-width cell -> DuckDB text (what duckdb_value_varchar / the chunk path's
  * duckdb_value_to_string hand to MoonBit, src/duckdb_native.c:224-238).  Returns length, -1 if the
@@ -1072,11 +1078,15 @@ int ora_render_cell(const ora_column *c, const uint8_t *p, char *out) {
     case T_UTINYINT: case T_USMALLINT: case T_UINTEGER:
       return sprintf(out, "%lld", (long long)load_i64(c, p, &ok));
     case T_UBIGINT: { uint64_t v; memcpy(&v, p, 8); return sprintf(out, "%llu", (unsigned long long)v); }
-    case T_FLOAT: { float v; memcpy(&v, p, 4); return ora_render_double((double)v, out); } /* UNPINNED (float shortest) */
+    case T_FLOAT: { float v; memcpy(&v, p, 4); return ora_render_float(v, out); } /* UNPINNED layout; digits float shortest */
     case T_DOUBLE: { double v; memcpy(&v, p, 8); return ora_render_double(v, out); }
-    case T_DATE: { int32_t v; memcpy(&v, p, 4); return ora_render_date(v, out); }
-    case T_TIMESTAMP: { int64_t v; memcpy(&v, p, 8); return ora_render_timestamp(v, 1000000, 0, out); }
-    case T_TIMESTAMP_TZ: { int64_t v; memcpy(&v, p, 8); return ora_render_timestamp(v, 1000000, 1, out); }
+    /* DuckDB stores 'infinity' / '-infinity' as DATE +-INT32_MAX and TIMESTAMP / TIMESTAMPTZ +-INT64_MAX and prints the words */
+    case T_DATE: { int32_t v; memcpy(&v, p, 4);
+      if (v == INT32_MAX || v == -INT32_MAX) return sprintf(out, "%s", v < 0 ? "-infinity" : "infinity");
+      return ora_render_date(v, out); }
+    case T_TIMESTAMP: case T_TIMESTAMP_TZ: { int64_t v; memcpy(&v, p, 8);
+      if (v == INT64_MAX || v == -INT64_MAX) return sprintf(out, "%s", v < 0 ? "-infinity" : "infinity");
+      return ora_render_timestamp(v, 1000000, c->type_id == T_TIMESTAMP_TZ, out); }
     case T_TIMESTAMP_S: { int64_t v; memcpy(&v, p, 8); return ora_render_timestamp(v, 1, 0, out); }
     case T_TIMESTAMP_MS: { int64_t v; memcpy(&v, p, 8); return ora_render_timestamp(v, 1000, 0, out); }
     case T_TIMESTAMP_NS: { int64_t v; memcpy(&v, p, 8); return ora_render_timestamp(v, 1000000000, 0, out); }

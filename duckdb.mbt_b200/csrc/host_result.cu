@@ -64,12 +64,17 @@ struct TypedOut {
   void *values = nullptr, *valid = nullptr, *offsets = nullptr, *data = nullptr;  // pinned
 };
 
-// ---- nested types (SURVEY.md 8f item 3).  The child level of a LIST / MAP column described by dmb_host_list.child_col:
-// every "leaf" is one vector family (one child vector per chunk, sizes[k] elements of it), staged as one flat slab.
-struct ListNode;
-struct Leaf {
+// the type of a column or of a nested leaf: what arrow_map needs of either
+struct ColType {
   std::string name;
   int32_t type_id = 0, phys = 0, dec_width = 0, dec_scale = 0, width = 0;
+};
+
+// ---- nested types (SURVEY.md 8f item 3).  The child level of a LIST / MAP column, in whichever form dmb_host_list gave
+// it (flat fixed-width fields or child_col): every "leaf" is one vector family (one child vector per chunk, sizes[k]
+// elements of it), staged as one flat slab.
+struct ListNode;
+struct Leaf : ColType {
   std::vector<const void *> data;      // [nchunks]
   std::vector<const void *> validity;  // [nchunks] or empty (no masks at all)
   // staged
@@ -91,9 +96,7 @@ struct ListNode {
   bool staged = false;
 };
 
-struct Col {
-  std::string name;
-  int32_t type_id = 0, phys = 0, dec_width = 0, dec_scale = 0, width = 0;
+struct Col : ColType {
   std::vector<const void *> data;
   std::vector<const void *> validity;  // entries may be NULL; empty = no masks at all
   bool any_validity = false;
@@ -101,21 +104,10 @@ struct Col {
   uint64_t heap_len = 0;
   bool force_large = false;  // export as large_utf8 / large_binary whatever the size (all parts of a sharded table agree)
   std::shared_ptr<EnumDict> dict;  // ENUM
-  // LIST: per-chunk child vectors
-  bool is_list = false;
-  int32_t child_type_id = 0, child_phys = 0, child_dec_width = 0, child_dec_scale = 0, child_width = 0;
-  std::vector<const void *> child_data;
-  std::vector<const void *> child_validity;  // empty = no masks at all
-  std::vector<uint64_t> child_sizes, child_base;  // child_base: element index of chunk k's child vector in the staged slab (nchunks + 1)
-  std::vector<int64_t> child_val_off;
-  uint8_t *d_child = nullptr;
-  uint64_t *d_child_validity = nullptr, *d_child_base = nullptr, *d_child_sizes = nullptr;
-  int64_t *d_child_val_off = nullptr;
-  bool child_staged = false;
   // STRUCT: the fields are columns of their own, appended behind the visible ones (indices into Result::cols)
   bool is_struct = false;
   std::vector<int> kids;
-  // LIST / MAP whose child is described as a column (VARCHAR, STRUCT, LIST children)
+  // LIST / MAP: the child level
   std::shared_ptr<ListNode> node;
   bool is_map = false;
   // device copy (lives as long as the result)
@@ -767,187 +759,18 @@ int32_t blob_text_source(Result *r, Scope &sc, int j, StringSource *src) {
   return 0;
 }
 
-// ------------------------------------------------------------------ LIST columns (kernels_list.cu)
-struct ListRun {
-  void *d_offsets = nullptr;
-  size_t offsets_bytes = 0;
-  uint8_t *d_child = nullptr;
-  uint64_t *d_child_bitmap = nullptr;
-  FixedRun validity;  // the LIST column's own bitmap / null count
-  unsigned long long *h_ctr = nullptr;  // pinned: [0] child elements [1] child nulls [2] error flags [3] parent null count
-  uint64_t capacity = 0;
-  uint8_t *d_child_out = nullptr;  // the child in its Arrow form (== d_child when it is exported as stored)
-  size_t child_out_bytes = 0;
-  cudaEvent_t done = nullptr;
-};
-
-// the child vectors of all chunks back to back on the device (gathered through a pinned arena: the vectors have different sizes)
-int32_t stage_list_child(Result *r, int j) {
-  Col &col = r->cols[(size_t)j];
-  if (col.child_staged) return 0;
-  CtxCore &c = *r->core;
-  const int64_t nch = r->nchunks;
-  const uint64_t total = col.child_base[(size_t)nch];
-  const size_t W = (size_t)col.child_width;
-  uint64_t words = 0;
-  for (int64_t k = 0; k < nch; ++k)
-    if (col.child_val_off[(size_t)k] >= 0) words += (col.child_sizes[(size_t)k] + 63) / 64 + 1;
-  uint8_t *arena = (uint8_t *)keep_pin(r, (size_t)total * W + 64);
-  uint64_t *warena = (uint64_t *)keep_pin(r, (size_t)(words + 2) * 8);
-  uint64_t *h_base = (uint64_t *)keep_pin(r, (size_t)(nch + 1) * 8);
-  uint64_t *h_sizes = (uint64_t *)keep_pin(r, (size_t)(nch + 1) * 8);
-  col.d_child_sizes = (uint64_t *)keep_dev(r, (size_t)(nch + 1) * 8);
-  int64_t *h_voff = (int64_t *)keep_pin(r, (size_t)(nch + 1) * 8);
-  col.d_child = (uint8_t *)keep_dev(r, (size_t)total * W + 64);
-  col.d_child_validity = (uint64_t *)keep_dev(r, (size_t)(words + 2) * 8);
-  col.d_child_base = (uint64_t *)keep_dev(r, (size_t)(nch + 1) * 8);
-  col.d_child_val_off = (int64_t *)keep_dev(r, (size_t)(nch + 1) * 8);
-  if (!arena || !warena || !h_base || !h_voff || !h_sizes || !col.d_child_sizes || !col.d_child || !col.d_child_validity || !col.d_child_base || !col.d_child_val_off) return -1;
-  memset(warena, 0, (size_t)(words + 2) * 8);
-  parallel_for(c, nch, [&](int64_t k) {
-    const uint64_t sz = col.child_sizes[(size_t)k];
-    if (sz) memcpy(arena + (size_t)col.child_base[(size_t)k] * W, col.child_data[(size_t)k], (size_t)sz * W);
-    if (col.child_val_off[(size_t)k] >= 0) memcpy(warena + col.child_val_off[(size_t)k], col.child_validity[(size_t)k], (size_t)((sz + 63) / 64) * 8);
-  });
-  memcpy(h_base, col.child_base.data(), (size_t)(nch + 1) * 8);
-  memcpy(h_voff, col.child_val_off.data(), (size_t)nch * 8);
-  if (nch) memcpy(h_sizes, col.child_sizes.data(), (size_t)nch * 8);
-  if (nch && check_cuda(cudaMemcpyAsync(col.d_child_sizes, h_sizes, (size_t)nch * 8, cudaMemcpyHostToDevice, c.s_in), "list child sizes H2D")) return -1;
-  if (total && check_cuda(cudaMemcpyAsync(col.d_child, arena, (size_t)total * W, cudaMemcpyHostToDevice, c.s_in), "list child H2D")) return -1;
-  if (words && check_cuda(cudaMemcpyAsync(col.d_child_validity, warena, (size_t)words * 8, cudaMemcpyHostToDevice, c.s_in), "list child masks H2D")) return -1;
-  if (check_cuda(cudaMemcpyAsync(col.d_child_base, h_base, (size_t)(nch + 1) * 8, cudaMemcpyHostToDevice, c.s_in), "list child base H2D")) return -1;
-  if (nch && check_cuda(cudaMemcpyAsync(col.d_child_val_off, h_voff, (size_t)nch * 8, cudaMemcpyHostToDevice, c.s_in), "list child mask offsets H2D")) return -1;
-  r->bytes_h2d += total * W + words * 8 + (uint64_t)(2 * nch + 1) * 8;
-  col.child_staged = true;
-  return 0;
-}
-
-// child_op: the child's fixed-width conversion (DMB_OP(child phys, dst)); children that are not exported as stored
-// (BOOLEAN -> bits, DECIMAL -> decimal128, INTERVAL -> month_day_nano) take a second pass over the gathered, dense child
-int32_t run_list(Result *r, Scope &sc, int j, int32_t child_op, bool child_as_stored, ListRun *out) {
-  Col &col = r->cols[(size_t)j];
-  CtxCore &c = *r->core;
-  const int64_t n = r->nrows, nch = r->nchunks;
-  if (stage_list_child(r, j)) return -1;  // before stage_column: its event then covers these copies too (same stream)
-  if (col.staged) {  // the entries were staged earlier: order the compute stream behind the child copies as well
-    cudaEvent_t e = sc.event(false);
-    if (!e) return -1;
-    cudaEventRecord(e, c.s_in);
-    if (check_cuda(cudaStreamWaitEvent(c.s_compute, e, 0), "wait list child")) return -1;
-  }
-  // the column's own validity bitmap + null count (also stages the entries)
-  if (run_fixed(r, sc, j, DMB_OP_VALIDITY_ONLY, 0, true, false, &out->validity)) return -1;
-  // upper bound of the child elements the export can hold: every element of every child vector, or (shared spans) more:
-  // sized exactly by a host pass over the entries
-  uint64_t cap = 0;
-  std::atomic<bool> outside{false};
-  {
-    std::vector<uint64_t> part((size_t)(nch > 0 ? nch : 1), 0);
-    parallel_for(c, nch, [&](int64_t k) {
-      const uint64_t *e = reinterpret_cast<const uint64_t *>(col.data[(size_t)k]);
-      const void *mask = col.validity.empty() ? nullptr : col.validity[(size_t)k];
-      uint64_t sum = 0;
-      const uint64_t csize = col.child_sizes[(size_t)k];
-      for (uint32_t i = 0; e && i < r->counts[(size_t)k]; ++i) {
-        if (!host_row_valid(mask, i)) continue;
-        if (e[2 * i] > csize || e[2 * i + 1] > csize - e[2 * i]) { outside.store(true); continue; }
-        sum += e[2 * i + 1];
-      }
-      part[(size_t)k] = sum;
-    });
-    for (uint64_t v : part) cap += v;
-  }
-  if (outside.load()) { set_error("LIST column %d: an entry reaches outside its chunk's child vector (offset + length > duckdb_list_vector_get_size)", j); return -1; }
-  if (cap > 0x7fffffffull) { set_error("LIST column %d: %llu child elements exceed int32 offsets; use smaller batches", j, (unsigned long long)cap); return -1; }
-  out->capacity = cap;
-  out->offsets_bytes = (size_t)(n + 1) * 4;
-  out->d_offsets = sc.dalloc(out->offsets_bytes + 64);
-  out->d_child = (uint8_t *)sc.dalloc((size_t)cap * (size_t)col.child_width + 64);
-  out->d_child_bitmap = (uint64_t *)sc.dalloc((size_t)((cap + DMB_VECTOR_SIZE - 1) / DMB_VECTOR_SIZE * DMB_VALIDITY_WORDS + 2) * 8);  // whole 32-word masks: the conversion pass reads it as chunk masks
-  unsigned long long *d_ctr = (unsigned long long *)sc.dalloc(16);
-  void *d_scratch = sc.dalloc(dmb_dev_list_scratch_bytes(nch) + 16);
-  out->h_ctr = (unsigned long long *)sc.palloc(32);
-  if (!out->d_offsets || !out->d_child || !out->d_child_bitmap || !d_ctr || !d_scratch || !out->h_ctr) return -1;
-  memset(out->h_ctr, 0, 32);
-  if (n == 0) return 0;
-  if (check_cuda(cudaMemsetAsync(d_ctr, 0, 16, c.s_compute), "list counters memset")) return -1;
-  dmb_list_job job;
-  memset(&job, 0, sizeof(job));
-  job.in_entries = col.d_data;
-  job.in_validity = col.d_validity;
-  job.vecs = col.d_vecs;
-  job.child_base = col.d_child_base;
-  job.child_data = col.d_child;
-  job.child_validity = col.child_validity.empty() ? nullptr : col.d_child_validity;
-  job.child_val_off = col.d_child_val_off;
-  job.out_offsets = out->d_offsets;
-  job.out_child = out->d_child;
-  job.out_child_validity = out->d_child_bitmap;
-  job.total = d_ctr;
-  job.child_null_count = d_ctr + 1;
-  job.child_width = col.child_width;
-  job.large = 0;
-  job.child_sizes = col.d_child_sizes;
-  cudaEvent_t k0 = sc.event(true), k1 = sc.event(true), done = sc.event(false);
-  if (!k0 || !k1 || !done) return -1;
-  cudaEventRecord(k0, c.s_compute);
-  if (dmb_dev_list_batch(&job, r->d_counts, r->d_row_off, nch, n, (int64_t)cap, d_scratch, c.s_compute)) return -1;
-  cudaEventRecord(k1, c.s_compute);
-  sc.kernel_spans.emplace_back(k0, k1);
-  out->d_child_out = out->d_child;
-  out->child_out_bytes = (size_t)cap * (size_t)col.child_width;
-  if (!child_as_stored && cap > 0) {
-    // the gathered child is a dense column: 2048-element "chunks", its bitmap = their 32-word masks back to back
-    const int32_t ow = dmb_op_out_width(child_op);
-    if (ow < 0) { set_error("LIST column %d: unsupported child conversion 0x%x", j, child_op); return -1; }
-    const int64_t nck = (int64_t)((cap + DMB_VECTOR_SIZE - 1) / DMB_VECTOR_SIZE);
-    std::vector<uint32_t> cc((size_t)nck, DMB_VECTOR_SIZE);
-    std::vector<int64_t> ro((size_t)nck + 1);
-    std::vector<dmb_vec_desc> vd((size_t)nck);
-    cc[(size_t)nck - 1] = (uint32_t)(cap - (uint64_t)(nck - 1) * DMB_VECTOR_SIZE);
-    for (int64_t k = 0; k < nck; ++k) {
-      ro[(size_t)k] = k * (int64_t)DMB_VECTOR_SIZE;
-      vd[(size_t)k].data_off = (uint64_t)k * DMB_VECTOR_SIZE * (uint64_t)col.child_width;
-      vd[(size_t)k].val_off = k * DMB_VALIDITY_WORDS;
-    }
-    ro[(size_t)nck] = (int64_t)cap;
-    uint32_t *d_cc = (uint32_t *)upload_job(sc, cc.data(), cc.size() * sizeof(uint32_t));
-    int64_t *d_ro = (int64_t *)upload_job(sc, ro.data(), ro.size() * sizeof(int64_t));
-    dmb_vec_desc *d_vd = (dmb_vec_desc *)upload_job(sc, vd.data(), vd.size() * sizeof(dmb_vec_desc));
-    out->child_out_bytes = ow == 0 ? (size_t)((cap + 7) / 8) : (size_t)cap * (size_t)ow;
-    out->d_child_out = (uint8_t *)sc.dalloc(out->child_out_bytes + 64);
-    if (!d_cc || !d_ro || !d_vd || !out->d_child_out) return -1;
-    dmb_fixed_job fj;
-    memset(&fj, 0, sizeof(fj));
-    fj.in_data = out->d_child;
-    fj.in_validity = out->d_child_bitmap;
-    fj.vecs = d_vd;
-    fj.out_values = out->d_child_out;
-    fj.op = child_op;
-    void *fjd = upload_job(sc, &fj, sizeof(fj));
-    if (!fjd) return -1;
-    if (dmb_dev_fixed_batch((const dmb_fixed_job *)fjd, &fj, 1, d_cc, d_ro, nck, (int64_t)cap, c.s_compute)) return -1;
-    cudaEventRecord(k1, c.s_compute);  // the span now covers the conversion pass
-  }
-  if (check_cuda(cudaMemcpyAsync(out->h_ctr, d_ctr, 16, cudaMemcpyDeviceToHost, c.s_compute), "list counters D2H")) return -1;
-  if (check_cuda(cudaMemcpyAsync(out->h_ctr + 2, d_scratch, 8, cudaMemcpyDeviceToHost, c.s_compute), "list flags D2H")) return -1;
-  if (check_cuda(cudaMemcpyAsync(out->h_ctr + 3, out->validity.d_null_count, 8, cudaMemcpyDeviceToHost, c.s_compute), "null count D2H")) return -1;
-  cudaEventRecord(done, c.s_compute);
-  out->done = done;
-  return 0;
-}
-
 // ------------------------------------------------------------------ DuckDB type -> Arrow
 struct ArrowMap {
   int32_t op = -1;      // fixed-width conversion, or -1 for strings
-  bool is_string = false, is_list = false;
-  bool is_nested = false;  // STRUCT / MAP / LIST with a described child: converted synchronously (nested_to_arrow)
+  bool is_string = false;
+  bool is_list = false;    // LIST of one fixed-width leaf: pipelined (run_list)
+  bool is_nested = false;  // STRUCT / MAP / every other LIST: converted synchronously (nested_to_arrow)
   std::string format, child_format;
   int32_t child_op = -1;
-  bool child_as_stored = true;
 };
 
-bool arrow_map(const Col &col, ArrowMap *m) {
+// the scalar and string types; the caller maps ENUM, STRUCT, MAP and LIST, which need more than the type
+bool type_arrow_map(const ColType &col, ArrowMap *m) {
   char buf[48];
   auto same = [&](const char *fmt) { m->op = DMB_OP(col.phys, DMB_DST_SAME); m->format = fmt; return true; };
   switch (col.type_id) {
@@ -980,9 +803,22 @@ bool arrow_map(const Col &col, ArrowMap *m) {
       snprintf(buf, sizeof(buf), "d:%d,%d", col.dec_width > 0 ? col.dec_width : 38, col.dec_scale);
       m->format = buf;
       return true;
+    case DMB_TYPE_VARCHAR: m->is_string = true; m->format = "u"; return true;
+    case DMB_TYPE_BLOB: m->is_string = true; m->format = "z"; return true;
+    default: set_error("column type %d has no Arrow mapping", col.type_id); return false;
+  }
+}
+
+// Arrow keeps these as DuckDB stores them: a gathered LIST child needs no second pass
+bool stored_as_arrow(const ColType &t, int32_t op) { return op == DMB_OP(t.phys, DMB_DST_SAME) || t.type_id == DMB_TYPE_HUGEINT; }
+
+bool arrow_map(const Col &col, ArrowMap *m) {
+  switch (col.type_id) {
     case DMB_TYPE_ENUM:  // dictionary-encoded: the indices as stored, the labels as the dictionary (export_column)
       if (!col.dict) { set_error("ENUM column without a dictionary"); return false; }
-      return same(col.phys == DMB_PHYS_U8 ? "C" : col.phys == DMB_PHYS_U16 ? "S" : "I");
+      m->op = DMB_OP(col.phys, DMB_DST_SAME);
+      m->format = col.phys == DMB_PHYS_U8 ? "C" : col.phys == DMB_PHYS_U16 ? "S" : "I";
+      return true;
     case DMB_TYPE_STRUCT:
       if (!col.is_struct) { set_error("STRUCT column without field vectors"); return false; }
       m->is_nested = true;
@@ -993,37 +829,32 @@ bool arrow_map(const Col &col, ArrowMap *m) {
       m->is_nested = true;
       m->format = "+m";
       return true;
-    case DMB_TYPE_LIST: {  // list<child>, child copied as stored
-      if (col.node) { m->is_nested = true; m->format = "+l"; return true; }
-      if (!col.is_list) { set_error("LIST column without child vectors"); return false; }
-      Col child;
-      child.type_id = col.child_type_id;
-      child.phys = col.child_phys;
-      child.dec_width = col.child_dec_width;
-      child.dec_scale = col.child_dec_scale;
-      ArrowMap cm;
-      if (child.type_id == DMB_TYPE_LIST || child.type_id == DMB_TYPE_ENUM || !arrow_map(child, &cm)) { set_error("LIST child type %d has no Arrow mapping here", child.type_id); return false; }
-      if (cm.is_string) { set_error("LIST child type %d: VARCHAR / BLOB children are not exported yet", child.type_id); return false; }
-      m->child_as_stored = cm.op == DMB_OP(child.phys, DMB_DST_SAME) || child.type_id == DMB_TYPE_HUGEINT;
-      m->child_op = cm.op;
-      m->is_list = true;
+    case DMB_TYPE_LIST: {  // (fill_column gives every LIST column its node)
       m->format = "+l";
+      const ListNode &node = *col.node;
+      if (node.kind != ListNode::kLeaf || node.leaves[0].phys == DMB_PHYS_STRING) { m->is_nested = true; return true; }
+      // one fixed-width leaf: a flat child may have any fixed-width type, and one without an Arrow mapping fails here,
+      // at export, so that the result's other columns still serve
+      const Leaf &leaf = node.leaves[0];
+      ArrowMap cm;
+      if (!type_arrow_map(leaf, &cm) || cm.is_string) { set_error("LIST child type %d has no Arrow mapping here", leaf.type_id); return false; }
+      m->is_list = true;
+      m->child_op = cm.op;
       m->child_format = cm.format;
       return true;
     }
-    case DMB_TYPE_VARCHAR: m->is_string = true; m->format = "u"; return true;
-    case DMB_TYPE_BLOB: m->is_string = true; m->format = "z"; return true;
-    default: set_error("column type %d has no Arrow mapping", col.type_id); return false;
+    default: return type_arrow_map(col, m);
   }
 }
 
 
-// ------------------------------------------------------------------ nested types: STRUCT, MAP, LIST of VARCHAR / STRUCT / LIST
+// ------------------------------------------------------------------ nested types: STRUCT, MAP, LIST
 // (SURVEY.md 8f item 3; the reference rejects them on its chunk path, src/duckdb_native.c:271-303, and has no Arrow
 // mapping: the contract is the Arrow format, checked with pyarrow in tests/test_gpu_nested.py.)
 //   STRUCT          the fields are columns of their own (hidden behind the visible ones): each is converted like a
 //                   top-level column; the parent contributes its validity bitmap
-//   LIST<x>         level by level on DENSE arrays: list_emit_kernel gathers every leaf vector family of the child
+//   LIST<x>         a ListNode, whether dmb_host_list gave the child in its flat fixed-width fields or as child_col.
+//                   Level by level on DENSE arrays: list_emit_kernel gathers every leaf vector family of the child
 //                   level through the entries (one launch per leaf: offsets are recomputed, the entries are tiny next
 //                   to the children); a gathered leaf is a dense column, so
 //                     fixed width     -> its Arrow form (second pass of fixed_batch_kernel when it is not stored that way)
@@ -1033,8 +864,9 @@ bool arrow_map(const Col &col, ArrowMap *m) {
 //                     LIST            -> the gathered inner entries (rebased onto the grandchild slab by the stager) are
 //                                        the entries of the next level: the same kernel again, over pseudo chunks
 //   MAP             LIST<STRUCT<key, value>> exported as Arrow map<key, value>
-// These columns are converted synchronously inside launch_arrow_col (no copy-in / copy-out overlap): they are not the
-// hot path.
+// A top-level LIST of one fixed-width leaf runs in materialise_arrow's pipeline (run_list: its copy-in, kernels and
+// copy-out overlap the neighbouring columns').  Every other nested column is converted synchronously inside
+// launch_arrow_col (nested_to_arrow: no copy-in / copy-out overlap).
 void copy_bits(uint64_t *dst, uint64_t dst_bit, const uint64_t *src, uint64_t nbits) {  // src bits [0, nbits) -> dst bits [dst_bit, ...); dst pre-zeroed
   for (uint64_t i = 0; i < nbits;) {
     const uint64_t d = dst_bit + i;
@@ -1054,7 +886,6 @@ bool leaf_from_column(const dmb_host_column &hc, int64_t nch, Leaf *leaf) {
   leaf->dec_scale = hc.dec_scale;
   leaf->width = dmb_phys_width(hc.phys);
   if (leaf->width <= 0) { set_error("nested column '%s': bad physical type %d", leaf->name.c_str(), hc.phys); return false; }
-  if (hc.type_id == DMB_TYPE_ENUM) { set_error("nested column '%s': ENUM inside LIST / MAP is not supported", leaf->name.c_str()); return false; }
   if (nch > 0 && !hc.data) { set_error("nested column '%s': no data pointers", leaf->name.c_str()); return false; }
   leaf->data.assign(hc.data, hc.data + nch);
   if (hc.validity) {
@@ -1066,23 +897,47 @@ bool leaf_from_column(const dmb_host_column &hc, int64_t nch, Leaf *leaf) {
   return true;
 }
 
+// the flat form of a list's child (child_type_id ... child_validity) as a column of its own
+dmb_host_column flat_child(const dmb_host_list &l) {
+  dmb_host_column f;
+  memset(&f, 0, sizeof(f));
+  f.name = "item";
+  f.type_id = l.child_type_id;
+  f.phys = l.child_phys;
+  f.dec_width = l.child_dec_width;
+  f.dec_scale = l.child_dec_scale;
+  f.data = l.child_data;
+  f.validity = l.child_validity;
+  return f;
+}
+
+// a node's per-chunk child sizes and their running sum
+std::shared_ptr<ListNode> sized_node(const uint64_t *sizes, int64_t nch) {
+  auto node = std::make_shared<ListNode>();
+  node->sizes.assign(sizes, sizes + nch);
+  node->base.assign((size_t)nch + 1, 0);
+  for (int64_t k = 0; k < nch; ++k) node->base[(size_t)k + 1] = node->base[(size_t)k] + node->sizes[(size_t)k];
+  return node;
+}
+
 // the child level of a LIST / MAP from its host description (dmb_host_list with child_col)
 std::shared_ptr<ListNode> build_node(const dmb_host_list *l, int64_t nch, int depth) {
   if (depth > 4) { set_error("LIST nesting deeper than 4 levels"); return nullptr; }
   const dmb_host_column *cc = l->child_col;
   if (!cc || (nch > 0 && !l->child_sizes)) { set_error("LIST column: child_col / child_sizes missing"); return nullptr; }
-  auto node = std::make_shared<ListNode>();
-  node->sizes.assign(l->child_sizes, l->child_sizes + nch);
-  node->base.assign((size_t)nch + 1, 0);
-  for (int64_t k = 0; k < nch; ++k) node->base[(size_t)k + 1] = node->base[(size_t)k] + node->sizes[(size_t)k];
+  auto node = sized_node(l->child_sizes, nch);
+  auto add_leaf = [&](const dmb_host_column &hc) {
+    if (hc.type_id == DMB_TYPE_ENUM) { set_error("nested column '%s': ENUM inside LIST / MAP is not supported", hc.name ? hc.name : ""); return false; }
+    node->leaves.emplace_back();
+    return leaf_from_column(hc, nch, &node->leaves.back());
+  };
   if (cc->type_id == DMB_TYPE_STRUCT) {
     if (!cc->struct_ || cc->struct_->nfields <= 0 || !cc->struct_->fields) { set_error("LIST<STRUCT>: no fields"); return nullptr; }
     node->kind = ListNode::kStruct;
     for (int32_t f = 0; f < cc->struct_->nfields; ++f) {
       const dmb_host_column &fc = cc->struct_->fields[f];
       if (fc.type_id == DMB_TYPE_STRUCT || fc.type_id == DMB_TYPE_LIST || fc.type_id == DMB_TYPE_MAP) { set_error("LIST<STRUCT>: field '%s' is itself nested (not supported)", fc.name ? fc.name : ""); return nullptr; }
-      node->leaves.emplace_back();
-      if (!leaf_from_column(fc, nch, &node->leaves.back())) return nullptr;
+      if (!add_leaf(fc)) return nullptr;
     }
     if (cc->validity) {
       node->struct_validity.validity.assign((const void *const *)cc->validity, (const void *const *)cc->validity + nch);
@@ -1094,43 +949,28 @@ std::shared_ptr<ListNode> build_node(const dmb_host_list *l, int64_t nch, int de
   } else if (cc->type_id == DMB_TYPE_LIST) {
     if (!cc->list) { set_error("LIST<LIST>: the inner list's child vectors are missing"); return nullptr; }
     node->kind = ListNode::kList;
-    node->leaves.emplace_back();
     dmb_host_column entries = *cc;
     entries.phys = DMB_PHYS_U128;
-    if (!leaf_from_column(entries, nch, &node->leaves.back())) return nullptr;
+    if (!add_leaf(entries)) return nullptr;
     dmb_host_list inner = *cc->list;
-    dmb_host_column flat;  // an inner list in the flat fixed-width form: wrap it as a column
-    if (!inner.child_col) {
-      memset(&flat, 0, sizeof(flat));
-      flat.name = "item";
-      flat.type_id = inner.child_type_id;
-      flat.phys = inner.child_phys;
-      flat.dec_width = inner.child_dec_width;
-      flat.dec_scale = inner.child_dec_scale;
-      flat.data = inner.child_data;
-      flat.validity = inner.child_validity;
-      inner.child_col = &flat;
-    }
+    const dmb_host_column flat = flat_child(inner);
+    if (!inner.child_col) inner.child_col = &flat;
     node->inner = build_node(&inner, nch, depth + 1);
     if (!node->inner) return nullptr;
   } else {
     node->kind = ListNode::kLeaf;
-    node->leaves.emplace_back();
-    if (!leaf_from_column(*cc, nch, &node->leaves.back())) return nullptr;
+    if (!add_leaf(*cc)) return nullptr;
   }
   return node;
 }
 
 // chunks [c0, c1) of a node (slice_result)
 std::shared_ptr<ListNode> slice_node(const ListNode &p, int64_t c0, int64_t c1) {
-  auto n = std::make_shared<ListNode>();
+  auto n = sized_node(p.sizes.data() + c0, c1 - c0);
   n->kind = p.kind;
-  n->sizes.assign(p.sizes.begin() + c0, p.sizes.begin() + c1);
-  n->base.assign((size_t)(c1 - c0) + 1, 0);
-  for (int64_t k = 0; k < c1 - c0; ++k) n->base[(size_t)k + 1] = n->base[(size_t)k] + n->sizes[(size_t)k];
   auto slice_leaf = [&](const Leaf &pl) {
     Leaf l;
-    l.name = pl.name; l.type_id = pl.type_id; l.phys = pl.phys; l.dec_width = pl.dec_width; l.dec_scale = pl.dec_scale; l.width = pl.width;
+    static_cast<ColType &>(l) = pl;
     if (!pl.data.empty()) l.data.assign(pl.data.begin() + c0, pl.data.begin() + c1);
     if (!pl.validity.empty()) l.validity.assign(pl.validity.begin() + c0, pl.validity.begin() + c1);
     return l;
@@ -1260,9 +1100,25 @@ struct GatherOut {
   void *d_offsets = nullptr;
   uint8_t *d_child = nullptr;
   uint64_t *d_bitmap = nullptr;  // whole 32-word masks: the next pass reads it as chunk masks
-  unsigned long long *h_ctr = nullptr;  // pinned: [0] elements [1] nulls [2] flags
+  unsigned long long *h_ctr = nullptr;  // pinned: [0] elements [1] nulls [2] flags [3] the parent's null count (run_list)
   cudaEvent_t done = nullptr;
 };
+
+// the entries of a LIST / MAP column itself, over its node's child slab
+EntrySrc column_entries(const Result *r, const Col &col, uint64_t cap) {
+  EntrySrc es;
+  es.d_entries = col.d_data;
+  es.d_validity = col.d_validity;
+  es.d_vecs = col.d_vecs;
+  es.d_counts = r->d_counts;
+  es.d_row_off = r->d_row_off;
+  es.nchunks = r->nchunks;
+  es.nrows = r->nrows;
+  es.d_child_base = col.node->d_base;
+  es.d_child_sizes = col.node->d_sizes;
+  es.cap = cap;
+  return es;
+}
 
 // metadata of a dense array of n elements cut into 2048-element pseudo chunks (masks: words [32 k, 32 k + 32) of a bitmap)
 struct Pseudo {
@@ -1340,15 +1196,44 @@ int32_t gather_leaf(Result *r, Scope &sc, const EntrySrc &es, const Leaf &leaf, 
   return 0;
 }
 
+// waits for a gather and decodes list_emit_kernel's error flags (every LIST path)
 int32_t check_gather(const GatherOut &g, uint64_t cap) {
-  if (check_cuda(cudaEventSynchronize(g.done), "nested gather wait")) return -1;
+  if (check_cuda(cudaEventSynchronize(g.done), "list gather wait")) return -1;
   const unsigned long long f = g.h_ctr[2];
   if (f & 8ull) { set_error("a LIST entry reaches outside its chunk's child vector (offset + length > duckdb_list_vector_get_size)"); return -1; }
-  if (f & 4ull) { set_error("a LIST chunk's look-back gave up waiting for its predecessors; run the call again"); return -1; }
+  if (f & 4ull) { set_error("a LIST chunk's look-back gave up waiting for its predecessors (GPU preempted or oversubscribed?); run the call again"); return -1; }
   if (f & 2ull) { set_error("a LIST chunk holds more than 4 G child elements"); return -1; }
   if (f & 1ull) { set_error("LIST child elements exceed int32 offsets; use smaller batches"); return -1; }
-  if (g.h_ctr[0] != cap) { set_error("nested column: the device gathered %llu child elements, the host counted %llu", g.h_ctr[0], (unsigned long long)cap); return -1; }
+  if (g.h_ctr[0] != cap) { set_error("LIST column: the device gathered %llu child elements, the host counted %llu", g.h_ctr[0], (unsigned long long)cap); return -1; }
   return 0;
+}
+
+// a gathered fixed-width leaf that Arrow stores differently (BOOLEAN -> bits, DECIMAL -> decimal128, INTERVAL ->
+// month_day_nano; `cap` > 0 elements): fixed_batch_kernel over the dense child as 2048-element pseudo chunks, the gathered
+// bitmap as their masks.  Returns the converted values (*bytes of them) on the compute stream.
+uint8_t *convert_gathered(Scope &sc, const Leaf &leaf, const GatherOut &g, uint64_t cap, int32_t op, size_t *bytes) {
+  const int32_t ow = dmb_op_out_width(op);
+  if (ow < 0) { set_error("LIST child '%s': unsupported conversion 0x%x", leaf.name.c_str(), op); return nullptr; }
+  Pseudo ps;
+  if (make_pseudo(sc, cap, (size_t)leaf.width, &ps)) return nullptr;
+  *bytes = ow == 0 ? (size_t)((cap + 7) / 8) : (size_t)cap * (size_t)ow;
+  uint8_t *d_out = (uint8_t *)sc.dalloc(*bytes + 64);
+  if (!d_out) return nullptr;
+  dmb_fixed_job fj;
+  memset(&fj, 0, sizeof(fj));
+  fj.in_data = g.d_child;
+  fj.in_validity = g.d_bitmap;
+  fj.vecs = ps.d_vecs;
+  fj.out_values = d_out;
+  fj.op = op;
+  void *fjd = upload_job(sc, &fj, sizeof(fj));
+  cudaEvent_t k0 = sc.event(true), k1 = sc.event(true);
+  if (!fjd || !k0 || !k1) return nullptr;
+  cudaEventRecord(k0, sc.c.s_compute);
+  if (dmb_dev_fixed_batch((const dmb_fixed_job *)fjd, &fj, 1, ps.d_counts, ps.d_row_off, ps.nchunks, (int64_t)cap, sc.c.s_compute)) return nullptr;
+  cudaEventRecord(k1, sc.c.s_compute);
+  sc.kernel_spans.emplace_back(k0, k1);
+  return d_out;
 }
 
 // a gathered leaf (dense, `cap` elements) -> its Arrow array in pinned memory.  Synchronous.
@@ -1385,13 +1270,8 @@ std::shared_ptr<ArrowColOut> leaf_to_arrow(Result *r, Scope &sc, const Leaf &lea
   o->length = (int64_t)cap;
   o->null_count = (int64_t)g.h_ctr[1];
   const size_t bm_bytes = (size_t)((cap + 7) / 8);
-  Col tmp;
-  tmp.type_id = leaf.type_id;
-  tmp.phys = leaf.phys;
-  tmp.dec_width = leaf.dec_width;
-  tmp.dec_scale = leaf.dec_scale;
   ArrowMap m;
-  if (!arrow_map(tmp, &m) || m.is_nested || m.is_list) { set_error("nested column '%s': child type %d has no Arrow mapping here", leaf.name.c_str(), leaf.type_id); return nullptr; }
+  if (!type_arrow_map(leaf, &m)) { set_error("nested column '%s': child type %d has no Arrow mapping here", leaf.name.c_str(), leaf.type_id); return nullptr; }
   o->format = m.format;
   if (m.is_string) {
     // the gathered string_t are a dense column: 2048-element pseudo chunks, the gathered bitmap as their masks, the
@@ -1429,29 +1309,13 @@ std::shared_ptr<ArrowColOut> leaf_to_arrow(Result *r, Scope &sc, const Leaf &lea
     }
     return pinned_copy(r, o, d_off, (size_t)(cap + 1) * 4, g.d_bitmap, bm_bytes, d_data, (size_t)h[0]);
   }
-  const bool as_stored = m.op == DMB_OP(leaf.phys, DMB_DST_SAME) || leaf.type_id == DMB_TYPE_HUGEINT;
-  if (as_stored || cap == 0) {
+  if (stored_as_arrow(leaf, m.op) || cap == 0) {
     const int ow = dmb_op_out_width(m.op);
     return pinned_copy(r, o, g.d_child, cap == 0 ? 0 : (size_t)cap * (size_t)(ow > 0 ? ow : leaf.width), g.d_bitmap, bm_bytes, nullptr, 0);
   }
-  // BOOLEAN -> bits, DECIMAL -> decimal128, INTERVAL -> month_day_nano: fixed_batch_kernel over the dense child
-  const int32_t ow = dmb_op_out_width(m.op);
-  if (ow < 0) { set_error("nested column '%s': unsupported child conversion 0x%x", leaf.name.c_str(), m.op); return nullptr; }
-  Pseudo ps;
-  if (make_pseudo(sc, cap, (size_t)leaf.width, &ps)) return nullptr;
-  const size_t out_bytes = ow == 0 ? (size_t)((cap + 7) / 8) : (size_t)cap * (size_t)ow;
-  uint8_t *d_out = (uint8_t *)sc.dalloc(out_bytes + 64);
+  size_t out_bytes = 0;
+  uint8_t *d_out = convert_gathered(sc, leaf, g, cap, m.op, &out_bytes);
   if (!d_out) return nullptr;
-  dmb_fixed_job fj;
-  memset(&fj, 0, sizeof(fj));
-  fj.in_data = g.d_child;
-  fj.in_validity = g.d_bitmap;
-  fj.vecs = ps.d_vecs;
-  fj.out_values = d_out;
-  fj.op = m.op;
-  void *fjd = upload_job(sc, &fj, sizeof(fj));
-  if (!fjd) return nullptr;
-  if (dmb_dev_fixed_batch((const dmb_fixed_job *)fjd, &fj, 1, ps.d_counts, ps.d_row_off, ps.nchunks, (int64_t)cap, c.s_compute)) return nullptr;
   return pinned_copy(r, o, d_out, out_bytes, g.d_bitmap, bm_bytes, nullptr, 0);
 }
 
@@ -1564,6 +1428,41 @@ int32_t nested_caps(Result *r, const Col &col, uint64_t *cap1, uint64_t *cap2) {
   return 0;
 }
 
+// A top-level LIST of one fixed-width leaf, launched in materialise_arrow's pipeline and copied out by drain_arrow_col
+struct ListRun {
+  FixedRun validity;  // the LIST column's own bitmap / null count
+  GatherOut g;        // done: after the conversion pass and the parent's null count as well
+  uint64_t cap = 0;
+  uint8_t *d_child_out = nullptr;  // the child in its Arrow form (== g.d_child when it is exported as stored)
+  size_t child_out_bytes = 0;
+};
+
+int32_t run_list(Result *r, Scope &sc, int j, int32_t child_op, ListRun *out) {
+  Col &col = r->cols[(size_t)j];
+  CtxCore &c = *r->core;
+  const Leaf &leaf = col.node->leaves[0];
+  // the child slab first: the entries' staging and the host pass below overlap its copy-in
+  if (stage_node(r, *col.node, false)) return -1;
+  // the column's own validity bitmap + null count (also stages the entries)
+  if (run_fixed(r, sc, j, DMB_OP_VALIDITY_ONLY, 0, true, false, &out->validity)) return -1;
+  cudaEvent_t e = sc.event(false);  // the child slab was copied on the copy-in stream
+  if (!e) return -1;
+  cudaEventRecord(e, c.s_in);
+  if (check_cuda(cudaStreamWaitEvent(c.s_compute, e, 0), "wait list child")) return -1;
+  uint64_t cap2 = 0;
+  if (nested_caps(r, col, &out->cap, &cap2)) return -1;
+  if (gather_leaf(r, sc, column_entries(r, col, out->cap), leaf, &out->g)) return -1;
+  out->d_child_out = out->g.d_child;
+  out->child_out_bytes = (size_t)out->cap * (size_t)leaf.width;
+  if (!stored_as_arrow(leaf, child_op) && out->cap > 0) {
+    out->d_child_out = convert_gathered(sc, leaf, out->g, out->cap, child_op, &out->child_out_bytes);
+    if (!out->d_child_out) return -1;
+  }
+  if (check_cuda(cudaMemcpyAsync(out->g.h_ctr + 3, out->validity.d_null_count, 8, cudaMemcpyDeviceToHost, c.s_compute), "null count D2H")) return -1;
+  cudaEventRecord(out->g.done, c.s_compute);
+  return 0;
+}
+
 struct Pending;
 int32_t launch_arrow_col(Result *r, Scope &sc, int j, int string_mode, Pending *p, size_t exact_cap);
 std::shared_ptr<ArrowColOut> convert_column_sync(Result *r, Scope &sc, int j);
@@ -1604,19 +1503,8 @@ std::shared_ptr<ArrowColOut> nested_to_arrow(Result *r, Scope &sc, int j) {
     if (!e) return nullptr;
     cudaEventRecord(e, c.s_in);
     if (check_cuda(cudaStreamWaitEvent(c.s_compute, e, 0), "wait nested children")) return nullptr;
-    EntrySrc es;
-    es.d_entries = col.d_data;
-    es.d_validity = col.d_validity;
-    es.d_vecs = col.d_vecs;
-    es.d_counts = r->d_counts;
-    es.d_row_off = r->d_row_off;
-    es.nchunks = r->nchunks;
-    es.nrows = n;
-    es.d_child_base = node.d_base;
-    es.d_child_sizes = node.d_sizes;
-    es.cap = cap1;
     GatherOut g1;
-    auto child = node_to_arrow(r, sc, es, node, cap2, &g1);
+    auto child = node_to_arrow(r, sc, column_entries(r, col, cap1), node, cap2, &g1);
     if (!child) return nullptr;
     const bool is_map = col.type_id == DMB_TYPE_MAP;
     o->format = is_map ? "+m" : "+l";
@@ -1663,8 +1551,13 @@ int32_t launch_arrow_col(Result *r, Scope &sc, int j, int string_mode, Pending *
   if (col.type_id == DMB_TYPE_ENUM) p->out->dict = col.dict;
   if (p->map.is_list) {
     p->lr = ListRun();
-    if (run_list(r, sc, j, p->map.child_op, p->map.child_as_stored, &p->lr)) return -1;
+    if (run_list(r, sc, j, p->map.child_op, &p->lr)) return -1;
     p->out->format = p->map.format;
+    auto ch = std::make_shared<ArrowColOut>();
+    ch->core = r->core;
+    ch->name = col.node->leaves[0].name.empty() ? "item" : col.node->leaves[0].name;
+    ch->format = p->map.child_format;
+    p->out->children.push_back(ch);
     return 0;
   }
   if (p->map.is_string) {
@@ -1688,43 +1581,26 @@ int32_t drain_arrow_col(Result *r, Scope &sc, Pending *p) {
   const int64_t n = r->nrows;
   if (p->map.is_list) {
     ListRun &l = p->lr;
-    o.values_bytes = l.offsets_bytes;
+    ArrowColOut &ch = *o.children[0];
+    if (check_gather(l.g, l.cap)) return -1;
+    o.values_bytes = (size_t)(n + 1) * 4;
     o.validity_bytes = l.validity.bitmap_bytes;
+    o.null_count = (int64_t)l.g.h_ctr[3];
+    ch.length = (int64_t)l.cap;
+    ch.null_count = (int64_t)l.g.h_ctr[1];
+    ch.values_bytes = l.child_out_bytes;
+    ch.validity_bytes = (size_t)((l.cap + 7) / 8);
     o.values = c.pin.alloc(o.values_bytes + 64);
     o.validity = c.pin.alloc(o.validity_bytes + 64);
-    auto ch = std::make_shared<ArrowColOut>();
-    ch->core = r->core;
-    ch->name = "item";
-    ch->format = p->map.child_format;
-    o.children.push_back(ch);
-    if (!o.values || !o.validity) return -1;
-    if (n == 0) {
-      memset(o.values, 0, o.values_bytes);
-      ch->values = c.pin.alloc(64);
-      ch->validity = c.pin.alloc(64);
-      return (ch->values && ch->validity) ? 0 : -1;
-    }
-    if (check_cuda(cudaEventSynchronize(l.done), "list kernel wait")) return -1;
-    if (l.h_ctr[2] & 8ull) { set_error("a LIST entry reaches outside its chunk's child vector (offset + length > duckdb_list_vector_get_size)"); return -1; }
-    if (l.h_ctr[2] & 4ull) { set_error("a LIST chunk's look-back gave up waiting for its predecessors (GPU preempted or oversubscribed?); run the call again"); return -1; }
-    if (l.h_ctr[2] & 2ull) { set_error("a LIST chunk holds more than 4 G child elements"); return -1; }
-    if (l.h_ctr[2] & 1ull) { set_error("LIST child elements exceed int32 offsets; use smaller batches"); return -1; }
-    const size_t total = (size_t)l.h_ctr[0];
-    ch->length = (int64_t)total;
-    ch->null_count = (int64_t)l.h_ctr[1];
-    ch->values_bytes = l.child_out_bytes;
-    if (total != l.capacity) { set_error("LIST column: the device gathered %zu child elements, the host counted %llu", total, (unsigned long long)l.capacity); return -1; }
-    ch->validity_bytes = (total + 7) / 8;
-    ch->values = c.pin.alloc(ch->values_bytes + 64);
-    ch->validity = c.pin.alloc(ch->validity_bytes + 64);
-    if (!ch->values || !ch->validity) return -1;
-    o.null_count = (int64_t)l.h_ctr[3];
-    if (check_cuda(cudaStreamWaitEvent(c.s_out, l.done, 0), "wait kernel")) return -1;
-    if (check_cuda(cudaMemcpyAsync(o.values, l.d_offsets, o.values_bytes, cudaMemcpyDeviceToHost, c.s_out), "list offsets D2H")) return -1;
+    ch.values = c.pin.alloc(ch.values_bytes + 64);
+    ch.validity = c.pin.alloc(ch.validity_bytes + 64);
+    if (!o.values || !o.validity || !ch.values || !ch.validity) return -1;
+    if (check_cuda(cudaStreamWaitEvent(c.s_out, l.g.done, 0), "wait kernel")) return -1;
+    if (check_cuda(cudaMemcpyAsync(o.values, l.g.d_offsets, o.values_bytes, cudaMemcpyDeviceToHost, c.s_out), "list offsets D2H")) return -1;
     if (o.validity_bytes && check_cuda(cudaMemcpyAsync(o.validity, l.validity.d_bitmap, o.validity_bytes, cudaMemcpyDeviceToHost, c.s_out), "bitmap D2H")) return -1;
-    if (ch->values_bytes && check_cuda(cudaMemcpyAsync(ch->values, l.d_child_out, ch->values_bytes, cudaMemcpyDeviceToHost, c.s_out), "list child D2H")) return -1;
-    if (ch->validity_bytes && check_cuda(cudaMemcpyAsync(ch->validity, l.d_child_bitmap, ch->validity_bytes, cudaMemcpyDeviceToHost, c.s_out), "list child bitmap D2H")) return -1;
-    r->bytes_d2h += o.values_bytes + o.validity_bytes + ch->values_bytes + ch->validity_bytes;
+    if (ch.values_bytes && check_cuda(cudaMemcpyAsync(ch.values, l.d_child_out, ch.values_bytes, cudaMemcpyDeviceToHost, c.s_out), "list child D2H")) return -1;
+    if (ch.validity_bytes && check_cuda(cudaMemcpyAsync(ch.validity, l.g.d_bitmap, ch.validity_bytes, cudaMemcpyDeviceToHost, c.s_out), "list child bitmap D2H")) return -1;
+    r->bytes_d2h += o.values_bytes + o.validity_bytes + ch.values_bytes + ch.validity_bytes;
     return 0;
   }
   if (p->map.is_string) {
@@ -1838,10 +1714,11 @@ int32_t materialise_arrow(Result *r) {
       for (int j = 0; j < ncols; ++j) {
         const Col &col = r->cols[(size_t)j];
         ArrowMap m;
-        const uint64_t list_bytes = col.is_list ? col.child_base.back() * (uint64_t)col.child_width : 0;
+        const bool mapped = arrow_map(col, &m);
+        const uint64_t list_bytes = mapped && m.is_list ? col.node->base.back() * (uint64_t)col.node->leaves[0].width : 0;
         w_in[(size_t)j] = (uint64_t)col.width * n + col.heap_len + list_bytes;
         uint64_t out = w_in[(size_t)j];
-        if (arrow_map(col, &m) && !m.is_nested && !m.is_list) {
+        if (mapped && !m.is_nested && !m.is_list) {
           if (m.is_string) out = 4 * n + (col.heap_len ? col.heap_len : 4 * n);  // (inlined bytes are not known before the kernel: a guess)
           else { const int32_t ow = dmb_op_out_width(m.op); out = ow > 0 ? (uint64_t)ow * n : n / 8; }
         }
@@ -2398,7 +2275,7 @@ namespace dmb {
 namespace {
 
 // One column of the batch -> r->cols[j] (already allocated).  STRUCT fields become columns of their own appended behind
-// the visible ones (Col::kids); a LIST / MAP whose child is described as a column gets a ListNode.
+// the visible ones (Col::kids); a LIST / MAP gets a ListNode, whichever form its child came in.
 bool fill_column(Result *r, int j, const dmb_host_column &hc, int64_t nch, const uint32_t *counts, int depth) {
   if (depth > 4) { set_error("column '%s': STRUCT nesting deeper than 4 levels", hc.name ? hc.name : ""); return false; }
   if (hc.type_id == DMB_TYPE_STRUCT) {
@@ -2459,46 +2336,28 @@ bool fill_column(Result *r, int j, const dmb_host_column &hc, int64_t nch, const
       if (d->offsets[d->size]) dict->data.assign(d->data, d->data + d->offsets[d->size]);
       col.dict = dict;
     }
-    if (hc.type_id == DMB_TYPE_LIST && !(hc.list && hc.list->child_col)) {
+    if (hc.type_id == DMB_TYPE_LIST || hc.type_id == DMB_TYPE_MAP) {
       const dmb_host_list *l = hc.list;
-      if (col.width != 16) { set_error("column %d: LIST vectors hold 16-byte list entries (phys DMB_PHYS_U128)", j); return false; }
-      if (!l || (nch > 0 && (!l->child_data || !l->child_sizes))) { set_error("column %d: LIST column without child vectors", j); return false; }
-      col.is_list = true;
-      col.child_type_id = l->child_type_id;
-      col.child_phys = l->child_phys;
-      col.child_dec_width = l->child_dec_width;
-      col.child_dec_scale = l->child_dec_scale;
-      col.child_width = dmb_phys_width(l->child_phys);
-      if (col.child_width <= 0 || l->child_phys == DMB_PHYS_STRING) { set_error("column %d: LIST child must be a fixed-width type (physical type %d)", j, l->child_phys); return false; }
-      col.child_data.assign(l->child_data, l->child_data + nch);
-      col.child_sizes.assign(l->child_sizes, l->child_sizes + nch);
-      if (l->child_validity) {
-        col.child_validity.assign((const void *const *)l->child_validity, (const void *const *)l->child_validity + nch);
-        bool any = false;
-        for (const void *p : col.child_validity) any |= p != nullptr;
-        if (!any) col.child_validity.clear();
-      }
-      col.child_base.assign((size_t)nch + 1, 0);
-      col.child_val_off.assign((size_t)(nch > 0 ? nch : 1), -1);
-      uint64_t words = 0;
-      for (int64_t k = 0; k < nch; ++k) {
-        if (col.child_sizes[(size_t)k] && !col.child_data[(size_t)k]) { set_error("column %d: chunk %lld has child elements but a null child pointer", j, (long long)k); return false; }
-        col.child_base[(size_t)k + 1] = col.child_base[(size_t)k] + col.child_sizes[(size_t)k];
-        if (!col.child_validity.empty() && col.child_validity[(size_t)k]) {
-          col.child_val_off[(size_t)k] = (int64_t)words;
-          words += (col.child_sizes[(size_t)k] + 63) / 64 + 1;
-        }
+      if (col.width != 16) { set_error("column %d: LIST / MAP vectors hold 16-byte list entries (phys DMB_PHYS_U128)", j); return false; }
+      if (l && l->child_col) {
+        col.node = build_node(l, nch, 0);
+        if (!col.node) return false;
+        col.is_map = hc.type_id == DMB_TYPE_MAP;
+      } else if (hc.type_id == DMB_TYPE_MAP) {
+        set_error("column %d: MAP column without its STRUCT<key, value> child (dmb_host_list.child_col)", j);
+        return false;
+      } else {
+        // the flat form: one leaf of any fixed-width type (build_node's refusals are for described children; a type without
+        // an Arrow mapping fails at export, and the result's other columns still serve)
+        if (!l || (nch > 0 && (!l->child_data || !l->child_sizes))) { set_error("column %d: LIST column without child vectors", j); return false; }
+        if (dmb_phys_width(l->child_phys) <= 0 || l->child_phys == DMB_PHYS_STRING) { set_error("column %d: LIST child must be a fixed-width type (physical type %d)", j, l->child_phys); return false; }
+        for (int64_t k = 0; k < nch; ++k)
+          if (l->child_sizes[k] && !l->child_data[k]) { set_error("column %d: chunk %lld has child elements but a null child pointer", j, (long long)k); return false; }
+        col.node = sized_node(l->child_sizes, nch);
+        col.node->leaves.emplace_back();
+        if (!leaf_from_column(flat_child(*l), nch, &col.node->leaves.back())) return false;
       }
     }
-    if ((hc.type_id == DMB_TYPE_LIST || hc.type_id == DMB_TYPE_MAP) && hc.list && hc.list->child_col) {
-    if (col.width != 16) { set_error("column %d: LIST / MAP vectors hold 16-byte list entries (phys DMB_PHYS_U128)", j); return false; }
-    col.node = build_node(hc.list, nch, 0);
-    if (!col.node) return false;
-    col.is_map = hc.type_id == DMB_TYPE_MAP;
-  } else if (hc.type_id == DMB_TYPE_MAP) {
-    set_error("column %d: MAP column without its STRUCT<key, value> child (dmb_host_list.child_col)", j);
-    return false;
-  }
   return true;
 }
 
@@ -2845,12 +2704,7 @@ Result *slice_result(const Result *p, const std::shared_ptr<CtxCore> &core, int6
   for (size_t j = 0; j < p->cols.size(); ++j) {
     const Col &pc = p->cols[j];
     Col &col = r->cols[j];
-    col.name = pc.name;
-    col.type_id = pc.type_id;
-    col.phys = pc.phys;
-    col.dec_width = pc.dec_width;
-    col.dec_scale = pc.dec_scale;
-    col.width = pc.width;
+    static_cast<ColType &>(col) = pc;
     col.force_large = pc.force_large;
     col.dict = pc.dict ? std::make_shared<EnumDict>() : nullptr;  // device copies are per result: own dictionary object
     if (pc.dict) {
@@ -2897,27 +2751,6 @@ Result *slice_result(const Result *p, const std::shared_ptr<CtxCore> &core, int6
     col.kids = pc.kids;  // (the hidden field columns are sliced like every other column, at the same indices)
     col.is_map = pc.is_map;
     if (pc.node) col.node = slice_node(*pc.node, c0, c1);
-    if (pc.is_list) {
-      col.is_list = true;
-      col.child_type_id = pc.child_type_id;
-      col.child_phys = pc.child_phys;
-      col.child_dec_width = pc.child_dec_width;
-      col.child_dec_scale = pc.child_dec_scale;
-      col.child_width = pc.child_width;
-      col.child_data.assign(pc.child_data.begin() + c0, pc.child_data.begin() + c1);
-      col.child_sizes.assign(pc.child_sizes.begin() + c0, pc.child_sizes.begin() + c1);
-      if (!pc.child_validity.empty()) col.child_validity.assign(pc.child_validity.begin() + c0, pc.child_validity.begin() + c1);
-      col.child_base.assign((size_t)r->nchunks + 1, 0);
-      col.child_val_off.assign((size_t)(r->nchunks > 0 ? r->nchunks : 1), -1);
-      uint64_t words = 0;
-      for (int64_t k = 0; k < r->nchunks; ++k) {
-        col.child_base[(size_t)k + 1] = col.child_base[(size_t)k] + col.child_sizes[(size_t)k];
-        if (!col.child_validity.empty() && col.child_validity[(size_t)k]) {
-          col.child_val_off[(size_t)k] = (int64_t)words;
-          words += (col.child_sizes[(size_t)k] + 63) / 64 + 1;
-        }
-      }
-    }
   }
   return r.release();
 }

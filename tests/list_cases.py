@@ -89,3 +89,12 @@ def as_column(lc, name, child_type, dec_width=0, dec_scale=0):
     col.list_child_validity = lc.child_validity
     col.list_child_val_off = lc.child_val_off
     return col
+
+
+def as_described_column(lc, name, child_type):
+    """the same LIST column with its child described as a column (dmb_host_list.child_col) instead of the flat fields"""
+    col = ch.Column(name, ch.T_LIST, ch.P_U128, lc.entries, lc.data_off, lc.validity, lc.val_off)
+    col.list_child_sizes = lc.child_sizes
+    col.list_child_col = ch.Column("item", child_type, ch.phys_of_type(child_type), lc.child_data, lc.child_base * np.uint64(lc.width),
+                                   lc.child_validity, lc.child_val_off)
+    return col

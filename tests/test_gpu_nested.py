@@ -12,6 +12,7 @@ pa = pytest.importorskip("pyarrow")
 
 from duckdb_mbt_b200 import chunks as ch  # noqa: E402
 
+import list_cases  # noqa: E402
 import nested_cases  # noqa: E402
 
 
@@ -89,3 +90,64 @@ def test_malformed_nested_entries_are_refused(ctx):
     with ar.ArrowResult.from_chunks(ctx, ch.ChunkBatch(counts, [col])) as res:
         with pytest.raises(ar.DuckDBError, match="outside its chunk's child vector"):
             res.to_arrow(0)
+
+
+def _int_rows(lc):
+    return [None if row is None else [None if v is None else int.from_bytes(v, "little", signed=True) for v in row] for row in lc.expected]
+
+
+@pytest.mark.parametrize("n,pattern,layout", [(9000, "ragged", "contiguous"), (6001, "full", "shuffled")])
+def test_flat_and_described_list_of_integer_export_the_same_array(ctx, n, pattern, layout):
+    """dmb_host_list's two forms of a fixed-width child (the flat child_* fields, child_col) are one column to the exporter"""
+    lc = list_cases.make_list_column(n, 4, pattern, 600 + n, layout)
+    other = ch.fixed_column("i", ch.T_INTEGER, np.arange(n, dtype=np.int32), lc.counts)
+    flat, described, i = _export(ctx, lc.counts, [list_cases.as_column(lc, "l", ch.T_INTEGER),
+                                                  list_cases.as_described_column(lc, "l", ch.T_INTEGER), other])
+    assert flat.type == described.type == pa.list_(pa.field("item", pa.int32()))
+    assert flat.equals(described)
+    assert flat.to_pylist() == described.to_pylist() == _int_rows(lc)
+    assert i.to_pylist() == list(range(n))
+
+
+@pytest.mark.parametrize("child_type,dec_width,dec_scale", [(ch.T_INTEGER, 0, 0), (ch.T_DECIMAL, 9, 2)], ids=["integer", "decimal"])
+def test_flat_list_in_stream_batches_across_chunks(ctx, child_type, dec_width, dec_scale):
+    """record batches of a flat LIST column (every batch a slice of several ragged chunks) concatenate to the single export"""
+    from duckdb_mbt_b200 import arrow_result as ar
+    n = 20_000
+    lc = list_cases.make_list_column(n, 4, "ragged", 71, "shuffled")
+    batch = ch.ChunkBatch(lc.counts, [list_cases.as_column(lc, "l", child_type, dec_width, dec_scale)])
+    with ar.ArrowResult.from_chunks(ctx, batch) as res:
+        whole = res.to_arrow(0)
+    with ar.ArrowResult.from_chunks(ctx, batch) as res:
+        parts = []
+        for b in res.to_stream(max_batch_rows=5000):
+            b.validate()
+            assert b.num_rows <= 5000
+            parts.append(b.column(0))
+    assert len(parts) > 2
+    got = pa.concat_arrays(parts)
+    assert got.type == whole.type
+    assert got.to_pylist() == whole.to_pylist()
+    if child_type == ch.T_INTEGER:
+        assert got.to_pylist() == _int_rows(lc)
+
+
+@pytest.mark.parametrize("stored_type,child_type", [(ch.T_UINTEGER, ch.T_ENUM), (ch.T_UUID, ch.T_LIST)], ids=["enum", "list"])
+def test_flat_list_child_without_arrow_mapping_fails_at_export(ctx, stored_type, child_type):
+    """a flat child whose type has no Arrow mapping here (ENUM, LIST given by type id) is accepted by from_chunks: the
+    result still serves its other columns, and only the Arrow export of that column fails"""
+    import ctypes as C
+    from duckdb_mbt_b200 import arrow_result as ar
+    from duckdb_mbt_b200 import native as nat
+    n = 3000
+    lc = list_cases.make_list_column(n, ch.PHYS_WIDTH[ch.phys_of_type(stored_type)], "ragged", 81, "contiguous")
+    other = ch.fixed_column("i", ch.T_INTEGER, np.arange(n, dtype=np.int32), lc.counts)
+    hb = ar.HostBatch(ch.ChunkBatch(lc.counts, [list_cases.as_column(lc, "l", stored_type), other]))
+    hb._cols[0].list.contents.child_type_id = child_type  # (the Python batch builder only knows mapped child types)
+    handle = ctx.lib.duckdb_mb_gpu_result_from_chunks(ctx.handle, C.byref(hb.struct))
+    assert not ctx.lib.duckdb_mb_is_null_arrow_result(handle), nat.last_error()
+    with ar.ArrowResult(ctx, handle, hb) as res:
+        assert np.array_equal(res.get_column_int32(1), np.arange(n, dtype=np.int32))
+        with pytest.raises(ar.DuckDBError, match="no Arrow mapping"):
+            res.to_arrow(0)
+        assert "LIST child type" in nat.last_error()

@@ -28,25 +28,79 @@ STATE_NAMES = ["NotCreated", "Ready", "RowInProgress", "Flushed", "Closed", "Err
 
 
 def _out_width(type_id: int, dec_width: int = 0) -> int:
+    if type_id == ch.T_LIST:
+        return 16  # duckdb_list_entry {uint64 offset, uint64 length}
     return ch.PHYS_WIDTH[ch.phys_of_type(type_id, dec_width)]
 
 
-class CollectedChunks:
-    """Default sink: copies every chunk out of the appender's pinned buffers."""
+# numpy dtype of a fixed-width LIST child value, by physical type (128-bit ones are decoded by hand)
+_CHILD_DTYPE = {ch.P_BOOL: np.uint8, ch.P_I8: np.int8, ch.P_I16: np.int16, ch.P_I32: np.int32, ch.P_I64: np.int64,
+                ch.P_U8: np.uint8, ch.P_U16: np.uint16, ch.P_U32: np.uint32, ch.P_U64: np.uint64,
+                ch.P_F32: np.float32, ch.P_F64: np.float64}
 
-    def __init__(self, type_ids: Sequence[int], dec_widths: Optional[Sequence[int]] = None):
+
+class CollectedChunks:
+    """Default sink: copies every chunk out of the appender's pinned buffers.
+
+    `list_children` maps a LIST column to its child type, `(child_type_id, child_dec_width)`; for those columns the
+    chunk's child vector is copied too (through Appender.list_child, valid only inside the sink call)."""
+
+    def __init__(self, type_ids: Sequence[int], dec_widths: Optional[Sequence[int]] = None, list_children: Optional[dict] = None):
         self.type_ids = list(type_ids)
         self.widths = [_out_width(t, (dec_widths or [0] * len(type_ids))[i]) for i, t in enumerate(type_ids)]
         self.counts: List[int] = []
         self.data: List[List[bytes]] = [[] for _ in type_ids]
         self.validity: List[List[np.ndarray]] = [[] for _ in type_ids]
+        self.list_children = dict(list_children or {})
+        self.child_data: dict = {c: [] for c in self.list_children}      # per chunk: child values, raw bytes
+        self.child_validity: dict = {c: [] for c in self.list_children}  # per chunk: ceil(size / 64) mask words
+        self.appender: Optional["Appender"] = None  # set by the Appender this sink is given to
 
     def __call__(self, count: int, vec_data, vec_validity) -> bool:
         self.counts.append(count)
         for c, w in enumerate(self.widths):
             self.data[c].append(C.string_at(vec_data[c], count * w))
             self.validity[c].append(np.frombuffer(C.string_at(vec_validity[c], 8 * ch.VALIDITY_WORDS), dtype=np.uint64).copy())
+        for c, (ct, dw) in self.list_children.items():
+            data, words, size = self.appender.list_child(c)
+            self.child_data[c].append(C.string_at(data, size * _out_width(ct, dw)) if size else b"")
+            nw = (size + 63) // 64
+            self.child_validity[c].append(np.frombuffer(C.string_at(words, 8 * nw), dtype=np.uint64).copy() if nw else np.zeros(0, np.uint64))
         return True
+
+    def list_values(self, c: int) -> list:
+        """LIST column `c` as Python lists (None: a NULL row or element).  Values: int (integers, DATE days,
+        TIME / TIMESTAMP ticks, DECIMAL unscaled, HUGEINT / UHUGEINT / UUID as 128-bit integers), float, bool, str
+        (VARCHAR) or bytes (BLOB).  Pointer string_t refer to the Arrow data buffer, which must still be alive."""
+        ct, dw = self.list_children[c]
+        phys = ch.phys_of_type(ct, dw)
+        out = []
+        for k, cnt in enumerate(self.counts):
+            ent = np.frombuffer(self.data[c][k], dtype=np.uint64).reshape(-1, 2)
+            valid = np.unpackbits(self.validity[c][k].view(np.uint8), bitorder="little")[:cnt].astype(bool)
+            raw = self.child_data[c][k]
+            size = len(raw) // _out_width(ct, dw)
+            cvalid = np.unpackbits(self.child_validity[c][k].view(np.uint8), bitorder="little")[:size].astype(bool)
+            if phys == ch.P_STRING:
+                e = np.frombuffer(raw, dtype=np.uint8).reshape(-1, 16)
+                vals = []
+                for i in range(size):
+                    ln = int(e[i, 0:4].view(np.uint32)[0])
+                    b = bytes(e[i, 4:4 + ln]) if ln <= 12 else C.string_at(int(e[i, 8:16].view(np.uint64)[0]), ln)
+                    vals.append(b.decode() if ct == ch.T_VARCHAR else b)
+            elif phys in (ch.P_I128, ch.P_U128):
+                vals = [int.from_bytes(raw[16 * i: 16 * i + 16], "little", signed=phys == ch.P_I128) for i in range(size)]
+            else:
+                vals = np.frombuffer(raw, dtype=_CHILD_DTYPE[phys]).tolist()
+                if phys == ch.P_BOOL:
+                    vals = [bool(v) for v in vals]
+            for i in range(cnt):
+                if not valid[i]:
+                    out.append(None)
+                    continue
+                o, ln = int(ent[i, 0]), int(ent[i, 1])
+                out.append([vals[j] if cvalid[j] else None for j in range(o, o + ln)])
+        return out
 
     @property
     def nrows(self) -> int:
@@ -82,6 +136,8 @@ class Appender:
             except Exception:  # noqa: BLE001 - a raising sink aborts the append
                 return 0
 
+        if isinstance(sink, CollectedChunks):
+            sink.appender = self
         self._cb = nat.CHUNK_SINK(_trampoline) if (sink is not None and not discard) else nat.CHUNK_SINK()
         ids = (C.c_int32 * n)(*self.type_ids)
         self.handle = self.lib.duckdb_mb_gpu_appender_create(ctx.handle, n, ids, self._cb, None)
@@ -142,6 +198,19 @@ class Appender:
     def set_decimal(self, col: int, width: int, scale: int):
         """The table column's DECIMAL(width, scale) (what duckdb_appender_column_type reports)."""
         self._check(self.lib.duckdb_mb_gpu_appender_set_decimal(self.handle, int(col), int(width), int(scale)), "set_decimal")
+
+    def set_list(self, col: int, child_type: int, dec_width: int = 0, dec_scale: int = 0):
+        """The LIST column's child type (what duckdb_list_type_child_type of duckdb_appender_column_type reports);
+        needed before an Arrow list reaches that column."""
+        self._check(self.lib.duckdb_mb_gpu_appender_set_list(self.handle, int(col), int(child_type), int(dec_width), int(dec_scale)),
+                    "set_list")
+
+    def list_child(self, col: int):
+        """Inside a sink call: (child values pointer, child mask pointer, child size) of LIST column `col`."""
+        data, words, size = C.c_void_p(), C.c_void_p(), C.c_uint64()
+        self._check(self.lib.duckdb_mb_gpu_appender_list_child(self.handle, int(col), C.byref(data), C.byref(words), C.byref(size)),
+                    "list_child")
+        return data.value, words.value, int(size.value)
 
     def append_decimal(self, width: int, scale: int, unscaled: int):  # src/duckdb_native.c:1447-1481 (hugeint parts)
         lo = unscaled & 0xFFFFFFFFFFFFFFFF

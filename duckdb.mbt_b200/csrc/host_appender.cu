@@ -41,13 +41,29 @@ struct RowBuf {  // one column of buffered rows (row API)
 // one column of a conversion request (host pointers, whole batch)
 struct ColInput {
   int rev_op = 0, w_in = 0, w_out = 0;
-  bool is_string = false, large = false, is_bits = false;
+  bool is_string = false, large = false, is_bits = false, is_list = false;
   const uint8_t *values = nullptr;       // fixed: first value of the slice; bits: bitmap base
   const uint8_t *validity = nullptr;     // Arrow bitmap base or NULL
   int64_t bit_offset = 0;                // array offset in bits (validity and bool values)
   const uint8_t *valid_bytes = nullptr;  // row API: one byte per row instead of a bitmap
-  const uint8_t *offsets = nullptr;      // strings: first offset of the slice
+  const uint8_t *offsets = nullptr;      // strings, lists: first offset of the slice
   const uint8_t *data = nullptr;         // strings: Arrow data buffer base
+  const ColInput *child = nullptr;       // lists: the child array, its rows are the list elements
+  int64_t child_len = 0;                 // lists: elements in the child array
+};
+
+// the table's child type of a LIST column (duckdb_mb_gpu_appender_set_list); type_id 0: not declared
+struct ListDecl {
+  int32_t type_id = 0, dec_width = 0, dec_scale = 0;
+};
+
+// what duckdb_mb_gpu_appender_list_child hands out during a sink call, per LIST column
+struct SinkList {
+  const uint8_t *values = nullptr;  // the sub-batch's child values, dense
+  const uint64_t *words = nullptr;  // the sub-batch's child masks, chunk k at cword[k]
+  const int64_t *bounds = nullptr;  // Arrow offsets at the sub-batch's chunk boundaries
+  const int64_t *cword = nullptr;
+  int w = 0;                        // bytes per child value
 };
 
 }  // namespace
@@ -68,7 +84,11 @@ struct duckdb_mb_gpu_appender {
   int64_t row_count = 0, flushed_row_count = 0, buffered_rows = 0;
   char error[256] = {0};
   std::vector<RowBuf> rows;
+  std::vector<ListDecl> lists;
+  std::vector<SinkList> sink_lists;  // valid while sink_chunk >= 0: chunk sink_chunk of the sub-batch being handed over
+  int64_t sink_chunk = -1;
   int64_t sub_rows = 4 << 20;
+  int64_t list_child_cap = 0;  // kListChildCap unless DMB_REV_LIST_CHILD_CAP says otherwise
   double t[4] = {0, 0, 0, 0};
   uint64_t bytes_h2d = 0, bytes_d2h = 0;
 };
@@ -174,33 +194,165 @@ bool map_format(App *a, int c, const char *fmt, int32_t type_id, ColInput *in) {
   return false;
 }
 
+// The child elements a sub-batch may hold per LIST column: a sub-batch ends at the 2048-row boundary before the chunk
+// that would take a LIST column past this many elements, but always holds at least one chunk, so one chunk's child
+// range is never split.  It bounds a slot's child buffers: 16 M elements are 256 MB of string_t or HUGEINT values.
+// DMB_REV_LIST_CHILD_CAP overrides it (tests force several sub-batches with it).
+constexpr int64_t kListChildCap = 16 << 20;
+
+bool grow(Scope &sc, uint8_t *&p, size_t &cap, size_t need, bool pinned = false) {
+  if (p && need <= cap) return true;  // the old block returns to the pool with the scope
+  cap = need + need / 8 + 64;
+  p = (uint8_t *)(pinned ? sc.palloc(cap) : sc.dalloc(cap));
+  return p != nullptr;
+}
+
+struct ListOut {  // one LIST column of a slot: the child vectors of the sub-batch and where each chunk's mask starts
+  uint8_t *d_child = nullptr, *h_child = nullptr;
+  uint8_t *d_words = nullptr, *h_words = nullptr;
+  size_t child_cap = 0, h_child_cap = 0, words_cap = 0, h_words_cap = 0;
+  int64_t *d_cword = nullptr, *h_cword = nullptr;
+  int64_t child_bytes = 0, words = 0;
+};
+
 struct Slot {  // device + pinned buffers of one in-flight sub-batch
   std::vector<uint8_t *> d_out, h_out;
   std::vector<uint64_t *> d_val, h_val;
+  std::vector<ListOut> lists;                     // [ncols], used by LIST columns
+  unsigned int *d_err = nullptr, *h_err = nullptr;  // [ncols]: rev_list_kernel error flags
   cudaEvent_t ev_out = nullptr;
   int64_t r0 = 0, r1 = 0;
   bool busy = false;
 };
 
-int32_t sink_slot(App *a, Slot &s, const std::vector<ColInput> &cols, int64_t nrows) {
+int32_t sink_slot(App *a, Slot &s, const std::vector<ColInput> &cols, const std::vector<std::vector<int64_t>> &bounds) {
   if (!s.busy) return 1;
   if (check_cuda(cudaEventSynchronize(s.ev_out), "appender copy-out wait")) return fail(a, "%s", duckdb_mb_gpu_last_error());
   s.busy = false;
-  if (!a->sink) return 1;
   const int nc = (int)cols.size();
+  for (int c = 0; c < nc; ++c)  // a malformed sub-batch reaches no sink
+    if (cols[(size_t)c].is_list && s.h_err[c])
+      return fail(a, "column %d: Arrow list offsets decrease within rows [%lld, %lld)", c, (long long)s.r0, (long long)s.r1);
+  if (!a->sink) return 1;
   std::vector<const void *> vd((size_t)nc);
   std::vector<const uint64_t *> vv((size_t)nc);
+  a->sink_lists.assign((size_t)nc, SinkList());
+  for (int c = 0; c < nc; ++c)
+    if (cols[(size_t)c].is_list) {
+      const ListOut &lo = s.lists[(size_t)c];
+      a->sink_lists[(size_t)c] = SinkList{lo.h_child, (const uint64_t *)lo.h_words, bounds[(size_t)c].data() + s.r0 / DMB_VECTOR_SIZE,
+                                          lo.h_cword, cols[(size_t)c].child->w_out};
+    }
   for (int64_t r = s.r0, k = 0; r < s.r1; r += DMB_VECTOR_SIZE, ++k) {
     const uint32_t count = (uint32_t)(s.r1 - r < DMB_VECTOR_SIZE ? s.r1 - r : DMB_VECTOR_SIZE);
     for (int c = 0; c < nc; ++c) {
       vd[(size_t)c] = s.h_out[(size_t)c] + (size_t)k * DMB_VECTOR_SIZE * (size_t)cols[(size_t)c].w_out;
       vv[(size_t)c] = s.h_val[(size_t)c] + (size_t)k * DMB_VALIDITY_WORDS;
     }
-    if (!a->sink(a->user, nc, count, vd.data(), vv.data())) return fail(a, "chunk sink aborted at row %lld", (long long)r);
+    a->sink_chunk = k;
+    const int32_t ok = a->sink(a->user, nc, count, vd.data(), vv.data());
+    a->sink_chunk = -1;
+    if (!ok) return fail(a, "chunk sink aborted at row %lld", (long long)r);
   }
-  (void)nrows;
   return 1;
 }
+
+struct InBuf {  // device inputs of one column in one slot
+  uint8_t *values = nullptr, *validity = nullptr, *offsets = nullptr, *data = nullptr;
+  uint8_t *masks = nullptr;  // row API: the masks built from the validity bytes
+  size_t values_cap = 0, validity_cap = 0, offsets_cap = 0, data_cap = 0;
+};
+
+// bits [p0, p1) of an Arrow bitmap -> `dst` (grown as needed); returns the bit offset of p0 there, -1 on failure
+int64_t stage_bits(App *a, Scope &sc, uint8_t *&dst, size_t &cap, const uint8_t *bm, int64_t p0, int64_t p1) {
+  CtxCore &c = *a->core;
+  const int64_t byte0 = p0 >> 3, byte1 = (p1 + 7) >> 3;
+  if (!grow(sc, dst, cap, (size_t)(byte1 - byte0) + 16) ||
+      stage_contiguous(c, c.s_in, dst, bm + byte0, (size_t)(byte1 - byte0), -1, &a->bytes_h2d)) return -1;
+  return p0 & 7;
+}
+
+// Arrow offset of `row` (strings, lists), read on the host
+int64_t offset_at(const ColInput &ci, int64_t row) {
+  if (ci.large) { int64_t v; memcpy(&v, ci.offsets + 8 * row, 8); return v; }
+  int32_t v; memcpy(&v, ci.offsets + 4 * row, 4); return v;
+}
+
+// Stage Arrow rows [r0, r1) of a column that is not a LIST and describe its conversion: `*fj` for a fixed-width
+// column, `*sj` for strings (the one that applies is filled).  `*d_validity` / `*bit_off`: the staged bitmap.
+int32_t stage_rows(App *a, Scope &sc, const ColInput &ci, InBuf &ib, int col, int64_t r0, int64_t r1, void *out, uint64_t *out_validity,
+                   dmb_rev_fixed_job *fj, dmb_rev_string_job *sj, const uint8_t **d_validity, int64_t *bit_off) {
+  CtxCore &c = *a->core;
+  const int64_t n = r1 - r0;
+  *d_validity = nullptr;
+  *bit_off = 0;
+  if (ci.validity) {
+    *bit_off = stage_bits(a, sc, ib.validity, ib.validity_cap, ci.validity, ci.bit_offset + r0, ci.bit_offset + r1);
+    if (*bit_off < 0) return fail(a, "%s", duckdb_mb_gpu_last_error());
+    *d_validity = ib.validity;
+  } else if (ci.valid_bytes) {  // row API: bytes here, masks built from them by dmb_dev_valid_bytes_to_masks
+    if (stage_contiguous(c, c.s_in, ib.validity, ci.valid_bytes + r0, (size_t)n, -1, &a->bytes_h2d)) return fail(a, "%s", duckdb_mb_gpu_last_error());
+    *d_validity = ib.masks;
+  }
+  if (ci.is_string) {
+    const int ow = ci.large ? 8 : 4;
+    if (!grow(sc, ib.offsets, ib.offsets_cap, (size_t)(n + 1) * (size_t)ow + 16) ||
+        stage_contiguous(c, c.s_in, ib.offsets, ci.offsets + (size_t)r0 * (size_t)ow, (size_t)(n + 1) * (size_t)ow, -1, &a->bytes_h2d))
+      return fail(a, "%s", duckdb_mb_gpu_last_error());
+    const int64_t o_first = offset_at(ci, r0), o_last = offset_at(ci, r1);
+    if (o_last < o_first || o_first < 0) return fail(a, "column %d: utf8 offsets are not monotonic", col);
+    const size_t dbytes = (size_t)(o_last - o_first);
+    if (!grow(sc, ib.data, ib.data_cap, dbytes + 64)) return fail(a, "%s", duckdb_mb_gpu_last_error());
+    if (dbytes && stage_contiguous(c, c.s_in, ib.data, ci.data + o_first, dbytes, -1, &a->bytes_h2d)) return fail(a, "%s", duckdb_mb_gpu_last_error());
+    memset(sj, 0, sizeof(*sj));
+    sj->in_offsets = ib.offsets;
+    sj->in_data = ib.data - o_first;  // indexed by absolute Arrow offsets
+    sj->in_validity = *d_validity;
+    sj->in_bit_offset = *bit_off;
+    sj->data_host_base = (uint64_t)(uintptr_t)ci.data;
+    sj->out = (dmb_string_t *)out;
+    sj->out_validity = out_validity;
+    sj->large_offsets = ci.large ? 1 : 0;
+    return 1;
+  }
+  memset(fj, 0, sizeof(*fj));
+  int64_t values_bit_off = *bit_off;
+  if (ci.is_bits) {
+    values_bit_off = stage_bits(a, sc, ib.values, ib.values_cap, ci.values, ci.bit_offset + r0, ci.bit_offset + r1);  // same array offset as the validity bitmap
+    if (values_bit_off < 0) return fail(a, "%s", duckdb_mb_gpu_last_error());
+  } else {
+    if (!grow(sc, ib.values, ib.values_cap, (size_t)n * (size_t)ci.w_in + 16) ||
+        stage_contiguous(c, c.s_in, ib.values, ci.values + (size_t)r0 * (size_t)ci.w_in, (size_t)n * (size_t)ci.w_in, -1, &a->bytes_h2d))
+      return fail(a, "%s", duckdb_mb_gpu_last_error());
+  }
+  fj->in_values = ib.values;
+  fj->in_validity = *d_validity;
+  fj->in_bit_offset = values_bit_off;
+  fj->out_data = out;
+  fj->out_validity = out_validity;
+  fj->op = ci.rev_op;
+  return 1;
+}
+
+}  // namespace
+}  // namespace dmb
+
+// end chunk (exclusive) of the sub-batch that starts at chunk k0: at most max_chunks chunks, and no LIST column holds
+// more than child_cap elements unless the sub-batch is that one chunk
+extern "C" int64_t dmb_rev_list_cut(const int64_t *const *bounds, int32_t nlists, int64_t nchunks, int64_t k0, int64_t max_chunks,
+                                    int64_t child_cap) {
+  const int64_t last = k0 + max_chunks < nchunks ? k0 + max_chunks : nchunks;
+  int64_t k1 = k0 + 1;
+  for (; k1 < last; ++k1) {
+    bool fits = true;
+    for (int32_t l = 0; l < nlists && fits; ++l) fits = bounds[l][k1 + 1] - bounds[l][k0] <= child_cap;
+    if (!fits) break;
+  }
+  return k1;
+}
+
+namespace dmb {
+namespace {
 
 // convert `nrows` rows described by `cols` and hand the chunks to the sink
 int32_t convert_rows(App *a, const std::vector<ColInput> &cols, int64_t nrows) {
@@ -212,156 +364,206 @@ int32_t convert_rows(App *a, const std::vector<ColInput> &cols, int64_t nrows) {
   const int nc = (int)cols.size();
   int64_t sub = a->sub_rows < nrows ? a->sub_rows : ((nrows + DMB_VECTOR_SIZE - 1) / DMB_VECTOR_SIZE) * DMB_VECTOR_SIZE;
   const int64_t sub_chunks = sub / DMB_VECTOR_SIZE;
+  // LIST columns: the Arrow offsets at every chunk boundary, read once; they cut the sub-batches and locate each
+  // chunk's child range
+  const int64_t nchunks = (nrows + DMB_VECTOR_SIZE - 1) / DMB_VECTOR_SIZE;
+  std::vector<std::vector<int64_t>> bounds((size_t)nc);
+  std::vector<const int64_t *> list_bounds;
+  for (int j = 0; j < nc; ++j) {
+    const ColInput &ci = cols[(size_t)j];
+    if (!ci.is_list) continue;
+    std::vector<int64_t> &b = bounds[(size_t)j];
+    b.resize((size_t)nchunks + 1);
+    for (int64_t k = 0; k <= nchunks; ++k) b[(size_t)k] = offset_at(ci, k * DMB_VECTOR_SIZE < nrows ? k * DMB_VECTOR_SIZE : nrows);
+    for (int64_t k = 0; k < nchunks; ++k)
+      if (b[(size_t)k + 1] < b[(size_t)k]) return fail(a, "column %d: Arrow list offsets decrease within rows [%lld, %lld)", j, (long long)(k * DMB_VECTOR_SIZE), (long long)((k + 1) * DMB_VECTOR_SIZE < nrows ? (k + 1) * DMB_VECTOR_SIZE : nrows));
+    if (b[0] < 0 || b[(size_t)nchunks] > ci.child_len) return fail(a, "column %d: Arrow list offsets leave the child array (%lld elements)", j, (long long)ci.child_len);
+    list_bounds.push_back(b.data());
+  }
+  std::vector<int64_t> cuts(1, 0);  // sub-batch b: chunks [cuts[b], cuts[b+1])
+  while (cuts.back() < nchunks)
+    cuts.push_back(dmb_rev_list_cut(list_bounds.data(), (int32_t)list_bounds.size(), nchunks, cuts.back(), sub_chunks, a->list_child_cap));
   Slot slots[2];
   Scope sc(c);
   cudaEvent_t in0 = sc.event(true), in1 = sc.event(true), out0 = sc.event(true), out1 = sc.event(true);
   if (!in0 || !in1 || !out0 || !out1) return fail(a, "%s", duckdb_mb_gpu_last_error());
-  const int nslots = nrows > sub ? 2 : 1;
+  const int nslots = cuts.size() > 2 ? 2 : 1;
   for (int s = 0; s < nslots; ++s) {
     slots[s].ev_out = sc.event(false);
+    slots[s].lists.resize((size_t)nc);
+    slots[s].d_err = (unsigned int *)sc.dalloc(sizeof(unsigned int) * (size_t)nc);
+    slots[s].h_err = (unsigned int *)sc.palloc(sizeof(unsigned int) * (size_t)nc);
+    if (!slots[s].ev_out || !slots[s].d_err || !slots[s].h_err) return fail(a, "%s", duckdb_mb_gpu_last_error());
     for (int j = 0; j < nc; ++j) {
       const size_t ob = (size_t)sub * (size_t)cols[(size_t)j].w_out, vb = (size_t)sub_chunks * DMB_VALIDITY_WORDS * 8;
       uint8_t *d = (uint8_t *)sc.dalloc(ob), *h = (uint8_t *)sc.palloc(ob);
       uint64_t *dv = (uint64_t *)sc.dalloc(vb), *hv = (uint64_t *)sc.palloc(vb);
-      if (!d || !h || !dv || !hv || !slots[s].ev_out) return fail(a, "%s", duckdb_mb_gpu_last_error());
+      if (!d || !h || !dv || !hv) return fail(a, "%s", duckdb_mb_gpu_last_error());
       slots[s].d_out.push_back(d);
       slots[s].h_out.push_back(h);
       slots[s].d_val.push_back(dv);
       slots[s].h_val.push_back(hv);
+      if (cols[(size_t)j].is_list) {
+        ListOut &lo = slots[s].lists[(size_t)j];
+        lo.d_cword = (int64_t *)sc.dalloc(sizeof(int64_t) * (size_t)(sub_chunks + 1));
+        lo.h_cword = (int64_t *)sc.palloc(sizeof(int64_t) * (size_t)(sub_chunks + 1));
+        if (!lo.d_cword || !lo.h_cword) return fail(a, "%s", duckdb_mb_gpu_last_error());
+      }
     }
   }
-  // per-slot device inputs
-  struct InBuf { uint8_t *values = nullptr, *validity = nullptr, *offsets = nullptr, *data = nullptr; size_t data_cap = 0; };
-  std::vector<InBuf> inbuf((size_t)nslots * (size_t)nc);
+  // per-slot device inputs: [slot][column], and the child arrays of LIST columns; sized up front for the columns that
+  // are not LISTs, grown on demand for the child ranges
+  std::vector<InBuf> inbuf((size_t)nslots * (size_t)nc), childbuf((size_t)nslots * (size_t)nc);
   for (int s = 0; s < nslots; ++s)
     for (int j = 0; j < nc; ++j) {
       const ColInput &ci = cols[(size_t)j];
       InBuf &ib = inbuf[(size_t)s * (size_t)nc + (size_t)j];
-      if (ci.is_string) ib.offsets = (uint8_t *)sc.dalloc((size_t)(sub + 1) * (ci.large ? 8 : 4) + 64);
-      else ib.values = (uint8_t *)sc.dalloc(ci.is_bits ? (size_t)(sub / 8 + 16) : (size_t)sub * (size_t)ci.w_in + 64);
-      if (ci.validity) ib.validity = (uint8_t *)sc.dalloc((size_t)(sub / 8 + 16) + 64);
-      else if (ci.valid_bytes) ib.validity = (uint8_t *)sc.dalloc((size_t)sub + (size_t)(sub / 8) + 128);  // bytes, then masks
-      if ((ci.is_string && !ib.offsets) || (!ci.is_string && !ib.values) || ((ci.validity || ci.valid_bytes) && !ib.validity))
-        return fail(a, "%s", duckdb_mb_gpu_last_error());
+      bool ok = true;
+      if (ci.is_string || ci.is_list) ok = grow(sc, ib.offsets, ib.offsets_cap, (size_t)(sub + 1) * (ci.large ? 8 : 4) + 64);
+      else ok = grow(sc, ib.values, ib.values_cap, ci.is_bits ? (size_t)(sub / 8 + 80) : (size_t)sub * (size_t)ci.w_in + 64);
+      if (ci.validity) ok = ok && grow(sc, ib.validity, ib.validity_cap, (size_t)(sub / 8 + 16) + 64);
+      else if (ci.valid_bytes) {
+        ok = ok && grow(sc, ib.validity, ib.validity_cap, (size_t)sub + 64);
+        ib.masks = (uint8_t *)sc.dalloc((size_t)(sub / 8) + 64);
+        ok = ok && ib.masks;
+      }
+      if (!ok) return fail(a, "%s", duckdb_mb_gpu_last_error());
     }
-  dmb_rev_fixed_job *h_jobs = (dmb_rev_fixed_job *)sc.palloc(sizeof(dmb_rev_fixed_job) * (size_t)nc * 2);
-  dmb_rev_fixed_job *d_jobs = (dmb_rev_fixed_job *)sc.dalloc(sizeof(dmb_rev_fixed_job) * (size_t)nc * 2);
+  // per slot: nc jobs of the columns, then one job per LIST column with a fixed-width child (a launch of its own)
+  dmb_rev_fixed_job *h_jobs = (dmb_rev_fixed_job *)sc.palloc(sizeof(dmb_rev_fixed_job) * (size_t)nc * 4);
+  dmb_rev_fixed_job *d_jobs = (dmb_rev_fixed_job *)sc.dalloc(sizeof(dmb_rev_fixed_job) * (size_t)nc * 4);
   if (!h_jobs || !d_jobs) return fail(a, "%s", duckdb_mb_gpu_last_error());
-  auto offset_at = [](const ColInput &ci, int64_t row) -> int64_t {
-    if (ci.large) { int64_t v; memcpy(&v, ci.offsets + 8 * row, 8); return v; }
-    int32_t v; memcpy(&v, ci.offsets + 4 * row, 4); return v;
-  };
   cudaEventRecord(in0, c.s_in);
   cudaEventRecord(out0, c.s_out);
-  int64_t b = 0;
-  for (int64_t r0 = 0; r0 < nrows; r0 += sub, ++b) {
-    const int64_t r1 = r0 + sub < nrows ? r0 + sub : nrows;
+  for (size_t b = 0; b + 1 < cuts.size(); ++b) {
+    const int64_t r0 = cuts[b] * DMB_VECTOR_SIZE, r1 = cuts[b + 1] * DMB_VECTOR_SIZE < nrows ? cuts[b + 1] * DMB_VECTOR_SIZE : nrows;
     const int64_t n = r1 - r0;
-    const int si = (int)(b % nslots);
+    const int64_t nch = cuts[b + 1] - cuts[b];
+    const int si = (int)(b % (size_t)nslots);
     Slot &slot = slots[si];
-    if (!sink_slot(a, slot, cols, nrows)) return 0;  // the slot's previous sub-batch leaves first
+    if (!sink_slot(a, slot, cols, bounds)) return 0;  // the slot's previous sub-batch leaves first
     // the job array of this slot is reused as well: its previous launch has completed (sink_slot waited)
-    dmb_rev_fixed_job *hj = h_jobs + (size_t)si * (size_t)nc, *dj = d_jobs + (size_t)si * (size_t)nc;
-    int nfixed = 0;
+    dmb_rev_fixed_job *hj = h_jobs + (size_t)si * (size_t)nc * 2, *dj = d_jobs + (size_t)si * (size_t)nc * 2;
+    int nfixed = 0, nchild_fixed = 0;
     cudaEvent_t ev_in = sc.event(false), ev_k = sc.event(false), k0 = sc.event(true), k1 = sc.event(true);
     if (!ev_in || !ev_k || !k0 || !k1) return fail(a, "%s", duckdb_mb_gpu_last_error());
-    struct StrLaunch { dmb_rev_string_job job; };
-    std::vector<StrLaunch> strs;
-    std::vector<std::pair<uint8_t *, int>> masks_from_bytes;  // (buffer, column)
+    std::vector<dmb_rev_string_job> strs;
+    std::vector<dmb_rev_list_job> lists;
+    std::vector<int64_t> child_rows;  // element count of each child job: fixed-width ones first, in job order
+    std::vector<int64_t> str_rows;
+    std::vector<int> masks_from_bytes;  // columns
     for (int j = 0; j < nc; ++j) {
       const ColInput &ci = cols[(size_t)j];
       InBuf &ib = inbuf[(size_t)si * (size_t)nc + (size_t)j];
       const uint8_t *d_validity = nullptr;
       int64_t bit_off = 0;
+      if (!ci.is_list) {
+        dmb_rev_string_job sj;
+        if (!stage_rows(a, sc, ci, ib, j, r0, r1, slot.d_out[(size_t)j], slot.d_val[(size_t)j], &hj[nfixed], &sj, &d_validity, &bit_off)) return 0;
+        if (ci.valid_bytes) masks_from_bytes.push_back(j);
+        if (ci.is_string) { strs.push_back(sj); str_rows.push_back(n); }
+        else ++nfixed;
+        continue;
+      }
+      // LIST: the list offsets and bitmap, then the child range [e0, e1) as a dense column of its own
+      const ColInput &cc = *ci.child;
+      ListOut &lo = slot.lists[(size_t)j];
+      const int64_t *bnd = bounds[(size_t)j].data() + cuts[b];
+      const int64_t e0 = bnd[0], e1 = bnd[nch], ne = e1 - e0;
+      const int ow = ci.large ? 8 : 4;
       if (ci.validity) {
-        const int64_t p0 = ci.bit_offset + r0, p1 = ci.bit_offset + r1;
-        const int64_t byte0 = p0 >> 3, byte1 = (p1 + 7) >> 3;
-        if (stage_contiguous(c, c.s_in, ib.validity, ci.validity + byte0, (size_t)(byte1 - byte0), -1, &a->bytes_h2d)) return fail(a, "%s", duckdb_mb_gpu_last_error());
+        bit_off = stage_bits(a, sc, ib.validity, ib.validity_cap, ci.validity, ci.bit_offset + r0, ci.bit_offset + r1);
+        if (bit_off < 0) return fail(a, "%s", duckdb_mb_gpu_last_error());
         d_validity = ib.validity;
-        bit_off = p0 & 7;
-      } else if (ci.valid_bytes) {
-        if (stage_contiguous(c, c.s_in, ib.validity, ci.valid_bytes + r0, (size_t)n, -1, &a->bytes_h2d)) return fail(a, "%s", duckdb_mb_gpu_last_error());
-        uint8_t *masks = ib.validity + (((size_t)sub + 63) & ~(size_t)63);
-        masks_from_bytes.emplace_back(ib.validity, j);
-        d_validity = masks;
-        bit_off = 0;
       }
-      if (ci.is_string) {
-        const int ow = ci.large ? 8 : 4;
-        if (stage_contiguous(c, c.s_in, ib.offsets, ci.offsets + (size_t)r0 * (size_t)ow, (size_t)(n + 1) * (size_t)ow, -1, &a->bytes_h2d)) return fail(a, "%s", duckdb_mb_gpu_last_error());
-        const int64_t o_first = offset_at(ci, r0), o_last = offset_at(ci, r1);
-        if (o_last < o_first || o_first < 0) return fail(a, "column %d: utf8 offsets are not monotonic", j);
-        const size_t dbytes = (size_t)(o_last - o_first);
-        if (dbytes + 64 > ib.data_cap) {  // grows to the largest sub-batch seen; old block returns to the pool with the scope
-          ib.data_cap = dbytes + dbytes / 8 + 64;
-          ib.data = (uint8_t *)sc.dalloc(ib.data_cap);
-          if (!ib.data) return fail(a, "%s", duckdb_mb_gpu_last_error());
-        }
-        if (dbytes && stage_contiguous(c, c.s_in, ib.data, ci.data + o_first, dbytes, -1, &a->bytes_h2d)) return fail(a, "%s", duckdb_mb_gpu_last_error());
-        StrLaunch sl;
-        memset(&sl.job, 0, sizeof(sl.job));
-        sl.job.in_offsets = ib.offsets;
-        sl.job.in_data = ib.data - o_first;  // indexed by absolute Arrow offsets
-        sl.job.in_validity = d_validity;
-        sl.job.in_bit_offset = bit_off;
-        sl.job.data_host_base = (uint64_t)(uintptr_t)ci.data;
-        sl.job.out = (dmb_string_t *)slot.d_out[(size_t)j];
-        sl.job.out_validity = slot.d_val[(size_t)j];
-        sl.job.large_offsets = ci.large ? 1 : 0;
-        strs.push_back(sl);
-      } else {
-        dmb_rev_fixed_job &job = hj[nfixed++];
-        memset(&job, 0, sizeof(job));
-        if (ci.is_bits) {
-          const int64_t p0 = ci.bit_offset + r0, p1 = ci.bit_offset + r1;
-          const int64_t byte0 = p0 >> 3, byte1 = (p1 + 7) >> 3;
-          if (stage_contiguous(c, c.s_in, ib.values, ci.values + byte0, (size_t)(byte1 - byte0), -1, &a->bytes_h2d)) return fail(a, "%s", duckdb_mb_gpu_last_error());
-          bit_off = p0 & 7;  // same array offset as the validity bitmap
-        } else {
-          if (stage_contiguous(c, c.s_in, ib.values, ci.values + (size_t)r0 * (size_t)ci.w_in, (size_t)n * (size_t)ci.w_in, -1, &a->bytes_h2d)) return fail(a, "%s", duckdb_mb_gpu_last_error());
-        }
-        job.in_values = ib.values;
-        job.in_validity = d_validity;
-        job.in_bit_offset = bit_off;
-        job.out_data = slot.d_out[(size_t)j];
-        job.out_validity = slot.d_val[(size_t)j];
-        job.op = ci.rev_op;
+      if (stage_contiguous(c, c.s_in, ib.offsets, ci.offsets + (size_t)r0 * (size_t)ow, (size_t)(n + 1) * (size_t)ow, -1, &a->bytes_h2d))
+        return fail(a, "%s", duckdb_mb_gpu_last_error());
+      lo.h_cword[0] = 0;
+      for (int64_t k = 0; k < nch; ++k) lo.h_cword[k + 1] = lo.h_cword[k] + (bnd[k + 1] - bnd[k] + 63) / 64;
+      lo.words = lo.h_cword[nch];
+      if (check_cuda(cudaMemcpyAsync(lo.d_cword, lo.h_cword, sizeof(int64_t) * (size_t)(nch + 1), cudaMemcpyHostToDevice, c.s_in), "child_word H2D"))
+        return fail(a, "%s", duckdb_mb_gpu_last_error());
+      a->bytes_h2d += sizeof(int64_t) * (uint64_t)(nch + 1);
+      const int64_t child_slots = cc.is_string ? ((ne + DMB_VECTOR_SIZE - 1) / DMB_VECTOR_SIZE) * DMB_VECTOR_SIZE : ne;  // rev_string_kernel fills whole vectors
+      lo.child_bytes = ne * cc.w_out;
+      if (!grow(sc, lo.d_child, lo.child_cap, (size_t)child_slots * (size_t)cc.w_out + 64) ||
+          !grow(sc, lo.h_child, lo.h_child_cap, (size_t)lo.child_bytes + 64, true) ||
+          !grow(sc, lo.d_words, lo.words_cap, (size_t)lo.words * 8 + 64) || !grow(sc, lo.h_words, lo.h_words_cap, (size_t)lo.words * 8 + 64, true))
+        return fail(a, "%s", duckdb_mb_gpu_last_error());
+      dmb_rev_list_job lj;
+      memset(&lj, 0, sizeof(lj));
+      if (ne > 0) {
+        dmb_rev_fixed_job *fj = &hj[nc + nchild_fixed];
+        dmb_rev_string_job sj;
+        const uint8_t *d_cvalidity = nullptr;
+        int64_t cbit_off = 0;
+        // out_validity NULL: the child masks are the list kernel's, per chunk
+        if (!stage_rows(a, sc, cc, childbuf[(size_t)si * (size_t)nc + (size_t)j], j, e0, e1, lo.d_child, nullptr, fj, &sj, &d_cvalidity, &cbit_off)) return 0;
+        if (cc.is_string) { strs.push_back(sj); str_rows.push_back(ne); }
+        else { ++nchild_fixed; child_rows.push_back(ne); }
+        lj.in_child_validity = d_cvalidity;
+        lj.child_bit_offset = cbit_off;
       }
+      lj.in_offsets = ib.offsets;
+      lj.in_validity = d_validity;
+      lj.in_bit_offset = bit_off;
+      lj.child_word = lo.d_cword;
+      lj.out_entries = slot.d_out[(size_t)j];
+      lj.out_validity = slot.d_val[(size_t)j];
+      lj.out_child_validity = (uint64_t *)lo.d_words;
+      lj.error = slot.d_err + j;
+      lj.large_offsets = ci.large ? 1 : 0;
+      lists.push_back(lj);
     }
     cudaEventRecord(ev_in, c.s_in);
     if (check_cuda(cudaStreamWaitEvent(c.s_compute, ev_in, 0), "wait copy-in")) return fail(a, "%s", duckdb_mb_gpu_last_error());
     cudaEventRecord(k0, c.s_compute);
-    for (auto &mb : masks_from_bytes) {
-      uint8_t *masks = mb.first + (((size_t)sub + 63) & ~(size_t)63);
-      if (dmb_dev_valid_bytes_to_masks(mb.first, (uint64_t *)masks, nullptr, n, c.s_compute)) return fail(a, "%s", duckdb_mb_gpu_last_error());
+    for (int j : masks_from_bytes) {
+      InBuf &ib = inbuf[(size_t)si * (size_t)nc + (size_t)j];
+      if (dmb_dev_valid_bytes_to_masks(ib.validity, (uint64_t *)ib.masks, nullptr, n, c.s_compute)) return fail(a, "%s", duckdb_mb_gpu_last_error());
     }
-    if (nfixed) {
-      if (check_cuda(cudaMemcpyAsync(dj, hj, sizeof(dmb_rev_fixed_job) * (size_t)nfixed, cudaMemcpyHostToDevice, c.s_compute), "job H2D")) return fail(a, "%s", duckdb_mb_gpu_last_error());
-      if (dmb_dev_rev_fixed_batch(dj, hj, nfixed, n, c.s_compute)) return fail(a, "%s", duckdb_mb_gpu_last_error());
+    if (nfixed || nchild_fixed) {
+      const size_t njobs = nchild_fixed ? (size_t)nc + (size_t)nchild_fixed : (size_t)nfixed;
+      if (check_cuda(cudaMemcpyAsync(dj, hj, sizeof(dmb_rev_fixed_job) * njobs, cudaMemcpyHostToDevice, c.s_compute), "job H2D")) return fail(a, "%s", duckdb_mb_gpu_last_error());
+      if (nfixed && dmb_dev_rev_fixed_batch(dj, hj, nfixed, n, c.s_compute)) return fail(a, "%s", duckdb_mb_gpu_last_error());
+      for (int i = 0; i < nchild_fixed; ++i)  // one launch per child: the launch takes one row count for all its jobs
+        if (dmb_dev_rev_fixed_batch(dj + nc + i, hj + nc + i, 1, child_rows[(size_t)i], c.s_compute)) return fail(a, "%s", duckdb_mb_gpu_last_error());
     }
-    for (auto &sl : strs)
-      if (dmb_dev_rev_string_batch(&sl.job, n, c.s_compute)) return fail(a, "%s", duckdb_mb_gpu_last_error());
+    for (size_t i = 0; i < strs.size(); ++i)
+      if (dmb_dev_rev_string_batch(&strs[i], str_rows[i], c.s_compute)) return fail(a, "%s", duckdb_mb_gpu_last_error());
+    if (!lists.empty() && check_cuda(cudaMemsetAsync(slot.d_err, 0, sizeof(unsigned int) * (size_t)nc, c.s_compute), "error flags reset"))
+      return fail(a, "%s", duckdb_mb_gpu_last_error());
+    for (auto &lj : lists)
+      if (dmb_dev_rev_list_batch(&lj, n, c.s_compute)) return fail(a, "%s", duckdb_mb_gpu_last_error());
     cudaEventRecord(k1, c.s_compute);
     sc.kernel_spans.emplace_back(k0, k1);
     cudaEventRecord(ev_k, c.s_compute);
     if (check_cuda(cudaStreamWaitEvent(c.s_out, ev_k, 0), "wait kernels")) return fail(a, "%s", duckdb_mb_gpu_last_error());
-    const int64_t nch = (n + DMB_VECTOR_SIZE - 1) / DMB_VECTOR_SIZE;
     for (int j = 0; j < nc; ++j) {
       const size_t ob = (size_t)n * (size_t)cols[(size_t)j].w_out, vb = (size_t)nch * DMB_VALIDITY_WORDS * 8;
       if (check_cuda(cudaMemcpyAsync(slot.h_out[(size_t)j], slot.d_out[(size_t)j], ob, cudaMemcpyDeviceToHost, c.s_out), "vectors D2H") ||
           check_cuda(cudaMemcpyAsync(slot.h_val[(size_t)j], slot.d_val[(size_t)j], vb, cudaMemcpyDeviceToHost, c.s_out), "validity D2H"))
         return fail(a, "%s", duckdb_mb_gpu_last_error());
       a->bytes_d2h += ob + vb;
+      if (!cols[(size_t)j].is_list) continue;
+      const ListOut &lo = slot.lists[(size_t)j];
+      if ((lo.child_bytes && check_cuda(cudaMemcpyAsync(lo.h_child, lo.d_child, (size_t)lo.child_bytes, cudaMemcpyDeviceToHost, c.s_out), "child D2H")) ||
+          (lo.words && check_cuda(cudaMemcpyAsync(lo.h_words, lo.d_words, (size_t)lo.words * 8, cudaMemcpyDeviceToHost, c.s_out), "child validity D2H")))
+        return fail(a, "%s", duckdb_mb_gpu_last_error());
+      a->bytes_d2h += (uint64_t)lo.child_bytes + (uint64_t)lo.words * 8;
     }
+    if (!lists.empty() && check_cuda(cudaMemcpyAsync(slot.h_err, slot.d_err, sizeof(unsigned int) * (size_t)nc, cudaMemcpyDeviceToHost, c.s_out), "error flags D2H"))
+      return fail(a, "%s", duckdb_mb_gpu_last_error());
     cudaEventRecord(slot.ev_out, c.s_out);
     slot.r0 = r0;
     slot.r1 = r1;
     slot.busy = true;
   }
   cudaEventRecord(in1, c.s_in);
+  const size_t nsub = cuts.size() - 1;
   for (int k = 0; k < nslots; ++k) {  // oldest first
-    Slot &slot = slots[(int)((b + k) % nslots)];
-    if (!sink_slot(a, slot, cols, nrows)) return 0;
+    Slot &slot = slots[(int)((nsub + (size_t)k) % (size_t)nslots)];
+    if (!sink_slot(a, slot, cols, bounds)) return 0;
   }
   cudaEventRecord(out1, c.s_out);
   if (check_cuda(cudaStreamSynchronize(c.s_out), "appender sync") || check_cuda(cudaStreamSynchronize(c.s_in), "appender sync"))
@@ -460,6 +662,82 @@ int32_t push_number(App *a, const char *cmd, int64_t iv, double dv, bool is_doub
   return 1;
 }
 
+// the buffers of one Arrow array (already mapped by map_format) at element `off`
+void bind_buffers(ColInput &ci, const ArrowArray *arr, int64_t off) {
+  static const uint8_t kNoData[16] = {0};
+  ci.bit_offset = off;
+  ci.validity = (arr->null_count != 0 && arr->n_buffers > 0) ? (const uint8_t *)arr->buffers[0] : nullptr;
+  if (ci.is_string || ci.is_list) {
+    ci.offsets = arr->n_buffers > 1 && arr->buffers[1] ? (const uint8_t *)arr->buffers[1] + (size_t)off * (ci.large ? 8 : 4) : nullptr;
+    if (ci.is_string) ci.data = arr->n_buffers > 2 && arr->buffers[2] ? (const uint8_t *)arr->buffers[2] : kNoData;
+  } else if (ci.is_bits) {
+    ci.values = arr->n_buffers > 1 ? (const uint8_t *)arr->buffers[1] : nullptr;
+  } else {
+    ci.values = arr->n_buffers > 1 && arr->buffers[1] ? (const uint8_t *)arr->buffers[1] + (size_t)off * (size_t)ci.w_in : nullptr;
+  }
+}
+
+const char *nested_name(const char *fmt) {
+  if (strcmp(fmt, "+l") == 0 || strcmp(fmt, "+L") == 0) return "LIST";
+  if (strcmp(fmt, "+s") == 0) return "STRUCT";
+  if (strcmp(fmt, "+m") == 0) return "MAP";
+  if (strcmp(fmt, "+vl") == 0 || strcmp(fmt, "+vL") == 0) return "list view";
+  if (strncmp(fmt, "+w:", 3) == 0) return "fixed_size_list";
+  return "nested type";
+}
+
+// Arrow list / large_list -> a LIST column whose child type the table declared (duckdb_mb_gpu_appender_set_list)
+bool map_list(App *a, int j, const ArrowArray *arr, const ArrowSchema *sch, ColInput *ci, ColInput *child) {
+  const char *fmt = sch->format;
+  if (strcmp(fmt, "+l") != 0 && strcmp(fmt, "+L") != 0) {
+    if (fmt[0] == '+') fail(a, "column %d: an Arrow %s ('%s') cannot be appended to a LIST column", j, nested_name(fmt), fmt);
+    else fail(a, "column %d: Arrow format '%s' cannot be appended to a LIST column", j, fmt);
+    return false;
+  }
+  const ListDecl &d = a->lists[(size_t)j];
+  if (!d.type_id) {
+    fail(a, "column %d: the LIST column's child type is not declared (duckdb_mb_gpu_appender_set_list)", j);
+    return false;
+  }
+  if (arr->n_children != 1 || sch->n_children != 1 || !arr->children[0] || !sch->children[0] || !sch->children[0]->format) {
+    fail(a, "column %d: an Arrow list needs exactly one child array", j);
+    return false;
+  }
+  const ArrowArray *carr = arr->children[0];
+  const char *cfmt = sch->children[0]->format;
+  if (cfmt[0] == '+') {
+    fail(a, "column %d: LIST<%s> cannot be appended (Arrow child format '%s')", j, nested_name(cfmt), cfmt);
+    return false;
+  }
+  if (!map_format(a, j, cfmt, d.type_id, child)) {
+    fail(a, "column %d: Arrow list child format '%s' does not match the declared child type %d", j, cfmt, d.type_id);
+    return false;
+  }
+  if (d.type_id == DMB_TYPE_DECIMAL) {  // the table's DECIMAL(w, s) sets the child vector's width; the scale must agree
+    const char *comma = strchr(cfmt, ',');
+    if (!comma || atoi(comma + 1) != d.dec_scale) {
+      fail(a, "column %d: Arrow list child '%s' does not have the declared scale %d", j, cfmt, d.dec_scale);
+      return false;
+    }
+    if (d.dec_width <= 4) { child->rev_op = DMB_REV_I128_TO_I16; child->w_out = 2; }
+    else if (d.dec_width <= 9) { child->rev_op = DMB_REV_I128_TO_I32; child->w_out = 4; }
+    else if (d.dec_width <= 18) { child->rev_op = DMB_REV_I128_TO_I64; child->w_out = 8; }
+    else { child->rev_op = DMB_REV_COPY16; child->w_out = 16; }
+  }
+  bind_buffers(*child, carr, carr->offset);
+  child->child_len = carr->length;
+  ci->is_list = true;
+  ci->large = fmt[1] == 'L';
+  ci->w_out = 16;  // duckdb_list_entry
+  ci->child = child;
+  ci->child_len = carr->length;
+  if (carr->length > 0 && ((child->is_string && !child->offsets) || (!child->is_string && !child->values))) {
+    fail(a, "column %d: the Arrow list child has no value buffer", j);
+    return false;
+  }
+  return true;
+}
+
 }  // namespace
 }  // namespace dmb
 
@@ -474,12 +752,15 @@ extern "C" duckdb_mb_gpu_appender *duckdb_mb_gpu_appender_create(duckdb_mb_gpu_c
   a->sink = sink;
   a->user = user;
   a->rows.resize((size_t)ncols);
+  a->lists.resize((size_t)ncols);
   for (int j = 0; j < ncols; ++j) {
     a->rows[(size_t)j].width = row_width(type_ids[j]);  // -1: column only reachable through Arrow batches
     a->rows[(size_t)j].offsets.assign(1, 0);
   }
   const char *env = getenv("DMB_REV_BATCH_ROWS");
   if (env && atoll(env) >= DMB_VECTOR_SIZE) a->sub_rows = (atoll(env) / DMB_VECTOR_SIZE) * DMB_VECTOR_SIZE;
+  const char *cap = getenv("DMB_REV_LIST_CHILD_CAP");
+  a->list_child_cap = cap && atoll(cap) > 0 ? atoll(cap) : kListChildCap;
   a->state = kReady;  // Create: NotCreated -> Ready
   return a;
 }
@@ -529,12 +810,14 @@ extern "C" int32_t duckdb_mb_gpu_append_arrow_batch(duckdb_mb_gpu_appender *a, c
     return 0;
   }
   const int64_t n = batch->length;
-  std::vector<ColInput> cols((size_t)a->ncols);
+  std::vector<ColInput> cols((size_t)a->ncols), children((size_t)a->ncols);
   for (int j = 0; j < a->ncols; ++j) {
     const ArrowArray *ch = batch->children[j];
     const ArrowSchema *cs = schema->children[j];
     ColInput &ci = cols[(size_t)j];
-    if (!ch || !cs || !cs->format || !map_format(a, j, cs->format, a->type_ids[(size_t)j], &ci)) {
+    const bool list = a->type_ids[(size_t)j] == DMB_TYPE_LIST;
+    if (!ch || !cs || !cs->format ||
+        !(list ? map_list(a, j, ch, cs, &ci, &children[(size_t)j]) : map_format(a, j, cs->format, a->type_ids[(size_t)j], &ci))) {
       if (!a->error[0]) fail(a, "append_arrow_batch: column %d is malformed", j);
       a->state = kError;
       return 0;
@@ -544,20 +827,8 @@ extern "C" int32_t duckdb_mb_gpu_append_arrow_batch(duckdb_mb_gpu_appender *a, c
       a->state = kError;
       return 0;
     }
-    const int64_t off = ch->offset + batch->offset;
-    ci.bit_offset = off;
-    ci.validity = (ch->null_count != 0 && ch->n_buffers > 0) ? (const uint8_t *)ch->buffers[0] : nullptr;
-    if (ci.is_string) {
-      ci.offsets = (const uint8_t *)ch->buffers[1] + (size_t)off * (ci.large ? 8 : 4);
-      ci.data = (const uint8_t *)ch->buffers[2];
-      static const uint8_t kNoData[16] = {0};
-      if (!ci.data) ci.data = kNoData;
-    } else if (ci.is_bits) {
-      ci.values = (const uint8_t *)ch->buffers[1];
-    } else {
-      ci.values = (const uint8_t *)ch->buffers[1] + (size_t)off * (size_t)ci.w_in;
-    }
-    if (n > 0 && ((ci.is_string && !ci.offsets) || (!ci.is_string && !ci.values))) {
+    bind_buffers(ci, ch, ch->offset + batch->offset);
+    if (n > 0 && (((ci.is_string || ci.is_list) && !ci.offsets) || (!ci.is_string && !ci.is_list && !ci.values))) {
       fail(a, "append_arrow_batch: column %d has no value buffer", j);
       a->state = kError;
       return 0;
@@ -676,6 +947,51 @@ extern "C" int32_t duckdb_mb_gpu_appender_set_decimal(duckdb_mb_gpu_appender *a,
   }
   rb.dec_prec = width;
   rb.dec_scale = scale;
+  return 1;
+}
+
+// the table column's LIST child type (duckdb_list_type_child_type(duckdb_appender_column_type(..)))
+extern "C" int32_t duckdb_mb_gpu_appender_set_list(duckdb_mb_gpu_appender *a, int32_t col, int32_t child_type_id, int32_t child_dec_width,
+                                                   int32_t child_dec_scale) {
+  if (!a) return 0;
+  if (col < 0 || col >= a->ncols || a->type_ids[(size_t)col] != DMB_TYPE_LIST) return fail(a, "appender_set_list: column %d is not a LIST column", col);
+  switch (child_type_id) {
+    case DMB_TYPE_LIST: return fail(a, "appender_set_list: column %d: LIST<LIST> cannot be appended", col);
+    case DMB_TYPE_STRUCT: return fail(a, "appender_set_list: column %d: LIST<STRUCT> cannot be appended", col);
+    case DMB_TYPE_MAP: return fail(a, "appender_set_list: column %d: LIST<MAP> cannot be appended", col);
+    case DMB_TYPE_DECIMAL:
+      if (child_dec_width < 1 || child_dec_width > 38 || child_dec_scale < 0 || child_dec_scale > child_dec_width)
+        return fail(a, "appender_set_list: column %d: DECIMAL(%d,%d) is not a type", col, child_dec_width, child_dec_scale);
+      break;
+    case DMB_TYPE_BOOLEAN: case DMB_TYPE_TINYINT: case DMB_TYPE_SMALLINT: case DMB_TYPE_INTEGER: case DMB_TYPE_BIGINT:
+    case DMB_TYPE_UTINYINT: case DMB_TYPE_USMALLINT: case DMB_TYPE_UINTEGER: case DMB_TYPE_UBIGINT: case DMB_TYPE_FLOAT:
+    case DMB_TYPE_DOUBLE: case DMB_TYPE_DATE: case DMB_TYPE_TIME: case DMB_TYPE_TIME_NS: case DMB_TYPE_TIME_TZ:
+    case DMB_TYPE_TIMESTAMP: case DMB_TYPE_TIMESTAMP_S: case DMB_TYPE_TIMESTAMP_MS: case DMB_TYPE_TIMESTAMP_NS:
+    case DMB_TYPE_TIMESTAMP_TZ: case DMB_TYPE_HUGEINT: case DMB_TYPE_UHUGEINT: case DMB_TYPE_UUID: case DMB_TYPE_VARCHAR:
+    case DMB_TYPE_BLOB:
+      break;
+    default:  // the child types map_format converts, and nothing else
+      return fail(a, "appender_set_list: column %d: LIST child type %d cannot be appended", col, child_type_id);
+  }
+  if (child_type_id != DMB_TYPE_DECIMAL) child_dec_width = child_dec_scale = 0;
+  ListDecl &d = a->lists[(size_t)col];
+  if (d.type_id && (d.type_id != child_type_id || d.dec_width != child_dec_width || d.dec_scale != child_dec_scale))
+    return fail(a, "appender_set_list: column %d already has LIST child type %d", col, d.type_id);
+  d = ListDecl{child_type_id, child_dec_width, child_dec_scale};
+  return 1;
+}
+
+// during a sink call: the child vector of LIST column `col` for the chunk being handed over
+extern "C" int32_t duckdb_mb_gpu_appender_list_child(duckdb_mb_gpu_appender *a, int32_t col, const void **data, const uint64_t **validity,
+                                                     uint64_t *size) {
+  if (!a || !data || !validity || !size) return 0;
+  if (a->sink_chunk < 0 || col < 0 || col >= a->ncols || (size_t)col >= a->sink_lists.size() || !a->sink_lists[(size_t)col].bounds)
+    return fail(a, "appender_list_child: column %d is not a LIST column of a chunk being handed to the sink", col);
+  const SinkList &l = a->sink_lists[(size_t)col];
+  const int64_t k = a->sink_chunk;
+  *data = l.values + (size_t)(l.bounds[k] - l.bounds[0]) * (size_t)l.w;
+  *validity = l.words + l.cword[k];
+  *size = (uint64_t)(l.bounds[k + 1] - l.bounds[k]);
   return 1;
 }
 

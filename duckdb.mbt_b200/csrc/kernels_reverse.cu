@@ -264,6 +264,82 @@ rev_string_kernel(dmb_rev_string_job job, int64_t nrows) {
   if (job.null_count && lane == 0 && nulls) atomicAdd(job.null_count, (unsigned long long)nulls);
 }
 
+// Arrow list offsets -> duckdb_list_entry + list masks (rows, two per thread in flight, offsets read like
+// rev_string_kernel), then every chunk's child mask (one 64-bit word per thread, funnel shifted from the dense child
+// bitmap so that chunk k's mask starts at its first element).
+template <bool LARGE>
+__global__ void __launch_bounds__(kThreads)
+rev_list_kernel(dmb_rev_list_job job, int64_t nrows) {
+  constexpr int U = 2;
+  using off_t = typename std::conditional<LARGE, long long, int>::type;
+  const off_t *off = reinterpret_cast<const off_t *>(job.in_offsets);
+  const int lane = threadIdx.x & 31;
+  const int64_t nchunks = (nrows + kVec - 1) / kVec;
+  const int64_t capacity = nchunks * (int64_t)kVec;  // a multiple of U * kThreads
+  const bool has_bm = job.in_validity != nullptr;
+  const BitSrc bs = bit_src(job.in_validity, job.in_bit_offset);
+  uint4 *out = reinterpret_cast<uint4 *>(job.out_entries);
+  uint32_t *out_val32 = reinterpret_cast<uint32_t *>(job.out_validity);
+  const int64_t off0 = (int64_t)__ldg(off);
+  int nulls = 0;
+  bool bad = false;
+  for (int64_t base = (int64_t)blockIdx.x * (U * kThreads); base < capacity; base += (int64_t)gridDim.x * (U * kThreads)) {
+    off_t o0[U], o1[U];
+    int64_t cbase[U];
+    uint32_t vb[U];
+#pragma unroll
+    for (int u = 0; u < U; ++u) {
+      const int64_t row = base + u * kThreads + threadIdx.x;
+      o0[u] = __ldg(off + (row < nrows ? row : nrows));
+      cbase[u] = (int64_t)__ldg(off + (row & ~(int64_t)(kVec - 1)));  // same address for the whole warp
+    }
+#pragma unroll
+    for (int u = 0; u < U; ++u) {
+      const int64_t row = base + u * kThreads + threadIdx.x;
+      const int64_t row0 = row - lane;
+      const int64_t left = nrows - row0;
+      const int live = left <= 0 ? 0 : (left < 32 ? (int)left : 32);
+      vb[u] = live == 0 ? 0u : (has_bm ? load_bits32(bs.w, bs.base + row0, live) : (live == 32 ? 0xffffffffu : ((1u << live) - 1u)));
+      if (lane == 0) {
+        out_val32[row >> 5] = vb[u];
+        nulls += live - __popc(vb[u]);
+      }
+      o1[u] = __shfl_down_sync(0xffffffffu, o0[u], 1);
+      if (lane == 31) o1[u] = __ldg(off + (row + 1 < nrows ? row + 1 : nrows));
+    }
+#pragma unroll
+    for (int u = 0; u < U; ++u) {
+      const int64_t row = base + u * kThreads + threadIdx.x;
+      uint4 e = make_uint4(0, 0, 0, 0);
+      if (row < nrows) {
+        const int64_t len = (int64_t)o1[u] - (int64_t)o0[u];
+        bad |= len < 0;
+        const uint64_t eo = (uint64_t)((int64_t)o0[u] - cbase[u]);
+        const uint64_t el = ((vb[u] >> lane) & 1u) && len > 0 ? (uint64_t)len : 0ull;
+        e = make_uint4((uint32_t)eo, (uint32_t)(eo >> 32), (uint32_t)el, (uint32_t)(el >> 32));
+      }
+      st_stream(out + row, e);
+    }
+  }
+  if (job.null_count && lane == 0 && nulls) atomicAdd(job.null_count, (unsigned long long)nulls);
+  if (__any_sync(0xffffffffu, bad) && lane == 0) atomicOr(job.error, 1u);
+  // child masks: word w belongs to the chunk k with child_word[k] <= w < child_word[k+1]
+  const int64_t nwords = __ldg(job.child_word + nchunks);
+  const bool has_cbm = job.in_child_validity != nullptr;
+  const BitSrc cs = bit_src(job.in_child_validity, job.child_bit_offset);
+  for (int64_t w = (int64_t)blockIdx.x * kThreads + threadIdx.x; w < nwords; w += (int64_t)gridDim.x * kThreads) {
+    int64_t lo = 0, hi = nchunks;
+    while (hi - lo > 1) {
+      const int64_t mid = (lo + hi) >> 1;
+      if (__ldg(job.child_word + mid) <= w) lo = mid; else hi = mid;
+    }
+    const int64_t r0 = lo * kVec, r1 = r0 + kVec < nrows ? r0 + kVec : nrows;
+    const int64_t e0 = (int64_t)__ldg(off + r0) - off0, size = (int64_t)__ldg(off + r1) - off0 - e0;
+    const BitSrc chunk_bits{cs.w, cs.base + e0};
+    __stcs(reinterpret_cast<unsigned long long *>(job.out_child_validity + w), rev_valid_word(chunk_bits, has_cbm, size, w - __ldg(job.child_word + lo)));
+  }
+}
+
 }  // namespace dmb
 
 using namespace dmb;
@@ -291,4 +367,20 @@ extern "C" int32_t dmb_dev_rev_string_batch(const dmb_rev_string_job *job, int64
   if (job->large_offsets) rev_string_kernel<true><<<gx, kThreads, 0, (cudaStream_t)stream>>>(*job, nrows);
   else rev_string_kernel<false><<<gx, kThreads, 0, (cudaStream_t)stream>>>(*job, nrows);
   return check_cuda(cudaGetLastError(), "rev_string_kernel launch");
+}
+
+extern "C" int32_t dmb_dev_rev_list_batch(const dmb_rev_list_job *job, int64_t nrows, void *stream) {
+  if (!job) { set_error("dmb_dev_rev_list_batch: job is null"); return -1; }
+  if (nrows <= 0) return 0;
+  if (!job->in_offsets || !job->child_word || !job->out_entries || !job->out_validity || !job->out_child_validity || !job->error) {
+    set_error("dmb_dev_rev_list_batch: a required pointer is null");
+    return -1;
+  }
+  int64_t capacity = ((nrows + kVec - 1) / kVec) * (int64_t)kVec;
+  int64_t blocks = capacity / (2 * kThreads);
+  int64_t max_grid = (int64_t)kNumSMs * 8;
+  int gx = (int)(blocks < max_grid ? blocks : max_grid);
+  if (job->large_offsets) rev_list_kernel<true><<<gx, kThreads, 0, (cudaStream_t)stream>>>(*job, nrows);
+  else rev_list_kernel<false><<<gx, kThreads, 0, (cudaStream_t)stream>>>(*job, nrows);
+  return check_cuda(cudaGetLastError(), "rev_list_kernel launch");
 }

@@ -53,6 +53,13 @@ class RevStringJob(C.Structure):
                 ("reserved", C.c_int32)]
 
 
+class RevListJob(C.Structure):
+    _fields_ = [("in_offsets", C.c_void_p), ("in_validity", C.c_void_p), ("in_bit_offset", C.c_int64),
+                ("in_child_validity", C.c_void_p), ("child_bit_offset", C.c_int64), ("child_word", C.c_void_p),
+                ("out_entries", C.c_void_p), ("out_validity", C.c_void_p), ("out_child_validity", C.c_void_p),
+                ("null_count", C.c_void_p), ("error", C.c_void_p), ("large_offsets", C.c_int32), ("reserved", C.c_int32)]
+
+
 class EnumDict(C.Structure):
     _fields_ = [("size", C.c_uint32), ("reserved", C.c_uint32), ("offsets", C.c_void_p), ("data", C.c_void_p)]
 
@@ -131,6 +138,7 @@ CHUNK_SINK = C.CFUNCTYPE(C.c_int32, C.c_void_p, C.c_int32, C.c_uint32, C.POINTER
 EXPORTED_SYMBOLS = [
     "dmb_dev_fixed_batch", "dmb_op_out_width", "dmb_phys_width", "dmb_dev_string_scratch_bytes",
     "dmb_dev_string_error", "dmb_dev_string_batch", "dmb_dev_set_lookback_limit_ns", "dmb_dev_rev_fixed_batch", "dmb_dev_rev_string_batch",
+    "dmb_dev_rev_list_batch", "dmb_rev_list_cut",
     "dmb_dev_valid_bytes_to_masks", "dmb_dev_make_string_t", "dmb_dev_blob_escape", "dmb_render_supported", "dmb_render_slot_bytes", "dmb_dev_render_text", "dmb_dev_enum_to_string_t", "dmb_dev_enum_utf8", "dmb_dev_list_scratch_bytes", "dmb_dev_list_batch",
     "duckdb_mb_gpu_last_error", "duckdb_mb_gpu_device_count", "duckdb_mb_gpu_bind_numa", "duckdb_mb_gpu_ctx_create",
     "duckdb_mb_gpu_ctx_destroy", "duckdb_mb_gpu_ctx_sync", "duckdb_mb_gpu_host_alloc", "duckdb_mb_gpu_host_free",
@@ -167,7 +175,8 @@ EXPORTED_SYMBOLS = [
     "duckdb_mb_gpu_append_varchar", "duckdb_mb_gpu_append_bool", "duckdb_mb_gpu_append_null", "duckdb_mb_gpu_append_date",
     "duckdb_mb_gpu_append_timestamp", "duckdb_mb_gpu_end_row", "duckdb_mb_gpu_append_blob", "duckdb_mb_gpu_append_decimal",
     "duckdb_mb_gpu_append_list_varchar", "duckdb_mb_gpu_append_struct_varchar", "duckdb_mb_gpu_append_map_varchar_varchar",
-    "duckdb_mb_gpu_append_interval", "duckdb_mb_gpu_appender_set_decimal",
+    "duckdb_mb_gpu_append_interval", "duckdb_mb_gpu_appender_set_decimal", "duckdb_mb_gpu_appender_set_list",
+    "duckdb_mb_gpu_appender_list_child",
 ]
 
 _lib = None
@@ -233,6 +242,12 @@ def lib():
     L.dmb_dev_rev_fixed_batch.argtypes = [vp, vp, i32, i64, vp]
     L.dmb_dev_rev_string_batch.restype = i32
     L.dmb_dev_rev_string_batch.argtypes = [C.POINTER(RevStringJob), i64, vp]
+    L.dmb_dev_rev_list_batch.restype = i32
+    L.dmb_dev_rev_list_batch.argtypes = [C.POINTER(RevListJob), i64, vp]
+    L.dmb_rev_list_cut.restype = i64
+    L.dmb_rev_list_cut.argtypes = [vp, i32, i64, i64, i64, i64]
+    L.duckdb_mb_gpu_appender_list_child.restype = i32
+    L.duckdb_mb_gpu_appender_list_child.argtypes = [vp, i32, C.POINTER(vp), C.POINTER(vp), C.POINTER(u64)]
     L.duckdb_mb_gpu_device_count.restype = i32
     L.duckdb_mb_gpu_ctx_create.restype = vp
     L.duckdb_mb_gpu_ctx_create.argtypes = [i32]
@@ -335,6 +350,7 @@ def lib():
                         ("append_date", [i32]), ("append_timestamp", [i64]), ("end_row", []),
                         ("append_blob", [C.c_char_p, i32]), ("append_decimal", [i32, i32, i64, i64]),
                         ("append_interval", [i32, i32, i64]), ("appender_set_decimal", [i32, i32, i32]),
+                        ("appender_set_list", [i32, i32, i32, i32]),
                         ("append_list_varchar", [vp, vp, i32]), ("append_struct_varchar", [vp, vp, vp, vp, i32]),
                         ("append_map_varchar_varchar", [vp, vp, vp, vp, i32])):
         f = getattr(L, "duckdb_mb_gpu_" + name)

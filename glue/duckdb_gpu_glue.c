@@ -299,10 +299,12 @@ duckdb_mb_stream *duckdb_mb_query_stream(duckdb_mb_connection *handle, moonbit_b
  * per finished 2048-row chunk; the sink fills a duckdb_data_chunk and appends it (the bulk door, :2109-2132). */
 typedef struct {
   duckdb_appender appender;
+  duckdb_mb_appender *lib; /* the library's handle: LIST children are read through it during a sink call */
   int32_t ncols;
   duckdb_logical_type *types;
   int32_t *type_ids;
   int32_t *widths;
+  int32_t *child_type_ids, *child_widths; /* LIST columns */
   duckdb_data_chunk chunk; /* reused: duckdb_append_data_chunk copies */
 } glue_sink;
 
@@ -313,8 +315,29 @@ static int32_t vector_width(duckdb_logical_type lt) {
     case DUCKDB_TYPE_SMALLINT: case DUCKDB_TYPE_USMALLINT: return 2;
     case DUCKDB_TYPE_INTEGER: case DUCKDB_TYPE_UINTEGER: case DUCKDB_TYPE_FLOAT: case DUCKDB_TYPE_DATE: return 4;
     case DUCKDB_TYPE_DECIMAL: { const int w = duckdb_decimal_width(lt); return w <= 4 ? 2 : w <= 9 ? 4 : w <= 18 ? 8 : 16; }
-    case DUCKDB_TYPE_VARCHAR: case DUCKDB_TYPE_BLOB: case DUCKDB_TYPE_INTERVAL: case DUCKDB_TYPE_HUGEINT: case DUCKDB_TYPE_UHUGEINT: case DUCKDB_TYPE_UUID: return 16;
+    case DUCKDB_TYPE_VARCHAR: case DUCKDB_TYPE_BLOB: case DUCKDB_TYPE_INTERVAL: case DUCKDB_TYPE_HUGEINT: case DUCKDB_TYPE_UHUGEINT: case DUCKDB_TYPE_UUID:
+    case DUCKDB_TYPE_LIST: return 16; /* LIST: duckdb_list_entry */
     default: return 8;
+  }
+}
+
+/* `count` rows of values + mask into vector v */
+static void fill_vector(duckdb_vector v, int32_t type_id, int32_t width, uint64_t count, const void *data, const uint64_t *mask) {
+  const int is_str = type_id == DUCKDB_TYPE_VARCHAR || type_id == DUCKDB_TYPE_BLOB;
+  if (!is_str) {
+    if (count) memcpy(duckdb_vector_get_data(v), data, (size_t)count * (size_t)width);
+  } else { /* the vector must own its strings: inlined entries are copied as they are, pointer entries assigned */
+    const dmb_string_t *e = (const dmb_string_t *)data;
+    dmb_string_t *out = (dmb_string_t *)duckdb_vector_get_data(v);
+    for (uint64_t i = 0; i < count; i++) {
+      if (mask && !((mask[i >> 6] >> (i & 63)) & 1ull)) continue;
+      if (e[i].length <= 12) out[i] = e[i];
+      else duckdb_vector_assign_string_element_len(v, i, (const char *)(uintptr_t)e[i].tail.ptr, e[i].length);
+    }
+  }
+  if (mask) {
+    duckdb_vector_ensure_validity_writable(v);
+    memcpy(duckdb_vector_get_validity(v), mask, 8 * (((size_t)count + 63) / 64));
   }
 }
 
@@ -323,22 +346,17 @@ static int32_t sink_chunk(void *user, int32_t ncols, uint32_t count, const void 
   if (ncols != s->ncols) return 0;
   for (int32_t c = 0; c < ncols; c++) {
     duckdb_vector v = duckdb_data_chunk_get_vector(s->chunk, (idx_t)c);
-    const uint64_t *mask = vec_validity[c];
-    const int is_str = s->type_ids[c] == DUCKDB_TYPE_VARCHAR || s->type_ids[c] == DUCKDB_TYPE_BLOB;
-    if (!is_str) {
-      memcpy(duckdb_vector_get_data(v), vec_data[c], (size_t)count * (size_t)s->widths[c]);
-    } else { /* the vector must own its strings: inlined entries are copied as they are, pointer entries assigned */
-      const dmb_string_t *e = (const dmb_string_t *)vec_data[c];
-      dmb_string_t *out = (dmb_string_t *)duckdb_vector_get_data(v);
-      for (uint32_t i = 0; i < count; i++) {
-        if (mask && !((mask[i >> 6] >> (i & 63)) & 1ull)) continue;
-        if (e[i].length <= 12) out[i] = e[i];
-        else duckdb_vector_assign_string_element_len(v, i, (const char *)(uintptr_t)e[i].tail.ptr, e[i].length);
-      }
-    }
-    if (mask) {
-      duckdb_vector_ensure_validity_writable(v);
-      memcpy(duckdb_vector_get_validity(v), mask, 8 * (((size_t)count + 63) / 64));
+    fill_vector(v, s->type_ids[c], s->widths[c], count, vec_data[c], vec_validity[c]);
+    if (s->type_ids[c] == DUCKDB_TYPE_LIST) { /* the entries index this chunk's own child vector */
+      const void *cdata = NULL;
+      const uint64_t *cmask = NULL;
+      uint64_t size = 0;
+      if (!duckdb_mb_gpu_appender_list_child(s->lib, c, &cdata, &cmask, &size)) return 0;
+      /* every call sets the size: the chunk is reused; the child is fetched after reserve, which may reallocate it */
+      if (duckdb_list_vector_reserve(v, (idx_t)size) != DuckDBSuccess || duckdb_list_vector_set_size(v, (idx_t)size) != DuckDBSuccess) return 0;
+      duckdb_vector child = duckdb_list_vector_get_child(v);
+      if (!child) return 0;
+      fill_vector(child, s->child_type_ids[c], s->child_widths[c], size, cdata, cmask);
     }
   }
   duckdb_data_chunk_set_size(s->chunk, count);
@@ -353,7 +371,7 @@ static void sink_destroy(void *user) {
   if (s->chunk) duckdb_destroy_data_chunk(&s->chunk);
   for (int32_t c = 0; c < s->ncols; c++) duckdb_destroy_logical_type(&s->types[c]);
   if (s->appender) duckdb_appender_destroy(&s->appender); /* (flushes what is left, like the reference's destroy :1083-1091) */
-  free(s->types); free(s->type_ids); free(s->widths); free(s);
+  free(s->types); free(s->type_ids); free(s->widths); free(s->child_type_ids); free(s->child_widths); free(s);
 }
 
 /* src/duckdb_native.c:1032-1081: NULL on failure (the reference sets no global error here either) */
@@ -376,6 +394,8 @@ duckdb_mb_appender *duckdb_mb_appender_create(duckdb_mb_connection *handle, moon
   s->types = (duckdb_logical_type *)calloc(nc, sizeof(duckdb_logical_type));
   s->type_ids = (int32_t *)calloc(nc, sizeof(int32_t));
   s->widths = (int32_t *)calloc(nc, sizeof(int32_t));
+  s->child_type_ids = (int32_t *)calloc(nc, sizeof(int32_t));
+  s->child_widths = (int32_t *)calloc(nc, sizeof(int32_t));
   for (int32_t c = 0; c < s->ncols; c++) {
     s->types[c] = duckdb_appender_column_type(s->appender, (idx_t)c);
     s->type_ids[c] = (int32_t)duckdb_get_type_id(s->types[c]);
@@ -384,10 +404,22 @@ duckdb_mb_appender *duckdb_mb_appender_create(duckdb_mb_connection *handle, moon
   s->chunk = duckdb_create_data_chunk(s->types, (idx_t)s->ncols);
   duckdb_mb_appender *a = duckdb_mb_gpu_appender_create(ctx, s->ncols, s->type_ids, sink_chunk, s);
   if (!a) { sink_destroy(s); return NULL; }
+  s->lib = a;
   duckdb_mb_gpu_appender_set_hooks(a, sink_flush, sink_destroy);
-  for (int32_t c = 0; c < s->ncols; c++)
+  for (int32_t c = 0; c < s->ncols; c++) {
     if (s->type_ids[c] == DUCKDB_TYPE_DECIMAL)
       duckdb_mb_gpu_appender_set_decimal(a, c, duckdb_decimal_width(s->types[c]), duckdb_decimal_scale(s->types[c]));
+    if (s->type_ids[c] == DUCKDB_TYPE_LIST) {
+      /* a child type the library refuses (LIST, STRUCT, ...) leaves the column undeclared: Arrow batches for it fail */
+      duckdb_logical_type child = duckdb_list_type_child_type(s->types[c]);
+      const duckdb_type ct = duckdb_get_type_id(child);
+      s->child_type_ids[c] = (int32_t)ct;
+      s->child_widths[c] = vector_width(child);
+      duckdb_mb_gpu_appender_set_list(a, c, (int32_t)ct, ct == DUCKDB_TYPE_DECIMAL ? duckdb_decimal_width(child) : 0,
+                                      ct == DUCKDB_TYPE_DECIMAL ? duckdb_decimal_scale(child) : 0);
+      duckdb_destroy_logical_type(&child);
+    }
+  }
   return a;
 }
 

@@ -74,6 +74,8 @@ void duckdb_vector_ensure_validity_writable(duckdb_vector vector);
 void duckdb_vector_assign_string_element_len(duckdb_vector vector, idx_t index, const char *str, idx_t str_len);
 duckdb_vector duckdb_list_vector_get_child(duckdb_vector vector);
 idx_t duckdb_list_vector_get_size(duckdb_vector vector);
+duckdb_state duckdb_list_vector_reserve(duckdb_vector vector, idx_t required_capacity);
+duckdb_state duckdb_list_vector_set_size(duckdb_vector vector, idx_t size);
 
 duckdb_type duckdb_get_type_id(duckdb_logical_type type);
 uint8_t duckdb_decimal_width(duckdb_logical_type type);

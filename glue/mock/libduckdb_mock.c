@@ -42,7 +42,11 @@ typedef struct mock_table {
 
 static mock_table *g_tables = NULL;
 
-typedef struct { int32_t type_id, dec_width, dec_scale, internal; const duckdb_mock_column *col; } mock_ltype;
+typedef struct {
+  int32_t type_id, dec_width, dec_scale, internal;
+  const duckdb_mock_column *col;                   /* served columns */
+  int32_t child_type_id, child_dec_width, child_dec_scale;  /* appender LIST columns */
+} mock_ltype;
 typedef struct { const mock_table *t; int64_t next_chunk; char error[128]; } mock_result;
 typedef struct mock_vec {
   const duckdb_mock_column *col;  /* served vector */
@@ -55,6 +59,8 @@ typedef struct mock_vec {
   uint8_t *buf;
   uint64_t *mask;
   char **strs;  /* owned copies of assigned strings */
+  idx_t cap;    /* rows buf holds: MOCK_VECTOR_SIZE, or a LIST child's reserved size */
+  idx_t list_size;
 } mock_vec;
 typedef struct { const mock_table *t; int64_t k; int32_t ncols; mock_vec *vecs; mock_vec *children; idx_t size; int created; } mock_chunk;
 
@@ -151,7 +157,8 @@ duckdb_vector duckdb_data_chunk_get_vector(duckdb_data_chunk chunk, idx_t col_id
 static void free_created_vec(mock_vec *v) {
   if (!v->created) return;
   free(v->buf); free(v->mask);
-  if (v->strs) { for (int i = 0; i < MOCK_VECTOR_SIZE; i++) free(v->strs[i]); free(v->strs); }
+  if (v->strs) { for (idx_t i = 0; i < v->cap; i++) free(v->strs[i]); free(v->strs); }
+  if (v->child) { free_created_vec(v->child); free(v->child); }
 }
 void duckdb_destroy_data_chunk(duckdb_data_chunk *chunk) {
   if (!chunk || !*chunk) return;
@@ -173,10 +180,12 @@ uint64_t *duckdb_vector_get_validity(duckdb_vector vector) {
 }
 duckdb_vector duckdb_list_vector_get_child(duckdb_vector vector) {
   mock_vec *v = (mock_vec *)vector;
-  return (v && !v->created && !v->is_child && v->col->child_data) ? (duckdb_vector)v->child : NULL;
+  if (v && v->created) return (duckdb_vector)v->child;
+  return (v && !v->is_child && v->col->child_data) ? (duckdb_vector)v->child : NULL;
 }
 idx_t duckdb_list_vector_get_size(duckdb_vector vector) {
   mock_vec *v = (mock_vec *)vector;
+  if (v->created) return v->list_size;
   return v->col->child_sizes ? v->col->child_sizes[v->chunk] : 0;
 }
 
@@ -192,7 +201,12 @@ duckdb_type duckdb_enum_internal_type(duckdb_logical_type type) {
 uint32_t duckdb_enum_dictionary_size(duckdb_logical_type type) { return ((mock_ltype *)type)->col->dict_size; }
 char *duckdb_enum_dictionary_value(duckdb_logical_type type, idx_t index) { return strdup(((mock_ltype *)type)->col->dict_values[index]); }
 duckdb_logical_type duckdb_list_type_child_type(duckdb_logical_type type) {
-  const duckdb_mock_column *c = ((mock_ltype *)type)->col;
+  const mock_ltype *t = (const mock_ltype *)type;
+  if (!t->col) { /* an appender column's type */
+    if (t->child_type_id == DUCKDB_TYPE_DECIMAL) return duckdb_create_decimal_type((uint8_t)t->child_dec_width, (uint8_t)t->child_dec_scale);
+    return duckdb_create_logical_type((duckdb_type)t->child_type_id);
+  }
+  const duckdb_mock_column *c = t->col;
   mock_ltype *lt = (mock_ltype *)calloc(1, sizeof(mock_ltype));
   lt->type_id = c->child_type_id; lt->internal = internal_of_width(c->child_width); lt->col = c;
   return (duckdb_logical_type)lt;
@@ -212,8 +226,16 @@ void duckdb_destroy_logical_type(duckdb_logical_type *type) { if (type && *type)
 void duckdb_free(void *ptr) { free(ptr); }
 
 /* ---- appender side: a "table" = its column types + every chunk that was appended */
-typedef struct { int32_t type_id, dec_width, dec_scale; } mock_coltype;
-typedef struct appended_chunk { idx_t size; uint8_t **data; uint64_t **mask; struct appended_chunk *next; } appended_chunk;
+typedef struct { int32_t type_id, dec_width, dec_scale, child_type_id, child_dec_width, child_dec_scale; } mock_coltype;
+typedef struct appended_chunk {
+  idx_t size;
+  uint8_t **data;
+  uint64_t **mask;
+  uint8_t **child_data;  /* LIST columns: the chunk's child vector */
+  uint64_t **child_mask;
+  idx_t *child_size;
+  struct appended_chunk *next;
+} appended_chunk;
 typedef struct mock_append_table {
   char *schema, *table;
   int32_t ncols;
@@ -241,13 +263,21 @@ static mock_append_table *find_append_table(const char *table) {
     if (strcmp(t->table, table) == 0) return t;
   return NULL;
 }
+/* the child type of a registered LIST column (what duckdb_list_type_child_type reports for it) */
+int32_t duckdb_mock_set_append_list_child(const char *table, int32_t col, int32_t child_type, int32_t dec_width, int32_t dec_scale) {
+  mock_append_table *t = find_append_table(table);
+  if (!t || col < 0 || col >= t->ncols) return 0;
+  t->types[col].child_type_id = child_type; t->types[col].child_dec_width = dec_width; t->types[col].child_dec_scale = dec_scale;
+  return 1;
+}
 static int type_width(int32_t type_id, int32_t dec_width) {
   switch (type_id) {
     case DUCKDB_TYPE_BOOLEAN: case DUCKDB_TYPE_TINYINT: case DUCKDB_TYPE_UTINYINT: return 1;
     case DUCKDB_TYPE_SMALLINT: case DUCKDB_TYPE_USMALLINT: return 2;
     case DUCKDB_TYPE_INTEGER: case DUCKDB_TYPE_UINTEGER: case DUCKDB_TYPE_FLOAT: case DUCKDB_TYPE_DATE: return 4;
     case DUCKDB_TYPE_DECIMAL: return dec_width <= 4 ? 2 : dec_width <= 9 ? 4 : dec_width <= 18 ? 8 : 16;
-    case DUCKDB_TYPE_VARCHAR: case DUCKDB_TYPE_BLOB: case DUCKDB_TYPE_INTERVAL: case DUCKDB_TYPE_HUGEINT: case DUCKDB_TYPE_UHUGEINT: case DUCKDB_TYPE_UUID: return 16;
+    case DUCKDB_TYPE_VARCHAR: case DUCKDB_TYPE_BLOB: case DUCKDB_TYPE_INTERVAL: case DUCKDB_TYPE_HUGEINT: case DUCKDB_TYPE_UHUGEINT: case DUCKDB_TYPE_UUID:
+    case DUCKDB_TYPE_LIST: return 16;
     default: return 8;
   }
 }
@@ -265,7 +295,9 @@ duckdb_logical_type duckdb_appender_column_type(duckdb_appender appender, idx_t 
   if (!a || !a->t || col_idx >= (idx_t)a->t->ncols) return NULL;
   const mock_coltype *ct = &a->t->types[col_idx];
   if (ct->type_id == DUCKDB_TYPE_DECIMAL) return duckdb_create_decimal_type((uint8_t)ct->dec_width, (uint8_t)ct->dec_scale);
-  return duckdb_create_logical_type((duckdb_type)ct->type_id);
+  mock_ltype *lt = (mock_ltype *)duckdb_create_logical_type((duckdb_type)ct->type_id);
+  lt->child_type_id = ct->child_type_id; lt->child_dec_width = ct->child_dec_width; lt->child_dec_scale = ct->child_dec_scale;
+  return (duckdb_logical_type)lt;
 }
 const char *duckdb_appender_error(duckdb_appender appender) { mock_appender *a = (mock_appender *)appender; return a && a->error[0] ? a->error : NULL; }
 duckdb_state duckdb_appender_flush(duckdb_appender appender) { mock_appender *a = (mock_appender *)appender; if (!a || !a->t) return DuckDBError; a->t->flushes++; return DuckDBSuccess; }
@@ -279,23 +311,61 @@ duckdb_data_chunk duckdb_create_data_chunk(duckdb_logical_type *types, idx_t col
     mock_vec *v = &ch->vecs[c];
     v->created = 1;
     v->ltype = *(mock_ltype *)types[c];
+    v->cap = MOCK_VECTOR_SIZE;
     v->buf = (uint8_t *)calloc(MOCK_VECTOR_SIZE, (size_t)type_width(v->ltype.type_id, v->ltype.dec_width));
+    if (v->ltype.type_id == DUCKDB_TYPE_LIST) { /* an empty child vector, grown by duckdb_list_vector_reserve */
+      v->child = (mock_vec *)calloc(1, sizeof(mock_vec));
+      v->child->created = 1;
+      v->child->is_child = 1;
+      v->child->ltype.type_id = v->ltype.child_type_id;
+      v->child->ltype.dec_width = v->ltype.child_dec_width;
+      v->child->ltype.dec_scale = v->ltype.child_dec_scale;
+    }
   }
   return (duckdb_data_chunk)ch;
+}
+duckdb_state duckdb_list_vector_reserve(duckdb_vector vector, idx_t required_capacity) {
+  mock_vec *v = (mock_vec *)vector;
+  if (!v || !v->created || !v->child) return DuckDBError;
+  mock_vec *c = v->child;
+  if (required_capacity <= c->cap) return DuckDBSuccess;
+  idx_t cap = c->cap * 2 > required_capacity ? c->cap * 2 : required_capacity;
+  const size_t w = (size_t)type_width(c->ltype.type_id, c->ltype.dec_width);
+  c->buf = (uint8_t *)realloc(c->buf, cap * w);
+  memset(c->buf + c->cap * w, 0, (cap - c->cap) * w);
+  if (c->mask) { /* new rows are valid */
+    const size_t old_words = (c->cap + 63) / 64, words = (cap + 63) / 64;
+    c->mask = (uint64_t *)realloc(c->mask, 8 * words);
+    memset(c->mask + old_words, 0xff, 8 * (words - old_words));
+    if (c->cap & 63) c->mask[old_words - 1] |= ~0ull << (c->cap & 63);
+  }
+  if (c->strs) { c->strs = (char **)realloc(c->strs, cap * sizeof(char *)); memset(c->strs + c->cap, 0, (cap - c->cap) * sizeof(char *)); }
+  c->cap = cap;
+  return DuckDBSuccess;
+}
+duckdb_state duckdb_list_vector_set_size(duckdb_vector vector, idx_t size) {
+  mock_vec *v = (mock_vec *)vector;
+  if (!v || !v->created || !v->child || size > v->child->cap) return DuckDBError;
+  v->list_size = size;
+  return DuckDBSuccess;
 }
 void duckdb_data_chunk_set_size(duckdb_data_chunk chunk, idx_t size) { ((mock_chunk *)chunk)->size = size; }
 void duckdb_vector_ensure_validity_writable(duckdb_vector vector) {
   mock_vec *v = (mock_vec *)vector;
-  if (v->created && !v->mask) { v->mask = (uint64_t *)malloc(8 * (MOCK_VECTOR_SIZE / 64)); memset(v->mask, 0xff, 8 * (MOCK_VECTOR_SIZE / 64)); }
+  if (v->created && !v->mask) {
+    const size_t words = v->cap ? (v->cap + 63) / 64 : 1;
+    v->mask = (uint64_t *)malloc(8 * words);
+    memset(v->mask, 0xff, 8 * words);
+  }
 }
 void duckdb_vector_assign_string_element_len(duckdb_vector vector, idx_t index, const char *str, idx_t str_len) {
   mock_vec *v = (mock_vec *)vector;
-  if (!v->created || index >= MOCK_VECTOR_SIZE) return;
+  if (!v->created || index >= v->cap) return;
   duckdb_string_t *e = (duckdb_string_t *)v->buf + index;
   memset(e, 0, sizeof(*e));
   e->value.inlined.length = (uint32_t)str_len;
   if (str_len <= 12) { memcpy(e->value.inlined.inlined, str, str_len); return; }
-  if (!v->strs) v->strs = (char **)calloc(MOCK_VECTOR_SIZE, sizeof(char *));
+  if (!v->strs) v->strs = (char **)calloc(v->cap, sizeof(char *));
   free(v->strs[index]);
   v->strs[index] = (char *)malloc(str_len);
   memcpy(v->strs[index], str, str_len);
@@ -310,6 +380,9 @@ duckdb_state duckdb_append_data_chunk(duckdb_appender appender, duckdb_data_chun
   ac->size = ch->size;
   ac->data = (uint8_t **)calloc((size_t)ch->ncols, sizeof(uint8_t *));
   ac->mask = (uint64_t **)calloc((size_t)ch->ncols, sizeof(uint64_t *));
+  ac->child_data = (uint8_t **)calloc((size_t)ch->ncols, sizeof(uint8_t *));
+  ac->child_mask = (uint64_t **)calloc((size_t)ch->ncols, sizeof(uint64_t *));
+  ac->child_size = (idx_t *)calloc((size_t)ch->ncols, sizeof(idx_t));
   for (int32_t c = 0; c < ch->ncols; c++) {
     mock_vec *v = &ch->vecs[c];
     const int w = type_width(a->t->types[c].type_id, a->t->types[c].dec_width);
@@ -325,6 +398,26 @@ duckdb_state duckdb_append_data_chunk(duckdb_appender appender, duckdb_data_chun
           char *copy = (char *)malloc(e[i].value.pointer.length);
           memcpy(copy, e[i].value.pointer.ptr, e[i].value.pointer.length);
           e[i].value.pointer.ptr = copy; /* (leaked with the table: test process) */
+        }
+      }
+    }
+    if (v->child) { /* LIST: the child vector, its first list_size rows */
+      const mock_vec *cv = v->child;
+      const idx_t size = v->list_size;
+      const size_t cw = (size_t)type_width(cv->ltype.type_id, cv->ltype.dec_width), words = (size + 63) / 64;
+      ac->child_size[c] = size;
+      ac->child_data[c] = (uint8_t *)malloc(size * cw + 1);
+      if (size) memcpy(ac->child_data[c], cv->buf, size * cw);
+      if (cv->mask) { ac->child_mask[c] = (uint64_t *)malloc(8 * words + 8); memcpy(ac->child_mask[c], cv->mask, 8 * words); }
+      if (cv->ltype.type_id == DUCKDB_TYPE_VARCHAR || cv->ltype.type_id == DUCKDB_TYPE_BLOB) {
+        duckdb_string_t *e = (duckdb_string_t *)ac->child_data[c];
+        for (idx_t i = 0; i < size; i++) {
+          if (ac->child_mask[c] && !((ac->child_mask[c][i >> 6] >> (i & 63)) & 1ull)) continue;
+          if (e[i].value.inlined.length > 12) {
+            char *copy = (char *)malloc(e[i].value.pointer.length);
+            memcpy(copy, e[i].value.pointer.ptr, e[i].value.pointer.length);
+            e[i].value.pointer.ptr = copy;
+          }
         }
       }
     }
@@ -350,4 +443,15 @@ int64_t duckdb_mock_appended_chunk(const char *table, int64_t k, int32_t col, co
   *data = ac->data[col];
   *mask = ac->mask[col];
   return (int64_t)ac->size;
+}
+/* chunk k, LIST column col: the child vector's values / mask pointers (mask NULL = all valid); returns the child size */
+int64_t duckdb_mock_appended_list_child(const char *table, int64_t k, int32_t col, const void **data, const uint64_t **mask) {
+  mock_append_table *t = find_append_table(table);
+  if (!t) return -1;
+  appended_chunk *ac = t->head;
+  for (int64_t i = 0; ac && i < k; i++) ac = ac->next;
+  if (!ac || col < 0 || col >= t->ncols || !ac->child_data[col]) return -1;
+  *data = ac->child_data[col];
+  *mask = ac->child_mask[col];
+  return (int64_t)ac->child_size[col];
 }

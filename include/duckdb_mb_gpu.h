@@ -379,6 +379,36 @@ typedef struct dmb_rev_string_job {
 
 int32_t dmb_dev_rev_string_batch(const dmb_rev_string_job *job, int64_t nrows, void *stream);
 
+/* Arrow list / large_list -> LIST vectors.  Row r of the slice gets duckdb_list_entry {off[r] - off[c0], off[r+1] - off[r]}
+ * (c0: the first row of r's 2048-row chunk), so each chunk's entries index that chunk's own child vector; a NULL row gets
+ * {off[r] - off[c0], 0}: DuckDB never sees a NULL row that owns elements.  The child values of the slice, Arrow elements
+ * [off[0], off[nrows]), are converted as a dense column by dmb_dev_rev_fixed_batch / dmb_dev_rev_string_batch; this
+ * kernel writes the entries, the list masks and each chunk's child mask, realigned to start at bit 0 of that chunk's
+ * first element. */
+typedef struct dmb_rev_list_job {
+  const void *in_offsets;          /* int32 (or int64 when large) offsets at the slice start: nrows + 1 entries  */
+  const uint8_t *in_validity;      /* list bitmap or NULL                                                       */
+  int64_t in_bit_offset;
+  const uint8_t *in_child_validity;  /* child bitmap or NULL                                                    */
+  int64_t child_bit_offset;        /* bit of element off[0]: child array offset + off[0]                        */
+  const int64_t *child_word;       /* [nchunks + 1]: chunk k's child mask starts at out_child_validity[child_word[k]] */
+  void *out_entries;               /* duckdb_list_entry slab: chunk k at k*2048 entries                         */
+  uint64_t *out_validity;          /* list mask slab: chunk k at k*32 words                                     */
+  uint64_t *out_child_validity;    /* ceil(size_k / 64) words per chunk, bits past size_k are 0                 */
+  unsigned long long *null_count;
+  unsigned int *error;             /* |= 1: a row with off[r+1] < off[r]                                       */
+  int32_t large_offsets;
+  int32_t reserved;
+} dmb_rev_list_job;
+
+int32_t dmb_dev_rev_list_batch(const dmb_rev_list_job *job, int64_t nrows, void *stream);
+/* the appender's sub-batch cut (host only): the end chunk (exclusive) of the sub-batch that starts at chunk k0.  It takes
+ * at most max_chunks chunks, and stops before the chunk that would give any of the nlists LIST columns more than
+ * child_cap child elements; the first chunk is always taken, so one chunk's child range is never split.
+ * bounds[l][k]: list l's Arrow offset at row 2048k (at the last row for k = nchunks). */
+int64_t dmb_rev_list_cut(const int64_t *const *bounds, int32_t nlists, int64_t nchunks, int64_t k0, int64_t max_chunks,
+                         int64_t child_cap);
+
 /* byte-per-row validity (MoonBit Array[Bool], src/duckdb_arrow_native.mbt:646-650) -> per-chunk
  * uint64 masks via warp ballots */
 int32_t dmb_dev_valid_bytes_to_masks(const uint8_t *valid_bytes, uint64_t *out_validity,
@@ -728,6 +758,19 @@ int32_t duckdb_mb_gpu_append_blob(duckdb_mb_gpu_appender *a, const uint8_t *byte
  * first value; values of another scale are cast like DuckDB's decimal -> decimal cast, out-of-range is an error. */
 int32_t duckdb_mb_gpu_appender_set_decimal(duckdb_mb_gpu_appender *a, int32_t col, int32_t width, int32_t scale);
 int32_t duckdb_mb_gpu_append_decimal(duckdb_mb_gpu_appender *a, int32_t width, int32_t scale, int64_t lower, int64_t upper);
+/* LIST columns take Arrow list / large_list arrays through duckdb_mb_gpu_append_arrow_batch.  The table's child type
+ * (duckdb_list_type_child_type of duckdb_appender_column_type) is declared first: the Arrow child format alone does not
+ * say it (`tsu:` is TIMESTAMP or TIMESTAMP_TZ, `L` UBIGINT or TIME_TZ).  Children: the types the reverse path converts
+ * (not INTERVAL or ENUM), VARCHAR and BLOB; LIST, STRUCT and MAP children are refused.  The row protocol refuses a
+ * table with a LIST column. */
+int32_t duckdb_mb_gpu_appender_set_list(duckdb_mb_gpu_appender *a, int32_t col, int32_t child_type_id, int32_t child_dec_width,
+                                        int32_t child_dec_scale);
+/* Only inside a dmb_chunk_sink call, for the chunk being handed over: LIST column `col`'s child vector.  vec_data[col] /
+ * vec_validity[col] of that call are the duckdb_list_entry vector and the list mask; the entries index this child.
+ * `*data`: `*size` values in DuckDB vector layout (string_t for VARCHAR / BLOB, pointers into the Arrow data buffer),
+ * `*validity`: ceil(size / 64) mask words.  Host memory of the appender, valid until the sink call returns. */
+int32_t duckdb_mb_gpu_appender_list_child(duckdb_mb_gpu_appender *a, int32_t col, const void **data, const uint64_t **validity,
+                                          uint64_t *size);
 int32_t duckdb_mb_gpu_append_interval(duckdb_mb_gpu_appender *a, int32_t months, int32_t days, int64_t micros); /* :1511 */
 /* LIST / STRUCT / MAP cells: the reference serialises them as text -- `["a", "b"]` (:1735-1790), `{"k": "v", ...}`
  * (:1792-1858 struct, :1860-1926 map), items copied without escaping -- and appends the text as one VARCHAR cell

@@ -42,7 +42,8 @@ _CHILD_DTYPE = {ch.P_BOOL: np.uint8, ch.P_I8: np.int8, ch.P_I16: np.int16, ch.P_
 class CollectedChunks:
     """Default sink: copies every chunk out of the appender's pinned buffers.
 
-    `list_children` maps a LIST column to its child type, `(child_type_id, child_dec_width)`; for those columns the
+    `dec_widths`: per column, the table's DECIMAL width (what `Appender.set_decimal` declares), which sets the vector's
+    physical width; the Arrow precision does not.  `list_children` maps a LIST column to its child type, `(child_type_id, child_dec_width)`; for those columns the
     chunk's child vector is copied too (through Appender.list_child, valid only inside the sink call)."""
 
     def __init__(self, type_ids: Sequence[int], dec_widths: Optional[Sequence[int]] = None, list_children: Optional[dict] = None):
@@ -196,7 +197,9 @@ class Appender:
         self._check(self.lib.duckdb_mb_gpu_append_blob(self.handle, data, len(data)), "append_blob")
 
     def set_decimal(self, col: int, width: int, scale: int):
-        """The table column's DECIMAL(width, scale) (what duckdb_appender_column_type reports)."""
+        """The table column's DECIMAL(width, scale) (what duckdb_appender_column_type reports).  Arrow batches are
+        converted to this width and must carry decimal128 at this scale with a precision <= width; without a declaration
+        the first Arrow batch (or row-API value) declares it."""
         self._check(self.lib.duckdb_mb_gpu_appender_set_decimal(self.handle, int(col), int(width), int(scale)), "set_decimal")
 
     def set_list(self, col: int, child_type: int, dec_width: int = 0, dec_scale: int = 0):

@@ -32,7 +32,9 @@ enum { kNotCreated = 0, kReady = 1, kRowInProgress = 2, kFlushed = 3, kClosed = 
 
 struct RowBuf {  // one column of buffered rows (row API)
   int width = 0;               // bytes per value; 0: string
-  int dec_prec = 0, dec_scale = 0;  // DECIMAL: the table column's precision / scale (0: not declared yet); values buffered as int128
+  // DECIMAL: the table column's width / scale (duckdb_mb_gpu_appender_set_decimal; 0: not declared yet, the first
+  // DECIMAL cell or Arrow batch declares it); values buffered as int128.  Arrow batches narrow to this width too.
+  int32_t dec_prec = 0, dec_scale = 0;
   std::vector<uint8_t> values, valid;
   std::vector<int32_t> offsets;  // strings: n+1 entries
   std::vector<uint8_t> data;
@@ -142,8 +144,58 @@ int copy_op(int w) {
   }
 }
 
-// Arrow format string of a child -> conversion for a DuckDB column of `type_id`
-bool map_format(App *a, int c, const char *fmt, int32_t type_id, ColInput *in) {
+// An Arrow decimal `fmt` ("d:p,s" or "d:p,s,bits") into a column of DuckDB DECIMAL(*w, *s); HUGEINT is DECIMAL(38, 0).
+// The values must be decimal128 with the column's scale and a precision that fits its width; they are narrowed to the
+// column's physical width (int16 / int32 / int64 / int128 for w <= 4 / 9 / 18 / 38), which keeps every value within
+// the Arrow precision exact.  *w == 0: the column is not declared yet, and this Arrow type declares it.
+bool map_decimal(App *a, int c, const char *what, const char *fmt, int32_t type_id, int32_t *w, int32_t *s, ColInput *in) {
+  // d:p,s[,bits]: each field one to three decimal digits, nothing else
+  long f[3] = {0, 0, 128};
+  int nf = 0;
+  const char *q = fmt + 2;
+  for (; nf < 3; ++nf) {
+    int digits = 0;
+    for (f[nf] = 0; *q >= '0' && *q <= '9' && digits < 3; ++q, ++digits) f[nf] = 10 * f[nf] + (*q - '0');
+    if (!digits || (*q != ',' && *q != '\0')) break;
+    if (*q++ == '\0') { ++nf; break; }
+  }
+  const long p = f[0], sc = f[1], bits = f[2];
+  char col[32];
+  if (type_id == DMB_TYPE_HUGEINT) snprintf(col, sizeof(col), "HUGEINT");
+  else if (*w) snprintf(col, sizeof(col), "DECIMAL(%d,%d)", *w, *s);
+  else snprintf(col, sizeof(col), "DECIMAL");
+  if (nf < 2 || q[-1] != '\0') {
+    fail(a, "column %d: Arrow %s '%s' is not a decimal format", c, what, fmt);
+    return false;
+  }
+  if (bits != 128) {
+    fail(a, "column %d: Arrow %s '%s' is a %ld-bit decimal; only decimal128 can be appended to a %s column", c, what, fmt, bits, col);
+    return false;
+  }
+  if (p < 1 || p > 38 || sc > p) {
+    fail(a, "column %d: Arrow %s '%s' is not a DECIMAL(width, scale) DuckDB can store", c, what, fmt);
+    return false;
+  }
+  if (*w == 0) { *w = (int32_t)p; *s = (int32_t)sc; }
+  if (sc != *s) {
+    fail(a, "column %d: Arrow %s '%s' has scale %ld; the column is %s", c, what, fmt, sc, col);
+    return false;
+  }
+  if (p > *w) {
+    fail(a, "column %d: Arrow %s '%s' has precision %ld; the column is %s", c, what, fmt, p, col);
+    return false;
+  }
+  in->w_in = 16;
+  if (*w <= 4) { in->rev_op = DMB_REV_I128_TO_I16; in->w_out = 2; }
+  else if (*w <= 9) { in->rev_op = DMB_REV_I128_TO_I32; in->w_out = 4; }
+  else if (*w <= 18) { in->rev_op = DMB_REV_I128_TO_I64; in->w_out = 8; }
+  else { in->rev_op = DMB_REV_COPY16; in->w_out = 16; }
+  return true;
+}
+
+// Arrow format string of a child -> conversion for a DuckDB column of `type_id`; `dec_w` / `dec_s`: the column's
+// DECIMAL(w, s) when it is one (w == 0: not declared yet, set from the Arrow type)
+bool map_format(App *a, int c, const char *what, const char *fmt, int32_t type_id, int32_t *dec_w, int32_t *dec_s, ColInput *in) {
   auto fixed = [&](int w) { in->rev_op = copy_op(w); in->w_in = w; in->w_out = w; return true; };
   auto is = [&](const char *f) { return strcmp(fmt, f) == 0; };
   auto starts = [&](const char *f) { return strncmp(fmt, f, strlen(f)) == 0; };
@@ -169,19 +221,14 @@ bool map_format(App *a, int c, const char *fmt, int32_t type_id, ColInput *in) {
     case DMB_TYPE_TIMESTAMP_S: if (starts("tss:")) return fixed(8); break;
     case DMB_TYPE_TIMESTAMP_MS: if (starts("tsm:")) return fixed(8); break;
     case DMB_TYPE_TIMESTAMP_NS: if (starts("tsn:")) return fixed(8); break;
-    case DMB_TYPE_HUGEINT: if (starts("d:")) return fixed(16); break;
-    case DMB_TYPE_UHUGEINT: case DMB_TYPE_UUID: if (is("w:16")) return fixed(16); break;
-    case DMB_TYPE_DECIMAL:
-      if (starts("d:")) {  // decimal128 -> the physical width DuckDB uses for this precision
-        int p = atoi(fmt + 2);
-        in->w_in = 16;
-        if (p <= 4) { in->rev_op = DMB_REV_I128_TO_I16; in->w_out = 2; }
-        else if (p <= 9) { in->rev_op = DMB_REV_I128_TO_I32; in->w_out = 4; }
-        else if (p <= 18) { in->rev_op = DMB_REV_I128_TO_I64; in->w_out = 8; }
-        else { in->rev_op = DMB_REV_COPY16; in->w_out = 16; }
-        return true;
+    case DMB_TYPE_HUGEINT:
+      if (starts("d:")) {  // the unscaled integer of a decimal128 with scale 0
+        int32_t w = 38, s = 0;
+        return map_decimal(a, c, what, fmt, type_id, &w, &s, in);
       }
       break;
+    case DMB_TYPE_UHUGEINT: case DMB_TYPE_UUID: if (is("w:16")) return fixed(16); break;
+    case DMB_TYPE_DECIMAL: if (starts("d:")) return map_decimal(a, c, what, fmt, type_id, dec_w, dec_s, in); break;
     case DMB_TYPE_VARCHAR:
       if (is("u") || is("U")) { in->is_string = true; in->large = is("U"); in->w_out = 16; return true; }
       break;
@@ -190,7 +237,7 @@ bool map_format(App *a, int c, const char *fmt, int32_t type_id, ColInput *in) {
       break;
     default: break;
   }
-  fail(a, "column %d: Arrow format '%s' cannot be appended to a column of DuckDB type %d", c, fmt, type_id);
+  fail(a, "column %d: Arrow %s '%s' cannot be appended to a column of DuckDB type %d", c, what, fmt, type_id);
   return false;
 }
 
@@ -709,20 +756,12 @@ bool map_list(App *a, int j, const ArrowArray *arr, const ArrowSchema *sch, ColI
     fail(a, "column %d: LIST<%s> cannot be appended (Arrow child format '%s')", j, nested_name(cfmt), cfmt);
     return false;
   }
-  if (!map_format(a, j, cfmt, d.type_id, child)) {
-    fail(a, "column %d: Arrow list child format '%s' does not match the declared child type %d", j, cfmt, d.type_id);
+  int32_t dec_w = d.dec_width, dec_s = d.dec_scale;  // a DECIMAL child: set_list declared it
+  if (!map_format(a, j, "list child format", cfmt, d.type_id, &dec_w, &dec_s, child)) {
+    const bool decimal_child = d.type_id == DMB_TYPE_DECIMAL || d.type_id == DMB_TYPE_HUGEINT;
+    if (!decimal_child || strncmp(cfmt, "d:", 2) != 0)  // map_decimal's refusal names its own reason
+      fail(a, "column %d: Arrow list child format '%s' does not match the declared child type %d", j, cfmt, d.type_id);
     return false;
-  }
-  if (d.type_id == DMB_TYPE_DECIMAL) {  // the table's DECIMAL(w, s) sets the child vector's width; the scale must agree
-    const char *comma = strchr(cfmt, ',');
-    if (!comma || atoi(comma + 1) != d.dec_scale) {
-      fail(a, "column %d: Arrow list child '%s' does not have the declared scale %d", j, cfmt, d.dec_scale);
-      return false;
-    }
-    if (d.dec_width <= 4) { child->rev_op = DMB_REV_I128_TO_I16; child->w_out = 2; }
-    else if (d.dec_width <= 9) { child->rev_op = DMB_REV_I128_TO_I32; child->w_out = 4; }
-    else if (d.dec_width <= 18) { child->rev_op = DMB_REV_I128_TO_I64; child->w_out = 8; }
-    else { child->rev_op = DMB_REV_COPY16; child->w_out = 16; }
   }
   bind_buffers(*child, carr, carr->offset);
   child->child_len = carr->length;
@@ -817,7 +856,8 @@ extern "C" int32_t duckdb_mb_gpu_append_arrow_batch(duckdb_mb_gpu_appender *a, c
     ColInput &ci = cols[(size_t)j];
     const bool list = a->type_ids[(size_t)j] == DMB_TYPE_LIST;
     if (!ch || !cs || !cs->format ||
-        !(list ? map_list(a, j, ch, cs, &ci, &children[(size_t)j]) : map_format(a, j, cs->format, a->type_ids[(size_t)j], &ci))) {
+        !(list ? map_list(a, j, ch, cs, &ci, &children[(size_t)j])
+               : map_format(a, j, "format", cs->format, a->type_ids[(size_t)j], &a->rows[(size_t)j].dec_prec, &a->rows[(size_t)j].dec_scale, &ci))) {
       if (!a->error[0]) fail(a, "append_arrow_batch: column %d is malformed", j);
       a->state = kError;
       return 0;

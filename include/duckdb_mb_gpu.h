@@ -755,7 +755,10 @@ int32_t duckdb_mb_gpu_append_timestamp(duckdb_mb_gpu_appender *a, int64_t micros
 int32_t duckdb_mb_gpu_append_blob(duckdb_mb_gpu_appender *a, const uint8_t *bytes, int32_t len);    /* :1397 */
 /* DECIMAL from hugeint parts (:1447-1481).  The column's DECIMAL(width, scale) comes from
  * duckdb_mb_gpu_appender_set_decimal (what duckdb_appender_column_type reports) or, failing that, from the
- * first value; values of another scale are cast like DuckDB's decimal -> decimal cast, out-of-range is an error. */
+ * first value; values of another scale are cast like DuckDB's decimal -> decimal cast, out-of-range is an error.
+ * Arrow batches are narrowed to the declared width too: a decimal128 column must have the declared scale and a
+ * precision <= the width (decimal32/64/256 and anything else are refused); an undeclared column takes both from its
+ * first Arrow batch. */
 int32_t duckdb_mb_gpu_appender_set_decimal(duckdb_mb_gpu_appender *a, int32_t col, int32_t width, int32_t scale);
 int32_t duckdb_mb_gpu_append_decimal(duckdb_mb_gpu_appender *a, int32_t width, int32_t scale, int64_t lower, int64_t upper);
 /* LIST columns take Arrow list / large_list arrays through duckdb_mb_gpu_append_arrow_batch.  The table's child type

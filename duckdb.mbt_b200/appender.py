@@ -33,6 +33,16 @@ def _out_width(type_id: int, dec_width: int = 0) -> int:
     return ch.PHYS_WIDTH[ch.phys_of_type(type_id, dec_width)]
 
 
+_ENUM_DTYPE = {ch.T_UTINYINT: np.uint8, ch.T_USMALLINT: np.uint16, ch.T_UINTEGER: np.uint32}
+
+
+def enum_dict(labels):
+    """(EnumDict, keep-alive) of `labels` (str or bytes) in the dmb_enum_dict layout"""
+    offs, data = ch.enum_dict_arrays([x.encode("utf-8") if isinstance(x, str) else bytes(x) for x in labels])
+    d = nat.EnumDict(len(labels), 0, offs.ctypes.data, data.ctypes.data)
+    return d, (offs, data)
+
+
 # numpy dtype of a fixed-width LIST child value, by physical type (128-bit ones are decoded by hand)
 _CHILD_DTYPE = {ch.P_BOOL: np.uint8, ch.P_I8: np.int8, ch.P_I16: np.int16, ch.P_I32: np.int32, ch.P_I64: np.int64,
                 ch.P_U8: np.uint8, ch.P_U16: np.uint16, ch.P_U32: np.uint32, ch.P_U64: np.uint64,
@@ -46,9 +56,13 @@ class CollectedChunks:
     physical width; the Arrow precision does not.  `list_children` maps a LIST column to its child type, `(child_type_id, child_dec_width)`; for those columns the
     chunk's child vector is copied too (through Appender.list_child, valid only inside the sink call)."""
 
-    def __init__(self, type_ids: Sequence[int], dec_widths: Optional[Sequence[int]] = None, list_children: Optional[dict] = None):
+    def __init__(self, type_ids: Sequence[int], dec_widths: Optional[Sequence[int]] = None, list_children: Optional[dict] = None,
+                 enums: Optional[dict] = None):
+        """`enums` maps an ENUM column to `(internal_type, labels)`: UTINYINT / USMALLINT / UINTEGER, the vector's width."""
         self.type_ids = list(type_ids)
-        self.widths = [_out_width(t, (dec_widths or [0] * len(type_ids))[i]) for i, t in enumerate(type_ids)]
+        self.enums = dict(enums or {})
+        self.widths = [np.dtype(_ENUM_DTYPE[self.enums[i][0]]).itemsize if t == ch.T_ENUM else
+                       _out_width(t, (dec_widths or [0] * len(type_ids))[i]) for i, t in enumerate(type_ids)]
         self.counts: List[int] = []
         self.data: List[List[bytes]] = [[] for _ in type_ids]
         self.validity: List[List[np.ndarray]] = [[] for _ in type_ids]
@@ -102,6 +116,15 @@ class CollectedChunks:
                 o, ln = int(ent[i, 0]), int(ent[i, 1])
                 out.append([vals[j] if cvalid[j] else None for j in range(o, o + ln)])
         return out
+
+    def enum_positions(self, c: int) -> np.ndarray:
+        """ENUM column `c`: the stored positions, in the column's internal width"""
+        return np.frombuffer(self.column_bytes(c), dtype=_ENUM_DTYPE[self.enums[c][0]])
+
+    def enum_values(self, c: int) -> list:
+        """ENUM column `c` as its labels (None: a NULL row)"""
+        labels = self.enums[c][1]
+        return [labels[int(p)] if v else None for p, v in zip(self.enum_positions(c), self.valid_bits(c))]
 
     @property
     def nrows(self) -> int:
@@ -207,6 +230,12 @@ class Appender:
         needed before an Arrow list reaches that column."""
         self._check(self.lib.duckdb_mb_gpu_appender_set_list(self.handle, int(col), int(child_type), int(dec_width), int(dec_scale)),
                     "set_list")
+
+    def set_enum(self, col: int, labels, internal_type: int):
+        """The ENUM column's labels (str or bytes, matched byte-exactly) and internal type (UTINYINT / USMALLINT / UINTEGER,
+        what duckdb_enum_internal_type reports); needed before Arrow arrays or append_varchar cells reach that column."""
+        d, keep = enum_dict(labels)
+        self._check(self.lib.duckdb_mb_gpu_appender_set_enum(self.handle, int(col), int(internal_type), C.byref(d)), "set_enum")
 
     def list_child(self, col: int):
         """Inside a sink call: (child values pointer, child mask pointer, child size) of LIST column `col`."""

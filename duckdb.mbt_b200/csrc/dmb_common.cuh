@@ -209,6 +209,38 @@ __device__ __forceinline__ uint4 enum_entry(const dmb_enum_job &job, uint32_t id
   return e;
 }
 
+// ---- ENUM labels -> positions (kernels_reverse.cu, dmb_rev_enum_table): one hash and one probe for the host that
+// builds the table and the device that reads it.  A label is keyed by its length, its first 12 bytes (zero padded, as
+// three little-endian words) and, past 12 bytes, its last 4; only labels longer than 16 bytes compare bytes beyond that.
+__host__ __device__ __forceinline__ uint32_t dmb_enum_hash(uint32_t len, uint32_t w0, uint32_t w1, uint32_t w2, uint32_t tail) {
+  uint32_t h = len * 0x9E3779B1u;
+  h = (h ^ w0) * 0x85EBCA77u; h ^= h >> 13;
+  h = (h ^ w1) * 0xC2B2AE3Du; h ^= h >> 16;
+  h = (h ^ w2) * 0x27D4EB2Fu; h ^= h >> 15;
+  h = (h ^ tail) * 0x165667B1u; h ^= h >> 16;
+  return h;
+}
+
+// position of the label with this key in `slots` (2 uint4 per slot, table_size - 1 = mask), or DMB_ENUM_CODE_MISSING.
+// `row`: the row's bytes; `label_off` / `label_data`: the ENUM's labels (read only for labels longer than 16 bytes).
+__host__ __device__ __forceinline__ uint32_t enum_probe(const uint4 *slots, uint32_t mask, uint32_t len, uint32_t w0, uint32_t w1,
+                                                        uint32_t w2, uint32_t tail, const uint8_t *row, const uint32_t *label_off,
+                                                        const uint8_t *label_data) {
+  const uint32_t h = dmb_enum_hash(len, w0, w1, w2, tail);
+  for (uint32_t i = h & mask;; i = (i + 1) & mask) {
+    const uint4 a = slots[2 * i];
+    if (a.x == DMB_ENUM_CODE_MISSING) return DMB_ENUM_CODE_MISSING;  // an empty slot ends the chain
+    if (a.y != len || a.z != h) continue;
+    const uint4 b = slots[2 * i + 1];
+    if (b.x != w0 || b.y != w1 || b.z != w2 || b.w != tail) continue;
+    bool eq = true;
+    if (len > 16) {
+      const uint8_t *l = label_data + label_off[a.x];
+      for (uint32_t k = 12; k < len - 4 && eq; ++k) eq = row[k] == l[k];
+    }
+    if (eq) return a.x;
+  }
+}
 
 // ---- decoupled look-back: status words (flag in bits 63..62, value below: one word, so no fences are needed) ----
 constexpr uint64_t kFlagAggregate = 1ull << 62;

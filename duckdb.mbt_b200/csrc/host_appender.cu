@@ -52,6 +52,20 @@ struct ColInput {
   const uint8_t *data = nullptr;         // strings: Arrow data buffer base
   const ColInput *child = nullptr;       // lists: the child array, its rows are the list elements
   int64_t child_len = 0;                 // lists: elements in the child array
+  // ENUM: labels (is_string) or Arrow dictionary indices (w_in bytes each) -> positions of w_out bytes
+  bool is_enum = false, index_signed = false, dict_large = false;
+  const uint8_t *dict_offsets = nullptr;  // dictionary indices: the Arrow dictionary (utf8 / large_utf8) at its own offset
+  const uint8_t *dict_data = nullptr, *dict_validity = nullptr;
+  int64_t dict_bit_offset = 0, dict_len = 0;
+};
+
+// an ENUM column's labels and internal width (duckdb_mb_gpu_appender_set_enum); width 0: not declared
+struct EnumDecl {
+  int32_t width = 0;
+  std::vector<uint32_t> offsets;
+  std::vector<uint8_t> data;
+  std::vector<uint4> slots;  // the lookup table (dmb_rev_enum_table), two uint4 per slot
+  uint32_t table_size = 0;
 };
 
 // the table's child type of a LIST column (duckdb_mb_gpu_appender_set_list); type_id 0: not declared
@@ -87,6 +101,7 @@ struct duckdb_mb_gpu_appender {
   char error[256] = {0};
   std::vector<RowBuf> rows;
   std::vector<ListDecl> lists;
+  std::vector<EnumDecl> enums;
   std::vector<SinkList> sink_lists;  // valid while sink_chunk >= 0: chunk sink_chunk of the sub-batch being handed over
   int64_t sink_chunk = -1;
   int64_t sub_rows = 4 << 20;
@@ -267,10 +282,45 @@ struct Slot {  // device + pinned buffers of one in-flight sub-batch
   std::vector<uint64_t *> d_val, h_val;
   std::vector<ListOut> lists;                     // [ncols], used by LIST columns
   unsigned int *d_err = nullptr, *h_err = nullptr;  // [ncols]: rev_list_kernel error flags
+  unsigned long long *d_eerr = nullptr, *h_eerr = nullptr;  // [ncols]: ENUM columns' first offending row (~0: none)
   cudaEvent_t ev_out = nullptr;
   int64_t r0 = 0, r1 = 0;
   bool busy = false;
 };
+
+// Arrow offset of `row` (strings, lists), read on the host
+int64_t offset_at(const ColInput &ci, int64_t row) {
+  if (ci.large) { int64_t v; memcpy(&v, ci.offsets + 8 * row, 8); return v; }
+  int32_t v; memcpy(&v, ci.offsets + 4 * row, 4); return v;
+}
+
+// the appender error for the first offending row of an ENUM column, rendered from the host buffers
+int32_t enum_error(App *a, int c, const ColInput &ci, int64_t row) {
+  const uint8_t *p;
+  int64_t len;
+  if (ci.is_string) {
+    const int64_t o0 = offset_at(ci, row);
+    p = ci.data + o0;
+    len = offset_at(ci, row + 1) - o0;
+  } else {
+    uint64_t raw = 0;
+    memcpy(&raw, ci.values + (size_t)row * (size_t)ci.w_in, (size_t)ci.w_in);
+    const int sh = 64 - 8 * ci.w_in;
+    const int64_t idx = ci.index_signed ? (int64_t)(raw << sh) >> sh : (int64_t)raw;
+    if (idx < 0 || idx >= ci.dict_len)
+      return fail(a, "column %d, row %lld: dictionary index %lld is outside the Arrow dictionary (%lld entries)", c, (long long)row,
+                  (long long)idx, (long long)ci.dict_len);
+    ColInput d;
+    d.offsets = ci.dict_offsets;
+    d.large = ci.dict_large;
+    const int64_t o0 = offset_at(d, idx);
+    p = ci.dict_data + o0;
+    len = offset_at(d, idx + 1) - o0;
+  }
+  const int shown = len > 160 ? 160 : (int)len;  // the message fits the 256-byte error buffer
+  return fail(a, "column %d, row %lld: '%.*s'%s is not a label of the ENUM", c, (long long)row, shown, (const char *)p,
+              len > shown ? "..." : "");
+}
 
 int32_t sink_slot(App *a, Slot &s, const std::vector<ColInput> &cols, const std::vector<std::vector<int64_t>> &bounds) {
   if (!s.busy) return 1;
@@ -280,6 +330,8 @@ int32_t sink_slot(App *a, Slot &s, const std::vector<ColInput> &cols, const std:
   for (int c = 0; c < nc; ++c)  // a malformed sub-batch reaches no sink
     if (cols[(size_t)c].is_list && s.h_err[c])
       return fail(a, "column %d: Arrow list offsets decrease within rows [%lld, %lld)", c, (long long)s.r0, (long long)s.r1);
+    else if (cols[(size_t)c].is_enum && s.h_eerr[c] != ~0ull)
+      return enum_error(a, c, cols[(size_t)c], s.r0 + (int64_t)s.h_eerr[c]);
   if (!a->sink) return 1;
   std::vector<const void *> vd((size_t)nc);
   std::vector<const uint64_t *> vv((size_t)nc);
@@ -317,12 +369,6 @@ int64_t stage_bits(App *a, Scope &sc, uint8_t *&dst, size_t &cap, const uint8_t 
   if (!grow(sc, dst, cap, (size_t)(byte1 - byte0) + 16) ||
       stage_contiguous(c, c.s_in, dst, bm + byte0, (size_t)(byte1 - byte0), -1, &a->bytes_h2d)) return -1;
   return p0 & 7;
-}
-
-// Arrow offset of `row` (strings, lists), read on the host
-int64_t offset_at(const ColInput &ci, int64_t row) {
-  if (ci.large) { int64_t v; memcpy(&v, ci.offsets + 8 * row, 8); return v; }
-  int32_t v; memcpy(&v, ci.offsets + 4 * row, 4); return v;
 }
 
 // Stage Arrow rows [r0, r1) of a column that is not a LIST and describe its conversion: `*fj` for a fixed-width
@@ -401,6 +447,76 @@ extern "C" int64_t dmb_rev_list_cut(const int64_t *const *bounds, int32_t nlists
 namespace dmb {
 namespace {
 
+// Once per conversion, before the first sub-batch's kernels: every ENUM column's lookup table and labels go to the
+// device, and for a dictionary column the Arrow dictionary too, whose labels the lookup kernel turns into the remap (one
+// code per dictionary entry) that the index kernel of every sub-batch reads.  `*base`: per column, the job fields that do
+// not change between sub-batches (empty when no column is an ENUM).
+int32_t stage_enums(App *a, Scope &sc, const std::vector<ColInput> &cols, std::vector<dmb_rev_enum_job> *base) {
+  CtxCore &c = *a->core;
+  base->clear();
+  std::vector<dmb_rev_enum_job> remaps;
+  std::vector<int64_t> remap_rows;
+  for (size_t j = 0; j < cols.size(); ++j) {
+    const ColInput &ci = cols[j];
+    if (!ci.is_enum) continue;
+    base->resize(cols.size());
+    const EnumDecl &e = a->enums[j];
+    dmb_rev_enum_job &ej = (*base)[j];
+    memset(&ej, 0, sizeof(ej));
+    ej.out_width = e.width;
+    const size_t tb = e.slots.size() * sizeof(uint4), ob = e.offsets.size() * 4;
+    uint8_t *table = (uint8_t *)sc.dalloc(tb), *loff = (uint8_t *)sc.dalloc(ob), *ldata = (uint8_t *)sc.dalloc(e.data.size() + 16);
+    if (!table || !loff || !ldata || stage_contiguous(c, c.s_in, table, e.slots.data(), tb, -1, &a->bytes_h2d) ||
+        stage_contiguous(c, c.s_in, loff, e.offsets.data(), ob, -1, &a->bytes_h2d) ||
+        (!e.data.empty() && stage_contiguous(c, c.s_in, ldata, e.data.data(), e.data.size(), -1, &a->bytes_h2d)))
+      return fail(a, "%s", duckdb_mb_gpu_last_error());
+    ej.table = table;
+    ej.table_size = e.table_size;
+    ej.label_offsets = (const uint32_t *)loff;
+    ej.label_data = ldata;
+    if (ci.is_string) continue;
+    ej.index_width = ci.w_in;
+    ej.index_signed = ci.index_signed ? 1 : 0;
+    ej.dict_len = ci.dict_len;
+    if (ci.dict_len == 0) continue;  // every valid row is out of range
+    // the Arrow dictionary as a string column of its own: its codes are the remap
+    ColInput d;
+    d.is_string = true;
+    d.large = ci.dict_large;
+    d.offsets = ci.dict_offsets;
+    d.data = ci.dict_data;
+    d.validity = ci.dict_validity;
+    d.bit_offset = ci.dict_bit_offset;
+    InBuf ib;
+    dmb_rev_fixed_job fj;
+    dmb_rev_string_job sj;
+    const uint8_t *d_validity = nullptr;
+    int64_t bit_off = 0;
+    uint32_t *remap = (uint32_t *)sc.dalloc(4 * (size_t)ci.dict_len);
+    if (!remap) return fail(a, "%s", duckdb_mb_gpu_last_error());
+    if (!stage_rows(a, sc, d, ib, (int)j, 0, ci.dict_len, nullptr, nullptr, &fj, &sj, &d_validity, &bit_off)) return 0;
+    dmb_rev_enum_job rj = ej;
+    rj.index_width = 0;
+    rj.out_width = 0;
+    rj.in_offsets = sj.in_offsets;
+    rj.in_data = sj.in_data;
+    rj.large_offsets = sj.large_offsets;
+    rj.in_validity = d_validity;
+    rj.in_bit_offset = bit_off;
+    rj.out = remap;
+    remaps.push_back(rj);
+    remap_rows.push_back(ci.dict_len);
+    ej.remap = remap;
+  }
+  if (remaps.empty()) return 1;
+  cudaEvent_t ev = sc.event(false);
+  if (!ev || check_cuda(cudaEventRecord(ev, c.s_in), "ENUM staging") || check_cuda(cudaStreamWaitEvent(c.s_compute, ev, 0), "wait ENUM staging"))
+    return fail(a, "%s", duckdb_mb_gpu_last_error());
+  for (size_t i = 0; i < remaps.size(); ++i)
+    if (dmb_dev_rev_enum_batch(&remaps[i], remap_rows[i], c.s_compute)) return fail(a, "%s", duckdb_mb_gpu_last_error());
+  return 1;
+}
+
 // convert `nrows` rows described by `cols` and hand the chunks to the sink
 int32_t convert_rows(App *a, const std::vector<ColInput> &cols, int64_t nrows) {
   if (nrows <= 0) return 1;
@@ -440,7 +556,9 @@ int32_t convert_rows(App *a, const std::vector<ColInput> &cols, int64_t nrows) {
     slots[s].lists.resize((size_t)nc);
     slots[s].d_err = (unsigned int *)sc.dalloc(sizeof(unsigned int) * (size_t)nc);
     slots[s].h_err = (unsigned int *)sc.palloc(sizeof(unsigned int) * (size_t)nc);
-    if (!slots[s].ev_out || !slots[s].d_err || !slots[s].h_err) return fail(a, "%s", duckdb_mb_gpu_last_error());
+    slots[s].d_eerr = (unsigned long long *)sc.dalloc(8 * (size_t)nc);
+    slots[s].h_eerr = (unsigned long long *)sc.palloc(8 * (size_t)nc);
+    if (!slots[s].ev_out || !slots[s].d_err || !slots[s].h_err || !slots[s].d_eerr || !slots[s].h_eerr) return fail(a, "%s", duckdb_mb_gpu_last_error());
     for (int j = 0; j < nc; ++j) {
       const size_t ob = (size_t)sub * (size_t)cols[(size_t)j].w_out, vb = (size_t)sub_chunks * DMB_VALIDITY_WORDS * 8;
       uint8_t *d = (uint8_t *)sc.dalloc(ob), *h = (uint8_t *)sc.palloc(ob);
@@ -482,6 +600,9 @@ int32_t convert_rows(App *a, const std::vector<ColInput> &cols, int64_t nrows) {
   if (!h_jobs || !d_jobs) return fail(a, "%s", duckdb_mb_gpu_last_error());
   cudaEventRecord(in0, c.s_in);
   cudaEventRecord(out0, c.s_out);
+  std::vector<dmb_rev_enum_job> enum_base;
+  if (!stage_enums(a, sc, cols, &enum_base)) return 0;
+  const bool any_enum = !enum_base.empty();
   for (size_t b = 0; b + 1 < cuts.size(); ++b) {
     const int64_t r0 = cuts[b] * DMB_VECTOR_SIZE, r1 = cuts[b + 1] * DMB_VECTOR_SIZE < nrows ? cuts[b + 1] * DMB_VECTOR_SIZE : nrows;
     const int64_t n = r1 - r0;
@@ -496,6 +617,7 @@ int32_t convert_rows(App *a, const std::vector<ColInput> &cols, int64_t nrows) {
     if (!ev_in || !ev_k || !k0 || !k1) return fail(a, "%s", duckdb_mb_gpu_last_error());
     std::vector<dmb_rev_string_job> strs;
     std::vector<dmb_rev_list_job> lists;
+    std::vector<dmb_rev_enum_job> enums;
     std::vector<int64_t> child_rows;  // element count of each child job: fixed-width ones first, in job order
     std::vector<int64_t> str_rows;
     std::vector<int> masks_from_bytes;  // columns
@@ -508,7 +630,22 @@ int32_t convert_rows(App *a, const std::vector<ColInput> &cols, int64_t nrows) {
         dmb_rev_string_job sj;
         if (!stage_rows(a, sc, ci, ib, j, r0, r1, slot.d_out[(size_t)j], slot.d_val[(size_t)j], &hj[nfixed], &sj, &d_validity, &bit_off)) return 0;
         if (ci.valid_bytes) masks_from_bytes.push_back(j);
-        if (ci.is_string) { strs.push_back(sj); str_rows.push_back(n); }
+        if (ci.is_enum) {
+          dmb_rev_enum_job ej = enum_base[(size_t)j];
+          if (ci.is_string) {
+            ej.in_offsets = sj.in_offsets;
+            ej.in_data = sj.in_data;
+            ej.large_offsets = sj.large_offsets;
+          } else {
+            ej.in_indices = hj[nfixed].in_values;  // (that job slot is reused by the next fixed-width column)
+          }
+          ej.in_validity = d_validity;
+          ej.in_bit_offset = bit_off;
+          ej.out = slot.d_out[(size_t)j];
+          ej.out_validity = slot.d_val[(size_t)j];
+          ej.error = slot.d_eerr + j;
+          enums.push_back(ej);
+        } else if (ci.is_string) { strs.push_back(sj); str_rows.push_back(n); }
         else ++nfixed;
         continue;
       }
@@ -578,6 +715,10 @@ int32_t convert_rows(App *a, const std::vector<ColInput> &cols, int64_t nrows) {
     }
     for (size_t i = 0; i < strs.size(); ++i)
       if (dmb_dev_rev_string_batch(&strs[i], str_rows[i], c.s_compute)) return fail(a, "%s", duckdb_mb_gpu_last_error());
+    if (any_enum && check_cuda(cudaMemsetAsync(slot.d_eerr, 0xff, 8 * (size_t)nc, c.s_compute), "ENUM error words reset"))
+      return fail(a, "%s", duckdb_mb_gpu_last_error());
+    for (auto &ej : enums)
+      if (dmb_dev_rev_enum_batch(&ej, n, c.s_compute)) return fail(a, "%s", duckdb_mb_gpu_last_error());
     if (!lists.empty() && check_cuda(cudaMemsetAsync(slot.d_err, 0, sizeof(unsigned int) * (size_t)nc, c.s_compute), "error flags reset"))
       return fail(a, "%s", duckdb_mb_gpu_last_error());
     for (auto &lj : lists)
@@ -600,6 +741,8 @@ int32_t convert_rows(App *a, const std::vector<ColInput> &cols, int64_t nrows) {
       a->bytes_d2h += (uint64_t)lo.child_bytes + (uint64_t)lo.words * 8;
     }
     if (!lists.empty() && check_cuda(cudaMemcpyAsync(slot.h_err, slot.d_err, sizeof(unsigned int) * (size_t)nc, cudaMemcpyDeviceToHost, c.s_out), "error flags D2H"))
+      return fail(a, "%s", duckdb_mb_gpu_last_error());
+    if (any_enum && check_cuda(cudaMemcpyAsync(slot.h_eerr, slot.d_eerr, 8 * (size_t)nc, cudaMemcpyDeviceToHost, c.s_out), "ENUM error words D2H"))
       return fail(a, "%s", duckdb_mb_gpu_last_error());
     cudaEventRecord(slot.ev_out, c.s_out);
     slot.r0 = r0;
@@ -634,6 +777,10 @@ int32_t flush_rows(App *a) {
     if (rb.width == 0) {
       ci.is_string = true;
       ci.w_out = 16;
+      if (a->type_ids[(size_t)j] == DMB_TYPE_ENUM) {  // labels -> positions (set_enum declared the column before begin_row)
+        ci.is_enum = true;
+        ci.w_out = a->enums[(size_t)j].width;
+      }
       ci.offsets = (const uint8_t *)rb.offsets.data();
       if (rb.data.empty()) rb.data.push_back(0);
       ci.data = rb.data.data();
@@ -777,6 +924,66 @@ bool map_list(App *a, int j, const ArrowArray *arr, const ArrowSchema *sch, ColI
   return true;
 }
 
+// an Arrow array for an ENUM column: a dictionary array (indices c C s S i I l L, labels u / U) or plain u / U labels
+bool map_enum(App *a, int j, const ArrowArray *arr, const ArrowSchema *sch, ColInput *ci) {
+  static const uint8_t kNoData[16] = {0};
+  const char *fmt = sch->format;
+  const EnumDecl &e = a->enums[(size_t)j];
+  if (!e.width) {
+    fail(a, "column %d: the ENUM column's labels are not declared (duckdb_mb_gpu_appender_set_enum)", j);
+    return false;
+  }
+  ci->is_enum = true;
+  ci->w_out = e.width;
+  const bool integer = strlen(fmt) == 1 && strchr("cCsSiIlL", fmt[0]);
+  if (!sch->dictionary) {
+    if (strcmp(fmt, "u") == 0 || strcmp(fmt, "U") == 0) {
+      ci->is_string = true;
+      ci->large = fmt[0] == 'U';
+      return true;
+    }
+    if (strcmp(fmt, "vu") == 0) fail(a, "column %d: Arrow string views ('vu') cannot be appended to an ENUM column", j);
+    else if (integer) fail(a, "column %d: a bare Arrow integer array ('%s') cannot be appended to an ENUM column: pass a dictionary array or utf8 labels", j, fmt);
+    else if (fmt[0] == '+') fail(a, "column %d: an Arrow %s ('%s') cannot be appended to an ENUM column", j, nested_name(fmt), fmt);
+    else fail(a, "column %d: Arrow format '%s' cannot be appended to an ENUM column", j, fmt);
+    return false;
+  }
+  const char *dfmt = sch->dictionary->format ? sch->dictionary->format : "";
+  if (!integer) {
+    fail(a, "column %d: Arrow dictionary index format '%s' cannot be appended to an ENUM column", j, fmt);
+    return false;
+  }
+  if (strcmp(dfmt, "u") != 0 && strcmp(dfmt, "U") != 0) {
+    fail(a, "column %d: an Arrow dictionary of '%s' values cannot be appended to an ENUM column (the labels must be utf8 or large_utf8)", j, dfmt);
+    return false;
+  }
+  const ArrowArray *d = arr->dictionary;
+  if (!d) {
+    fail(a, "column %d: the Arrow dictionary array is missing", j);
+    return false;
+  }
+  const char f = fmt[0];
+  ci->w_in = f == 'c' || f == 'C' ? 1 : f == 's' || f == 'S' ? 2 : f == 'i' || f == 'I' ? 4 : 8;
+  ci->rev_op = copy_op(ci->w_in);
+  ci->index_signed = f >= 'a' && f <= 'z';
+  ci->dict_large = dfmt[0] == 'U';
+  ci->dict_len = d->length;
+  ci->dict_bit_offset = d->offset;
+  ci->dict_validity = (d->null_count != 0 && d->n_buffers > 0) ? (const uint8_t *)d->buffers[0] : nullptr;
+  ci->dict_offsets = d->n_buffers > 1 && d->buffers[1] ? (const uint8_t *)d->buffers[1] + (size_t)d->offset * (ci->dict_large ? 8 : 4) : nullptr;
+  ci->dict_data = d->n_buffers > 2 && d->buffers[2] ? (const uint8_t *)d->buffers[2] : kNoData;
+  if (d->length > 0 && !ci->dict_offsets) {
+    fail(a, "column %d: the Arrow dictionary has no offsets buffer", j);
+    return false;
+  }
+  return true;
+}
+
+// the current cell of a row in progress belongs to an ENUM column
+bool enum_cell(App *a) {
+  return a->state == kRowInProgress && a->cur_col < a->ncols && a->type_ids[(size_t)a->cur_col] == DMB_TYPE_ENUM;
+}
+
 }  // namespace
 }  // namespace dmb
 
@@ -792,6 +999,7 @@ extern "C" duckdb_mb_gpu_appender *duckdb_mb_gpu_appender_create(duckdb_mb_gpu_c
   a->user = user;
   a->rows.resize((size_t)ncols);
   a->lists.resize((size_t)ncols);
+  a->enums.resize((size_t)ncols);
   for (int j = 0; j < ncols; ++j) {
     a->rows[(size_t)j].width = row_width(type_ids[j]);  // -1: column only reachable through Arrow batches
     a->rows[(size_t)j].offsets.assign(1, 0);
@@ -854,10 +1062,11 @@ extern "C" int32_t duckdb_mb_gpu_append_arrow_batch(duckdb_mb_gpu_appender *a, c
     const ArrowArray *ch = batch->children[j];
     const ArrowSchema *cs = schema->children[j];
     ColInput &ci = cols[(size_t)j];
-    const bool list = a->type_ids[(size_t)j] == DMB_TYPE_LIST;
+    const bool list = a->type_ids[(size_t)j] == DMB_TYPE_LIST, en = a->type_ids[(size_t)j] == DMB_TYPE_ENUM;
     if (!ch || !cs || !cs->format ||
         !(list ? map_list(a, j, ch, cs, &ci, &children[(size_t)j])
-               : map_format(a, j, "format", cs->format, a->type_ids[(size_t)j], &a->rows[(size_t)j].dec_prec, &a->rows[(size_t)j].dec_scale, &ci))) {
+               : en ? map_enum(a, j, ch, cs, &ci)
+                    : map_format(a, j, "format", cs->format, a->type_ids[(size_t)j], &a->rows[(size_t)j].dec_prec, &a->rows[(size_t)j].dec_scale, &ci))) {
       if (!a->error[0]) fail(a, "append_arrow_batch: column %d is malformed", j);
       a->state = kError;
       return 0;
@@ -885,8 +1094,14 @@ extern "C" int32_t duckdb_mb_gpu_append_arrow_batch(duckdb_mb_gpu_appender *a, c
 extern "C" int32_t duckdb_mb_gpu_begin_row(duckdb_mb_gpu_appender *a) {
   if (!a) return 0;
   if (a->state != kReady && a->state != kFlushed) return illegal(a, "begin_row");
-  for (int j = 0; j < a->ncols; ++j)
+  for (int j = 0; j < a->ncols; ++j) {
+    if (a->type_ids[(size_t)j] == DMB_TYPE_ENUM && !a->enums[(size_t)j].width) {
+      fail(a, "begin_row: ENUM column %d has no declared labels (duckdb_mb_gpu_appender_set_enum)", j);
+      a->state = kError;
+      return 0;
+    }
     if (a->rows[(size_t)j].width < 0) { fail(a, "begin_row: column %d (type %d) is only appendable through Arrow batches", j, a->type_ids[(size_t)j]); a->state = kError; return 0; }
+  }
   a->state = kRowInProgress;
   a->cur_col = 0;
   return 1;
@@ -900,6 +1115,7 @@ extern "C" int32_t duckdb_mb_gpu_append_timestamp(duckdb_mb_gpu_appender *a, int
 
 // BLOB cell (src/duckdb_native.c:1397-1415): the bytes as they are, no UTF-8 requirement
 extern "C" int32_t duckdb_mb_gpu_append_blob(duckdb_mb_gpu_appender *a, const uint8_t *bytes, int32_t len) {
+  if (a && enum_cell(a)) return type_mismatch(a, "append_blob");  // an ENUM cell takes VARCHAR labels only
   return duckdb_mb_gpu_append_varchar(a, bytes, len);
 }
 
@@ -912,7 +1128,8 @@ void put_quoted(std::vector<uint8_t> &t, const uint8_t *p, int32_t len) {
   if (p && len > 0) t.insert(t.end(), p, p + len);
   t.push_back('"');
 }
-int32_t append_text_cell(duckdb_mb_gpu_appender *a, std::vector<uint8_t> &t) {
+int32_t append_text_cell(duckdb_mb_gpu_appender *a, const char *cmd, std::vector<uint8_t> &t) {
+  if (enum_cell(a)) return type_mismatch(a, cmd);
   size_t n = 0;
   while (n < t.size() && t[n] != 0) ++n;  // strlen of the reference's buffer
   return duckdb_mb_gpu_append_varchar(a, t.data(), (int32_t)n);
@@ -929,7 +1146,7 @@ extern "C" int32_t duckdb_mb_gpu_append_list_varchar(duckdb_mb_gpu_appender *a, 
     put_quoted(t, values[i], lens[i]);
   }
   t.push_back(']');
-  return append_text_cell(a, t);
+  return append_text_cell(a, "append_list_varchar", t);
 }
 
 static int32_t append_pairs(duckdb_mb_gpu_appender *a, const char *what, const uint8_t *const *keys, const int32_t *key_lens,
@@ -946,7 +1163,7 @@ static int32_t append_pairs(duckdb_mb_gpu_appender *a, const char *what, const u
     put_quoted(t, values[i], value_lens[i]);
   }
   t.push_back('}');
-  return append_text_cell(a, t);
+  return append_text_cell(a, what, t);
 }
 
 extern "C" int32_t duckdb_mb_gpu_append_struct_varchar(duckdb_mb_gpu_appender *a, const uint8_t *const *names, const int32_t *name_lens,
@@ -1018,6 +1235,48 @@ extern "C" int32_t duckdb_mb_gpu_appender_set_list(duckdb_mb_gpu_appender *a, in
   if (d.type_id && (d.type_id != child_type_id || d.dec_width != child_dec_width || d.dec_scale != child_dec_scale))
     return fail(a, "appender_set_list: column %d already has LIST child type %d", col, d.type_id);
   d = ListDecl{child_type_id, child_dec_width, child_dec_scale};
+  return 1;
+}
+
+// the table column's ENUM type (duckdb_enum_dictionary_size / _value, duckdb_enum_internal_type of duckdb_appender_column_type)
+extern "C" int32_t duckdb_mb_gpu_appender_set_enum(duckdb_mb_gpu_appender *a, int32_t col, int32_t internal_type_id, const dmb_enum_dict *dict) {
+  if (!a) return 0;
+  if (col < 0 || col >= a->ncols || a->type_ids[(size_t)col] != DMB_TYPE_ENUM) return fail(a, "appender_set_enum: column %d is not an ENUM column", col);
+  int32_t w;
+  uint64_t most;
+  switch (internal_type_id) {
+    case DMB_TYPE_UTINYINT: w = 1; most = 1ull << 8; break;
+    case DMB_TYPE_USMALLINT: w = 2; most = 1ull << 16; break;
+    case DMB_TYPE_UINTEGER: w = 4; most = 1ull << 30; break;  // (the lookup table takes 2^31 slots at most)
+    default: return fail(a, "appender_set_enum: column %d: internal type %d is not UTINYINT, USMALLINT or UINTEGER", col, internal_type_id);
+  }
+  if (!dict) return fail(a, "appender_set_enum: column %d: no dictionary", col);
+  if ((uint64_t)dict->size > most)
+    return fail(a, "appender_set_enum: column %d: %u labels are more than internal type %d can index (%llu)", col, dict->size, internal_type_id,
+                (unsigned long long)most);
+  if (dict->size && (!dict->offsets || dict->offsets[0] != 0)) return fail(a, "appender_set_enum: column %d: malformed offsets (offsets[0] must be 0)", col);
+  for (uint32_t i = 0; i < dict->size; ++i)
+    if (dict->offsets[i + 1] < dict->offsets[i]) return fail(a, "appender_set_enum: column %d: malformed offsets (decreasing at label %u)", col, i);
+  const uint32_t bytes = dict->size ? dict->offsets[dict->size] : 0;
+  if (bytes && !dict->data) return fail(a, "appender_set_enum: column %d: malformed offsets (labels without data)", col);
+  EnumDecl e;
+  e.width = w;
+  e.offsets.assign(dict->offsets ? dict->offsets : nullptr, dict->offsets ? dict->offsets + dict->size + 1 : nullptr);
+  if (e.offsets.empty()) e.offsets.push_back(0);
+  e.data.assign((const uint8_t *)dict->data, (const uint8_t *)dict->data + bytes);
+  EnumDecl &cur = a->enums[(size_t)col];
+  if (cur.width) {
+    if (cur.width != e.width || cur.offsets != e.offsets || cur.data != e.data)
+      return fail(a, "appender_set_enum: column %d already has a different ENUM declaration", col);
+    return 1;
+  }
+  e.table_size = 16;
+  while (e.table_size < 2 * (uint64_t)dict->size) e.table_size *= 2;
+  e.slots.resize(2 * (size_t)e.table_size);
+  const dmb_enum_dict copy{dict->size, 0, e.offsets.data(), (const char *)e.data.data()};
+  if (!dmb_rev_enum_table(&copy, e.table_size, e.slots.data())) return fail(a, "appender_set_enum: column %d: %s", col, duckdb_mb_gpu_last_error());
+  cur = std::move(e);
+  a->rows[(size_t)col].width = 0;  // the row protocol buffers VARCHAR labels
   return 1;
 }
 

@@ -340,9 +340,235 @@ rev_list_kernel(dmb_rev_list_job job, int64_t nrows) {
   }
 }
 
+// ---- ENUM: labels -> positions (dmb_rev_enum_job).  One row per thread; a warp's 32 rows share one validity word, which
+// is also the mask word the ballot of the rows that got a position writes.
+extern __shared__ uint4 rev_enum_smem[];  // the lookup table or the remap, when it fits
+constexpr int kEnumSmemBytes = 48 << 10;
+
+// row `row` of a final-vector or remap launch: `code` is a position, DMB_ENUM_CODE_NULL or DMB_ENUM_CODE_MISSING (unused
+// when the row is NULL).  Called by every lane of the warp.
+__device__ __forceinline__ void enum_emit(const dmb_rev_enum_job &job, int64_t row, int64_t nrows, uint32_t vb, uint32_t code, int &nulls,
+                                          unsigned long long &first_bad) {
+  const int lane = threadIdx.x & 31;
+  const bool in = row < nrows, valid = (vb >> lane) & 1u;
+  if (job.out_width == 0) {
+    if (in) __stcs(reinterpret_cast<unsigned int *>(job.out) + row, valid ? code : DMB_ENUM_CODE_NULL);
+    return;
+  }
+  const bool ok = valid && code < DMB_ENUM_CODE_NULL;
+  if (valid && code == DMB_ENUM_CODE_MISSING && (unsigned long long)row < first_bad) first_bad = (unsigned long long)row;
+  const uint32_t word = __ballot_sync(0xffffffffu, ok);
+  const uint32_t v = ok ? code : 0u;
+  switch (job.out_width) {
+    case 1: reinterpret_cast<uint8_t *>(job.out)[row] = (uint8_t)v; break;
+    case 2: __stcs(reinterpret_cast<unsigned short *>(job.out) + row, (unsigned short)v); break;
+    default: __stcs(reinterpret_cast<unsigned int *>(job.out) + row, v); break;
+  }
+  if (lane == 0) {
+    reinterpret_cast<uint32_t *>(job.out_validity)[row >> 5] = word;
+    const int64_t left = nrows - row;
+    nulls += (left <= 0 ? 0 : (left < 32 ? (int)left : 32)) - __popc(word);
+  }
+}
+
+__device__ __forceinline__ void enum_finish(const dmb_rev_enum_job &job, int nulls, unsigned long long first_bad) {
+  if (first_bad != ~0ull) atomicMin(job.error, first_bad);
+  if (job.null_count && (threadIdx.x & 31) == 0 && nulls) atomicAdd(job.null_count, (unsigned long long)nulls);
+}
+
+// utf8 rows -> positions through the lookup table.  Offsets are read one per lane (lane 31 loads one more), the first 12
+// bytes of a row by 4 aligned words + funnel shifts, as in rev_string_kernel.
+template <bool LARGE>
+__global__ void __launch_bounds__(kThreads)
+rev_enum_string_kernel(dmb_rev_enum_job job, int64_t nrows, int64_t capacity, int smem) {
+  using off_t = typename std::conditional<LARGE, long long, int>::type;
+  const uint4 *tab = reinterpret_cast<const uint4 *>(job.table);
+  if (smem) {
+    for (uint32_t i = threadIdx.x; i < 2 * job.table_size; i += kThreads) rev_enum_smem[i] = __ldg(tab + i);
+    __syncthreads();
+    tab = rev_enum_smem;
+  }
+  const uint32_t mask = job.table_size - 1;
+  const off_t *off = reinterpret_cast<const off_t *>(job.in_offsets);
+  const int lane = threadIdx.x & 31;
+  const bool has_bm = job.in_validity != nullptr;
+  const BitSrc bs = bit_src(job.in_validity, job.in_bit_offset);
+  int nulls = 0;
+  unsigned long long first_bad = ~0ull;
+  for (int64_t base = (int64_t)blockIdx.x * kThreads; base < capacity; base += (int64_t)gridDim.x * kThreads) {
+    const int64_t row = base + threadIdx.x, row0 = row - lane;
+    const off_t o0 = __ldg(off + (row < nrows ? row : nrows));
+    const int64_t left = nrows - row0;
+    const int live = left <= 0 ? 0 : (left < 32 ? (int)left : 32);
+    const uint32_t vb = live == 0 ? 0u : (has_bm ? load_bits32(bs.w, bs.base + row0, live) : (live == 32 ? 0xffffffffu : ((1u << live) - 1u)));
+    off_t o1 = __shfl_down_sync(0xffffffffu, o0, 1);
+    if (lane == 31) o1 = __ldg(off + (row + 1 < nrows ? row + 1 : nrows));
+    uint32_t code = DMB_ENUM_CODE_MISSING;
+    if ((vb >> lane) & 1u) {
+      const uint32_t len = (uint32_t)(o1 - o0);
+      const uint8_t *q = job.in_data + o0;
+      const uint32_t *b32 = reinterpret_cast<const uint32_t *>(reinterpret_cast<uintptr_t>(q) & ~(uintptr_t)3);
+      const uint32_t sh = (uint32_t)(reinterpret_cast<uintptr_t>(q) & 3u) * 8u;
+      const uint32_t a0 = __ldg(b32), a1 = __ldg(b32 + 1), a2 = __ldg(b32 + 2), a3 = __ldg(b32 + 3);
+      auto keep = [](uint32_t word, int nb) { return nb >= 4 ? word : (nb <= 0 ? 0u : (word & ((1u << (8 * nb)) - 1u))); };
+      const uint32_t w0 = keep(__funnelshift_r(a0, a1, sh), (int)len), w1 = keep(__funnelshift_r(a1, a2, sh), (int)len - 4),
+                     w2 = keep(__funnelshift_r(a2, a3, sh), (int)len - 8);
+      uint32_t tail = 0;
+      if (len > 12u) {
+        const uint8_t *t = q + len - 4;
+        const uint32_t *t32 = reinterpret_cast<const uint32_t *>(reinterpret_cast<uintptr_t>(t) & ~(uintptr_t)3);
+        tail = __funnelshift_r(__ldg(t32), __ldg(t32 + 1), (uint32_t)(reinterpret_cast<uintptr_t>(t) & 3u) * 8u);
+      }
+      code = enum_probe(tab, mask, len, w0, w1, w2, tail, q, job.label_offsets, job.label_data);
+    }
+    enum_emit(job, row, nrows, vb, code, nulls, first_bad);
+  }
+  enum_finish(job, nulls, first_bad);
+}
+
+// Arrow dictionary indices -> positions through the remap (the codes of the dictionary's labels); four rows per thread
+// in flight, each warp's loads and stores contiguous.
+template <typename I>
+__global__ void __launch_bounds__(kThreads)
+rev_enum_index_kernel(dmb_rev_enum_job job, int64_t nrows, int64_t capacity, int smem) {
+  constexpr int U = 4;
+  constexpr int kShift = 64 - 8 * (int)sizeof(I);
+  const uint32_t *remap = job.remap;
+  if (smem) {
+    uint32_t *s = reinterpret_cast<uint32_t *>(rev_enum_smem);
+    for (int64_t i = threadIdx.x; i < job.dict_len; i += kThreads) s[i] = __ldg(remap + i);
+    __syncthreads();
+    remap = s;
+  }
+  const I *in = reinterpret_cast<const I *>(job.in_indices);
+  const int lane = threadIdx.x & 31;
+  const bool has_bm = job.in_validity != nullptr;
+  const BitSrc bs = bit_src(job.in_validity, job.in_bit_offset);
+  int nulls = 0;
+  unsigned long long first_bad = ~0ull;
+  for (int64_t base = (int64_t)blockIdx.x * (U * kThreads); base < capacity; base += (int64_t)gridDim.x * (U * kThreads)) {
+    I raw[U];
+    uint32_t vb[U];
+#pragma unroll
+    for (int u = 0; u < U; ++u) {
+      const int64_t row = base + u * kThreads + threadIdx.x;
+      raw[u] = row < nrows ? __ldcs(in + row) : I(0);
+    }
+#pragma unroll
+    for (int u = 0; u < U; ++u) {
+      const int64_t row0 = base + u * kThreads + threadIdx.x - lane;
+      const int64_t left = nrows - row0;
+      const int live = left <= 0 ? 0 : (left < 32 ? (int)left : 32);
+      vb[u] = live == 0 ? 0u : (has_bm ? load_bits32(bs.w, bs.base + row0, live) : (live == 32 ? 0xffffffffu : ((1u << live) - 1u)));
+    }
+#pragma unroll
+    for (int u = 0; u < U; ++u) {
+      const int64_t row = base + u * kThreads + threadIdx.x;
+      // sign- or zero-extended; an unsigned 64-bit index past 2^63 comes out negative, i.e. out of range as well
+      const int64_t idx = job.index_signed ? (int64_t)((uint64_t)raw[u] << kShift) >> kShift : (int64_t)(uint64_t)raw[u];
+      uint32_t code = DMB_ENUM_CODE_MISSING;
+      if (((vb[u] >> lane) & 1u) && idx >= 0 && idx < job.dict_len) code = remap[idx];
+      enum_emit(job, row, nrows, vb[u], code, nulls, first_bad);
+    }
+  }
+  enum_finish(job, nulls, first_bad);
+}
+
+// the key of a label on the host: what rev_enum_string_kernel computes from the row's bytes
+void enum_host_key(const uint8_t *p, uint32_t len, uint32_t *w, uint32_t *tail) {
+  uint8_t b[12] = {0};
+  if (len) memcpy(b, p, len < 12 ? len : 12);
+  memcpy(w, b, 12);
+  *tail = 0;
+  if (len > 12) memcpy(tail, p + len - 4, 4);
+}
+
 }  // namespace dmb
 
 using namespace dmb;
+
+extern "C" int32_t dmb_rev_enum_table(const dmb_enum_dict *d, uint32_t table_size, void *slots) {
+  if (!d || !slots || (d->size && !d->offsets)) { set_error("dmb_rev_enum_table: null dictionary or table"); return 0; }
+  if (table_size == 0 || (table_size & (table_size - 1)) || table_size <= d->size) {
+    set_error("dmb_rev_enum_table: a table of %u slots cannot hold %u labels (a power of two above the label count)", table_size, d->size);
+    return 0;
+  }
+  if (d->size && (d->offsets[0] != 0 || (d->offsets[d->size] && !d->data))) { set_error("ENUM dictionary offsets must start at 0 and come with data"); return 0; }
+  for (uint32_t i = 0; i < d->size; ++i)
+    if (d->offsets[i + 1] < d->offsets[i]) { set_error("ENUM dictionary offsets are not monotonic at label %u", i); return 0; }
+  uint4 *s = static_cast<uint4 *>(slots);
+  for (uint32_t i = 0; i < table_size; ++i) {
+    s[2 * i] = make_uint4(DMB_ENUM_CODE_MISSING, 0, 0, 0);
+    s[2 * i + 1] = make_uint4(0, 0, 0, 0);
+  }
+  const uint8_t *data = reinterpret_cast<const uint8_t *>(d->data);
+  for (uint32_t p = 0; p < d->size; ++p) {
+    const uint8_t *q = data + d->offsets[p];
+    const uint32_t len = d->offsets[p + 1] - d->offsets[p];
+    uint32_t w[3], tail;
+    enum_host_key(q, len, w, &tail);
+    const uint32_t dup = enum_probe(s, table_size - 1, len, w[0], w[1], w[2], tail, q, d->offsets, data);
+    if (dup != DMB_ENUM_CODE_MISSING) {
+      set_error("ENUM labels %u and %u are both '%.*s'", dup, p, (int)(len < 64 ? len : 64), (const char *)q);
+      return 0;
+    }
+    uint32_t i = dmb_enum_hash(len, w[0], w[1], w[2], tail) & (table_size - 1);
+    while (s[2 * i].x != DMB_ENUM_CODE_MISSING) i = (i + 1) & (table_size - 1);
+    s[2 * i] = make_uint4(p, len, dmb_enum_hash(len, w[0], w[1], w[2], tail), 0);
+    s[2 * i + 1] = make_uint4(w[0], w[1], w[2], tail);
+  }
+  return 1;
+}
+
+extern "C" int64_t dmb_rev_enum_lookup(const void *slots, uint32_t table_size, const dmb_enum_dict *d, const uint8_t *bytes, uint32_t len) {
+  if (!slots || !d || table_size == 0 || (len && !bytes)) return -1;
+  uint32_t w[3], tail;
+  enum_host_key(bytes, len, w, &tail);
+  const uint32_t p = enum_probe(static_cast<const uint4 *>(slots), table_size - 1, len, w[0], w[1], w[2], tail, bytes, d->offsets,
+                                reinterpret_cast<const uint8_t *>(d->data));
+  return p == DMB_ENUM_CODE_MISSING ? -1 : (int64_t)p;
+}
+
+extern "C" int32_t dmb_dev_rev_enum_batch(const dmb_rev_enum_job *job, int64_t nrows, void *stream) {
+  if (!job) { set_error("dmb_dev_rev_enum_batch: job is null"); return -1; }
+  if (nrows <= 0) return 0;
+  const int ow = job->out_width, iw = job->index_width;
+  if ((ow != 0 && ow != 1 && ow != 2 && ow != 4) || (iw != 0 && iw != 1 && iw != 2 && iw != 4 && iw != 8) || (ow == 0 && iw != 0)) {
+    set_error("dmb_dev_rev_enum_batch: out_width %d / index_width %d", ow, iw);
+    return -1;
+  }
+  if (!job->out || (ow && (!job->out_validity || !job->error)) ||
+      (iw == 0 && (!job->in_offsets || !job->in_data || !job->table || !job->label_offsets || !job->table_size ||
+                   (job->table_size & (job->table_size - 1)))) ||
+      (iw && (!job->in_indices || job->dict_len < 0 || (job->dict_len && !job->remap)))) {
+    set_error("dmb_dev_rev_enum_batch: a required pointer is null or the table size is not a power of two");
+    return -1;
+  }
+  const int64_t chunks = ((nrows + kVec - 1) / kVec) * (int64_t)kVec;
+  const int64_t max_grid = (int64_t)kNumSMs * 8;
+  cudaStream_t st = (cudaStream_t)stream;
+  if (iw == 0) {
+    const int64_t capacity = ow ? chunks : ((nrows + 31) / 32) * 32;  // remap mode: codes only, no masks to fill
+    const size_t tb = (size_t)job->table_size * DMB_ENUM_SLOT_BYTES;
+    const int smem = tb <= (size_t)kEnumSmemBytes ? (int)tb : 0;
+    const int64_t blocks = (capacity + kThreads - 1) / kThreads;
+    const int gx = (int)(blocks < max_grid ? blocks : max_grid);
+    if (job->large_offsets) rev_enum_string_kernel<true><<<gx, kThreads, smem, st>>>(*job, nrows, capacity, smem);
+    else rev_enum_string_kernel<false><<<gx, kThreads, smem, st>>>(*job, nrows, capacity, smem);
+    return check_cuda(cudaGetLastError(), "rev_enum_string_kernel launch");
+  }
+  const size_t rb = (size_t)job->dict_len * 4;
+  const int smem = rb <= (size_t)kEnumSmemBytes ? (int)((rb + 15) & ~(size_t)15) : 0;
+  const int64_t blocks = chunks / (4 * kThreads);
+  const int gx = (int)(blocks < max_grid ? blocks : max_grid);
+  switch (iw) {
+    case 1: rev_enum_index_kernel<uint8_t><<<gx, kThreads, smem, st>>>(*job, nrows, chunks, smem); break;
+    case 2: rev_enum_index_kernel<unsigned short><<<gx, kThreads, smem, st>>>(*job, nrows, chunks, smem); break;
+    case 4: rev_enum_index_kernel<unsigned int><<<gx, kThreads, smem, st>>>(*job, nrows, chunks, smem); break;
+    default: rev_enum_index_kernel<unsigned long long><<<gx, kThreads, smem, st>>>(*job, nrows, chunks, smem); break;
+  }
+  return check_cuda(cudaGetLastError(), "rev_enum_index_kernel launch");
+}
 
 extern "C" int32_t dmb_dev_rev_fixed_batch(const dmb_rev_fixed_job *jobs_dev, const dmb_rev_fixed_job *jobs_host,
                                            int32_t njobs, int64_t nrows, void *stream) {

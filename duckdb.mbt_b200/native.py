@@ -60,6 +60,17 @@ class RevListJob(C.Structure):
                 ("null_count", C.c_void_p), ("error", C.c_void_p), ("large_offsets", C.c_int32), ("reserved", C.c_int32)]
 
 
+class RevEnumJob(C.Structure):
+    _fields_ = [("in_offsets", C.c_void_p), ("in_data", C.c_void_p), ("in_indices", C.c_void_p), ("in_validity", C.c_void_p),
+                ("in_bit_offset", C.c_int64), ("remap", C.c_void_p), ("dict_len", C.c_int64), ("table", C.c_void_p),
+                ("label_offsets", C.c_void_p), ("label_data", C.c_void_p), ("out", C.c_void_p), ("out_validity", C.c_void_p),
+                ("null_count", C.c_void_p), ("error", C.c_void_p), ("table_size", C.c_uint32), ("out_width", C.c_int32),
+                ("index_width", C.c_int32), ("index_signed", C.c_int32), ("large_offsets", C.c_int32), ("reserved", C.c_int32)]
+
+
+ENUM_CODE_NULL, ENUM_CODE_MISSING, ENUM_SLOT_BYTES = 0xFFFFFFFE, 0xFFFFFFFF, 32
+
+
 class EnumDict(C.Structure):
     _fields_ = [("size", C.c_uint32), ("reserved", C.c_uint32), ("offsets", C.c_void_p), ("data", C.c_void_p)]
 
@@ -138,7 +149,7 @@ CHUNK_SINK = C.CFUNCTYPE(C.c_int32, C.c_void_p, C.c_int32, C.c_uint32, C.POINTER
 EXPORTED_SYMBOLS = [
     "dmb_dev_fixed_batch", "dmb_op_out_width", "dmb_phys_width", "dmb_dev_string_scratch_bytes",
     "dmb_dev_string_error", "dmb_dev_string_batch", "dmb_dev_set_lookback_limit_ns", "dmb_dev_rev_fixed_batch", "dmb_dev_rev_string_batch",
-    "dmb_dev_rev_list_batch", "dmb_rev_list_cut",
+    "dmb_dev_rev_list_batch", "dmb_rev_list_cut", "dmb_dev_rev_enum_batch", "dmb_rev_enum_table", "dmb_rev_enum_lookup",
     "dmb_dev_valid_bytes_to_masks", "dmb_dev_make_string_t", "dmb_dev_blob_escape", "dmb_render_supported", "dmb_render_slot_bytes", "dmb_dev_render_text", "dmb_dev_enum_to_string_t", "dmb_dev_enum_utf8", "dmb_dev_list_scratch_bytes", "dmb_dev_list_batch",
     "duckdb_mb_gpu_last_error", "duckdb_mb_gpu_device_count", "duckdb_mb_gpu_bind_numa", "duckdb_mb_gpu_ctx_create",
     "duckdb_mb_gpu_ctx_destroy", "duckdb_mb_gpu_ctx_sync", "duckdb_mb_gpu_host_alloc", "duckdb_mb_gpu_host_free",
@@ -176,7 +187,7 @@ EXPORTED_SYMBOLS = [
     "duckdb_mb_gpu_append_timestamp", "duckdb_mb_gpu_end_row", "duckdb_mb_gpu_append_blob", "duckdb_mb_gpu_append_decimal",
     "duckdb_mb_gpu_append_list_varchar", "duckdb_mb_gpu_append_struct_varchar", "duckdb_mb_gpu_append_map_varchar_varchar",
     "duckdb_mb_gpu_append_interval", "duckdb_mb_gpu_appender_set_decimal", "duckdb_mb_gpu_appender_set_list",
-    "duckdb_mb_gpu_appender_list_child",
+    "duckdb_mb_gpu_appender_list_child", "duckdb_mb_gpu_appender_set_enum",
 ]
 
 _lib = None
@@ -244,6 +255,14 @@ def lib():
     L.dmb_dev_rev_string_batch.argtypes = [C.POINTER(RevStringJob), i64, vp]
     L.dmb_dev_rev_list_batch.restype = i32
     L.dmb_dev_rev_list_batch.argtypes = [C.POINTER(RevListJob), i64, vp]
+    L.dmb_dev_rev_enum_batch.restype = i32
+    L.dmb_dev_rev_enum_batch.argtypes = [C.POINTER(RevEnumJob), i64, vp]
+    L.dmb_rev_enum_table.restype = i32
+    L.dmb_rev_enum_table.argtypes = [C.POINTER(EnumDict), C.c_uint32, vp]
+    L.dmb_rev_enum_lookup.restype = i64
+    L.dmb_rev_enum_lookup.argtypes = [vp, C.c_uint32, C.POINTER(EnumDict), vp, C.c_uint32]
+    L.duckdb_mb_gpu_appender_set_enum.restype = i32
+    L.duckdb_mb_gpu_appender_set_enum.argtypes = [vp, i32, i32, C.POINTER(EnumDict)]
     L.dmb_rev_list_cut.restype = i64
     L.dmb_rev_list_cut.argtypes = [vp, i32, i64, i64, i64, i64]
     L.duckdb_mb_gpu_appender_list_child.restype = i32

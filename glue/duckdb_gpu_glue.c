@@ -137,6 +137,27 @@ static int32_t phys_of(duckdb_type t, duckdb_type internal) {
   }
 }
 
+/* An ENUM type's labels (duckdb_enum_dictionary_size / _value) packed as a dmb_enum_dict; *offs / *bytes are the caller's
+ * to free.  Returns the label count. */
+static uint32_t read_enum_dict(duckdb_logical_type lt, uint32_t **offs_out, char **bytes_out) {
+  const uint32_t size = duckdb_enum_dictionary_size(lt);
+  uint32_t *offs = (uint32_t *)calloc((size_t)size + 1, sizeof(uint32_t));
+  size_t cap = 64, pos = 0;
+  char *bytes = (char *)malloc(cap);
+  for (uint32_t i = 0; i < size; i++) {
+    char *label = duckdb_enum_dictionary_value(lt, i);
+    const size_t n = label ? strlen(label) : 0;
+    if (pos + n + 1 > cap) { while (pos + n + 1 > cap) cap *= 2; bytes = (char *)realloc(bytes, cap); }
+    if (n) memcpy(bytes + pos, label, n);
+    pos += n;
+    offs[i + 1] = (uint32_t)pos;
+    duckdb_free(label);
+  }
+  *offs_out = offs;
+  *bytes_out = bytes;
+  return size;
+}
+
 /* Run `sql` and wrap every chunk of its result in a library result handle.  NULL + last error on failure. */
 static duckdb_mb_arrow_result *glue_query(duckdb_mb_connection *handle, moonbit_bytes_t sql) {
   duckdb_mb_gpu_ctx *ctx = glue_ctx();
@@ -191,19 +212,9 @@ static duckdb_mb_arrow_result *glue_query(duckdb_mb_connection *handle, moonbit_
       internal = duckdb_decimal_internal_type(lt);
     } else if (t == DUCKDB_TYPE_ENUM) {
       internal = duckdb_enum_internal_type(lt);
-      const uint32_t size = duckdb_enum_dictionary_size(lt);
-      uint32_t *offs = (uint32_t *)calloc((size_t)size + 1, sizeof(uint32_t));
-      size_t cap = 64, pos = 0;
-      char *bytes = (char *)malloc(cap);
-      for (uint32_t i = 0; i < size; i++) {
-        char *label = duckdb_enum_dictionary_value(lt, i);
-        const size_t n = label ? strlen(label) : 0;
-        if (pos + n + 1 > cap) { while (pos + n + 1 > cap) cap *= 2; bytes = (char *)realloc(bytes, cap); }
-        if (n) memcpy(bytes + pos, label, n);
-        pos += n;
-        offs[i + 1] = (uint32_t)pos;
-        duckdb_free(label);
-      }
+      uint32_t *offs;
+      char *bytes;
+      const uint32_t size = read_enum_dict(lt, &offs, &bytes);
       o->dict_offsets[c] = offs;
       o->dict_data[c] = bytes;
       o->dicts[c].size = size;
@@ -317,6 +328,7 @@ static int32_t vector_width(duckdb_logical_type lt) {
     case DUCKDB_TYPE_DECIMAL: { const int w = duckdb_decimal_width(lt); return w <= 4 ? 2 : w <= 9 ? 4 : w <= 18 ? 8 : 16; }
     case DUCKDB_TYPE_VARCHAR: case DUCKDB_TYPE_BLOB: case DUCKDB_TYPE_INTERVAL: case DUCKDB_TYPE_HUGEINT: case DUCKDB_TYPE_UHUGEINT: case DUCKDB_TYPE_UUID:
     case DUCKDB_TYPE_LIST: return 16; /* LIST: duckdb_list_entry */
+    case DUCKDB_TYPE_ENUM: { const duckdb_type it = duckdb_enum_internal_type(lt); return it == DUCKDB_TYPE_UTINYINT ? 1 : it == DUCKDB_TYPE_USMALLINT ? 2 : 4; }
     default: return 8;
   }
 }
@@ -418,6 +430,19 @@ duckdb_mb_appender *duckdb_mb_appender_create(duckdb_mb_connection *handle, moon
       duckdb_mb_gpu_appender_set_list(a, c, (int32_t)ct, ct == DUCKDB_TYPE_DECIMAL ? duckdb_decimal_width(child) : 0,
                                       ct == DUCKDB_TYPE_DECIMAL ? duckdb_decimal_scale(child) : 0);
       duckdb_destroy_logical_type(&child);
+    }
+    if (s->type_ids[c] == DUCKDB_TYPE_ENUM) {
+      /* a refused declaration leaves the column undeclared: appends to it fail and name duckdb_mb_gpu_appender_set_enum */
+      dmb_enum_dict d;
+      uint32_t *offs;
+      char *bytes;
+      memset(&d, 0, sizeof(d));
+      d.size = read_enum_dict(s->types[c], &offs, &bytes);
+      d.offsets = offs;
+      d.data = bytes;
+      duckdb_mb_gpu_appender_set_enum(a, c, (int32_t)duckdb_enum_internal_type(s->types[c]), &d);
+      free(offs);
+      free(bytes);
     }
   }
   return a;

@@ -46,6 +46,7 @@ typedef struct {
   int32_t type_id, dec_width, dec_scale, internal;
   const duckdb_mock_column *col;                   /* served columns */
   int32_t child_type_id, child_dec_width, child_dec_scale;  /* appender LIST columns */
+  int32_t enum_width; uint32_t enum_size; char **enum_labels;  /* appender ENUM columns (owned by the append table) */
 } mock_ltype;
 typedef struct { const mock_table *t; int64_t next_chunk; char error[128]; } mock_result;
 typedef struct mock_vec {
@@ -194,12 +195,20 @@ duckdb_type duckdb_get_type_id(duckdb_logical_type type) { return type ? (duckdb
 uint8_t duckdb_decimal_width(duckdb_logical_type type) { return (uint8_t)((mock_ltype *)type)->dec_width; }
 uint8_t duckdb_decimal_scale(duckdb_logical_type type) { return (uint8_t)((mock_ltype *)type)->dec_scale; }
 duckdb_type duckdb_decimal_internal_type(duckdb_logical_type type) { return (duckdb_type)((mock_ltype *)type)->internal; }
+/* served columns answer from their registration, appender columns from duckdb_mock_set_append_enum */
 duckdb_type duckdb_enum_internal_type(duckdb_logical_type type) {
-  const duckdb_mock_column *c = ((mock_ltype *)type)->col;
-  return c->width == 1 ? DUCKDB_TYPE_UTINYINT : c->width == 2 ? DUCKDB_TYPE_USMALLINT : DUCKDB_TYPE_UINTEGER;
+  const mock_ltype *t = (const mock_ltype *)type;
+  const int w = t->col ? t->col->width : t->enum_width;
+  return w == 1 ? DUCKDB_TYPE_UTINYINT : w == 2 ? DUCKDB_TYPE_USMALLINT : DUCKDB_TYPE_UINTEGER;
 }
-uint32_t duckdb_enum_dictionary_size(duckdb_logical_type type) { return ((mock_ltype *)type)->col->dict_size; }
-char *duckdb_enum_dictionary_value(duckdb_logical_type type, idx_t index) { return strdup(((mock_ltype *)type)->col->dict_values[index]); }
+uint32_t duckdb_enum_dictionary_size(duckdb_logical_type type) {
+  const mock_ltype *t = (const mock_ltype *)type;
+  return t->col ? t->col->dict_size : t->enum_size;
+}
+char *duckdb_enum_dictionary_value(duckdb_logical_type type, idx_t index) {
+  const mock_ltype *t = (const mock_ltype *)type;
+  return strdup(t->col ? t->col->dict_values[index] : t->enum_labels[index]);
+}
 duckdb_logical_type duckdb_list_type_child_type(duckdb_logical_type type) {
   const mock_ltype *t = (const mock_ltype *)type;
   if (!t->col) { /* an appender column's type */
@@ -226,7 +235,10 @@ void duckdb_destroy_logical_type(duckdb_logical_type *type) { if (type && *type)
 void duckdb_free(void *ptr) { free(ptr); }
 
 /* ---- appender side: a "table" = its column types + every chunk that was appended */
-typedef struct { int32_t type_id, dec_width, dec_scale, child_type_id, child_dec_width, child_dec_scale; } mock_coltype;
+typedef struct {
+  int32_t type_id, dec_width, dec_scale, child_type_id, child_dec_width, child_dec_scale;
+  int32_t enum_width; uint32_t enum_size; char **enum_labels;  /* ENUM: internal width and labels */
+} mock_coltype;
 typedef struct appended_chunk {
   idx_t size;
   uint8_t **data;
@@ -270,8 +282,20 @@ int32_t duckdb_mock_set_append_list_child(const char *table, int32_t col, int32_
   t->types[col].child_type_id = child_type; t->types[col].child_dec_width = dec_width; t->types[col].child_dec_scale = dec_scale;
   return 1;
 }
-static int type_width(int32_t type_id, int32_t dec_width) {
+/* the labels and internal width (1 / 2 / 4 bytes) of a registered ENUM column (what duckdb_enum_* report for it) */
+int32_t duckdb_mock_set_append_enum(const char *table, int32_t col, int32_t internal_width, uint32_t nlabels, const char *const *labels) {
+  mock_append_table *t = find_append_table(table);
+  if (!t || col < 0 || col >= t->ncols) return 0;
+  mock_coltype *ct = &t->types[col];
+  ct->enum_width = internal_width;
+  ct->enum_size = nlabels;
+  ct->enum_labels = (char **)calloc(nlabels ? nlabels : 1, sizeof(char *)); /* (leaked with the table: test process) */
+  for (uint32_t i = 0; i < nlabels; i++) ct->enum_labels[i] = strdup(labels[i]);
+  return 1;
+}
+static int type_width(int32_t type_id, int32_t dec_width, int32_t enum_width) {
   switch (type_id) {
+    case DUCKDB_TYPE_ENUM: return enum_width;
     case DUCKDB_TYPE_BOOLEAN: case DUCKDB_TYPE_TINYINT: case DUCKDB_TYPE_UTINYINT: return 1;
     case DUCKDB_TYPE_SMALLINT: case DUCKDB_TYPE_USMALLINT: return 2;
     case DUCKDB_TYPE_INTEGER: case DUCKDB_TYPE_UINTEGER: case DUCKDB_TYPE_FLOAT: case DUCKDB_TYPE_DATE: return 4;
@@ -297,6 +321,7 @@ duckdb_logical_type duckdb_appender_column_type(duckdb_appender appender, idx_t 
   if (ct->type_id == DUCKDB_TYPE_DECIMAL) return duckdb_create_decimal_type((uint8_t)ct->dec_width, (uint8_t)ct->dec_scale);
   mock_ltype *lt = (mock_ltype *)duckdb_create_logical_type((duckdb_type)ct->type_id);
   lt->child_type_id = ct->child_type_id; lt->child_dec_width = ct->child_dec_width; lt->child_dec_scale = ct->child_dec_scale;
+  lt->enum_width = ct->enum_width; lt->enum_size = ct->enum_size; lt->enum_labels = ct->enum_labels;
   return (duckdb_logical_type)lt;
 }
 const char *duckdb_appender_error(duckdb_appender appender) { mock_appender *a = (mock_appender *)appender; return a && a->error[0] ? a->error : NULL; }
@@ -312,7 +337,7 @@ duckdb_data_chunk duckdb_create_data_chunk(duckdb_logical_type *types, idx_t col
     v->created = 1;
     v->ltype = *(mock_ltype *)types[c];
     v->cap = MOCK_VECTOR_SIZE;
-    v->buf = (uint8_t *)calloc(MOCK_VECTOR_SIZE, (size_t)type_width(v->ltype.type_id, v->ltype.dec_width));
+    v->buf = (uint8_t *)calloc(MOCK_VECTOR_SIZE, (size_t)type_width(v->ltype.type_id, v->ltype.dec_width, v->ltype.enum_width));
     if (v->ltype.type_id == DUCKDB_TYPE_LIST) { /* an empty child vector, grown by duckdb_list_vector_reserve */
       v->child = (mock_vec *)calloc(1, sizeof(mock_vec));
       v->child->created = 1;
@@ -330,7 +355,7 @@ duckdb_state duckdb_list_vector_reserve(duckdb_vector vector, idx_t required_cap
   mock_vec *c = v->child;
   if (required_capacity <= c->cap) return DuckDBSuccess;
   idx_t cap = c->cap * 2 > required_capacity ? c->cap * 2 : required_capacity;
-  const size_t w = (size_t)type_width(c->ltype.type_id, c->ltype.dec_width);
+  const size_t w = (size_t)type_width(c->ltype.type_id, c->ltype.dec_width, 0);
   c->buf = (uint8_t *)realloc(c->buf, cap * w);
   memset(c->buf + c->cap * w, 0, (cap - c->cap) * w);
   if (c->mask) { /* new rows are valid */
@@ -385,7 +410,7 @@ duckdb_state duckdb_append_data_chunk(duckdb_appender appender, duckdb_data_chun
   ac->child_size = (idx_t *)calloc((size_t)ch->ncols, sizeof(idx_t));
   for (int32_t c = 0; c < ch->ncols; c++) {
     mock_vec *v = &ch->vecs[c];
-    const int w = type_width(a->t->types[c].type_id, a->t->types[c].dec_width);
+    const int w = type_width(a->t->types[c].type_id, a->t->types[c].dec_width, a->t->types[c].enum_width);
     const int is_str = a->t->types[c].type_id == DUCKDB_TYPE_VARCHAR || a->t->types[c].type_id == DUCKDB_TYPE_BLOB;
     ac->data[c] = (uint8_t *)malloc((size_t)MOCK_VECTOR_SIZE * (size_t)w);
     memcpy(ac->data[c], v->buf, (size_t)MOCK_VECTOR_SIZE * (size_t)w);
@@ -404,7 +429,7 @@ duckdb_state duckdb_append_data_chunk(duckdb_appender appender, duckdb_data_chun
     if (v->child) { /* LIST: the child vector, its first list_size rows */
       const mock_vec *cv = v->child;
       const idx_t size = v->list_size;
-      const size_t cw = (size_t)type_width(cv->ltype.type_id, cv->ltype.dec_width), words = (size + 63) / 64;
+      const size_t cw = (size_t)type_width(cv->ltype.type_id, cv->ltype.dec_width, 0), words = (size + 63) / 64;
       ac->child_size[c] = size;
       ac->child_data[c] = (uint8_t *)malloc(size * cw + 1);
       if (size) memcpy(ac->child_data[c], cv->buf, size * cw);

@@ -409,6 +409,51 @@ int32_t dmb_dev_rev_list_batch(const dmb_rev_list_job *job, int64_t nrows, void 
 int64_t dmb_rev_list_cut(const int64_t *const *bounds, int32_t nlists, int64_t nchunks, int64_t k0, int64_t max_chunks,
                          int64_t child_cap);
 
+/* Labels -> DuckDB ENUM positions.  Two conversions, one job:
+ *   strings (index_width 0): utf8 / large_utf8 rows are looked up byte-exactly in an open-addressing table of the ENUM's
+ *     labels (dmb_rev_enum_table); with out_width 0 ("remap" mode) the rows are an Arrow dictionary and each gets one
+ *     uint32 code in `out` (a position, DMB_ENUM_CODE_NULL for a NULL entry, DMB_ENUM_CODE_MISSING for a label the ENUM
+ *     lacks), no masks and no error;
+ *   dictionary indices (index_width 1/2/4/8, signed or not): row r's position is remap[index] (remap: the codes of the
+ *     Arrow dictionary, dict_len entries).
+ * Otherwise the output is final vectors: positions of out_width (1/2/4) bytes, chunk k at k*2048*out_width bytes, masks
+ * at k*32 words.  A NULL row, and a valid row whose dictionary entry is NULL, is NULL with payload 0.  A valid row whose
+ * label is not in the ENUM, or whose index is outside [0, dict_len), is an error: *error takes the smallest such row
+ * (atomicMin; the caller sets it to ~0 first) and the row is written as NULL. */
+struct dmb_enum_dict;
+#define DMB_ENUM_CODE_NULL 0xFFFFFFFEu
+#define DMB_ENUM_CODE_MISSING 0xFFFFFFFFu
+#define DMB_ENUM_SLOT_BYTES 32 /* one lookup-table slot: {position, length, hash, 0} {first 12 bytes, last 4 bytes} */
+typedef struct dmb_rev_enum_job {
+  const void *in_offsets;          /* strings: int32 (or int64 when large) offsets at the slice start: nrows + 1 entries */
+  const uint8_t *in_data;          /* strings: device copy of the data buffer, indexed by the offsets                    */
+  const void *in_indices;          /* indices: the first index of the slice                                              */
+  const uint8_t *in_validity;      /* bitmap or NULL                                                                      */
+  int64_t in_bit_offset;
+  const uint32_t *remap;           /* indices: [dict_len] codes                                                           */
+  int64_t dict_len;
+  const void *table;               /* strings: table_size slots of DMB_ENUM_SLOT_BYTES                                    */
+  const uint32_t *label_offsets;   /* strings: the ENUM's labels (dmb_enum_dict layout), read for labels > 16 bytes      */
+  const uint8_t *label_data;
+  void *out;
+  uint64_t *out_validity;
+  unsigned long long *null_count;
+  unsigned long long *error;
+  uint32_t table_size;             /* a power of two                                                                      */
+  int32_t out_width;               /* 1 / 2 / 4; 0: remap mode (strings only)                                             */
+  int32_t index_width;             /* 1 / 2 / 4 / 8; 0: strings                                                           */
+  int32_t index_signed;
+  int32_t large_offsets;
+  int32_t reserved;
+} dmb_rev_enum_job;
+
+int32_t dmb_dev_rev_enum_batch(const dmb_rev_enum_job *job, int64_t nrows, void *stream);
+/* host only: the lookup table of `dict` in table_size slots (a power of two above the label count), what
+ * dmb_dev_rev_enum_batch probes.  Returns 0 with the last error set for a table that is too small or a duplicate label. */
+int32_t dmb_rev_enum_table(const struct dmb_enum_dict *dict, uint32_t table_size, void *slots);
+/* host only: the position of `bytes` in such a table, -1 when it is not a label (the device's probe, run on the host) */
+int64_t dmb_rev_enum_lookup(const void *slots, uint32_t table_size, const struct dmb_enum_dict *dict, const uint8_t *bytes, uint32_t len);
+
 /* byte-per-row validity (MoonBit Array[Bool], src/duckdb_arrow_native.mbt:646-650) -> per-chunk
  * uint64 masks via warp ballots */
 int32_t dmb_dev_valid_bytes_to_masks(const uint8_t *valid_bytes, uint64_t *out_validity,
@@ -774,6 +819,14 @@ int32_t duckdb_mb_gpu_appender_set_list(duckdb_mb_gpu_appender *a, int32_t col, 
  * `*validity`: ceil(size / 64) mask words.  Host memory of the appender, valid until the sink call returns. */
 int32_t duckdb_mb_gpu_appender_list_child(duckdb_mb_gpu_appender *a, int32_t col, const void **data, const uint64_t **validity,
                                           uint64_t *size);
+/* ENUM columns: the type's labels (duckdb_enum_dictionary_value, copied) and its internal type (duckdb_enum_internal_type:
+ * UTINYINT / USMALLINT / UINTEGER), which is the width of the vector.  Refused: a column that is not ENUM, another
+ * internal type, more labels than it can index, a duplicate label, malformed offsets, a second, different declaration.
+ * A declared column then takes dictionary-encoded Arrow arrays (indices c C s S i I l L, dictionary u / U) and plain u / U
+ * arrays, and append_varchar / append_null cells of the row protocol; each label is matched byte-exactly.  A valid row
+ * whose label is not in the ENUM, or whose dictionary index is out of range, fails the append before its sub-batch reaches
+ * the sink; a row whose dictionary entry is NULL is NULL. */
+int32_t duckdb_mb_gpu_appender_set_enum(duckdb_mb_gpu_appender *a, int32_t col, int32_t internal_type_id, const dmb_enum_dict *dict);
 int32_t duckdb_mb_gpu_append_interval(duckdb_mb_gpu_appender *a, int32_t months, int32_t days, int64_t micros); /* :1511 */
 /* LIST / STRUCT / MAP cells: the reference serialises them as text -- `["a", "b"]` (:1735-1790), `{"k": "v", ...}`
  * (:1792-1858 struct, :1860-1926 map), items copied without escaping -- and appends the text as one VARCHAR cell

@@ -49,6 +49,38 @@ _CHILD_DTYPE = {ch.P_BOOL: np.uint8, ch.P_I8: np.int8, ch.P_I16: np.int16, ch.P_
                 ch.P_F32: np.float32, ch.P_F64: np.float64}
 
 
+def _values(raw: bytes, ct: int, dw: int, size: int) -> list:
+    """`size` values of a vector of type `ct` (DECIMAL width `dw`) as Python values, the forms `list_values` gives"""
+    phys = ch.phys_of_type(ct, dw)
+    if phys == ch.P_STRING:
+        e = np.frombuffer(raw, dtype=np.uint8).reshape(-1, 16)
+        vals = []
+        for i in range(size):
+            ln = int(e[i, 0:4].view(np.uint32)[0])
+            b = bytes(e[i, 4:4 + ln]) if ln <= 12 else C.string_at(int(e[i, 8:16].view(np.uint64)[0]), ln)
+            vals.append(b.decode() if ct == ch.T_VARCHAR else b)
+        return vals
+    if phys in (ch.P_I128, ch.P_U128):
+        return [int.from_bytes(raw[16 * i: 16 * i + 16], "little", signed=phys == ch.P_I128) for i in range(size)]
+    vals = np.frombuffer(raw, dtype=_CHILD_DTYPE[phys], count=size).tolist()
+    return [bool(v) for v in vals] if phys == ch.P_BOOL else vals
+
+
+def _field_spec(spec) -> tuple:
+    """(name, type_id, extra) of a STRUCT field spec: extra is the DECIMAL width, an ENUM's (internal type, labels) or a
+    nested STRUCT's field specs"""
+    name, t, *rest = spec
+    return name, t, (rest[0] if rest else None)
+
+
+def _field_width(t: int, extra) -> int:
+    if t == ch.T_STRUCT:
+        return 0
+    if t == ch.T_ENUM:
+        return np.dtype(_ENUM_DTYPE[extra[0]]).itemsize
+    return _out_width(t, extra or 0)
+
+
 class CollectedChunks:
     """Default sink: copies every chunk out of the appender's pinned buffers.
 
@@ -57,11 +89,15 @@ class CollectedChunks:
     chunk's child vector is copied too (through Appender.list_child, valid only inside the sink call)."""
 
     def __init__(self, type_ids: Sequence[int], dec_widths: Optional[Sequence[int]] = None, list_children: Optional[dict] = None,
-                 enums: Optional[dict] = None):
-        """`enums` maps an ENUM column to `(internal_type, labels)`: UTINYINT / USMALLINT / UINTEGER, the vector's width."""
+                 enums: Optional[dict] = None, structs: Optional[dict] = None):
+        """`enums` maps an ENUM column to `(internal_type, labels)`: UTINYINT / USMALLINT / UINTEGER, the vector's width.
+        `structs` maps a STRUCT column to its field specs `(name, type_id[, extra])`, extra: a DECIMAL field's width, an
+        ENUM field's `(internal_type, labels)`, a STRUCT field's own field specs; the field vectors are copied too (through
+        Appender.struct_field, valid only inside the sink call)."""
         self.type_ids = list(type_ids)
         self.enums = dict(enums or {})
-        self.widths = [np.dtype(_ENUM_DTYPE[self.enums[i][0]]).itemsize if t == ch.T_ENUM else
+        self.structs = dict(structs or {})
+        self.widths = [np.dtype(_ENUM_DTYPE[self.enums[i][0]]).itemsize if t == ch.T_ENUM else 0 if t == ch.T_STRUCT else
                        _out_width(t, (dec_widths or [0] * len(type_ids))[i]) for i, t in enumerate(type_ids)]
         self.counts: List[int] = []
         self.data: List[List[bytes]] = [[] for _ in type_ids]
@@ -69,26 +105,73 @@ class CollectedChunks:
         self.list_children = dict(list_children or {})
         self.child_data: dict = {c: [] for c in self.list_children}      # per chunk: child values, raw bytes
         self.child_validity: dict = {c: [] for c in self.list_children}  # per chunk: ceil(size / 64) mask words
+        self.field_data: dict = {}      # (column, field, nested field, ...) -> per chunk: the field's values, raw bytes
+        self.field_validity: dict = {}  # the same keys -> per chunk: 32 mask words
         self.appender: Optional["Appender"] = None  # set by the Appender this sink is given to
 
     def __call__(self, count: int, vec_data, vec_validity) -> bool:
         self.counts.append(count)
         for c, w in enumerate(self.widths):
-            self.data[c].append(C.string_at(vec_data[c], count * w))
+            self.data[c].append(C.string_at(vec_data[c], count * w) if w else b"")
             self.validity[c].append(np.frombuffer(C.string_at(vec_validity[c], 8 * ch.VALIDITY_WORDS), dtype=np.uint64).copy())
         for c, (ct, dw) in self.list_children.items():
             data, words, size = self.appender.list_child(c)
             self.child_data[c].append(C.string_at(data, size * _out_width(ct, dw)) if size else b"")
             nw = (size + 63) // 64
             self.child_validity[c].append(np.frombuffer(C.string_at(words, 8 * nw), dtype=np.uint64).copy() if nw else np.zeros(0, np.uint64))
+        for c, fields in self.structs.items():
+            self._copy_fields(c, (c,), fields, count)
         return True
+
+    def _copy_fields(self, col: int, key: tuple, fields, count: int) -> None:
+        for f, spec in enumerate(fields):
+            _, t, extra = _field_spec(spec)
+            data, words = self.appender.struct_field(col, f)
+            w = _field_width(t, extra)
+            self.field_data.setdefault(key + (f,), []).append(C.string_at(data, count * w) if w else b"")
+            self.field_validity.setdefault(key + (f,), []).append(
+                np.frombuffer(C.string_at(words, 8 * ch.VALIDITY_WORDS), dtype=np.uint64).copy())
+            if t == ch.T_STRUCT:
+                self._copy_fields(self.appender.struct_first[col] + f, key + (f,), extra, count)
+
+    def _bits(self, words: list) -> np.ndarray:
+        out = [np.unpackbits(m.view(np.uint8), bitorder="little")[:cnt].astype(bool) for m, cnt in zip(words, self.counts)]
+        return np.concatenate(out) if out else np.zeros(0, dtype=bool)
+
+    def field_bytes(self, key: tuple) -> bytes:
+        """the field vector of `key` = (column, field, nested field, ...), every chunk's values"""
+        return b"".join(self.field_data[key])
+
+    def field_valid_bits(self, key: tuple) -> np.ndarray:
+        """bool per row of the field vector of `key`"""
+        return self._bits(self.field_validity[key])
+
+    def struct_values(self, c: int) -> list:
+        """STRUCT column `c` as dicts of its fields (None: a NULL row or field), in the shape pyarrow's `to_pylist` gives;
+        field values in the forms of `list_values`, ENUM fields as their labels"""
+        return self._struct_rows((c,), self.structs[c], self.valid_bits(c))
+
+    def _struct_rows(self, key: tuple, fields, valid) -> list:
+        cols = []
+        for f, spec in enumerate(fields):
+            name, t, extra = _field_spec(spec)
+            fk = key + (f,)
+            fvalid = self.field_valid_bits(fk)
+            if t == ch.T_STRUCT:
+                vals = self._struct_rows(fk, extra, fvalid)
+            elif t == ch.T_ENUM:
+                pos = np.frombuffer(self.field_bytes(fk), dtype=_ENUM_DTYPE[extra[0]])
+                vals = [extra[1][int(p)] for p in pos]
+            else:
+                vals = [v for k, cnt in enumerate(self.counts) for v in _values(self.field_data[fk][k], t, extra or 0, cnt)]
+            cols.append((name, [v if ok else None for v, ok in zip(vals, fvalid)]))
+        return [{n: v[i] for n, v in cols} if valid[i] else None for i in range(len(valid))]
 
     def list_values(self, c: int) -> list:
         """LIST column `c` as Python lists (None: a NULL row or element).  Values: int (integers, DATE days,
         TIME / TIMESTAMP ticks, DECIMAL unscaled, HUGEINT / UHUGEINT / UUID as 128-bit integers), float, bool, str
         (VARCHAR) or bytes (BLOB).  Pointer string_t refer to the Arrow data buffer, which must still be alive."""
         ct, dw = self.list_children[c]
-        phys = ch.phys_of_type(ct, dw)
         out = []
         for k, cnt in enumerate(self.counts):
             ent = np.frombuffer(self.data[c][k], dtype=np.uint64).reshape(-1, 2)
@@ -96,19 +179,7 @@ class CollectedChunks:
             raw = self.child_data[c][k]
             size = len(raw) // _out_width(ct, dw)
             cvalid = np.unpackbits(self.child_validity[c][k].view(np.uint8), bitorder="little")[:size].astype(bool)
-            if phys == ch.P_STRING:
-                e = np.frombuffer(raw, dtype=np.uint8).reshape(-1, 16)
-                vals = []
-                for i in range(size):
-                    ln = int(e[i, 0:4].view(np.uint32)[0])
-                    b = bytes(e[i, 4:4 + ln]) if ln <= 12 else C.string_at(int(e[i, 8:16].view(np.uint64)[0]), ln)
-                    vals.append(b.decode() if ct == ch.T_VARCHAR else b)
-            elif phys in (ch.P_I128, ch.P_U128):
-                vals = [int.from_bytes(raw[16 * i: 16 * i + 16], "little", signed=phys == ch.P_I128) for i in range(size)]
-            else:
-                vals = np.frombuffer(raw, dtype=_CHILD_DTYPE[phys]).tolist()
-                if phys == ch.P_BOOL:
-                    vals = [bool(v) for v in vals]
+            vals = _values(raw, ct, dw, size)
             for i in range(cnt):
                 if not valid[i]:
                     out.append(None)
@@ -150,6 +221,7 @@ class Appender:
         self.lib = ctx.lib
         self.ctx = ctx
         self.type_ids = list(type_ids)
+        self.struct_first: dict = {}  # STRUCT column or field column -> its first field column (set_struct)
         self._sink_py = sink
         n = len(self.type_ids)
 
@@ -236,6 +308,24 @@ class Appender:
         what duckdb_enum_internal_type reports); needed before Arrow arrays or append_varchar cells reach that column."""
         d, keep = enum_dict(labels)
         self._check(self.lib.duckdb_mb_gpu_appender_set_enum(self.handle, int(col), int(internal_type), C.byref(d)), "set_enum")
+
+    def set_struct(self, col: int, field_types: Sequence[int]) -> int:
+        """A STRUCT column's field types (what duckdb_struct_type_child_type of duckdb_appender_column_type reports), by
+        position; needed before an Arrow struct reaches that column.  Returns the first of the field columns the fields
+        become, which set_decimal / set_enum / set_struct take to declare DECIMAL and ENUM fields and nested STRUCTs."""
+        ids = (C.c_int32 * max(len(field_types), 1))(*field_types)
+        first = C.c_int32(-1)
+        self._check(self.lib.duckdb_mb_gpu_appender_set_struct(self.handle, int(col), len(field_types), ids, C.byref(first)), "set_struct")
+        self.struct_first[int(col)] = first.value
+        return first.value
+
+    def struct_field(self, col: int, field: int):
+        """Inside a sink call: (values pointer or None for a STRUCT field, mask pointer) of field `field` of STRUCT column
+        `col` (a table column or a field column) for the chunk being handed over."""
+        data, words = C.c_void_p(), C.c_void_p()
+        self._check(self.lib.duckdb_mb_gpu_appender_struct_field(self.handle, int(col), int(field), C.byref(data), C.byref(words)),
+                    "struct_field")
+        return data.value, words.value
 
     def list_child(self, col: int):
         """Inside a sink call: (child values pointer, child mask pointer, child size) of LIST column `col`."""

@@ -18,6 +18,8 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include <string>
+
 #include "host_common.hpp"
 
 namespace dmb {
@@ -57,6 +59,10 @@ struct ColInput {
   const uint8_t *dict_offsets = nullptr;  // dictionary indices: the Arrow dictionary (utf8 / large_utf8) at its own offset
   const uint8_t *dict_data = nullptr, *dict_validity = nullptr;
   int64_t dict_bit_offset = 0, dict_len = 0;
+  // STRUCT: a mask and no payload (w_out 0).  Field columns follow the table's columns; `parent`: the STRUCT column
+  // whose masks a field column's rows are ANDed with (-1: a table column)
+  bool is_struct = false;
+  int parent = -1;
 };
 
 // an ENUM column's labels and internal width (duckdb_mb_gpu_appender_set_enum); width 0: not declared
@@ -71,6 +77,20 @@ struct EnumDecl {
 // the table's child type of a LIST column (duckdb_mb_gpu_appender_set_list); type_id 0: not declared
 struct ListDecl {
   int32_t type_id = 0, dec_width = 0, dec_scale = 0;
+};
+
+// a STRUCT column's fields (duckdb_mb_gpu_appender_set_struct): field columns first .. first + types.size() - 1;
+// first -1: not declared
+struct StructDecl {
+  int32_t first = -1;
+  std::vector<int32_t> types;
+};
+
+// what duckdb_mb_gpu_appender_struct_field hands out during a sink call, per column: the sub-batch's vectors and masks
+struct SinkCol {
+  const uint8_t *data = nullptr;  // NULL for a STRUCT column
+  const uint64_t *masks = nullptr;
+  int w = 0;
 };
 
 // what duckdb_mb_gpu_appender_list_child hands out during a sink call, per LIST column
@@ -89,7 +109,7 @@ using namespace dmb;
 
 struct duckdb_mb_gpu_appender {
   std::shared_ptr<CtxCore> core;
-  int32_t ncols = 0;
+  int32_t ncols = 0;                    // table columns; field columns of STRUCTs follow them in the per-column vectors
   std::vector<int32_t> type_ids;
   dmb_chunk_sink sink = nullptr;
   void *user = nullptr;
@@ -102,7 +122,10 @@ struct duckdb_mb_gpu_appender {
   std::vector<RowBuf> rows;
   std::vector<ListDecl> lists;
   std::vector<EnumDecl> enums;
-  std::vector<SinkList> sink_lists;  // valid while sink_chunk >= 0: chunk sink_chunk of the sub-batch being handed over
+  std::vector<StructDecl> structs;
+  std::vector<int32_t> parent, field_index;  // field columns: the STRUCT column and the position in it (-1: table column)
+  std::vector<SinkList> sink_lists;
+  std::vector<SinkCol> sink_cols;  // valid while sink_chunk >= 0, every column and field column  // valid while sink_chunk >= 0: chunk sink_chunk of the sub-batch being handed over
   int64_t sink_chunk = -1;
   int64_t sub_rows = 4 << 20;
   int64_t list_child_cap = 0;  // kListChildCap unless DMB_REV_LIST_CHILD_CAP says otherwise
@@ -122,6 +145,13 @@ int32_t fail(App *a, const char *fmt, ...) {
   va_end(ap);
   set_error("%s", a->error);
   return 0;
+}
+
+// how messages name column c: "column 3", or for a field column the table column and the field path, "column 2, field 1.0"
+std::string col_name(const App *a, int c) {
+  std::string path;
+  for (; c >= a->ncols; c = a->parent[(size_t)c]) path = std::to_string(a->field_index[(size_t)c]) + (path.empty() ? "" : "." + path);
+  return "column " + std::to_string(c) + (path.empty() ? "" : ", field " + path);
 }
 
 // any command the model does not allow in the current state moves it to Error
@@ -163,7 +193,7 @@ int copy_op(int w) {
 // The values must be decimal128 with the column's scale and a precision that fits its width; they are narrowed to the
 // column's physical width (int16 / int32 / int64 / int128 for w <= 4 / 9 / 18 / 38), which keeps every value within
 // the Arrow precision exact.  *w == 0: the column is not declared yet, and this Arrow type declares it.
-bool map_decimal(App *a, int c, const char *what, const char *fmt, int32_t type_id, int32_t *w, int32_t *s, ColInput *in) {
+bool map_decimal(App *a, const char *cn, const char *what, const char *fmt, int32_t type_id, int32_t *w, int32_t *s, ColInput *in) {
   // d:p,s[,bits]: each field one to three decimal digits, nothing else
   long f[3] = {0, 0, 128};
   int nf = 0;
@@ -180,24 +210,24 @@ bool map_decimal(App *a, int c, const char *what, const char *fmt, int32_t type_
   else if (*w) snprintf(col, sizeof(col), "DECIMAL(%d,%d)", *w, *s);
   else snprintf(col, sizeof(col), "DECIMAL");
   if (nf < 2 || q[-1] != '\0') {
-    fail(a, "column %d: Arrow %s '%s' is not a decimal format", c, what, fmt);
+    fail(a, "%s: Arrow %s '%s' is not a decimal format", cn, what, fmt);
     return false;
   }
   if (bits != 128) {
-    fail(a, "column %d: Arrow %s '%s' is a %ld-bit decimal; only decimal128 can be appended to a %s column", c, what, fmt, bits, col);
+    fail(a, "%s: Arrow %s '%s' is a %ld-bit decimal; only decimal128 can be appended to a %s column", cn, what, fmt, bits, col);
     return false;
   }
   if (p < 1 || p > 38 || sc > p) {
-    fail(a, "column %d: Arrow %s '%s' is not a DECIMAL(width, scale) DuckDB can store", c, what, fmt);
+    fail(a, "%s: Arrow %s '%s' is not a DECIMAL(width, scale) DuckDB can store", cn, what, fmt);
     return false;
   }
   if (*w == 0) { *w = (int32_t)p; *s = (int32_t)sc; }
   if (sc != *s) {
-    fail(a, "column %d: Arrow %s '%s' has scale %ld; the column is %s", c, what, fmt, sc, col);
+    fail(a, "%s: Arrow %s '%s' has scale %ld; the column is %s", cn, what, fmt, sc, col);
     return false;
   }
   if (p > *w) {
-    fail(a, "column %d: Arrow %s '%s' has precision %ld; the column is %s", c, what, fmt, p, col);
+    fail(a, "%s: Arrow %s '%s' has precision %ld; the column is %s", cn, what, fmt, p, col);
     return false;
   }
   in->w_in = 16;
@@ -210,7 +240,7 @@ bool map_decimal(App *a, int c, const char *what, const char *fmt, int32_t type_
 
 // Arrow format string of a child -> conversion for a DuckDB column of `type_id`; `dec_w` / `dec_s`: the column's
 // DECIMAL(w, s) when it is one (w == 0: not declared yet, set from the Arrow type)
-bool map_format(App *a, int c, const char *what, const char *fmt, int32_t type_id, int32_t *dec_w, int32_t *dec_s, ColInput *in) {
+bool map_format(App *a, const char *cn, const char *what, const char *fmt, int32_t type_id, int32_t *dec_w, int32_t *dec_s, ColInput *in) {
   auto fixed = [&](int w) { in->rev_op = copy_op(w); in->w_in = w; in->w_out = w; return true; };
   auto is = [&](const char *f) { return strcmp(fmt, f) == 0; };
   auto starts = [&](const char *f) { return strncmp(fmt, f, strlen(f)) == 0; };
@@ -239,11 +269,11 @@ bool map_format(App *a, int c, const char *what, const char *fmt, int32_t type_i
     case DMB_TYPE_HUGEINT:
       if (starts("d:")) {  // the unscaled integer of a decimal128 with scale 0
         int32_t w = 38, s = 0;
-        return map_decimal(a, c, what, fmt, type_id, &w, &s, in);
+        return map_decimal(a, cn, what, fmt, type_id, &w, &s, in);
       }
       break;
     case DMB_TYPE_UHUGEINT: case DMB_TYPE_UUID: if (is("w:16")) return fixed(16); break;
-    case DMB_TYPE_DECIMAL: if (starts("d:")) return map_decimal(a, c, what, fmt, type_id, dec_w, dec_s, in); break;
+    case DMB_TYPE_DECIMAL: if (starts("d:")) return map_decimal(a, cn, what, fmt, type_id, dec_w, dec_s, in); break;
     case DMB_TYPE_VARCHAR:
       if (is("u") || is("U")) { in->is_string = true; in->large = is("U"); in->w_out = 16; return true; }
       break;
@@ -252,7 +282,7 @@ bool map_format(App *a, int c, const char *what, const char *fmt, int32_t type_i
       break;
     default: break;
   }
-  fail(a, "column %d: Arrow %s '%s' cannot be appended to a column of DuckDB type %d", c, what, fmt, type_id);
+  fail(a, "%s: Arrow %s '%s' cannot be appended to a column of DuckDB type %d", cn, what, fmt, type_id);
   return false;
 }
 
@@ -295,7 +325,7 @@ int64_t offset_at(const ColInput &ci, int64_t row) {
 }
 
 // the appender error for the first offending row of an ENUM column, rendered from the host buffers
-int32_t enum_error(App *a, int c, const ColInput &ci, int64_t row) {
+int32_t enum_error(App *a, const char *cn, const ColInput &ci, int64_t row) {
   const uint8_t *p;
   int64_t len;
   if (ci.is_string) {
@@ -308,7 +338,7 @@ int32_t enum_error(App *a, int c, const ColInput &ci, int64_t row) {
     const int sh = 64 - 8 * ci.w_in;
     const int64_t idx = ci.index_signed ? (int64_t)(raw << sh) >> sh : (int64_t)raw;
     if (idx < 0 || idx >= ci.dict_len)
-      return fail(a, "column %d, row %lld: dictionary index %lld is outside the Arrow dictionary (%lld entries)", c, (long long)row,
+      return fail(a, "%s, row %lld: dictionary index %lld is outside the Arrow dictionary (%lld entries)", cn, (long long)row,
                   (long long)idx, (long long)ci.dict_len);
     ColInput d;
     d.offsets = ci.dict_offsets;
@@ -318,7 +348,7 @@ int32_t enum_error(App *a, int c, const ColInput &ci, int64_t row) {
     len = offset_at(d, idx + 1) - o0;
   }
   const int shown = len > 160 ? 160 : (int)len;  // the message fits the 256-byte error buffer
-  return fail(a, "column %d, row %lld: '%.*s'%s is not a label of the ENUM", c, (long long)row, shown, (const char *)p,
+  return fail(a, "%s, row %lld: '%.*s'%s is not a label of the ENUM", cn, (long long)row, shown, (const char *)p,
               len > shown ? "..." : "");
 }
 
@@ -331,11 +361,17 @@ int32_t sink_slot(App *a, Slot &s, const std::vector<ColInput> &cols, const std:
     if (cols[(size_t)c].is_list && s.h_err[c])
       return fail(a, "column %d: Arrow list offsets decrease within rows [%lld, %lld)", c, (long long)s.r0, (long long)s.r1);
     else if (cols[(size_t)c].is_enum && s.h_eerr[c] != ~0ull)
-      return enum_error(a, c, cols[(size_t)c], s.r0 + (int64_t)s.h_eerr[c]);
+      return enum_error(a, col_name(a, c).c_str(), cols[(size_t)c], s.r0 + (int64_t)s.h_eerr[c]);
   if (!a->sink) return 1;
-  std::vector<const void *> vd((size_t)nc);
-  std::vector<const uint64_t *> vv((size_t)nc);
+  const int nt = a->ncols;  // the sink sees the table's columns; field columns through duckdb_mb_gpu_appender_struct_field
+  std::vector<const void *> vd((size_t)nt);
+  std::vector<const uint64_t *> vv((size_t)nt);
   a->sink_lists.assign((size_t)nc, SinkList());
+  a->sink_cols.assign((size_t)nc, SinkCol());
+  for (int c = 0; c < nc; ++c) {
+    const int w = cols[(size_t)c].w_out;
+    a->sink_cols[(size_t)c] = SinkCol{w ? s.h_out[(size_t)c] : nullptr, s.h_val[(size_t)c], w};
+  }
   for (int c = 0; c < nc; ++c)
     if (cols[(size_t)c].is_list) {
       const ListOut &lo = s.lists[(size_t)c];
@@ -344,12 +380,13 @@ int32_t sink_slot(App *a, Slot &s, const std::vector<ColInput> &cols, const std:
     }
   for (int64_t r = s.r0, k = 0; r < s.r1; r += DMB_VECTOR_SIZE, ++k) {
     const uint32_t count = (uint32_t)(s.r1 - r < DMB_VECTOR_SIZE ? s.r1 - r : DMB_VECTOR_SIZE);
-    for (int c = 0; c < nc; ++c) {
-      vd[(size_t)c] = s.h_out[(size_t)c] + (size_t)k * DMB_VECTOR_SIZE * (size_t)cols[(size_t)c].w_out;
+    for (int c = 0; c < nt; ++c) {
+      const int w = cols[(size_t)c].w_out;
+      vd[(size_t)c] = w ? s.h_out[(size_t)c] + (size_t)k * DMB_VECTOR_SIZE * (size_t)w : nullptr;
       vv[(size_t)c] = s.h_val[(size_t)c] + (size_t)k * DMB_VALIDITY_WORDS;
     }
     a->sink_chunk = k;
-    const int32_t ok = a->sink(a->user, nc, count, vd.data(), vv.data());
+    const int32_t ok = a->sink(a->user, nt, count, vd.data(), vv.data());
     a->sink_chunk = -1;
     if (!ok) return fail(a, "chunk sink aborted at row %lld", (long long)r);
   }
@@ -561,9 +598,9 @@ int32_t convert_rows(App *a, const std::vector<ColInput> &cols, int64_t nrows) {
     if (!slots[s].ev_out || !slots[s].d_err || !slots[s].h_err || !slots[s].d_eerr || !slots[s].h_eerr) return fail(a, "%s", duckdb_mb_gpu_last_error());
     for (int j = 0; j < nc; ++j) {
       const size_t ob = (size_t)sub * (size_t)cols[(size_t)j].w_out, vb = (size_t)sub_chunks * DMB_VALIDITY_WORDS * 8;
-      uint8_t *d = (uint8_t *)sc.dalloc(ob), *h = (uint8_t *)sc.palloc(ob);
+      uint8_t *d = ob ? (uint8_t *)sc.dalloc(ob) : nullptr, *h = ob ? (uint8_t *)sc.palloc(ob) : nullptr;  // STRUCT: no payload
       uint64_t *dv = (uint64_t *)sc.dalloc(vb), *hv = (uint64_t *)sc.palloc(vb);
-      if (!d || !h || !dv || !hv) return fail(a, "%s", duckdb_mb_gpu_last_error());
+      if ((ob && (!d || !h)) || !dv || !hv) return fail(a, "%s", duckdb_mb_gpu_last_error());
       slots[s].d_out.push_back(d);
       slots[s].h_out.push_back(h);
       slots[s].d_val.push_back(dv);
@@ -575,6 +612,34 @@ int32_t convert_rows(App *a, const std::vector<ColInput> &cols, int64_t nrows) {
         if (!lo.d_cword || !lo.h_cword) return fail(a, "%s", duckdb_mb_gpu_last_error());
       }
     }
+  }
+  // STRUCT columns: a column is "masked" when it or an ancestor STRUCT has an Arrow bitmap.  Then rev_mask_kernel writes
+  // its masks from its bitmap AND its parent's masks, and for each field that is not a STRUCT the parent's masks AND the
+  // field's bitmap into comb[slot][field], which the field's conversion reads as its validity.  Jobs of nesting level d
+  // read the masks of level d - 1: one launch per level.  (A field column's number is above its parent's.)
+  std::vector<char> masked((size_t)nc, 0);
+  std::vector<int> depth((size_t)nc, 0);
+  int levels = 0;
+  for (int j = 0; j < nc; ++j) {
+    const ColInput &ci = cols[(size_t)j];
+    const int p = ci.parent;
+    depth[(size_t)j] = p < 0 ? 0 : depth[(size_t)p] + 1;
+    if (ci.is_struct) masked[(size_t)j] = ci.validity != nullptr || (p >= 0 && masked[(size_t)p]);
+    if (ci.is_struct || (p >= 0 && masked[(size_t)p])) levels = depth[(size_t)j] + 1 > levels ? depth[(size_t)j] + 1 : levels;
+  }
+  std::vector<uint64_t *> comb((size_t)nslots * (size_t)nc, nullptr);
+  dmb_rev_mask_job *h_mjobs = nullptr, *d_mjobs = nullptr;
+  if (levels) {
+    h_mjobs = (dmb_rev_mask_job *)sc.palloc(sizeof(dmb_rev_mask_job) * (size_t)nc * 2);
+    d_mjobs = (dmb_rev_mask_job *)sc.dalloc(sizeof(dmb_rev_mask_job) * (size_t)nc * 2);
+    if (!h_mjobs || !d_mjobs) return fail(a, "%s", duckdb_mb_gpu_last_error());
+    for (int s = 0; s < nslots; ++s)
+      for (int j = 0; j < nc; ++j)
+        if (!cols[(size_t)j].is_struct && cols[(size_t)j].parent >= 0 && masked[(size_t)cols[(size_t)j].parent]) {
+          uint64_t *&cb = comb[(size_t)s * (size_t)nc + (size_t)j];
+          cb = (uint64_t *)sc.dalloc((size_t)(sub_chunks + 1) * DMB_VALIDITY_WORDS * 8);  // + 1 chunk: a BOOLEAN field's bit phase
+          if (!cb) return fail(a, "%s", duckdb_mb_gpu_last_error());
+        }
   }
   // per-slot device inputs: [slot][column], and the child arrays of LIST columns; sized up front for the columns that
   // are not LISTs, grown on demand for the child ranges
@@ -621,15 +686,38 @@ int32_t convert_rows(App *a, const std::vector<ColInput> &cols, int64_t nrows) {
     std::vector<int64_t> child_rows;  // element count of each child job: fixed-width ones first, in job order
     std::vector<int64_t> str_rows;
     std::vector<int> masks_from_bytes;  // columns
+    std::vector<std::vector<dmb_rev_mask_job>> mask_levels((size_t)levels);
     for (int j = 0; j < nc; ++j) {
       const ColInput &ci = cols[(size_t)j];
       InBuf &ib = inbuf[(size_t)si * (size_t)nc + (size_t)j];
       const uint8_t *d_validity = nullptr;
       int64_t bit_off = 0;
+      const bool under_mask = ci.parent >= 0 && masked[(size_t)ci.parent];
+      const uint8_t *parent_masks = under_mask ? (const uint8_t *)slot.d_val[(size_t)ci.parent] : nullptr;
+      if (ci.is_struct) {  // its masks only: own bitmap AND the parent's masks
+        if (ci.validity) {
+          bit_off = stage_bits(a, sc, ib.validity, ib.validity_cap, ci.validity, ci.bit_offset + r0, ci.bit_offset + r1);
+          if (bit_off < 0) return fail(a, "%s", duckdb_mb_gpu_last_error());
+          d_validity = ib.validity;
+        }
+        mask_levels[(size_t)depth[(size_t)j]].push_back(dmb_rev_mask_job{parent_masks, 0, d_validity, bit_off, slot.d_val[(size_t)j], 0});
+        continue;
+      }
       if (!ci.is_list) {
         dmb_rev_string_job sj;
         if (!stage_rows(a, sc, ci, ib, j, r0, r1, slot.d_out[(size_t)j], slot.d_val[(size_t)j], &hj[nfixed], &sj, &d_validity, &bit_off)) return 0;
         if (ci.valid_bytes) masks_from_bytes.push_back(j);
+        if (under_mask) {  // the conversion reads parent masks AND own bitmap; a BOOLEAN field at its values' bit phase
+          uint64_t *cb = comb[(size_t)si * (size_t)nc + (size_t)j];
+          const int64_t phase = ci.is_bits ? hj[nfixed].in_bit_offset : 0;
+          mask_levels[(size_t)depth[(size_t)j]].push_back(dmb_rev_mask_job{parent_masks, 0, d_validity, bit_off, cb, phase});
+          d_validity = (const uint8_t *)cb;
+          bit_off = phase;
+          hj[nfixed].in_validity = d_validity;
+          hj[nfixed].in_bit_offset = phase;
+          sj.in_validity = d_validity;
+          sj.in_bit_offset = 0;
+        }
         if (ci.is_enum) {
           dmb_rev_enum_job ej = enum_base[(size_t)j];
           if (ci.is_string) {
@@ -706,6 +794,16 @@ int32_t convert_rows(App *a, const std::vector<ColInput> &cols, int64_t nrows) {
       InBuf &ib = inbuf[(size_t)si * (size_t)nc + (size_t)j];
       if (dmb_dev_valid_bytes_to_masks(ib.validity, (uint64_t *)ib.masks, nullptr, n, c.s_compute)) return fail(a, "%s", duckdb_mb_gpu_last_error());
     }
+    if (levels) {  // STRUCT masks and the combined bitmaps of the fields, level by level, before the conversions read them
+      dmb_rev_mask_job *hm = h_mjobs + (size_t)si * (size_t)nc, *dm = d_mjobs + (size_t)si * (size_t)nc;
+      size_t nm = 0;
+      for (const auto &lv : mask_levels)
+        for (const auto &mj : lv) hm[nm++] = mj;
+      if (nm && check_cuda(cudaMemcpyAsync(dm, hm, sizeof(dmb_rev_mask_job) * nm, cudaMemcpyHostToDevice, c.s_compute), "mask job H2D"))
+        return fail(a, "%s", duckdb_mb_gpu_last_error());
+      for (size_t l = 0, at = 0; l < mask_levels.size(); at += mask_levels[l].size(), ++l)
+        if (dmb_dev_rev_mask_batch(dm + at, hm + at, (int32_t)mask_levels[l].size(), n, c.s_compute)) return fail(a, "%s", duckdb_mb_gpu_last_error());
+    }
     if (nfixed || nchild_fixed) {
       const size_t njobs = nchild_fixed ? (size_t)nc + (size_t)nchild_fixed : (size_t)nfixed;
       if (check_cuda(cudaMemcpyAsync(dj, hj, sizeof(dmb_rev_fixed_job) * njobs, cudaMemcpyHostToDevice, c.s_compute), "job H2D")) return fail(a, "%s", duckdb_mb_gpu_last_error());
@@ -729,7 +827,7 @@ int32_t convert_rows(App *a, const std::vector<ColInput> &cols, int64_t nrows) {
     if (check_cuda(cudaStreamWaitEvent(c.s_out, ev_k, 0), "wait kernels")) return fail(a, "%s", duckdb_mb_gpu_last_error());
     for (int j = 0; j < nc; ++j) {
       const size_t ob = (size_t)n * (size_t)cols[(size_t)j].w_out, vb = (size_t)nch * DMB_VALIDITY_WORDS * 8;
-      if (check_cuda(cudaMemcpyAsync(slot.h_out[(size_t)j], slot.d_out[(size_t)j], ob, cudaMemcpyDeviceToHost, c.s_out), "vectors D2H") ||
+      if ((ob && check_cuda(cudaMemcpyAsync(slot.h_out[(size_t)j], slot.d_out[(size_t)j], ob, cudaMemcpyDeviceToHost, c.s_out), "vectors D2H")) ||
           check_cuda(cudaMemcpyAsync(slot.h_val[(size_t)j], slot.d_val[(size_t)j], vb, cudaMemcpyDeviceToHost, c.s_out), "validity D2H"))
         return fail(a, "%s", duckdb_mb_gpu_last_error());
       a->bytes_d2h += ob + vb;
@@ -904,7 +1002,7 @@ bool map_list(App *a, int j, const ArrowArray *arr, const ArrowSchema *sch, ColI
     return false;
   }
   int32_t dec_w = d.dec_width, dec_s = d.dec_scale;  // a DECIMAL child: set_list declared it
-  if (!map_format(a, j, "list child format", cfmt, d.type_id, &dec_w, &dec_s, child)) {
+  if (!map_format(a, col_name(a, j).c_str(), "list child format", cfmt, d.type_id, &dec_w, &dec_s, child)) {
     const bool decimal_child = d.type_id == DMB_TYPE_DECIMAL || d.type_id == DMB_TYPE_HUGEINT;
     if (!decimal_child || strncmp(cfmt, "d:", 2) != 0)  // map_decimal's refusal names its own reason
       fail(a, "column %d: Arrow list child format '%s' does not match the declared child type %d", j, cfmt, d.type_id);
@@ -924,13 +1022,36 @@ bool map_list(App *a, int j, const ArrowArray *arr, const ArrowSchema *sch, ColI
   return true;
 }
 
+// an Arrow struct array for a STRUCT column whose fields are declared (duckdb_mb_gpu_appender_set_struct); map_column maps
+// the fields
+bool map_struct(App *a, int j, const char *cn, const ArrowArray *arr, const ArrowSchema *sch, ColInput *ci) {
+  const char *fmt = sch->format;
+  if (strcmp(fmt, "+s") != 0) {
+    if (fmt[0] == '+') fail(a, "%s: an Arrow %s ('%s') cannot be appended to a STRUCT column", cn, nested_name(fmt), fmt);
+    else fail(a, "%s: Arrow format '%s' cannot be appended to a STRUCT column", cn, fmt);
+    return false;
+  }
+  const StructDecl &d = a->structs[(size_t)j];
+  if (d.first < 0) {
+    fail(a, "%s: the STRUCT column's fields are not declared (duckdb_mb_gpu_appender_set_struct)", cn);
+    return false;
+  }
+  if (arr->n_children != (int64_t)d.types.size() || sch->n_children != (int64_t)d.types.size() || !arr->children || !sch->children) {
+    fail(a, "%s: the Arrow struct has %lld fields, the STRUCT column %d", cn, (long long)arr->n_children, (int)d.types.size());
+    return false;
+  }
+  ci->is_struct = true;
+  ci->w_out = 0;
+  return true;
+}
+
 // an Arrow array for an ENUM column: a dictionary array (indices c C s S i I l L, labels u / U) or plain u / U labels
-bool map_enum(App *a, int j, const ArrowArray *arr, const ArrowSchema *sch, ColInput *ci) {
+bool map_enum(App *a, int j, const char *cn, const ArrowArray *arr, const ArrowSchema *sch, ColInput *ci) {
   static const uint8_t kNoData[16] = {0};
   const char *fmt = sch->format;
   const EnumDecl &e = a->enums[(size_t)j];
   if (!e.width) {
-    fail(a, "column %d: the ENUM column's labels are not declared (duckdb_mb_gpu_appender_set_enum)", j);
+    fail(a, "%s: the ENUM column's labels are not declared (duckdb_mb_gpu_appender_set_enum)", cn);
     return false;
   }
   ci->is_enum = true;
@@ -942,24 +1063,24 @@ bool map_enum(App *a, int j, const ArrowArray *arr, const ArrowSchema *sch, ColI
       ci->large = fmt[0] == 'U';
       return true;
     }
-    if (strcmp(fmt, "vu") == 0) fail(a, "column %d: Arrow string views ('vu') cannot be appended to an ENUM column", j);
-    else if (integer) fail(a, "column %d: a bare Arrow integer array ('%s') cannot be appended to an ENUM column: pass a dictionary array or utf8 labels", j, fmt);
-    else if (fmt[0] == '+') fail(a, "column %d: an Arrow %s ('%s') cannot be appended to an ENUM column", j, nested_name(fmt), fmt);
-    else fail(a, "column %d: Arrow format '%s' cannot be appended to an ENUM column", j, fmt);
+    if (strcmp(fmt, "vu") == 0) fail(a, "%s: Arrow string views ('vu') cannot be appended to an ENUM column", cn);
+    else if (integer) fail(a, "%s: a bare Arrow integer array ('%s') cannot be appended to an ENUM column: pass a dictionary array or utf8 labels", cn, fmt);
+    else if (fmt[0] == '+') fail(a, "%s: an Arrow %s ('%s') cannot be appended to an ENUM column", cn, nested_name(fmt), fmt);
+    else fail(a, "%s: Arrow format '%s' cannot be appended to an ENUM column", cn, fmt);
     return false;
   }
   const char *dfmt = sch->dictionary->format ? sch->dictionary->format : "";
   if (!integer) {
-    fail(a, "column %d: Arrow dictionary index format '%s' cannot be appended to an ENUM column", j, fmt);
+    fail(a, "%s: Arrow dictionary index format '%s' cannot be appended to an ENUM column", cn, fmt);
     return false;
   }
   if (strcmp(dfmt, "u") != 0 && strcmp(dfmt, "U") != 0) {
-    fail(a, "column %d: an Arrow dictionary of '%s' values cannot be appended to an ENUM column (the labels must be utf8 or large_utf8)", j, dfmt);
+    fail(a, "%s: an Arrow dictionary of '%s' values cannot be appended to an ENUM column (the labels must be utf8 or large_utf8)", cn, dfmt);
     return false;
   }
   const ArrowArray *d = arr->dictionary;
   if (!d) {
-    fail(a, "column %d: the Arrow dictionary array is missing", j);
+    fail(a, "%s: the Arrow dictionary array is missing", cn);
     return false;
   }
   const char f = fmt[0];
@@ -973,7 +1094,51 @@ bool map_enum(App *a, int j, const ArrowArray *arr, const ArrowSchema *sch, ColI
   ci->dict_offsets = d->n_buffers > 1 && d->buffers[1] ? (const uint8_t *)d->buffers[1] + (size_t)d->offset * (ci->dict_large ? 8 : 4) : nullptr;
   ci->dict_data = d->n_buffers > 2 && d->buffers[2] ? (const uint8_t *)d->buffers[2] : kNoData;
   if (d->length > 0 && !ci->dict_offsets) {
-    fail(a, "column %d: the Arrow dictionary has no offsets buffer", j);
+    fail(a, "%s: the Arrow dictionary has no offsets buffer", cn);
+    return false;
+  }
+  return true;
+}
+
+// Arrow array `arr` -> column j (a table column or a field column) of `cols`: row i of the batch is logical row at + i of
+// `arr`.  A STRUCT maps its fields the same way, at arr->offset + at: in the Arrow C data interface a struct's offset is not
+// applied to its children.
+bool map_column(App *a, int j, const ArrowArray *arr, const ArrowSchema *sch, int64_t at, int64_t n, std::vector<ColInput> &cols,
+                std::vector<ColInput> &children) {
+  const std::string name = col_name(a, j);
+  const char *cn = name.c_str();
+  const bool field = j >= a->ncols;
+  ColInput &ci = cols[(size_t)j];
+  const int32_t t = a->type_ids[(size_t)j];
+  if (arr && sch && sch->format && field && sch->format[0] == '+' && t != DMB_TYPE_STRUCT) {
+    fail(a, "%s: an Arrow %s field ('%s') cannot be appended to a STRUCT", cn, nested_name(sch->format), sch->format);
+    return false;
+  }
+  if (!arr || !sch || !sch->format ||
+      !(t == DMB_TYPE_LIST ? map_list(a, j, arr, sch, &ci, &children[(size_t)j])
+        : t == DMB_TYPE_ENUM ? map_enum(a, j, cn, arr, sch, &ci)
+        : t == DMB_TYPE_STRUCT ? map_struct(a, j, cn, arr, sch, &ci)
+                               : map_format(a, cn, field ? "field format" : "format", sch->format, t, &a->rows[(size_t)j].dec_prec,
+                                            &a->rows[(size_t)j].dec_scale, &ci))) {
+    if (!a->error[0]) fail(a, "append_arrow_batch: %s is malformed", cn);
+    return false;
+  }
+  if (arr->length < at + n) {
+    if (field) fail(a, "append_arrow_batch: %s is shorter than the rows it is read at (%lld of %lld)", cn, (long long)arr->length, (long long)(at + n));
+    else fail(a, "append_arrow_batch: %s is shorter than the batch", cn);
+    return false;
+  }
+  bind_buffers(ci, arr, arr->offset + at);
+  if (ci.is_struct) {
+    const StructDecl &d = a->structs[(size_t)j];
+    for (int f = 0; f < (int)d.types.size(); ++f) {
+      cols[(size_t)(d.first + f)].parent = j;
+      if (!map_column(a, d.first + f, arr->children[f], sch->children[f], arr->offset + at, n, cols, children)) return false;
+    }
+    return true;
+  }
+  if (n > 0 && (((ci.is_string || ci.is_list) && !ci.offsets) || (!ci.is_string && !ci.is_list && !ci.values))) {
+    fail(a, "append_arrow_batch: %s has no value buffer", cn);
     return false;
   }
   return true;
@@ -1000,6 +1165,9 @@ extern "C" duckdb_mb_gpu_appender *duckdb_mb_gpu_appender_create(duckdb_mb_gpu_c
   a->rows.resize((size_t)ncols);
   a->lists.resize((size_t)ncols);
   a->enums.resize((size_t)ncols);
+  a->structs.resize((size_t)ncols);
+  a->parent.assign((size_t)ncols, -1);
+  a->field_index.assign((size_t)ncols, -1);
   for (int j = 0; j < ncols; ++j) {
     a->rows[(size_t)j].width = row_width(type_ids[j]);  // -1: column only reachable through Arrow batches
     a->rows[(size_t)j].offsets.assign(1, 0);
@@ -1057,32 +1225,13 @@ extern "C" int32_t duckdb_mb_gpu_append_arrow_batch(duckdb_mb_gpu_appender *a, c
     return 0;
   }
   const int64_t n = batch->length;
-  std::vector<ColInput> cols((size_t)a->ncols), children((size_t)a->ncols);
-  for (int j = 0; j < a->ncols; ++j) {
-    const ArrowArray *ch = batch->children[j];
-    const ArrowSchema *cs = schema->children[j];
-    ColInput &ci = cols[(size_t)j];
-    const bool list = a->type_ids[(size_t)j] == DMB_TYPE_LIST, en = a->type_ids[(size_t)j] == DMB_TYPE_ENUM;
-    if (!ch || !cs || !cs->format ||
-        !(list ? map_list(a, j, ch, cs, &ci, &children[(size_t)j])
-               : en ? map_enum(a, j, ch, cs, &ci)
-                    : map_format(a, j, "format", cs->format, a->type_ids[(size_t)j], &a->rows[(size_t)j].dec_prec, &a->rows[(size_t)j].dec_scale, &ci))) {
-      if (!a->error[0]) fail(a, "append_arrow_batch: column %d is malformed", j);
+  const size_t total = a->type_ids.size();  // table columns and field columns
+  std::vector<ColInput> cols(total), children(total);
+  for (int j = 0; j < a->ncols; ++j)
+    if (!map_column(a, j, batch->children[j], schema->children[j], batch->offset, n, cols, children)) {
       a->state = kError;
       return 0;
     }
-    if (ch->length < batch->offset + n) {
-      fail(a, "append_arrow_batch: column %d is shorter than the batch", j);
-      a->state = kError;
-      return 0;
-    }
-    bind_buffers(ci, ch, ch->offset + batch->offset);
-    if (n > 0 && (((ci.is_string || ci.is_list) && !ci.offsets) || (!ci.is_string && !ci.is_list && !ci.values))) {
-      fail(a, "append_arrow_batch: column %d has no value buffer", j);
-      a->state = kError;
-      return 0;
-    }
-  }
   if (!flush_rows(a)) { a->state = kError; return 0; }  // keep row order with earlier row-API appends
   if (!convert_rows(a, cols, n)) { a->state = kError; return 0; }
   a->row_count += n;
@@ -1193,7 +1342,7 @@ extern "C" int32_t duckdb_mb_gpu_append_interval(duckdb_mb_gpu_appender *a, int3
 // the table column's DECIMAL(width, scale) (duckdb_appender_column_type -> duckdb_decimal_width / _scale)
 extern "C" int32_t duckdb_mb_gpu_appender_set_decimal(duckdb_mb_gpu_appender *a, int32_t col, int32_t width, int32_t scale) {
   if (!a) return 0;
-  if (col < 0 || col >= a->ncols || a->type_ids[(size_t)col] != DMB_TYPE_DECIMAL || width < 1 || width > 38 || scale < 0 || scale > width) {
+  if (col < 0 || col >= (int32_t)a->type_ids.size() || a->type_ids[(size_t)col] != DMB_TYPE_DECIMAL || width < 1 || width > 38 || scale < 0 || scale > width) {
     fail(a, "appender_set_decimal: column %d is not a DECIMAL column or DECIMAL(%d,%d) is not a type", col, width, scale);
     return 0;
   }
@@ -1241,7 +1390,7 @@ extern "C" int32_t duckdb_mb_gpu_appender_set_list(duckdb_mb_gpu_appender *a, in
 // the table column's ENUM type (duckdb_enum_dictionary_size / _value, duckdb_enum_internal_type of duckdb_appender_column_type)
 extern "C" int32_t duckdb_mb_gpu_appender_set_enum(duckdb_mb_gpu_appender *a, int32_t col, int32_t internal_type_id, const dmb_enum_dict *dict) {
   if (!a) return 0;
-  if (col < 0 || col >= a->ncols || a->type_ids[(size_t)col] != DMB_TYPE_ENUM) return fail(a, "appender_set_enum: column %d is not an ENUM column", col);
+  if (col < 0 || col >= (int32_t)a->type_ids.size() || a->type_ids[(size_t)col] != DMB_TYPE_ENUM) return fail(a, "appender_set_enum: column %d is not an ENUM column", col);
   int32_t w;
   uint64_t most;
   switch (internal_type_id) {
@@ -1277,6 +1426,71 @@ extern "C" int32_t duckdb_mb_gpu_appender_set_enum(duckdb_mb_gpu_appender *a, in
   if (!dmb_rev_enum_table(&copy, e.table_size, e.slots.data())) return fail(a, "appender_set_enum: column %d: %s", col, duckdb_mb_gpu_last_error());
   cur = std::move(e);
   a->rows[(size_t)col].width = 0;  // the row protocol buffers VARCHAR labels
+  return 1;
+}
+
+// the table's field types of a STRUCT column (duckdb_struct_type_child_count / _child_type), or of a STRUCT field column:
+// they become field columns, numbered from the current column count on
+extern "C" int32_t duckdb_mb_gpu_appender_set_struct(duckdb_mb_gpu_appender *a, int32_t col, int32_t nfields, const int32_t *field_type_ids,
+                                                     int32_t *first_field) {
+  if (!a) return 0;
+  if (col < 0 || col >= (int32_t)a->type_ids.size() || a->type_ids[(size_t)col] != DMB_TYPE_STRUCT)
+    return fail(a, "appender_set_struct: column %d is not a STRUCT column", col);
+  if (nfields <= 0 || !field_type_ids) return fail(a, "appender_set_struct: column %d: a STRUCT needs at least one field", col);
+  for (int32_t f = 0; f < nfields; ++f) {
+    const int32_t t = field_type_ids[f];
+    switch (t) {
+      case DMB_TYPE_LIST: return fail(a, "appender_set_struct: column %d, field %d: LIST fields cannot be appended", col, f);
+      case DMB_TYPE_MAP: return fail(a, "appender_set_struct: column %d, field %d: MAP fields cannot be appended", col, f);
+      case DMB_TYPE_BOOLEAN: case DMB_TYPE_TINYINT: case DMB_TYPE_SMALLINT: case DMB_TYPE_INTEGER: case DMB_TYPE_BIGINT:
+      case DMB_TYPE_UTINYINT: case DMB_TYPE_USMALLINT: case DMB_TYPE_UINTEGER: case DMB_TYPE_UBIGINT: case DMB_TYPE_FLOAT:
+      case DMB_TYPE_DOUBLE: case DMB_TYPE_DATE: case DMB_TYPE_TIME: case DMB_TYPE_TIME_NS: case DMB_TYPE_TIME_TZ:
+      case DMB_TYPE_TIMESTAMP: case DMB_TYPE_TIMESTAMP_S: case DMB_TYPE_TIMESTAMP_MS: case DMB_TYPE_TIMESTAMP_NS:
+      case DMB_TYPE_TIMESTAMP_TZ: case DMB_TYPE_HUGEINT: case DMB_TYPE_UHUGEINT: case DMB_TYPE_UUID: case DMB_TYPE_VARCHAR:
+      case DMB_TYPE_BLOB: case DMB_TYPE_DECIMAL: case DMB_TYPE_ENUM: case DMB_TYPE_STRUCT:
+        break;
+      default:  // the types map_column converts, and nothing else
+        return fail(a, "appender_set_struct: column %d, field %d: field type %d cannot be appended", col, f, t);
+    }
+  }
+  StructDecl &d = a->structs[(size_t)col];
+  if (d.first >= 0) {
+    if (d.types != std::vector<int32_t>(field_type_ids, field_type_ids + nfields))
+      return fail(a, "appender_set_struct: column %d already has a different STRUCT declaration (%d fields)", col, (int)d.types.size());
+    if (first_field) *first_field = d.first;
+    return 1;
+  }
+  const int32_t first = (int32_t)a->type_ids.size();
+  d.first = first;
+  d.types.assign(field_type_ids, field_type_ids + nfields);
+  for (int32_t f = 0; f < nfields; ++f) {
+    a->type_ids.push_back(field_type_ids[f]);
+    a->parent.push_back(col);
+    a->field_index.push_back(f);
+    RowBuf rb;
+    rb.width = row_width(field_type_ids[f]);
+    rb.offsets.assign(1, 0);
+    a->rows.push_back(std::move(rb));
+    a->lists.emplace_back();
+    a->enums.emplace_back();
+    a->structs.emplace_back();  // (moves `d`)
+  }
+  if (first_field) *first_field = first;
+  return 1;
+}
+
+// during a sink call: field `field` of STRUCT column `col` for the chunk being handed over
+extern "C" int32_t duckdb_mb_gpu_appender_struct_field(duckdb_mb_gpu_appender *a, int32_t col, int32_t field, const void **data,
+                                                       const uint64_t **validity) {
+  if (!a || !data || !validity) return 0;
+  if (a->sink_chunk < 0 || col < 0 || (size_t)col >= a->sink_cols.size() || a->type_ids[(size_t)col] != DMB_TYPE_STRUCT)
+    return fail(a, "appender_struct_field: column %d is not a STRUCT column of a chunk being handed to the sink", col);
+  const StructDecl &d = a->structs[(size_t)col];
+  if (field < 0 || field >= (int32_t)d.types.size()) return fail(a, "appender_struct_field: column %d has no field %d", col, field);
+  const SinkCol &f = a->sink_cols[(size_t)(d.first + field)];
+  const int64_t k = a->sink_chunk;
+  *data = f.data ? f.data + (size_t)k * DMB_VECTOR_SIZE * (size_t)f.w : nullptr;
+  *validity = f.masks + (size_t)k * DMB_VALIDITY_WORDS;
   return 1;
 }
 

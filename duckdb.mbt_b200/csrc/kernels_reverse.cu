@@ -340,6 +340,38 @@ rev_list_kernel(dmb_rev_list_job job, int64_t nrows) {
   }
 }
 
+// bits [r0, r0 + 64) of a row bitmap (bit k: row r0 + k), 0 outside rows [0, nrows); r0 > -64.  An absent bitmap is all
+// valid.
+__device__ __forceinline__ uint64_t rev_mask_bits64(const BitSrc &bs, bool has_bm, int64_t nrows, int64_t r0) {
+  const int lead = r0 < 0 ? (int)(-r0) : 0;  // the first word of an output at a bit phase starts before row 0
+  const int64_t first = r0 + lead, left = nrows - first;
+  if (left <= 0) return 0ull;
+  const int live = left < 64 - lead ? (int)left : 64 - lead;
+  uint64_t v;
+  if (!has_bm) {
+    v = live == 64 ? ~0ull : ((1ull << live) - 1ull);
+  } else {
+    const uint64_t lo = load_bits32(bs.w, bs.base + first, live < 32 ? live : 32);
+    const uint64_t hi = live > 32 ? load_bits32(bs.w, bs.base + first + 32, live - 32) : 0u;
+    v = lo | (hi << 32);
+  }
+  return v << lead;
+}
+
+// STRUCT validity: out = a AND b over nrows rows, written as whole 64-bit words from bit out_bit_offset on, every bit
+// outside [out_bit_offset, out_bit_offset + nrows) zero.  One thread per output word; grid.y = job.
+__global__ void __launch_bounds__(kThreads)
+rev_mask_kernel(const dmb_rev_mask_job *__restrict__ jobs, int64_t nrows) {
+  const dmb_rev_mask_job job = jobs[blockIdx.y];
+  const int64_t nwords = ((job.out_bit_offset + nrows + kVec - 1) / kVec) * DMB_VALIDITY_WORDS;
+  const BitSrc a = bit_src(job.in_a, job.a_bit_offset), b = bit_src(job.in_b, job.b_bit_offset);
+  const bool has_a = job.in_a != nullptr, has_b = job.in_b != nullptr;
+  for (int64_t w = (int64_t)blockIdx.x * kThreads + threadIdx.x; w < nwords; w += (int64_t)gridDim.x * kThreads) {
+    const int64_t r0 = (w << 6) - job.out_bit_offset;
+    __stcs(reinterpret_cast<unsigned long long *>(job.out + w), rev_mask_bits64(a, has_a, nrows, r0) & rev_mask_bits64(b, has_b, nrows, r0));
+  }
+}
+
 // ---- ENUM: labels -> positions (dmb_rev_enum_job).  One row per thread; a warp's 32 rows share one validity word, which
 // is also the mask word the ballot of the rows that got a position writes.
 extern __shared__ uint4 rev_enum_smem[];  // the lookup table or the remap, when it fits
@@ -581,6 +613,24 @@ extern "C" int32_t dmb_dev_rev_fixed_batch(const dmb_rev_fixed_job *jobs_dev, co
   int gx = (int)(blocks < 1 ? 1 : (blocks < max_grid ? blocks : max_grid));
   rev_fixed_kernel<<<dim3(gx, njobs), kThreads, 0, (cudaStream_t)stream>>>(jobs_dev, nrows);
   return check_cuda(cudaGetLastError(), "rev_fixed_kernel launch");
+}
+
+extern "C" int32_t dmb_dev_rev_mask_batch(const dmb_rev_mask_job *jobs_dev, const dmb_rev_mask_job *jobs_host, int32_t njobs,
+                                          int64_t nrows, void *stream) {
+  if (njobs <= 0 || nrows <= 0) return 0;
+  if (!jobs_dev || !jobs_host) { set_error("dmb_dev_rev_mask_batch: jobs is null"); return -1; }
+  if (njobs > 65535) { set_error("dmb_dev_rev_mask_batch: %d jobs (at most 65535)", njobs); return -1; }
+  for (int32_t j = 0; j < njobs; ++j)
+    if (!jobs_host[j].out || jobs_host[j].out_bit_offset < 0 || jobs_host[j].out_bit_offset > 63 || jobs_host[j].a_bit_offset < 0 ||
+        jobs_host[j].b_bit_offset < 0) {
+      set_error("dmb_dev_rev_mask_batch: job %d has no output or a bit offset out of range", j);
+      return -1;
+    }
+  const int64_t words = ((nrows + 63 + kVec - 1) / kVec) * DMB_VALIDITY_WORDS;  // the most any job writes
+  const int64_t blocks = (words + kThreads - 1) / kThreads, max_grid = (int64_t)kNumSMs * 8;
+  const int gx = (int)(blocks < max_grid ? blocks : max_grid);
+  rev_mask_kernel<<<dim3(gx, njobs), kThreads, 0, (cudaStream_t)stream>>>(jobs_dev, nrows);
+  return check_cuda(cudaGetLastError(), "rev_mask_kernel launch");
 }
 
 extern "C" int32_t dmb_dev_rev_string_batch(const dmb_rev_string_job *job, int64_t nrows, void *stream) {

@@ -60,6 +60,11 @@ class RevListJob(C.Structure):
                 ("null_count", C.c_void_p), ("error", C.c_void_p), ("large_offsets", C.c_int32), ("reserved", C.c_int32)]
 
 
+class RevMaskJob(C.Structure):
+    _fields_ = [("in_a", C.c_void_p), ("a_bit_offset", C.c_int64), ("in_b", C.c_void_p), ("b_bit_offset", C.c_int64),
+                ("out", C.c_void_p), ("out_bit_offset", C.c_int64)]
+
+
 class RevEnumJob(C.Structure):
     _fields_ = [("in_offsets", C.c_void_p), ("in_data", C.c_void_p), ("in_indices", C.c_void_p), ("in_validity", C.c_void_p),
                 ("in_bit_offset", C.c_int64), ("remap", C.c_void_p), ("dict_len", C.c_int64), ("table", C.c_void_p),
@@ -149,7 +154,7 @@ CHUNK_SINK = C.CFUNCTYPE(C.c_int32, C.c_void_p, C.c_int32, C.c_uint32, C.POINTER
 EXPORTED_SYMBOLS = [
     "dmb_dev_fixed_batch", "dmb_op_out_width", "dmb_phys_width", "dmb_dev_string_scratch_bytes",
     "dmb_dev_string_error", "dmb_dev_string_batch", "dmb_dev_set_lookback_limit_ns", "dmb_dev_rev_fixed_batch", "dmb_dev_rev_string_batch",
-    "dmb_dev_rev_list_batch", "dmb_rev_list_cut", "dmb_dev_rev_enum_batch", "dmb_rev_enum_table", "dmb_rev_enum_lookup",
+    "dmb_dev_rev_list_batch", "dmb_dev_rev_mask_batch", "dmb_rev_list_cut", "dmb_dev_rev_enum_batch", "dmb_rev_enum_table", "dmb_rev_enum_lookup",
     "dmb_dev_valid_bytes_to_masks", "dmb_dev_make_string_t", "dmb_dev_blob_escape", "dmb_render_supported", "dmb_render_slot_bytes", "dmb_dev_render_text", "dmb_dev_enum_to_string_t", "dmb_dev_enum_utf8", "dmb_dev_list_scratch_bytes", "dmb_dev_list_batch",
     "duckdb_mb_gpu_last_error", "duckdb_mb_gpu_device_count", "duckdb_mb_gpu_bind_numa", "duckdb_mb_gpu_ctx_create",
     "duckdb_mb_gpu_ctx_destroy", "duckdb_mb_gpu_ctx_sync", "duckdb_mb_gpu_host_alloc", "duckdb_mb_gpu_host_free",
@@ -187,7 +192,8 @@ EXPORTED_SYMBOLS = [
     "duckdb_mb_gpu_append_timestamp", "duckdb_mb_gpu_end_row", "duckdb_mb_gpu_append_blob", "duckdb_mb_gpu_append_decimal",
     "duckdb_mb_gpu_append_list_varchar", "duckdb_mb_gpu_append_struct_varchar", "duckdb_mb_gpu_append_map_varchar_varchar",
     "duckdb_mb_gpu_append_interval", "duckdb_mb_gpu_appender_set_decimal", "duckdb_mb_gpu_appender_set_list",
-    "duckdb_mb_gpu_appender_list_child", "duckdb_mb_gpu_appender_set_enum",
+    "duckdb_mb_gpu_appender_list_child", "duckdb_mb_gpu_appender_set_enum", "duckdb_mb_gpu_appender_set_struct",
+    "duckdb_mb_gpu_appender_struct_field",
 ]
 
 _lib = None
@@ -255,6 +261,12 @@ def lib():
     L.dmb_dev_rev_string_batch.argtypes = [C.POINTER(RevStringJob), i64, vp]
     L.dmb_dev_rev_list_batch.restype = i32
     L.dmb_dev_rev_list_batch.argtypes = [C.POINTER(RevListJob), i64, vp]
+    L.dmb_dev_rev_mask_batch.restype = i32
+    L.dmb_dev_rev_mask_batch.argtypes = [vp, vp, i32, i64, vp]
+    L.duckdb_mb_gpu_appender_set_struct.restype = i32
+    L.duckdb_mb_gpu_appender_set_struct.argtypes = [vp, i32, i32, vp, C.POINTER(i32)]
+    L.duckdb_mb_gpu_appender_struct_field.restype = i32
+    L.duckdb_mb_gpu_appender_struct_field.argtypes = [vp, i32, i32, C.POINTER(vp), C.POINTER(vp)]
     L.dmb_dev_rev_enum_batch.restype = i32
     L.dmb_dev_rev_enum_batch.argtypes = [C.POINTER(RevEnumJob), i64, vp]
     L.dmb_rev_enum_table.restype = i32

@@ -316,6 +316,10 @@ typedef struct {
   int32_t *type_ids;
   int32_t *widths;
   int32_t *child_type_ids, *child_widths; /* LIST columns */
+  /* every table column and field column of the library's handle (duckdb_mb_gpu_appender_set_struct numbers the fields
+   * of STRUCT columns after the table's columns): type, vector width and, for a STRUCT, its first field column */
+  struct { int32_t type_id, width, first, nfields; } *all;
+  int32_t nall;
   duckdb_data_chunk chunk; /* reused: duckdb_append_data_chunk copies */
 } glue_sink;
 
@@ -329,6 +333,7 @@ static int32_t vector_width(duckdb_logical_type lt) {
     case DUCKDB_TYPE_VARCHAR: case DUCKDB_TYPE_BLOB: case DUCKDB_TYPE_INTERVAL: case DUCKDB_TYPE_HUGEINT: case DUCKDB_TYPE_UHUGEINT: case DUCKDB_TYPE_UUID:
     case DUCKDB_TYPE_LIST: return 16; /* LIST: duckdb_list_entry */
     case DUCKDB_TYPE_ENUM: { const duckdb_type it = duckdb_enum_internal_type(lt); return it == DUCKDB_TYPE_UTINYINT ? 1 : it == DUCKDB_TYPE_USMALLINT ? 2 : 4; }
+    case DUCKDB_TYPE_STRUCT: return 0; /* a mask and one child vector per field */
     default: return 8;
   }
 }
@@ -337,7 +342,7 @@ static int32_t vector_width(duckdb_logical_type lt) {
 static void fill_vector(duckdb_vector v, int32_t type_id, int32_t width, uint64_t count, const void *data, const uint64_t *mask) {
   const int is_str = type_id == DUCKDB_TYPE_VARCHAR || type_id == DUCKDB_TYPE_BLOB;
   if (!is_str) {
-    if (count) memcpy(duckdb_vector_get_data(v), data, (size_t)count * (size_t)width);
+    if (count && width) memcpy(duckdb_vector_get_data(v), data, (size_t)count * (size_t)width);
   } else { /* the vector must own its strings: inlined entries are copied as they are, pointer entries assigned */
     const dmb_string_t *e = (const dmb_string_t *)data;
     dmb_string_t *out = (dmb_string_t *)duckdb_vector_get_data(v);
@@ -351,6 +356,21 @@ static void fill_vector(duckdb_vector v, int32_t type_id, int32_t width, uint64_
     duckdb_vector_ensure_validity_writable(v);
     memcpy(duckdb_vector_get_validity(v), mask, 8 * (((size_t)count + 63) / 64));
   }
+}
+
+/* the fields of STRUCT column `col` (a table column or a field column) into STRUCT vector v, recursively */
+static int32_t fill_struct(glue_sink *s, duckdb_vector v, int32_t col, uint64_t count) {
+  for (int32_t f = 0; f < s->all[col].nfields; f++) {
+    const int32_t fc = s->all[col].first + f;
+    const void *data = NULL;
+    const uint64_t *mask = NULL;
+    if (!duckdb_mb_gpu_appender_struct_field(s->lib, col, f, &data, &mask)) return 0;
+    duckdb_vector child = duckdb_struct_vector_get_child(v, (idx_t)f);
+    if (!child) return 0;
+    fill_vector(child, s->all[fc].type_id, s->all[fc].width, count, data, mask);
+    if (s->all[fc].type_id == DUCKDB_TYPE_STRUCT && !fill_struct(s, child, fc, count)) return 0;
+  }
+  return 1;
 }
 
 static int32_t sink_chunk(void *user, int32_t ncols, uint32_t count, const void *const *vec_data, const uint64_t *const *vec_validity) {
@@ -370,6 +390,7 @@ static int32_t sink_chunk(void *user, int32_t ncols, uint32_t count, const void 
       if (!child) return 0;
       fill_vector(child, s->child_type_ids[c], s->child_widths[c], size, cdata, cmask);
     }
+    if (s->type_ids[c] == DUCKDB_TYPE_STRUCT && !fill_struct(s, v, c, count)) return 0;
   }
   duckdb_data_chunk_set_size(s->chunk, count);
   return duckdb_append_data_chunk(s->appender, s->chunk) == DuckDBSuccess ? 1 : 0;
@@ -383,7 +404,56 @@ static void sink_destroy(void *user) {
   if (s->chunk) duckdb_destroy_data_chunk(&s->chunk);
   for (int32_t c = 0; c < s->ncols; c++) duckdb_destroy_logical_type(&s->types[c]);
   if (s->appender) duckdb_appender_destroy(&s->appender); /* (flushes what is left, like the reference's destroy :1083-1091) */
-  free(s->types); free(s->type_ids); free(s->widths); free(s->child_type_ids); free(s->child_widths); free(s);
+  free(s->types); free(s->type_ids); free(s->widths); free(s->child_type_ids); free(s->child_widths); free(s->all); free(s);
+}
+
+/* column c's type that the library must be told: DECIMAL width / scale, ENUM labels, STRUCT fields (recursively, through
+ * the field columns duckdb_mb_gpu_appender_set_struct numbers).  A refused declaration leaves the column undeclared:
+ * Arrow batches for it fail and name the declaration they lack. */
+static void declare_column(glue_sink *s, duckdb_mb_appender *a, int32_t c, duckdb_logical_type lt) {
+  const duckdb_type t = duckdb_get_type_id(lt);
+  if (t == DUCKDB_TYPE_DECIMAL) duckdb_mb_gpu_appender_set_decimal(a, c, duckdb_decimal_width(lt), duckdb_decimal_scale(lt));
+  if (t == DUCKDB_TYPE_ENUM) {
+    dmb_enum_dict d;
+    uint32_t *offs;
+    char *bytes;
+    memset(&d, 0, sizeof(d));
+    d.size = read_enum_dict(lt, &offs, &bytes);
+    d.offsets = offs;
+    d.data = bytes;
+    duckdb_mb_gpu_appender_set_enum(a, c, (int32_t)duckdb_enum_internal_type(lt), &d);
+    free(offs);
+    free(bytes);
+  }
+  if (t == DUCKDB_TYPE_STRUCT) {
+    const int32_t n = (int32_t)duckdb_struct_type_child_count(lt);
+    duckdb_logical_type *ft = (duckdb_logical_type *)calloc((size_t)(n > 0 ? n : 1), sizeof(duckdb_logical_type));
+    int32_t *ids = (int32_t *)calloc((size_t)(n > 0 ? n : 1), sizeof(int32_t));
+    int32_t first = -1;
+    for (int32_t f = 0; f < n; f++) {
+      ft[f] = duckdb_struct_type_child_type(lt, (idx_t)f);
+      ids[f] = (int32_t)duckdb_get_type_id(ft[f]);
+    }
+    if (ft && ids && duckdb_mb_gpu_appender_set_struct(a, c, n, ids, &first)) {
+      void *grown = realloc(s->all, sizeof(*s->all) * (size_t)(first + n));
+      if (grown) {
+        s->all = grown;
+        s->nall = first + n;
+        s->all[c].first = first;
+        s->all[c].nfields = n;
+        for (int32_t f = 0; f < n; f++) {
+          s->all[first + f].type_id = ids[f];
+          s->all[first + f].width = vector_width(ft[f]);
+          s->all[first + f].first = -1;
+          s->all[first + f].nfields = 0;
+        }
+        for (int32_t f = 0; f < n; f++) declare_column(s, a, first + f, ft[f]);
+      }
+    }
+    for (int32_t f = 0; f < n; f++) duckdb_destroy_logical_type(&ft[f]);
+    free(ft);
+    free(ids);
+  }
 }
 
 /* src/duckdb_native.c:1032-1081: NULL on failure (the reference sets no global error here either) */
@@ -408,10 +478,15 @@ duckdb_mb_appender *duckdb_mb_appender_create(duckdb_mb_connection *handle, moon
   s->widths = (int32_t *)calloc(nc, sizeof(int32_t));
   s->child_type_ids = (int32_t *)calloc(nc, sizeof(int32_t));
   s->child_widths = (int32_t *)calloc(nc, sizeof(int32_t));
+  s->all = calloc(nc, sizeof(*s->all));
+  s->nall = s->ncols;
   for (int32_t c = 0; c < s->ncols; c++) {
     s->types[c] = duckdb_appender_column_type(s->appender, (idx_t)c);
     s->type_ids[c] = (int32_t)duckdb_get_type_id(s->types[c]);
     s->widths[c] = vector_width(s->types[c]);
+    s->all[c].type_id = s->type_ids[c];
+    s->all[c].width = s->widths[c];
+    s->all[c].first = -1;
   }
   s->chunk = duckdb_create_data_chunk(s->types, (idx_t)s->ncols);
   duckdb_mb_appender *a = duckdb_mb_gpu_appender_create(ctx, s->ncols, s->type_ids, sink_chunk, s);
@@ -419,8 +494,7 @@ duckdb_mb_appender *duckdb_mb_appender_create(duckdb_mb_connection *handle, moon
   s->lib = a;
   duckdb_mb_gpu_appender_set_hooks(a, sink_flush, sink_destroy);
   for (int32_t c = 0; c < s->ncols; c++) {
-    if (s->type_ids[c] == DUCKDB_TYPE_DECIMAL)
-      duckdb_mb_gpu_appender_set_decimal(a, c, duckdb_decimal_width(s->types[c]), duckdb_decimal_scale(s->types[c]));
+    declare_column(s, a, c, s->types[c]);
     if (s->type_ids[c] == DUCKDB_TYPE_LIST) {
       /* a child type the library refuses (LIST, STRUCT, ...) leaves the column undeclared: Arrow batches for it fail */
       duckdb_logical_type child = duckdb_list_type_child_type(s->types[c]);
@@ -430,19 +504,6 @@ duckdb_mb_appender *duckdb_mb_appender_create(duckdb_mb_connection *handle, moon
       duckdb_mb_gpu_appender_set_list(a, c, (int32_t)ct, ct == DUCKDB_TYPE_DECIMAL ? duckdb_decimal_width(child) : 0,
                                       ct == DUCKDB_TYPE_DECIMAL ? duckdb_decimal_scale(child) : 0);
       duckdb_destroy_logical_type(&child);
-    }
-    if (s->type_ids[c] == DUCKDB_TYPE_ENUM) {
-      /* a refused declaration leaves the column undeclared: appends to it fail and name duckdb_mb_gpu_appender_set_enum */
-      dmb_enum_dict d;
-      uint32_t *offs;
-      char *bytes;
-      memset(&d, 0, sizeof(d));
-      d.size = read_enum_dict(s->types[c], &offs, &bytes);
-      d.offsets = offs;
-      d.data = bytes;
-      duckdb_mb_gpu_appender_set_enum(a, c, (int32_t)duckdb_enum_internal_type(s->types[c]), &d);
-      free(offs);
-      free(bytes);
     }
   }
   return a;

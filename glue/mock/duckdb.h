@@ -76,6 +76,7 @@ duckdb_vector duckdb_list_vector_get_child(duckdb_vector vector);
 idx_t duckdb_list_vector_get_size(duckdb_vector vector);
 duckdb_state duckdb_list_vector_reserve(duckdb_vector vector, idx_t required_capacity);
 duckdb_state duckdb_list_vector_set_size(duckdb_vector vector, idx_t size);
+duckdb_vector duckdb_struct_vector_get_child(duckdb_vector vector, idx_t index);
 
 duckdb_type duckdb_get_type_id(duckdb_logical_type type);
 uint8_t duckdb_decimal_width(duckdb_logical_type type);
@@ -85,6 +86,8 @@ duckdb_type duckdb_enum_internal_type(duckdb_logical_type type);
 uint32_t duckdb_enum_dictionary_size(duckdb_logical_type type);
 char *duckdb_enum_dictionary_value(duckdb_logical_type type, idx_t index);
 duckdb_logical_type duckdb_list_type_child_type(duckdb_logical_type type);
+idx_t duckdb_struct_type_child_count(duckdb_logical_type type);
+duckdb_logical_type duckdb_struct_type_child_type(duckdb_logical_type type, idx_t index);
 duckdb_logical_type duckdb_create_logical_type(duckdb_type type);
 duckdb_logical_type duckdb_create_decimal_type(uint8_t width, uint8_t scale);
 void duckdb_destroy_logical_type(duckdb_logical_type *type);

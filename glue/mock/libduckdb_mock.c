@@ -42,9 +42,11 @@ typedef struct mock_table {
 
 static mock_table *g_tables = NULL;
 
+struct mock_coltype;
 typedef struct {
   int32_t type_id, dec_width, dec_scale, internal;
   const duckdb_mock_column *col;                   /* served columns */
+  const struct mock_coltype *node;                 /* appender columns: the registered type (STRUCT fields) */
   int32_t child_type_id, child_dec_width, child_dec_scale;  /* appender LIST columns */
   int32_t enum_width; uint32_t enum_size; char **enum_labels;  /* appender ENUM columns (owned by the append table) */
 } mock_ltype;
@@ -54,6 +56,8 @@ typedef struct mock_vec {
   int64_t chunk;
   int is_child;
   struct mock_vec *child;         /* LIST: the chunk's child vector */
+  struct mock_vec *fields;        /* created STRUCT vector: one vector per field */
+  int32_t nfields;
   /* created (appender side) vector */
   int created;
   mock_ltype ltype;
@@ -160,6 +164,8 @@ static void free_created_vec(mock_vec *v) {
   free(v->buf); free(v->mask);
   if (v->strs) { for (idx_t i = 0; i < v->cap; i++) free(v->strs[i]); free(v->strs); }
   if (v->child) { free_created_vec(v->child); free(v->child); }
+  for (int32_t f = 0; f < v->nfields; f++) free_created_vec(&v->fields[f]);
+  free(v->fields);
 }
 void duckdb_destroy_data_chunk(duckdb_data_chunk *chunk) {
   if (!chunk || !*chunk) return;
@@ -235,10 +241,18 @@ void duckdb_destroy_logical_type(duckdb_logical_type *type) { if (type && *type)
 void duckdb_free(void *ptr) { free(ptr); }
 
 /* ---- appender side: a "table" = its column types + every chunk that was appended */
-typedef struct {
+typedef struct mock_coltype {
   int32_t type_id, dec_width, dec_scale, child_type_id, child_dec_width, child_dec_scale;
   int32_t enum_width; uint32_t enum_size; char **enum_labels;  /* ENUM: internal width and labels */
+  int32_t nfields; struct mock_coltype *fields;                /* STRUCT */
 } mock_coltype;
+/* a STRUCT column's appended vectors: per field its payload (MOCK_VECTOR_SIZE rows) and mask, nested STRUCTs inside */
+typedef struct app_vec {
+  uint8_t *data;
+  uint64_t *mask;
+  int32_t nfields;
+  struct app_vec *fields;
+} app_vec;
 typedef struct appended_chunk {
   idx_t size;
   uint8_t **data;
@@ -246,6 +260,7 @@ typedef struct appended_chunk {
   uint8_t **child_data;  /* LIST columns: the chunk's child vector */
   uint64_t **child_mask;
   idx_t *child_size;
+  app_vec **structs;     /* STRUCT columns: the field vectors */
   struct appended_chunk *next;
 } appended_chunk;
 typedef struct mock_append_table {
@@ -282,16 +297,48 @@ int32_t duckdb_mock_set_append_list_child(const char *table, int32_t col, int32_
   t->types[col].child_type_id = child_type; t->types[col].child_dec_width = dec_width; t->types[col].child_dec_scale = dec_scale;
   return 1;
 }
-/* the labels and internal width (1 / 2 / 4 bytes) of a registered ENUM column (what duckdb_enum_* report for it) */
-int32_t duckdb_mock_set_append_enum(const char *table, int32_t col, int32_t internal_width, uint32_t nlabels, const char *const *labels) {
+/* column col of a registered table, or the field at path[0..depth) inside it (NULL when there is none) */
+static mock_coltype *find_coltype(const char *table, int32_t col, const int32_t *path, int32_t depth) {
   mock_append_table *t = find_append_table(table);
-  if (!t || col < 0 || col >= t->ncols) return 0;
+  if (!t || col < 0 || col >= t->ncols) return NULL;
   mock_coltype *ct = &t->types[col];
+  for (int32_t d = 0; d < depth; d++) {
+    if (path[d] < 0 || path[d] >= ct->nfields) return NULL;
+    ct = &ct->fields[path[d]];
+  }
+  return ct;
+}
+/* the fields of a registered STRUCT column, or of a STRUCT field at path[0..depth) inside it (what
+ * duckdb_struct_type_child_count / _child_type report); a field's ENUM labels come from duckdb_mock_set_append_enum_field */
+int32_t duckdb_mock_set_append_struct(const char *table, int32_t col, const int32_t *path, int32_t depth, int32_t nfields,
+                                      const int32_t *type_ids, const int32_t *dec_widths, const int32_t *dec_scales) {
+  mock_coltype *ct = find_coltype(table, col, path, depth);
+  if (!ct || ct->type_id != DUCKDB_TYPE_STRUCT || nfields <= 0) return 0;
+  ct->nfields = nfields;
+  ct->fields = (mock_coltype *)calloc((size_t)nfields, sizeof(mock_coltype)); /* (leaked with the table: test process) */
+  for (int32_t f = 0; f < nfields; f++) {
+    ct->fields[f].type_id = type_ids[f];
+    ct->fields[f].dec_width = dec_widths ? dec_widths[f] : 0;
+    ct->fields[f].dec_scale = dec_scales ? dec_scales[f] : 0;
+  }
+  return 1;
+}
+static int32_t set_enum(mock_coltype *ct, int32_t internal_width, uint32_t nlabels, const char *const *labels) {
+  if (!ct) return 0;
   ct->enum_width = internal_width;
   ct->enum_size = nlabels;
   ct->enum_labels = (char **)calloc(nlabels ? nlabels : 1, sizeof(char *)); /* (leaked with the table: test process) */
   for (uint32_t i = 0; i < nlabels; i++) ct->enum_labels[i] = strdup(labels[i]);
   return 1;
+}
+/* the labels and internal width (1 / 2 / 4 bytes) of a registered ENUM column (what duckdb_enum_* report for it) */
+int32_t duckdb_mock_set_append_enum(const char *table, int32_t col, int32_t internal_width, uint32_t nlabels, const char *const *labels) {
+  return set_enum(find_coltype(table, col, NULL, 0), internal_width, nlabels, labels);
+}
+/* the same for an ENUM field at path[0..depth) of a STRUCT column */
+int32_t duckdb_mock_set_append_enum_field(const char *table, int32_t col, const int32_t *path, int32_t depth, int32_t internal_width,
+                                          uint32_t nlabels, const char *const *labels) {
+  return set_enum(find_coltype(table, col, path, depth), internal_width, nlabels, labels);
 }
 static int type_width(int32_t type_id, int32_t dec_width, int32_t enum_width) {
   switch (type_id) {
@@ -314,40 +361,65 @@ duckdb_state duckdb_appender_create(duckdb_connection connection, const char *sc
   return DuckDBSuccess;
 }
 idx_t duckdb_appender_column_count(duckdb_appender appender) { mock_appender *a = (mock_appender *)appender; return a && a->t ? (idx_t)a->t->ncols : 0; }
-duckdb_logical_type duckdb_appender_column_type(duckdb_appender appender, idx_t col_idx) {
-  mock_appender *a = (mock_appender *)appender;
-  if (!a || !a->t || col_idx >= (idx_t)a->t->ncols) return NULL;
-  const mock_coltype *ct = &a->t->types[col_idx];
+static duckdb_logical_type ltype_of(const mock_coltype *ct) {
   if (ct->type_id == DUCKDB_TYPE_DECIMAL) return duckdb_create_decimal_type((uint8_t)ct->dec_width, (uint8_t)ct->dec_scale);
   mock_ltype *lt = (mock_ltype *)duckdb_create_logical_type((duckdb_type)ct->type_id);
   lt->child_type_id = ct->child_type_id; lt->child_dec_width = ct->child_dec_width; lt->child_dec_scale = ct->child_dec_scale;
   lt->enum_width = ct->enum_width; lt->enum_size = ct->enum_size; lt->enum_labels = ct->enum_labels;
+  lt->node = ct;
   return (duckdb_logical_type)lt;
+}
+duckdb_logical_type duckdb_appender_column_type(duckdb_appender appender, idx_t col_idx) {
+  mock_appender *a = (mock_appender *)appender;
+  if (!a || !a->t || col_idx >= (idx_t)a->t->ncols) return NULL;
+  return ltype_of(&a->t->types[col_idx]);
+}
+/* appender-side STRUCT types (duckdb_mock_set_append_struct) */
+idx_t duckdb_struct_type_child_count(duckdb_logical_type type) {
+  const mock_ltype *t = (const mock_ltype *)type;
+  return t && t->node ? (idx_t)t->node->nfields : 0;
+}
+duckdb_logical_type duckdb_struct_type_child_type(duckdb_logical_type type, idx_t index) {
+  const mock_ltype *t = (const mock_ltype *)type;
+  return t && t->node && index < (idx_t)t->node->nfields ? ltype_of(&t->node->fields[index]) : NULL;
 }
 const char *duckdb_appender_error(duckdb_appender appender) { mock_appender *a = (mock_appender *)appender; return a && a->error[0] ? a->error : NULL; }
 duckdb_state duckdb_appender_flush(duckdb_appender appender) { mock_appender *a = (mock_appender *)appender; if (!a || !a->t) return DuckDBError; a->t->flushes++; return DuckDBSuccess; }
 duckdb_state duckdb_appender_destroy(duckdb_appender *appender) { if (appender && *appender) { free(*appender); *appender = NULL; } return DuckDBSuccess; }
 
+static void init_created_vec(mock_vec *v, const mock_ltype *lt) {
+  v->created = 1;
+  v->ltype = *lt;
+  v->cap = MOCK_VECTOR_SIZE;
+  v->buf = (uint8_t *)calloc(MOCK_VECTOR_SIZE, (size_t)type_width(v->ltype.type_id, v->ltype.dec_width, v->ltype.enum_width));
+  if (v->ltype.type_id == DUCKDB_TYPE_LIST) { /* an empty child vector, grown by duckdb_list_vector_reserve */
+    v->child = (mock_vec *)calloc(1, sizeof(mock_vec));
+    v->child->created = 1;
+    v->child->is_child = 1;
+    v->child->ltype.type_id = v->ltype.child_type_id;
+    v->child->ltype.dec_width = v->ltype.child_dec_width;
+    v->child->ltype.dec_scale = v->ltype.child_dec_scale;
+  }
+  if (v->ltype.type_id == DUCKDB_TYPE_STRUCT && lt->node) { /* one vector per field */
+    v->nfields = lt->node->nfields;
+    v->fields = (mock_vec *)calloc((size_t)(v->nfields > 0 ? v->nfields : 1), sizeof(mock_vec));
+    for (int32_t f = 0; f < v->nfields; f++) {
+      duckdb_logical_type ft = ltype_of(&lt->node->fields[f]);
+      init_created_vec(&v->fields[f], (const mock_ltype *)ft);
+      duckdb_destroy_logical_type(&ft);
+    }
+  }
+}
 duckdb_data_chunk duckdb_create_data_chunk(duckdb_logical_type *types, idx_t column_count) {
   mock_chunk *ch = (mock_chunk *)calloc(1, sizeof(mock_chunk));
   ch->created = 1; ch->ncols = (int32_t)column_count;
   ch->vecs = (mock_vec *)calloc((size_t)(column_count ? column_count : 1), sizeof(mock_vec));
-  for (idx_t c = 0; c < column_count; c++) {
-    mock_vec *v = &ch->vecs[c];
-    v->created = 1;
-    v->ltype = *(mock_ltype *)types[c];
-    v->cap = MOCK_VECTOR_SIZE;
-    v->buf = (uint8_t *)calloc(MOCK_VECTOR_SIZE, (size_t)type_width(v->ltype.type_id, v->ltype.dec_width, v->ltype.enum_width));
-    if (v->ltype.type_id == DUCKDB_TYPE_LIST) { /* an empty child vector, grown by duckdb_list_vector_reserve */
-      v->child = (mock_vec *)calloc(1, sizeof(mock_vec));
-      v->child->created = 1;
-      v->child->is_child = 1;
-      v->child->ltype.type_id = v->ltype.child_type_id;
-      v->child->ltype.dec_width = v->ltype.child_dec_width;
-      v->child->ltype.dec_scale = v->ltype.child_dec_scale;
-    }
-  }
+  for (idx_t c = 0; c < column_count; c++) init_created_vec(&ch->vecs[c], (const mock_ltype *)types[c]);
   return (duckdb_data_chunk)ch;
+}
+duckdb_vector duckdb_struct_vector_get_child(duckdb_vector vector, idx_t index) {
+  mock_vec *v = (mock_vec *)vector;
+  return v && v->created && index < (idx_t)v->nfields ? (duckdb_vector)&v->fields[index] : NULL;
 }
 duckdb_state duckdb_list_vector_reserve(duckdb_vector vector, idx_t required_capacity) {
   mock_vec *v = (mock_vec *)vector;
@@ -397,6 +469,33 @@ void duckdb_vector_assign_string_element_len(duckdb_vector vector, idx_t index, 
   memcpy(e->value.pointer.prefix, str, 4);
   e->value.pointer.ptr = v->strs[index];
 }
+/* the table owns its strings: copy what the valid pointer entries of `size` string_t refer to */
+static void own_strings(uint8_t *data, const uint64_t *mask, idx_t size) {
+  duckdb_string_t *e = (duckdb_string_t *)data;
+  for (idx_t i = 0; i < size; i++) {
+    if (mask && !((mask[i >> 6] >> (i & 63)) & 1ull)) continue;
+    if (e[i].value.inlined.length > 12) {
+      char *copy = (char *)malloc(e[i].value.pointer.length);
+      memcpy(copy, e[i].value.pointer.ptr, e[i].value.pointer.length);
+      e[i].value.pointer.ptr = copy; /* (leaked with the table: test process) */
+    }
+  }
+}
+/* a created STRUCT vector's fields, recursively */
+static void copy_fields(app_vec *out, const mock_vec *v, idx_t size) {
+  out->nfields = v->nfields;
+  out->fields = (app_vec *)calloc((size_t)(v->nfields > 0 ? v->nfields : 1), sizeof(app_vec));
+  for (int32_t f = 0; f < v->nfields; f++) {
+    const mock_vec *fv = &v->fields[f];
+    app_vec *o = &out->fields[f];
+    const size_t w = (size_t)type_width(fv->ltype.type_id, fv->ltype.dec_width, fv->ltype.enum_width);
+    o->data = (uint8_t *)malloc((size_t)MOCK_VECTOR_SIZE * w + 1);
+    memcpy(o->data, fv->buf, (size_t)MOCK_VECTOR_SIZE * w);
+    if (fv->mask) { o->mask = (uint64_t *)malloc(8 * (MOCK_VECTOR_SIZE / 64)); memcpy(o->mask, fv->mask, 8 * (MOCK_VECTOR_SIZE / 64)); }
+    if (fv->ltype.type_id == DUCKDB_TYPE_VARCHAR || fv->ltype.type_id == DUCKDB_TYPE_BLOB) own_strings(o->data, o->mask, size);
+    if (fv->nfields) copy_fields(o, fv, size);
+  }
+}
 duckdb_state duckdb_append_data_chunk(duckdb_appender appender, duckdb_data_chunk chunk) {
   mock_appender *a = (mock_appender *)appender;
   mock_chunk *ch = (mock_chunk *)chunk;
@@ -408,6 +507,7 @@ duckdb_state duckdb_append_data_chunk(duckdb_appender appender, duckdb_data_chun
   ac->child_data = (uint8_t **)calloc((size_t)ch->ncols, sizeof(uint8_t *));
   ac->child_mask = (uint64_t **)calloc((size_t)ch->ncols, sizeof(uint64_t *));
   ac->child_size = (idx_t *)calloc((size_t)ch->ncols, sizeof(idx_t));
+  ac->structs = (app_vec **)calloc((size_t)ch->ncols, sizeof(app_vec *));
   for (int32_t c = 0; c < ch->ncols; c++) {
     mock_vec *v = &ch->vecs[c];
     const int w = type_width(a->t->types[c].type_id, a->t->types[c].dec_width, a->t->types[c].enum_width);
@@ -425,6 +525,10 @@ duckdb_state duckdb_append_data_chunk(duckdb_appender appender, duckdb_data_chun
           e[i].value.pointer.ptr = copy; /* (leaked with the table: test process) */
         }
       }
+    }
+    if (v->nfields) { /* STRUCT: the field vectors */
+      ac->structs[c] = (app_vec *)calloc(1, sizeof(app_vec));
+      copy_fields(ac->structs[c], v, ch->size);
     }
     if (v->child) { /* LIST: the child vector, its first list_size rows */
       const mock_vec *cv = v->child;
@@ -479,4 +583,22 @@ int64_t duckdb_mock_appended_list_child(const char *table, int64_t k, int32_t co
   *data = ac->child_data[col];
   *mask = ac->child_mask[col];
   return (int64_t)ac->child_size[col];
+}
+/* chunk k, STRUCT column col: the vector of the field at path[0..depth) (depth >= 1), its values / mask pointers (mask NULL = all
+ * valid); returns the chunk size */
+int64_t duckdb_mock_appended_struct_field(const char *table, int64_t k, int32_t col, const int32_t *path, int32_t depth, const void **data,
+                                          const uint64_t **mask) {
+  mock_append_table *t = find_append_table(table);
+  if (!t) return -1;
+  appended_chunk *ac = t->head;
+  for (int64_t i = 0; ac && i < k; i++) ac = ac->next;
+  if (!ac || col < 0 || col >= t->ncols || !ac->structs[col] || depth < 1) return -1;
+  const app_vec *v = ac->structs[col];
+  for (int32_t d = 0; d < depth; d++) {
+    if (path[d] < 0 || path[d] >= v->nfields) return -1;
+    v = &v->fields[path[d]];
+  }
+  *data = v->data;
+  *mask = v->mask;
+  return (int64_t)ac->size;
 }

@@ -402,6 +402,25 @@ typedef struct dmb_rev_list_job {
 } dmb_rev_list_job;
 
 int32_t dmb_dev_rev_list_batch(const dmb_rev_list_job *job, int64_t nrows, void *stream);
+
+/* STRUCT validity: out = in_a AND in_b over nrows rows (row r: bit a_bit_offset + r of in_a, bit b_bit_offset + r of in_b;
+ * an absent bitmap is all valid), written from bit out_bit_offset (0..63) of `out` on as a dense bitmap of whole chunks:
+ * ceil((out_bit_offset + nrows) / 2048) * 32 words, every bit outside [out_bit_offset, out_bit_offset + nrows) zero.
+ * At bit offset 0 from a sub-batch's first row that is the DuckDB mask slab (chunk k at k*32 words): the appender writes a
+ * STRUCT column's masks this way (its own bitmap AND its parent STRUCT's masks), and the combined bitmap that a field's
+ * conversion reads as its validity (the parent's masks AND the field's own bitmap; for a BOOLEAN field at the bit phase
+ * of its staged values).  jobs_dev: device array, jobs_host: its host mirror; grid.y = job. */
+typedef struct dmb_rev_mask_job {
+  const uint8_t *in_a;   /* bitmap bytes or NULL */
+  int64_t a_bit_offset;
+  const uint8_t *in_b;   /* bitmap bytes or NULL */
+  int64_t b_bit_offset;
+  uint64_t *out;
+  int64_t out_bit_offset;
+} dmb_rev_mask_job;
+
+int32_t dmb_dev_rev_mask_batch(const dmb_rev_mask_job *jobs_dev, const dmb_rev_mask_job *jobs_host, int32_t njobs, int64_t nrows,
+                               void *stream);
 /* the appender's sub-batch cut (host only): the end chunk (exclusive) of the sub-batch that starts at chunk k0.  It takes
  * at most max_chunks chunks, and stops before the chunk that would give any of the nlists LIST columns more than
  * child_cap child elements; the first chunk is always taken, so one chunk's child range is never split.
@@ -827,6 +846,25 @@ int32_t duckdb_mb_gpu_appender_list_child(duckdb_mb_gpu_appender *a, int32_t col
  * whose label is not in the ENUM, or whose dictionary index is out of range, fails the append before its sub-batch reaches
  * the sink; a row whose dictionary entry is NULL is NULL. */
 int32_t duckdb_mb_gpu_appender_set_enum(duckdb_mb_gpu_appender *a, int32_t col, int32_t internal_type_id, const dmb_enum_dict *dict);
+/* STRUCT columns take Arrow struct arrays ('+s') through duckdb_mb_gpu_append_arrow_batch.  The table's field types
+ * (duckdb_struct_type_child_type of duckdb_appender_column_type) are declared first.  The fields become "field columns",
+ * numbered *first_field .. *first_field + nfields - 1: numbering starts at the table's column count and follows declaration
+ * order across all STRUCT columns.  set_decimal, set_enum and set_struct take a field column as they take a table column,
+ * which declares DECIMAL and ENUM fields and nested STRUCTs.  Fields: the types the reverse path converts at top level,
+ * DECIMAL, VARCHAR, BLOB, ENUM and STRUCT.  Refused by name: a column that is not STRUCT, zero fields, LIST and MAP
+ * fields, any other field type, and a second declaration that differs from the first.
+ * Arrow fields match by position (names are not compared).  A NULL struct row makes every field NULL at that row,
+ * recursively, with payload 0, as DuckDB stores it; a label missing from an ENUM field is an error only under a valid
+ * struct row.  In the sink call, vec_data[col] of a STRUCT column is NULL and vec_validity[col] is the struct's mask (its
+ * own NULLs AND those of its ancestors).  The row protocol refuses a table with a STRUCT column. */
+int32_t duckdb_mb_gpu_appender_set_struct(duckdb_mb_gpu_appender *a, int32_t col, int32_t nfields, const int32_t *field_type_ids,
+                                          int32_t *first_field);
+/* Only inside a dmb_chunk_sink call, for the chunk being handed over: field `field` of STRUCT column `col` (a table column
+ * or a field column).  `*data`: the chunk's count values in DuckDB vector layout (string_t for VARCHAR / BLOB, pointers
+ * into the Arrow data buffer), NULL for a STRUCT field; `*validity`: 32 mask words with the ancestors' NULLs folded in.
+ * Host memory of the appender, valid until the sink call returns. */
+int32_t duckdb_mb_gpu_appender_struct_field(duckdb_mb_gpu_appender *a, int32_t col, int32_t field, const void **data,
+                                            const uint64_t **validity);
 int32_t duckdb_mb_gpu_append_interval(duckdb_mb_gpu_appender *a, int32_t months, int32_t days, int64_t micros); /* :1511 */
 /* LIST / STRUCT / MAP cells: the reference serialises them as text -- `["a", "b"]` (:1735-1790), `{"k": "v", ...}`
  * (:1792-1858 struct, :1860-1926 map), items copied without escaping -- and appends the text as one VARCHAR cell

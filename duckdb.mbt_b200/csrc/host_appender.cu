@@ -56,9 +56,16 @@ struct ColInput {
   int64_t child_len = 0;                 // lists: elements in the child array
   // ENUM: labels (is_string) or Arrow dictionary indices (w_in bytes each) -> positions of w_out bytes
   bool is_enum = false, index_signed = false, dict_large = false;
-  const uint8_t *dict_offsets = nullptr;  // dictionary indices: the Arrow dictionary (utf8 / large_utf8) at its own offset
+  const uint8_t *dict_offsets = nullptr;  // dictionary indices: the Arrow dictionary's offsets (views when dict_view) at its own offset
   const uint8_t *dict_data = nullptr, *dict_validity = nullptr;
   int64_t dict_bit_offset = 0, dict_len = 0;
+  // VARCHAR / BLOB from Arrow string views (is_view: `values` the 16-byte views of the slice) or from an Arrow dictionary of
+  // strings (is_dict: `values` the indices, the dictionary in the dict_* fields; dict_view: its values are views).
+  // view_bufs / view_sizes / nviews: the data buffers of those views and their sizes
+  bool is_view = false, is_dict = false, dict_view = false;
+  const void *const *view_bufs = nullptr;
+  const int64_t *view_sizes = nullptr;
+  int64_t nviews = 0;
   // STRUCT: a mask and no payload (w_out 0).  Field columns follow the table's columns; `parent`: the STRUCT column
   // whose masks a field column's rows are ANDed with (-1: a table column)
   bool is_struct = false;
@@ -276,9 +283,11 @@ bool map_format(App *a, const char *cn, const char *what, const char *fmt, int32
     case DMB_TYPE_DECIMAL: if (starts("d:")) return map_decimal(a, cn, what, fmt, type_id, dec_w, dec_s, in); break;
     case DMB_TYPE_VARCHAR:
       if (is("u") || is("U")) { in->is_string = true; in->large = is("U"); in->w_out = 16; return true; }
+      if (is("vu")) { fixed(16); in->is_view = true; return true; }
       break;
     case DMB_TYPE_BLOB:
       if (is("z") || is("Z")) { in->is_string = true; in->large = is("Z"); in->w_out = 16; return true; }
+      if (is("vz")) { fixed(16); in->is_view = true; return true; }
       break;
     default: break;
   }
@@ -302,9 +311,10 @@ bool grow(Scope &sc, uint8_t *&p, size_t &cap, size_t need, bool pinned = false)
 struct ListOut {  // one LIST column of a slot: the child vectors of the sub-batch and where each chunk's mask starts
   uint8_t *d_child = nullptr, *h_child = nullptr;
   uint8_t *d_words = nullptr, *h_words = nullptr;
-  size_t child_cap = 0, h_child_cap = 0, words_cap = 0, h_words_cap = 0;
+  uint8_t *d_dense = nullptr;  // a dictionary child: the element validity the gather writes, bit 0 = element e0
+  size_t child_cap = 0, h_child_cap = 0, words_cap = 0, h_words_cap = 0, dense_cap = 0;
   int64_t *d_cword = nullptr, *h_cword = nullptr;
-  int64_t child_bytes = 0, words = 0;
+  int64_t child_bytes = 0, words = 0, e0 = 0;
 };
 
 struct Slot {  // device + pinned buffers of one in-flight sub-batch
@@ -312,7 +322,9 @@ struct Slot {  // device + pinned buffers of one in-flight sub-batch
   std::vector<uint64_t *> d_val, h_val;
   std::vector<ListOut> lists;                     // [ncols], used by LIST columns
   unsigned int *d_err = nullptr, *h_err = nullptr;  // [ncols]: rev_list_kernel error flags
-  unsigned long long *d_eerr = nullptr, *h_eerr = nullptr;  // [ncols]: ENUM columns' first offending row (~0: none)
+  // [ncols]: the first offending row of an ENUM, view or dictionary column, or element of a LIST column's view or
+  // dictionary child (~0: none)
+  unsigned long long *d_eerr = nullptr, *h_eerr = nullptr;
   cudaEvent_t ev_out = nullptr;
   int64_t r0 = 0, r1 = 0;
   bool busy = false;
@@ -324,6 +336,35 @@ int64_t offset_at(const ColInput &ci, int64_t row) {
   int32_t v; memcpy(&v, ci.offsets + 4 * row, 4); return v;
 }
 
+// the Arrow dictionary index of `row`, read on the host; false (with the appender error, `what` naming the row) when it
+// is outside the dictionary
+bool dict_index_at(App *a, const char *cn, const char *what, const ColInput &ci, int64_t row, int64_t *idx) {
+  uint64_t raw = 0;
+  memcpy(&raw, ci.values + (size_t)row * (size_t)ci.w_in, (size_t)ci.w_in);
+  const int sh = 64 - 8 * ci.w_in;
+  *idx = ci.index_signed ? (int64_t)(raw << sh) >> sh : (int64_t)raw;
+  if (*idx >= 0 && *idx < ci.dict_len) return true;
+  fail(a, "%s, %s %lld: dictionary index %lld is outside the Arrow dictionary (%lld entries)", cn, what, (long long)row, (long long)*idx,
+       (long long)ci.dict_len);
+  return false;
+}
+
+// the appender error for the first offending row of a VARCHAR / BLOB column read from string views or a dictionary,
+// rendered from the host buffers (`what`: "row", "list element" or "dictionary entry")
+int32_t string_error(App *a, const char *cn, const char *what, const ColInput &ci, int64_t row) {
+  int64_t idx;
+  if (ci.is_dict) return dict_index_at(a, cn, what, ci, row, &idx) ? fail(a, "%s, %s %lld: malformed", cn, what, (long long)row) : 0;
+  int32_t v[4];
+  memcpy(v, ci.values + (size_t)row * 16, 16);
+  const long long r = (long long)row;
+  if (v[0] < 0) return fail(a, "%s, %s %lld: string view length %d is negative", cn, what, r, v[0]);
+  if ((uint32_t)v[2] >= (uint64_t)ci.nviews)
+    return fail(a, "%s, %s %lld: string view buffer index %u is outside the array's %lld data buffers", cn, what, r, (uint32_t)v[2], (long long)ci.nviews);
+  if (v[3] < 0) return fail(a, "%s, %s %lld: string view offset %d is negative", cn, what, r, v[3]);
+  return fail(a, "%s, %s %lld: string view bytes [%d, %lld) pass the end of data buffer %d (%lld bytes)", cn, what, r, v[3],
+              (long long)v[3] + v[0], v[2], (long long)ci.view_sizes[v[2]]);
+}
+
 // the appender error for the first offending row of an ENUM column, rendered from the host buffers
 int32_t enum_error(App *a, const char *cn, const ColInput &ci, int64_t row) {
   const uint8_t *p;
@@ -333,13 +374,8 @@ int32_t enum_error(App *a, const char *cn, const ColInput &ci, int64_t row) {
     p = ci.data + o0;
     len = offset_at(ci, row + 1) - o0;
   } else {
-    uint64_t raw = 0;
-    memcpy(&raw, ci.values + (size_t)row * (size_t)ci.w_in, (size_t)ci.w_in);
-    const int sh = 64 - 8 * ci.w_in;
-    const int64_t idx = ci.index_signed ? (int64_t)(raw << sh) >> sh : (int64_t)raw;
-    if (idx < 0 || idx >= ci.dict_len)
-      return fail(a, "%s, row %lld: dictionary index %lld is outside the Arrow dictionary (%lld entries)", cn, (long long)row,
-                  (long long)idx, (long long)ci.dict_len);
+    int64_t idx;
+    if (!dict_index_at(a, cn, "row", ci, row, &idx)) return 0;
     ColInput d;
     d.offsets = ci.dict_offsets;
     d.large = ci.dict_large;
@@ -352,16 +388,52 @@ int32_t enum_error(App *a, const char *cn, const ColInput &ci, int64_t row) {
               len > shown ? "..." : "");
 }
 
-int32_t sink_slot(App *a, Slot &s, const std::vector<ColInput> &cols, const std::vector<std::vector<int64_t>> &bounds) {
+// the conversion of column `ci` itself, or of its LIST child, reports its first offending row in the slot's error word
+bool uses_error_word(const ColInput &ci) {
+  const ColInput &x = ci.is_list ? *ci.child : ci;
+  return x.is_enum || x.is_view || x.is_dict;
+}
+
+// the Arrow dictionary of a dictionary column as a column of its own: utf8 / large_utf8 / binary / large_binary or views
+ColInput dict_values(const ColInput &ci) {
+  ColInput d;
+  d.is_string = !ci.dict_view;
+  d.is_view = ci.dict_view;
+  d.large = ci.dict_large;
+  d.offsets = ci.dict_offsets;
+  d.data = ci.dict_data;
+  d.validity = ci.dict_validity;
+  d.bit_offset = ci.dict_bit_offset;
+  d.w_out = 16;
+  if (ci.dict_view) {
+    d.values = ci.dict_offsets;
+    d.w_in = 16;
+    d.rev_op = DMB_REV_COPY16;
+    d.view_bufs = ci.view_bufs;
+    d.view_sizes = ci.view_sizes;
+    d.nviews = ci.nviews;
+  }
+  return d;
+}
+
+// `h_derr`: per column, the first malformed string view of a dictionary of views (~0: none; NULL: no such dictionary)
+int32_t sink_slot(App *a, Slot &s, const std::vector<ColInput> &cols, const std::vector<std::vector<int64_t>> &bounds,
+                  const unsigned long long *h_derr) {
   if (!s.busy) return 1;
   if (check_cuda(cudaEventSynchronize(s.ev_out), "appender copy-out wait")) return fail(a, "%s", duckdb_mb_gpu_last_error());
   s.busy = false;
   const int nc = (int)cols.size();
-  for (int c = 0; c < nc; ++c)  // a malformed sub-batch reaches no sink
-    if (cols[(size_t)c].is_list && s.h_err[c])
+  for (int c = 0; c < nc; ++c) {  // a malformed sub-batch reaches no sink
+    const ColInput &ci = cols[(size_t)c];
+    const ColInput &x = ci.is_list ? *ci.child : ci;
+    if (h_derr && h_derr[c] != ~0ull) return string_error(a, col_name(a, c).c_str(), "dictionary entry", dict_values(x), (int64_t)h_derr[c]);
+    if (ci.is_list && s.h_err[c])
       return fail(a, "column %d: Arrow list offsets decrease within rows [%lld, %lld)", c, (long long)s.r0, (long long)s.r1);
-    else if (cols[(size_t)c].is_enum && s.h_eerr[c] != ~0ull)
-      return enum_error(a, col_name(a, c).c_str(), cols[(size_t)c], s.r0 + (int64_t)s.h_eerr[c]);
+    if (!uses_error_word(ci) || s.h_eerr[c] == ~0ull) continue;
+    if (ci.is_enum) return enum_error(a, col_name(a, c).c_str(), ci, s.r0 + (int64_t)s.h_eerr[c]);
+    if (ci.is_list) return string_error(a, col_name(a, c).c_str(), "list element", x, s.lists[(size_t)c].e0 + (int64_t)s.h_eerr[c]);
+    return string_error(a, col_name(a, c).c_str(), "row", ci, s.r0 + (int64_t)s.h_eerr[c]);
+  }
   if (!a->sink) return 1;
   const int nt = a->ncols;  // the sink sees the table's columns; field columns through duckdb_mb_gpu_appender_struct_field
   std::vector<const void *> vd((size_t)nt);
@@ -484,21 +556,96 @@ extern "C" int64_t dmb_rev_list_cut(const int64_t *const *bounds, int32_t nlists
 namespace dmb {
 namespace {
 
-// Once per conversion, before the first sub-batch's kernels: every ENUM column's lookup table and labels go to the
-// device, and for a dictionary column the Arrow dictionary too, whose labels the lookup kernel turns into the remap (one
-// code per dictionary entry) that the index kernel of every sub-batch reads.  `*base`: per column, the job fields that do
-// not change between sub-batches (empty when no column is an ENUM).
-int32_t stage_enums(App *a, Scope &sc, const std::vector<ColInput> &cols, std::vector<dmb_rev_enum_job> *base) {
+// per column, the job fields of its conversion (or its LIST child's) that do not change between sub-batches
+struct CallTables {
+  std::vector<dmb_rev_enum_job> enums;  // ENUM columns
+  std::vector<dmb_rev_view_job> views;  // string views: the table of data buffers
+  std::vector<dmb_rev_dict_job> dicts;  // dictionaries of strings: the string_t table of the entries
+  unsigned long long *d_err = nullptr, *h_err = nullptr;  // a dictionary of views: its first malformed entry (~0: none)
+};
+
+// Once per conversion, before the first sub-batch's kernels:
+//  * every ENUM column's lookup table and labels go to the device, and for a dictionary column the Arrow dictionary too,
+//    whose labels the lookup kernel turns into the remap (one code per dictionary entry) that the index kernel of every
+//    sub-batch reads;
+//  * a string view column's data buffers become a device table of {host base, size};
+//  * a VARCHAR / BLOB dictionary column's dictionary is converted to string_t by the string or view kernel, the table
+//    every sub-batch's gather reads, and its NULL entries are marked.
+int32_t stage_tables(App *a, Scope &sc, const std::vector<ColInput> &cols, CallTables *t) {
   CtxCore &c = *a->core;
-  base->clear();
+  const size_t nc = cols.size();
+  t->enums.assign(nc, dmb_rev_enum_job());
+  t->views.assign(nc, dmb_rev_view_job());
+  t->dicts.assign(nc, dmb_rev_dict_job());
   std::vector<dmb_rev_enum_job> remaps;
   std::vector<int64_t> remap_rows;
-  for (size_t j = 0; j < cols.size(); ++j) {
-    const ColInput &ci = cols[j];
+  std::vector<dmb_rev_string_job> str_builds;
+  std::vector<dmb_rev_view_job> view_builds;
+  std::vector<int64_t> str_rows, view_rows;
+  std::vector<std::pair<dmb_string_t *, std::pair<const uint64_t *, int64_t>>> marks;
+  // the {host base, size} table of a view array's data buffers
+  auto buffer_table = [&](const ColInput &v, const dmb_view_buffer **out) {
+    std::vector<dmb_view_buffer> hb((size_t)v.nviews);
+    for (int64_t i = 0; i < v.nviews; ++i) hb[(size_t)i] = dmb_view_buffer{(uint64_t)(uintptr_t)v.view_bufs[i], v.view_sizes[i]};
+    void *d = sc.dalloc(hb.size() * sizeof(dmb_view_buffer) + 16);
+    if (!d || (!hb.empty() && stage_contiguous(c, c.s_in, d, hb.data(), hb.size() * sizeof(dmb_view_buffer), -1, &a->bytes_h2d))) return false;
+    *out = (const dmb_view_buffer *)d;
+    return true;
+  };
+  for (size_t j = 0; j < nc; ++j) {
+    const ColInput &ci = cols[j].is_list ? *cols[j].child : cols[j];
+    if (ci.is_view) {
+      dmb_rev_view_job &vj = t->views[j];
+      vj.nbuffers = ci.nviews;
+      if (!buffer_table(ci, &vj.buffers)) return fail(a, "%s", duckdb_mb_gpu_last_error());
+      continue;
+    }
+    if (ci.is_dict) {
+      dmb_rev_dict_job &dj = t->dicts[j];
+      dj.index_width = ci.w_in;
+      dj.index_signed = ci.index_signed ? 1 : 0;
+      dj.dict_len = ci.dict_len;
+      if (ci.dict_len == 0) continue;  // every valid row is out of range
+      const ColInput d = dict_values(ci);
+      const int64_t cap = ((ci.dict_len + DMB_VECTOR_SIZE - 1) / DMB_VECTOR_SIZE) * DMB_VECTOR_SIZE;  // the kernels fill whole chunks
+      dmb_string_t *table = (dmb_string_t *)sc.dalloc((size_t)cap * sizeof(dmb_string_t));
+      uint64_t *masks = (uint64_t *)sc.dalloc((size_t)cap / 8);
+      if (!table || !masks) return fail(a, "%s", duckdb_mb_gpu_last_error());
+      InBuf ib;
+      dmb_rev_fixed_job fj;
+      dmb_rev_string_job sj;
+      const uint8_t *d_validity = nullptr;
+      int64_t bit_off = 0;
+      if (!stage_rows(a, sc, d, ib, (int)j, 0, ci.dict_len, table, masks, &fj, &sj, &d_validity, &bit_off)) return 0;
+      if (d.is_view) {
+        if (!t->d_err) {
+          t->d_err = (unsigned long long *)sc.dalloc(8 * nc);
+          t->h_err = (unsigned long long *)sc.palloc(8 * nc);
+          if (!t->d_err || !t->h_err) return fail(a, "%s", duckdb_mb_gpu_last_error());
+        }
+        dmb_rev_view_job vj;
+        memset(&vj, 0, sizeof(vj));
+        vj.nbuffers = d.nviews;
+        if (!buffer_table(d, &vj.buffers)) return fail(a, "%s", duckdb_mb_gpu_last_error());
+        vj.in_views = fj.in_values;
+        vj.in_validity = d_validity;
+        vj.in_bit_offset = bit_off;
+        vj.out = table;
+        vj.out_validity = masks;
+        vj.error = t->d_err + j;
+        view_builds.push_back(vj);
+        view_rows.push_back(ci.dict_len);
+      } else {
+        str_builds.push_back(sj);
+        str_rows.push_back(ci.dict_len);
+      }
+      if (d.validity) marks.push_back({table, {masks, ci.dict_len}});
+      dj.table = table;
+      continue;
+    }
     if (!ci.is_enum) continue;
-    base->resize(cols.size());
     const EnumDecl &e = a->enums[j];
-    dmb_rev_enum_job &ej = (*base)[j];
+    dmb_rev_enum_job &ej = t->enums[j];
     memset(&ej, 0, sizeof(ej));
     ej.out_width = e.width;
     const size_t tb = e.slots.size() * sizeof(uint4), ob = e.offsets.size() * 4;
@@ -516,14 +663,7 @@ int32_t stage_enums(App *a, Scope &sc, const std::vector<ColInput> &cols, std::v
     ej.index_signed = ci.index_signed ? 1 : 0;
     ej.dict_len = ci.dict_len;
     if (ci.dict_len == 0) continue;  // every valid row is out of range
-    // the Arrow dictionary as a string column of its own: its codes are the remap
-    ColInput d;
-    d.is_string = true;
-    d.large = ci.dict_large;
-    d.offsets = ci.dict_offsets;
-    d.data = ci.dict_data;
-    d.validity = ci.dict_validity;
-    d.bit_offset = ci.dict_bit_offset;
+    const ColInput d = dict_values(ci);  // its codes are the remap
     InBuf ib;
     dmb_rev_fixed_job fj;
     dmb_rev_string_job sj;
@@ -545,12 +685,23 @@ int32_t stage_enums(App *a, Scope &sc, const std::vector<ColInput> &cols, std::v
     remap_rows.push_back(ci.dict_len);
     ej.remap = remap;
   }
-  if (remaps.empty()) return 1;
+  if (remaps.empty() && str_builds.empty() && view_builds.empty()) return 1;
   cudaEvent_t ev = sc.event(false);
-  if (!ev || check_cuda(cudaEventRecord(ev, c.s_in), "ENUM staging") || check_cuda(cudaStreamWaitEvent(c.s_compute, ev, 0), "wait ENUM staging"))
+  if (!ev || check_cuda(cudaEventRecord(ev, c.s_in), "dictionary staging") || check_cuda(cudaStreamWaitEvent(c.s_compute, ev, 0), "wait dictionary staging"))
     return fail(a, "%s", duckdb_mb_gpu_last_error());
   for (size_t i = 0; i < remaps.size(); ++i)
     if (dmb_dev_rev_enum_batch(&remaps[i], remap_rows[i], c.s_compute)) return fail(a, "%s", duckdb_mb_gpu_last_error());
+  for (size_t i = 0; i < str_builds.size(); ++i)
+    if (dmb_dev_rev_string_batch(&str_builds[i], str_rows[i], c.s_compute)) return fail(a, "%s", duckdb_mb_gpu_last_error());
+  if (t->d_err && check_cuda(cudaMemsetAsync(t->d_err, 0xff, 8 * nc, c.s_compute), "dictionary error words reset"))
+    return fail(a, "%s", duckdb_mb_gpu_last_error());
+  for (size_t i = 0; i < view_builds.size(); ++i)
+    if (dmb_dev_rev_view_batch(&view_builds[i], view_rows[i], c.s_compute)) return fail(a, "%s", duckdb_mb_gpu_last_error());
+  for (const auto &m : marks)
+    if (dmb_dev_rev_dict_mark(m.first, m.second.first, m.second.second, c.s_compute)) return fail(a, "%s", duckdb_mb_gpu_last_error());
+  // read back before the first sub-batch's kernels, so before its copy-out, which sink_slot waits for
+  if (t->d_err && check_cuda(cudaMemcpyAsync(t->h_err, t->d_err, 8 * nc, cudaMemcpyDeviceToHost, c.s_compute), "dictionary error words D2H"))
+    return fail(a, "%s", duckdb_mb_gpu_last_error());
   return 1;
 }
 
@@ -665,16 +816,17 @@ int32_t convert_rows(App *a, const std::vector<ColInput> &cols, int64_t nrows) {
   if (!h_jobs || !d_jobs) return fail(a, "%s", duckdb_mb_gpu_last_error());
   cudaEventRecord(in0, c.s_in);
   cudaEventRecord(out0, c.s_out);
-  std::vector<dmb_rev_enum_job> enum_base;
-  if (!stage_enums(a, sc, cols, &enum_base)) return 0;
-  const bool any_enum = !enum_base.empty();
+  CallTables tabs;
+  if (!stage_tables(a, sc, cols, &tabs)) return 0;
+  bool any_err = false;  // some conversion reports rows in the slot's error words
+  for (const ColInput &ci : cols) any_err = any_err || uses_error_word(ci);
   for (size_t b = 0; b + 1 < cuts.size(); ++b) {
     const int64_t r0 = cuts[b] * DMB_VECTOR_SIZE, r1 = cuts[b + 1] * DMB_VECTOR_SIZE < nrows ? cuts[b + 1] * DMB_VECTOR_SIZE : nrows;
     const int64_t n = r1 - r0;
     const int64_t nch = cuts[b + 1] - cuts[b];
     const int si = (int)(b % (size_t)nslots);
     Slot &slot = slots[si];
-    if (!sink_slot(a, slot, cols, bounds)) return 0;  // the slot's previous sub-batch leaves first
+    if (!sink_slot(a, slot, cols, bounds, tabs.h_err)) return 0;  // the slot's previous sub-batch leaves first
     // the job array of this slot is reused as well: its previous launch has completed (sink_slot waited)
     dmb_rev_fixed_job *hj = h_jobs + (size_t)si * (size_t)nc * 2, *dj = d_jobs + (size_t)si * (size_t)nc * 2;
     int nfixed = 0, nchild_fixed = 0;
@@ -683,6 +835,9 @@ int32_t convert_rows(App *a, const std::vector<ColInput> &cols, int64_t nrows) {
     std::vector<dmb_rev_string_job> strs;
     std::vector<dmb_rev_list_job> lists;
     std::vector<dmb_rev_enum_job> enums;
+    std::vector<dmb_rev_view_job> views;
+    std::vector<dmb_rev_dict_job> dicts;
+    std::vector<int64_t> view_rows, dict_rows;
     std::vector<int64_t> child_rows;  // element count of each child job: fixed-width ones first, in job order
     std::vector<int64_t> str_rows;
     std::vector<int> masks_from_bytes;  // columns
@@ -719,7 +874,7 @@ int32_t convert_rows(App *a, const std::vector<ColInput> &cols, int64_t nrows) {
           sj.in_bit_offset = 0;
         }
         if (ci.is_enum) {
-          dmb_rev_enum_job ej = enum_base[(size_t)j];
+          dmb_rev_enum_job ej = tabs.enums[(size_t)j];
           if (ci.is_string) {
             ej.in_offsets = sj.in_offsets;
             ej.in_data = sj.in_data;
@@ -733,6 +888,26 @@ int32_t convert_rows(App *a, const std::vector<ColInput> &cols, int64_t nrows) {
           ej.out_validity = slot.d_val[(size_t)j];
           ej.error = slot.d_eerr + j;
           enums.push_back(ej);
+        } else if (ci.is_view) {
+          dmb_rev_view_job vj = tabs.views[(size_t)j];
+          vj.in_views = hj[nfixed].in_values;  // (that job slot is reused by the next fixed-width column)
+          vj.in_validity = d_validity;
+          vj.in_bit_offset = bit_off;
+          vj.out = (dmb_string_t *)slot.d_out[(size_t)j];
+          vj.out_validity = slot.d_val[(size_t)j];
+          vj.error = slot.d_eerr + j;
+          views.push_back(vj);
+          view_rows.push_back(n);
+        } else if (ci.is_dict) {
+          dmb_rev_dict_job dj = tabs.dicts[(size_t)j];
+          dj.in_indices = hj[nfixed].in_values;
+          dj.in_validity = d_validity;
+          dj.in_bit_offset = bit_off;
+          dj.out = (dmb_string_t *)slot.d_out[(size_t)j];
+          dj.out_validity = slot.d_val[(size_t)j];
+          dj.error = slot.d_eerr + j;
+          dicts.push_back(dj);
+          dict_rows.push_back(n);
         } else if (ci.is_string) { strs.push_back(sj); str_rows.push_back(n); }
         else ++nfixed;
         continue;
@@ -756,9 +931,13 @@ int32_t convert_rows(App *a, const std::vector<ColInput> &cols, int64_t nrows) {
       if (check_cuda(cudaMemcpyAsync(lo.d_cword, lo.h_cword, sizeof(int64_t) * (size_t)(nch + 1), cudaMemcpyHostToDevice, c.s_in), "child_word H2D"))
         return fail(a, "%s", duckdb_mb_gpu_last_error());
       a->bytes_h2d += sizeof(int64_t) * (uint64_t)(nch + 1);
-      const int64_t child_slots = cc.is_string ? ((ne + DMB_VECTOR_SIZE - 1) / DMB_VECTOR_SIZE) * DMB_VECTOR_SIZE : ne;  // rev_string_kernel fills whole vectors
+      // the string, view and dictionary kernels fill whole vectors
+      const bool whole = cc.is_string || cc.is_view || cc.is_dict;
+      const int64_t child_slots = whole ? ((ne + DMB_VECTOR_SIZE - 1) / DMB_VECTOR_SIZE) * DMB_VECTOR_SIZE : ne;
       lo.child_bytes = ne * cc.w_out;
+      lo.e0 = e0;
       if (!grow(sc, lo.d_child, lo.child_cap, (size_t)child_slots * (size_t)cc.w_out + 64) ||
+          (cc.is_dict && !grow(sc, lo.d_dense, lo.dense_cap, (size_t)child_slots / 8 + 64)) ||
           !grow(sc, lo.h_child, lo.h_child_cap, (size_t)lo.child_bytes + 64, true) ||
           !grow(sc, lo.d_words, lo.words_cap, (size_t)lo.words * 8 + 64) || !grow(sc, lo.h_words, lo.h_words_cap, (size_t)lo.words * 8 + 64, true))
         return fail(a, "%s", duckdb_mb_gpu_last_error());
@@ -771,7 +950,30 @@ int32_t convert_rows(App *a, const std::vector<ColInput> &cols, int64_t nrows) {
         int64_t cbit_off = 0;
         // out_validity NULL: the child masks are the list kernel's, per chunk
         if (!stage_rows(a, sc, cc, childbuf[(size_t)si * (size_t)nc + (size_t)j], j, e0, e1, lo.d_child, nullptr, fj, &sj, &d_cvalidity, &cbit_off)) return 0;
-        if (cc.is_string) { strs.push_back(sj); str_rows.push_back(ne); }
+        // A view or dictionary child is judged by its own bitmap alone: an element the child marks valid is checked even in
+        // the segment of a NULL list row, which Arrow's validation of the child array requires as well.
+        if (cc.is_view) {
+          dmb_rev_view_job vj = tabs.views[(size_t)j];
+          vj.in_views = fj->in_values;  // (that job slot is reused by the next child)
+          vj.in_validity = d_cvalidity;
+          vj.in_bit_offset = cbit_off;
+          vj.out = (dmb_string_t *)lo.d_child;
+          vj.error = slot.d_eerr + j;
+          views.push_back(vj);
+          view_rows.push_back(ne);
+        } else if (cc.is_dict) {  // a NULL dictionary entry makes an element NULL: the list kernel reads the gather's bitmap
+          dmb_rev_dict_job dj = tabs.dicts[(size_t)j];
+          dj.in_indices = fj->in_values;
+          dj.in_validity = d_cvalidity;
+          dj.in_bit_offset = cbit_off;
+          dj.out = (dmb_string_t *)lo.d_child;
+          dj.out_validity = (uint64_t *)lo.d_dense;
+          dj.error = slot.d_eerr + j;
+          dicts.push_back(dj);
+          dict_rows.push_back(ne);
+          d_cvalidity = lo.d_dense;
+          cbit_off = 0;
+        } else if (cc.is_string) { strs.push_back(sj); str_rows.push_back(ne); }
         else { ++nchild_fixed; child_rows.push_back(ne); }
         lj.in_child_validity = d_cvalidity;
         lj.child_bit_offset = cbit_off;
@@ -813,10 +1015,14 @@ int32_t convert_rows(App *a, const std::vector<ColInput> &cols, int64_t nrows) {
     }
     for (size_t i = 0; i < strs.size(); ++i)
       if (dmb_dev_rev_string_batch(&strs[i], str_rows[i], c.s_compute)) return fail(a, "%s", duckdb_mb_gpu_last_error());
-    if (any_enum && check_cuda(cudaMemsetAsync(slot.d_eerr, 0xff, 8 * (size_t)nc, c.s_compute), "ENUM error words reset"))
+    if (any_err && check_cuda(cudaMemsetAsync(slot.d_eerr, 0xff, 8 * (size_t)nc, c.s_compute), "error words reset"))
       return fail(a, "%s", duckdb_mb_gpu_last_error());
     for (auto &ej : enums)
       if (dmb_dev_rev_enum_batch(&ej, n, c.s_compute)) return fail(a, "%s", duckdb_mb_gpu_last_error());
+    for (size_t i = 0; i < views.size(); ++i)
+      if (dmb_dev_rev_view_batch(&views[i], view_rows[i], c.s_compute)) return fail(a, "%s", duckdb_mb_gpu_last_error());
+    for (size_t i = 0; i < dicts.size(); ++i)
+      if (dmb_dev_rev_dict_batch(&dicts[i], dict_rows[i], c.s_compute)) return fail(a, "%s", duckdb_mb_gpu_last_error());
     if (!lists.empty() && check_cuda(cudaMemsetAsync(slot.d_err, 0, sizeof(unsigned int) * (size_t)nc, c.s_compute), "error flags reset"))
       return fail(a, "%s", duckdb_mb_gpu_last_error());
     for (auto &lj : lists)
@@ -840,7 +1046,7 @@ int32_t convert_rows(App *a, const std::vector<ColInput> &cols, int64_t nrows) {
     }
     if (!lists.empty() && check_cuda(cudaMemcpyAsync(slot.h_err, slot.d_err, sizeof(unsigned int) * (size_t)nc, cudaMemcpyDeviceToHost, c.s_out), "error flags D2H"))
       return fail(a, "%s", duckdb_mb_gpu_last_error());
-    if (any_enum && check_cuda(cudaMemcpyAsync(slot.h_eerr, slot.d_eerr, 8 * (size_t)nc, cudaMemcpyDeviceToHost, c.s_out), "ENUM error words D2H"))
+    if (any_err && check_cuda(cudaMemcpyAsync(slot.h_eerr, slot.d_eerr, 8 * (size_t)nc, cudaMemcpyDeviceToHost, c.s_out), "error words D2H"))
       return fail(a, "%s", duckdb_mb_gpu_last_error());
     cudaEventRecord(slot.ev_out, c.s_out);
     slot.r0 = r0;
@@ -851,7 +1057,7 @@ int32_t convert_rows(App *a, const std::vector<ColInput> &cols, int64_t nrows) {
   const size_t nsub = cuts.size() - 1;
   for (int k = 0; k < nslots; ++k) {  // oldest first
     Slot &slot = slots[(int)((nsub + (size_t)k) % (size_t)nslots)];
-    if (!sink_slot(a, slot, cols, bounds)) return 0;
+    if (!sink_slot(a, slot, cols, bounds, tabs.h_err)) return 0;
   }
   cudaEventRecord(out1, c.s_out);
   if (check_cuda(cudaStreamSynchronize(c.s_out), "appender sync") || check_cuda(cudaStreamSynchronize(c.s_in), "appender sync"))
@@ -964,6 +1170,11 @@ void bind_buffers(ColInput &ci, const ArrowArray *arr, int64_t off) {
     if (ci.is_string) ci.data = arr->n_buffers > 2 && arr->buffers[2] ? (const uint8_t *)arr->buffers[2] : kNoData;
   } else if (ci.is_bits) {
     ci.values = arr->n_buffers > 1 ? (const uint8_t *)arr->buffers[1] : nullptr;
+  } else if (ci.is_view) {  // validity, views, the data buffers, their sizes
+    ci.values = arr->n_buffers > 1 && arr->buffers[1] ? (const uint8_t *)arr->buffers[1] + (size_t)off * 16 : nullptr;
+    ci.nviews = arr->n_buffers >= 3 ? arr->n_buffers - 3 : 0;
+    ci.view_bufs = arr->buffers + 2;
+    ci.view_sizes = arr->n_buffers >= 3 ? (const int64_t *)arr->buffers[arr->n_buffers - 1] : nullptr;
   } else {
     ci.values = arr->n_buffers > 1 && arr->buffers[1] ? (const uint8_t *)arr->buffers[1] + (size_t)off * (size_t)ci.w_in : nullptr;
   }
@@ -976,6 +1187,85 @@ const char *nested_name(const char *fmt) {
   if (strcmp(fmt, "+vl") == 0 || strcmp(fmt, "+vL") == 0) return "list view";
   if (strncmp(fmt, "+w:", 3) == 0) return "fixed_size_list";
   return "nested type";
+}
+
+// a string view array's buffers: validity, views, k data buffers, then the k sizes.  With k = 0 the sizes buffer is empty,
+// and Arrow C++ exports it as NULL: an all-NULL, empty or all-inline array.
+bool check_views(App *a, const char *cn, const ArrowArray *arr) {
+  if (arr->n_buffers < 3) {
+    fail(a, "%s: the Arrow string view array is malformed: it has %lld buffers, and needs validity, views, its data buffers and "
+         "their sizes (at least 3)", cn, (long long)arr->n_buffers);
+    return false;
+  }
+  if (arr->n_buffers > 3 && !arr->buffers[arr->n_buffers - 1]) {
+    fail(a, "%s: the Arrow string view array is malformed: its %lld data buffers come without their sizes", cn,
+         (long long)(arr->n_buffers - 3));
+    return false;
+  }
+  return true;
+}
+
+// the index width and signedness of an Arrow dictionary's index format, false when it is not an integer format
+bool map_dict_indices(const char *fmt, ColInput *ci) {
+  if (strlen(fmt) != 1 || !strchr("cCsSiIlL", fmt[0])) return false;
+  const char f = fmt[0];
+  ci->w_in = f == 'c' || f == 'C' ? 1 : f == 's' || f == 'S' ? 2 : f == 'i' || f == 'I' ? 4 : 8;
+  ci->rev_op = copy_op(ci->w_in);
+  ci->index_signed = f >= 'a' && f <= 'z';
+  return true;
+}
+
+// the Arrow dictionary `d` (values of format `dfmt`: u U z Z, or vu vz) into the dict_* fields of `ci`
+bool bind_dict(App *a, const char *cn, const ArrowArray *d, const char *dfmt, ColInput *ci) {
+  static const uint8_t kNoData[16] = {0};
+  if (!d) {
+    fail(a, "%s: the Arrow dictionary array is missing", cn);
+    return false;
+  }
+  ci->dict_view = dfmt[0] == 'v';
+  ci->dict_large = dfmt[0] == 'U' || dfmt[0] == 'Z';
+  ci->dict_len = d->length;
+  ci->dict_bit_offset = d->offset;
+  ci->dict_validity = (d->null_count != 0 && d->n_buffers > 0) ? (const uint8_t *)d->buffers[0] : nullptr;
+  const int ew = ci->dict_view ? 16 : ci->dict_large ? 8 : 4;
+  ci->dict_offsets = d->n_buffers > 1 && d->buffers[1] ? (const uint8_t *)d->buffers[1] + (size_t)d->offset * (size_t)ew : nullptr;
+  if (ci->dict_view) {
+    if (!check_views(a, cn, d)) return false;
+    ci->nviews = d->n_buffers - 3;
+    ci->view_bufs = d->buffers + 2;
+    ci->view_sizes = (const int64_t *)d->buffers[d->n_buffers - 1];
+  } else {
+    ci->dict_data = d->n_buffers > 2 && d->buffers[2] ? (const uint8_t *)d->buffers[2] : kNoData;
+  }
+  if (d->length > 0 && !ci->dict_offsets) {
+    fail(a, "%s: the Arrow dictionary has no %s buffer", cn, ci->dict_view ? "views" : "offsets");
+    return false;
+  }
+  return true;
+}
+
+// an Arrow dictionary array (indices c C s S i I l L) of strings for a VARCHAR (u U vu) or BLOB (z Z vz) column, table column,
+// field or LIST child
+bool map_string_dict(App *a, const char *cn, const ArrowArray *arr, const ArrowSchema *sch, int32_t type_id, ColInput *ci) {
+  const char *fmt = sch->format;
+  const char *dfmt = sch->dictionary->format ? sch->dictionary->format : "";
+  const bool blob = type_id == DMB_TYPE_BLOB;
+  const char *col = blob ? "BLOB" : "VARCHAR";
+  if (!map_dict_indices(fmt, ci)) {
+    fail(a, "%s: Arrow dictionary index format '%s' cannot be appended to a %s column", cn, fmt, col);
+    return false;
+  }
+  static const char *const kValues[2][3] = {{"u", "U", "vu"}, {"z", "Z", "vz"}};
+  bool ok = false;
+  for (const char *f : kValues[blob ? 1 : 0]) ok = ok || strcmp(dfmt, f) == 0;
+  if (!ok) {
+    fail(a, "%s: an Arrow dictionary of '%s' values cannot be appended to a %s column", cn, dfmt, col);
+    return false;
+  }
+  if (!bind_dict(a, cn, arr->dictionary, dfmt, ci)) return false;
+  ci->is_dict = true;
+  ci->w_out = 16;
+  return true;
 }
 
 // Arrow list / large_list -> a LIST column whose child type the table declared (duckdb_mb_gpu_appender_set_list)
@@ -1002,13 +1292,17 @@ bool map_list(App *a, int j, const ArrowArray *arr, const ArrowSchema *sch, ColI
     return false;
   }
   int32_t dec_w = d.dec_width, dec_s = d.dec_scale;  // a DECIMAL child: set_list declared it
-  if (!map_format(a, col_name(a, j).c_str(), "list child format", cfmt, d.type_id, &dec_w, &dec_s, child)) {
+  const std::string cn = col_name(a, j);
+  if ((d.type_id == DMB_TYPE_VARCHAR || d.type_id == DMB_TYPE_BLOB) && sch->children[0]->dictionary) {
+    if (!map_string_dict(a, cn.c_str(), carr, sch->children[0], d.type_id, child)) return false;
+  } else if (!map_format(a, cn.c_str(), "list child format", cfmt, d.type_id, &dec_w, &dec_s, child)) {
     const bool decimal_child = d.type_id == DMB_TYPE_DECIMAL || d.type_id == DMB_TYPE_HUGEINT;
     if (!decimal_child || strncmp(cfmt, "d:", 2) != 0)  // map_decimal's refusal names its own reason
       fail(a, "column %d: Arrow list child format '%s' does not match the declared child type %d", j, cfmt, d.type_id);
     return false;
   }
   bind_buffers(*child, carr, carr->offset);
+  if (child->is_view && !check_views(a, cn.c_str(), carr)) return false;
   child->child_len = carr->length;
   ci->is_list = true;
   ci->large = fmt[1] == 'L';
@@ -1047,7 +1341,6 @@ bool map_struct(App *a, int j, const char *cn, const ArrowArray *arr, const Arro
 
 // an Arrow array for an ENUM column: a dictionary array (indices c C s S i I l L, labels u / U) or plain u / U labels
 bool map_enum(App *a, int j, const char *cn, const ArrowArray *arr, const ArrowSchema *sch, ColInput *ci) {
-  static const uint8_t kNoData[16] = {0};
   const char *fmt = sch->format;
   const EnumDecl &e = a->enums[(size_t)j];
   if (!e.width) {
@@ -1078,26 +1371,8 @@ bool map_enum(App *a, int j, const char *cn, const ArrowArray *arr, const ArrowS
     fail(a, "%s: an Arrow dictionary of '%s' values cannot be appended to an ENUM column (the labels must be utf8 or large_utf8)", cn, dfmt);
     return false;
   }
-  const ArrowArray *d = arr->dictionary;
-  if (!d) {
-    fail(a, "%s: the Arrow dictionary array is missing", cn);
-    return false;
-  }
-  const char f = fmt[0];
-  ci->w_in = f == 'c' || f == 'C' ? 1 : f == 's' || f == 'S' ? 2 : f == 'i' || f == 'I' ? 4 : 8;
-  ci->rev_op = copy_op(ci->w_in);
-  ci->index_signed = f >= 'a' && f <= 'z';
-  ci->dict_large = dfmt[0] == 'U';
-  ci->dict_len = d->length;
-  ci->dict_bit_offset = d->offset;
-  ci->dict_validity = (d->null_count != 0 && d->n_buffers > 0) ? (const uint8_t *)d->buffers[0] : nullptr;
-  ci->dict_offsets = d->n_buffers > 1 && d->buffers[1] ? (const uint8_t *)d->buffers[1] + (size_t)d->offset * (ci->dict_large ? 8 : 4) : nullptr;
-  ci->dict_data = d->n_buffers > 2 && d->buffers[2] ? (const uint8_t *)d->buffers[2] : kNoData;
-  if (d->length > 0 && !ci->dict_offsets) {
-    fail(a, "%s: the Arrow dictionary has no offsets buffer", cn);
-    return false;
-  }
-  return true;
+  map_dict_indices(fmt, ci);
+  return bind_dict(a, cn, arr->dictionary, dfmt, ci);
 }
 
 // Arrow array `arr` -> column j (a table column or a field column) of `cols`: row i of the batch is logical row at + i of
@@ -1118,6 +1393,7 @@ bool map_column(App *a, int j, const ArrowArray *arr, const ArrowSchema *sch, in
       !(t == DMB_TYPE_LIST ? map_list(a, j, arr, sch, &ci, &children[(size_t)j])
         : t == DMB_TYPE_ENUM ? map_enum(a, j, cn, arr, sch, &ci)
         : t == DMB_TYPE_STRUCT ? map_struct(a, j, cn, arr, sch, &ci)
+        : (t == DMB_TYPE_VARCHAR || t == DMB_TYPE_BLOB) && sch->dictionary ? map_string_dict(a, cn, arr, sch, t, &ci)
                                : map_format(a, cn, field ? "field format" : "format", sch->format, t, &a->rows[(size_t)j].dec_prec,
                                             &a->rows[(size_t)j].dec_scale, &ci))) {
     if (!a->error[0]) fail(a, "append_arrow_batch: %s is malformed", cn);
@@ -1129,6 +1405,7 @@ bool map_column(App *a, int j, const ArrowArray *arr, const ArrowSchema *sch, in
     return false;
   }
   bind_buffers(ci, arr, arr->offset + at);
+  if (ci.is_view && !check_views(a, cn, arr)) return false;
   if (ci.is_struct) {
     const StructDecl &d = a->structs[(size_t)j];
     for (int f = 0; f < (int)d.types.size(); ++f) {

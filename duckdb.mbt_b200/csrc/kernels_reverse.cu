@@ -18,6 +18,25 @@
 
 namespace dmb {
 
+// rows of the warp whose first row is row0 that lie below nrows (0..32)
+__device__ __forceinline__ int rev_warp_live(int64_t nrows, int64_t row0) {
+  const int64_t left = nrows - row0;
+  return left <= 0 ? 0 : (left < 32 ? (int)left : 32);
+}
+
+// the validity word of that warp: bit k for row row0 + k, 0 past the live rows; an absent bitmap is all valid
+__device__ __forceinline__ uint32_t rev_warp_bits(const BitSrc &bs, bool has_bm, int live, int64_t row0) {
+  return live == 0 ? 0u : (has_bm ? load_bits32(bs.w, bs.base + row0, live) : (live == 32 ? 0xffffffffu : ((1u << live) - 1u)));
+}
+
+// an Arrow dictionary index, sign- or zero-extended; an unsigned 64-bit index past 2^63 comes out negative, i.e. out of
+// range as well
+template <typename I>
+__device__ __forceinline__ int64_t rev_dict_index(I raw, bool is_signed) {
+  constexpr int kShift = 64 - 8 * (int)sizeof(I);
+  return is_signed ? (int64_t)((uint64_t)raw << kShift) >> kShift : (int64_t)(uint64_t)raw;
+}
+
 // 64 validity bits for output word w (rows 64w..64w+63), rows >= nrows are 0
 __device__ __forceinline__ uint64_t rev_valid_word(const BitSrc &bs, bool has_bm, int64_t nrows, int64_t w) {
   const int64_t r0 = w << 6;
@@ -374,7 +393,7 @@ rev_mask_kernel(const dmb_rev_mask_job *__restrict__ jobs, int64_t nrows) {
 
 // ---- ENUM: labels -> positions (dmb_rev_enum_job).  One row per thread; a warp's 32 rows share one validity word, which
 // is also the mask word the ballot of the rows that got a position writes.
-extern __shared__ uint4 rev_enum_smem[];  // the lookup table or the remap, when it fits
+extern __shared__ uint4 rev_enum_smem[];  // the lookup table, the remap or a dictionary's string_t table, when it fits
 constexpr int kEnumSmemBytes = 48 << 10;
 
 // row `row` of a final-vector or remap launch: `code` is a position, DMB_ENUM_CODE_NULL or DMB_ENUM_CODE_MISSING (unused
@@ -464,7 +483,6 @@ template <typename I>
 __global__ void __launch_bounds__(kThreads)
 rev_enum_index_kernel(dmb_rev_enum_job job, int64_t nrows, int64_t capacity, int smem) {
   constexpr int U = 4;
-  constexpr int kShift = 64 - 8 * (int)sizeof(I);
   const uint32_t *remap = job.remap;
   if (smem) {
     uint32_t *s = reinterpret_cast<uint32_t *>(rev_enum_smem);
@@ -489,21 +507,147 @@ rev_enum_index_kernel(dmb_rev_enum_job job, int64_t nrows, int64_t capacity, int
 #pragma unroll
     for (int u = 0; u < U; ++u) {
       const int64_t row0 = base + u * kThreads + threadIdx.x - lane;
-      const int64_t left = nrows - row0;
-      const int live = left <= 0 ? 0 : (left < 32 ? (int)left : 32);
-      vb[u] = live == 0 ? 0u : (has_bm ? load_bits32(bs.w, bs.base + row0, live) : (live == 32 ? 0xffffffffu : ((1u << live) - 1u)));
+      vb[u] = rev_warp_bits(bs, has_bm, rev_warp_live(nrows, row0), row0);
     }
 #pragma unroll
     for (int u = 0; u < U; ++u) {
       const int64_t row = base + u * kThreads + threadIdx.x;
-      // sign- or zero-extended; an unsigned 64-bit index past 2^63 comes out negative, i.e. out of range as well
-      const int64_t idx = job.index_signed ? (int64_t)((uint64_t)raw[u] << kShift) >> kShift : (int64_t)(uint64_t)raw[u];
+      const int64_t idx = rev_dict_index(raw[u], job.index_signed != 0);
       uint32_t code = DMB_ENUM_CODE_MISSING;
       if (((vb[u] >> lane) & 1u) && idx >= 0 && idx < job.dict_len) code = remap[idx];
       enum_emit(job, row, nrows, vb[u], code, nulls, first_bad);
     }
   }
   enum_finish(job, nulls, first_bad);
+}
+
+// ---- VARCHAR / BLOB from Arrow string views (dmb_rev_view_job): a 16 B -> 16 B streaming transform, four rows per thread
+// in flight; a warp's 32 rows share one validity word, which is also the mask word.
+__device__ __forceinline__ uint32_t keep_bytes(uint32_t word, int nb) { return nb >= 4 ? word : (nb <= 0 ? 0u : (word & ((1u << (8 * nb)) - 1u))); }
+
+__global__ void __launch_bounds__(kThreads)
+rev_view_kernel(dmb_rev_view_job job, int64_t nrows, int64_t capacity) {
+  constexpr int U = 4;
+  const uint4 *in = reinterpret_cast<const uint4 *>(job.in_views);
+  const longlong2 *bufs = reinterpret_cast<const longlong2 *>(job.buffers);
+  const int lane = threadIdx.x & 31;
+  const bool has_bm = job.in_validity != nullptr;
+  const BitSrc bs = bit_src(job.in_validity, job.in_bit_offset);
+  uint4 *out = reinterpret_cast<uint4 *>(job.out);
+  uint32_t *out_val32 = reinterpret_cast<uint32_t *>(job.out_validity);
+  int nulls = 0;
+  unsigned long long first_bad = ~0ull;
+  for (int64_t base = (int64_t)blockIdx.x * (U * kThreads); base < capacity; base += (int64_t)gridDim.x * (U * kThreads)) {
+    uint4 v[U];
+    uint32_t vb[U];
+#pragma unroll
+    for (int u = 0; u < U; ++u) {
+      const int64_t row = base + u * kThreads + threadIdx.x;
+      v[u] = row < nrows ? ld_stream(in + row) : make_uint4(0, 0, 0, 0);
+    }
+#pragma unroll
+    for (int u = 0; u < U; ++u) {
+      const int64_t row0 = base + u * kThreads + threadIdx.x - lane;
+      const int live = rev_warp_live(nrows, row0);
+      vb[u] = rev_warp_bits(bs, has_bm, live, row0);
+      if (lane == 0) {
+        if (out_val32) out_val32[row0 >> 5] = vb[u];
+        nulls += live - __popc(vb[u]);
+      }
+    }
+#pragma unroll
+    for (int u = 0; u < U; ++u) {
+      const int64_t row = base + u * kThreads + threadIdx.x;
+      uint4 e = make_uint4(0, 0, 0, 0);
+      if ((vb[u] >> lane) & 1u) {
+        const int len = (int)v[u].x;
+        bool bad = len < 0;
+        if (len >= 0 && len <= 12) {
+          e = make_uint4(v[u].x, keep_bytes(v[u].y, len), keep_bytes(v[u].z, len - 4), keep_bytes(v[u].w, len - 8));
+        } else if (len > 12) {
+          const uint32_t idx = v[u].z;
+          const int off = (int)v[u].w;
+          bad = (int64_t)idx >= job.nbuffers || off < 0;
+          if (!bad) {
+            const longlong2 b = __ldg(bufs + idx);
+            bad = (int64_t)off + len > b.y;
+            const uint64_t p = (uint64_t)b.x + (uint64_t)off;
+            if (!bad) e = make_uint4(v[u].x, v[u].y, (uint32_t)p, (uint32_t)(p >> 32));
+          }
+        }
+        if (bad && (unsigned long long)row < first_bad) first_bad = (unsigned long long)row;
+      }
+      st_stream(out + row, e);
+    }
+  }
+  if (first_bad != ~0ull) atomicMin(job.error, first_bad);
+  if (job.null_count && lane == 0 && nulls) atomicAdd(job.null_count, (unsigned long long)nulls);
+}
+
+// ---- VARCHAR / BLOB from Arrow dictionary indices (dmb_rev_dict_job): row r takes table[index] (one 16-byte entry, from
+// shared memory when the table fits); four rows per thread in flight, the mask word is the ballot of the rows that got a
+// valid entry.
+template <typename I>
+__global__ void __launch_bounds__(kThreads)
+rev_dict_kernel(dmb_rev_dict_job job, int64_t nrows, int64_t capacity, int smem) {
+  constexpr int U = 4;
+  const uint4 *tab = reinterpret_cast<const uint4 *>(job.table);
+  if (smem) {
+    for (int64_t i = threadIdx.x; i < job.dict_len; i += kThreads) rev_enum_smem[i] = __ldg(tab + i);
+    __syncthreads();
+    tab = rev_enum_smem;
+  }
+  const I *in = reinterpret_cast<const I *>(job.in_indices);
+  const int lane = threadIdx.x & 31;
+  const bool has_bm = job.in_validity != nullptr;
+  const BitSrc bs = bit_src(job.in_validity, job.in_bit_offset);
+  uint4 *out = reinterpret_cast<uint4 *>(job.out);
+  uint32_t *out_val32 = reinterpret_cast<uint32_t *>(job.out_validity);
+  int nulls = 0;
+  unsigned long long first_bad = ~0ull;
+  for (int64_t base = (int64_t)blockIdx.x * (U * kThreads); base < capacity; base += (int64_t)gridDim.x * (U * kThreads)) {
+    I raw[U];
+    uint32_t vb[U];
+#pragma unroll
+    for (int u = 0; u < U; ++u) {
+      const int64_t row = base + u * kThreads + threadIdx.x;
+      raw[u] = row < nrows ? __ldcs(in + row) : I(0);
+    }
+#pragma unroll
+    for (int u = 0; u < U; ++u) {
+      const int64_t row0 = base + u * kThreads + threadIdx.x - lane;
+      vb[u] = rev_warp_bits(bs, has_bm, rev_warp_live(nrows, row0), row0);
+    }
+#pragma unroll
+    for (int u = 0; u < U; ++u) {
+      const int64_t row = base + u * kThreads + threadIdx.x;
+      const int64_t idx = rev_dict_index(raw[u], job.index_signed != 0);
+      uint4 e = make_uint4(0, 0, 0, 0);
+      bool ok = false;
+      if ((vb[u] >> lane) & 1u) {
+        if (idx < 0 || idx >= job.dict_len) {
+          if ((unsigned long long)row < first_bad) first_bad = (unsigned long long)row;
+        } else {
+          const uint4 t = tab[idx];
+          ok = t.x != DMB_DICT_ENTRY_NULL;
+          if (ok) e = t;
+        }
+      }
+      const uint32_t word = __ballot_sync(0xffffffffu, ok);
+      st_stream(out + row, e);
+      if (lane == 0) {
+        out_val32[row >> 5] = word;
+        nulls += rev_warp_live(nrows, row) - __popc(word);
+      }
+    }
+  }
+  if (first_bad != ~0ull) atomicMin(job.error, first_bad);
+  if (job.null_count && lane == 0 && nulls) atomicAdd(job.null_count, (unsigned long long)nulls);
+}
+
+__global__ void rev_dict_mark_kernel(dmb_string_t *table, const uint64_t *masks, int64_t n) {
+  for (int64_t i = (int64_t)blockIdx.x * kThreads + threadIdx.x; i < n; i += (int64_t)gridDim.x * kThreads)
+    if (!((__ldg(masks + (i >> 6)) >> (i & 63)) & 1ull)) reinterpret_cast<uint32_t *>(table + i)[0] = DMB_DICT_ENTRY_NULL;
 }
 
 // the key of a label on the host: what rev_enum_string_kernel computes from the row's bytes
@@ -600,6 +744,53 @@ extern "C" int32_t dmb_dev_rev_enum_batch(const dmb_rev_enum_job *job, int64_t n
     default: rev_enum_index_kernel<unsigned long long><<<gx, kThreads, smem, st>>>(*job, nrows, chunks, smem); break;
   }
   return check_cuda(cudaGetLastError(), "rev_enum_index_kernel launch");
+}
+
+extern "C" int32_t dmb_dev_rev_view_batch(const dmb_rev_view_job *job, int64_t nrows, void *stream) {
+  if (!job) { set_error("dmb_dev_rev_view_batch: job is null"); return -1; }
+  if (nrows <= 0) return 0;
+  if (!job->in_views || !job->out || !job->error || job->nbuffers < 0 || (job->nbuffers && !job->buffers) ||
+      (reinterpret_cast<uintptr_t>(job->in_views) & 15u)) {
+    set_error("dmb_dev_rev_view_batch: a required pointer is null or the views are not 16-byte aligned");
+    return -1;
+  }
+  const int64_t capacity = ((nrows + kVec - 1) / kVec) * (int64_t)kVec;  // a multiple of 4 * kThreads
+  const int64_t blocks = capacity / (4 * kThreads), max_grid = (int64_t)kNumSMs * 8;
+  const int gx = (int)(blocks < max_grid ? blocks : max_grid);
+  rev_view_kernel<<<gx, kThreads, 0, (cudaStream_t)stream>>>(*job, nrows, capacity);
+  return check_cuda(cudaGetLastError(), "rev_view_kernel launch");
+}
+
+extern "C" int32_t dmb_dev_rev_dict_batch(const dmb_rev_dict_job *job, int64_t nrows, void *stream) {
+  if (!job) { set_error("dmb_dev_rev_dict_batch: job is null"); return -1; }
+  if (nrows <= 0) return 0;
+  const int iw = job->index_width;
+  if (iw != 1 && iw != 2 && iw != 4 && iw != 8) { set_error("dmb_dev_rev_dict_batch: index_width %d", iw); return -1; }
+  if (!job->in_indices || !job->out || !job->out_validity || !job->error || job->dict_len < 0 || (job->dict_len && !job->table)) {
+    set_error("dmb_dev_rev_dict_batch: a required pointer is null");
+    return -1;
+  }
+  const int64_t capacity = ((nrows + kVec - 1) / kVec) * (int64_t)kVec;
+  const size_t tb = (size_t)job->dict_len * sizeof(dmb_string_t);
+  const int smem = tb <= (size_t)kEnumSmemBytes ? (int)tb : 0;
+  const int64_t blocks = capacity / (4 * kThreads), max_grid = (int64_t)kNumSMs * 8;
+  const int gx = (int)(blocks < max_grid ? blocks : max_grid);
+  cudaStream_t st = (cudaStream_t)stream;
+  switch (iw) {
+    case 1: rev_dict_kernel<uint8_t><<<gx, kThreads, smem, st>>>(*job, nrows, capacity, smem); break;
+    case 2: rev_dict_kernel<unsigned short><<<gx, kThreads, smem, st>>>(*job, nrows, capacity, smem); break;
+    case 4: rev_dict_kernel<unsigned int><<<gx, kThreads, smem, st>>>(*job, nrows, capacity, smem); break;
+    default: rev_dict_kernel<unsigned long long><<<gx, kThreads, smem, st>>>(*job, nrows, capacity, smem); break;
+  }
+  return check_cuda(cudaGetLastError(), "rev_dict_kernel launch");
+}
+
+extern "C" int32_t dmb_dev_rev_dict_mark(dmb_string_t *table, const uint64_t *masks, int64_t n, void *stream) {
+  if (n <= 0) return 0;
+  if (!table || !masks) { set_error("dmb_dev_rev_dict_mark: table or masks is null"); return -1; }
+  const int64_t blocks = (n + kThreads - 1) / kThreads, max_grid = (int64_t)kNumSMs * 8;
+  rev_dict_mark_kernel<<<(int)(blocks < max_grid ? blocks : max_grid), kThreads, 0, (cudaStream_t)stream>>>(table, masks, n);
+  return check_cuda(cudaGetLastError(), "rev_dict_mark_kernel launch");
 }
 
 extern "C" int32_t dmb_dev_rev_fixed_batch(const dmb_rev_fixed_job *jobs_dev, const dmb_rev_fixed_job *jobs_host,

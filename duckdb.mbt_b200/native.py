@@ -76,6 +76,25 @@ class RevEnumJob(C.Structure):
 ENUM_CODE_NULL, ENUM_CODE_MISSING, ENUM_SLOT_BYTES = 0xFFFFFFFE, 0xFFFFFFFF, 32
 
 
+class ViewBuffer(C.Structure):
+    _fields_ = [("host_base", C.c_uint64), ("size", C.c_int64)]
+
+
+class RevViewJob(C.Structure):
+    _fields_ = [("in_views", C.c_void_p), ("in_validity", C.c_void_p), ("in_bit_offset", C.c_int64), ("buffers", C.c_void_p),
+                ("nbuffers", C.c_int64), ("out", C.c_void_p), ("out_validity", C.c_void_p), ("null_count", C.c_void_p),
+                ("error", C.c_void_p)]
+
+
+class RevDictJob(C.Structure):
+    _fields_ = [("in_indices", C.c_void_p), ("in_validity", C.c_void_p), ("in_bit_offset", C.c_int64), ("table", C.c_void_p),
+                ("dict_len", C.c_int64), ("out", C.c_void_p), ("out_validity", C.c_void_p), ("null_count", C.c_void_p),
+                ("error", C.c_void_p), ("index_width", C.c_int32), ("index_signed", C.c_int32)]
+
+
+DICT_ENTRY_NULL = 0xFFFFFFFF
+
+
 class EnumDict(C.Structure):
     _fields_ = [("size", C.c_uint32), ("reserved", C.c_uint32), ("offsets", C.c_void_p), ("data", C.c_void_p)]
 
@@ -155,6 +174,7 @@ EXPORTED_SYMBOLS = [
     "dmb_dev_fixed_batch", "dmb_op_out_width", "dmb_phys_width", "dmb_dev_string_scratch_bytes",
     "dmb_dev_string_error", "dmb_dev_string_batch", "dmb_dev_set_lookback_limit_ns", "dmb_dev_rev_fixed_batch", "dmb_dev_rev_string_batch",
     "dmb_dev_rev_list_batch", "dmb_dev_rev_mask_batch", "dmb_rev_list_cut", "dmb_dev_rev_enum_batch", "dmb_rev_enum_table", "dmb_rev_enum_lookup",
+    "dmb_dev_rev_view_batch", "dmb_dev_rev_dict_batch", "dmb_dev_rev_dict_mark",
     "dmb_dev_valid_bytes_to_masks", "dmb_dev_make_string_t", "dmb_dev_blob_escape", "dmb_render_supported", "dmb_render_slot_bytes", "dmb_dev_render_text", "dmb_dev_enum_to_string_t", "dmb_dev_enum_utf8", "dmb_dev_list_scratch_bytes", "dmb_dev_list_batch",
     "duckdb_mb_gpu_last_error", "duckdb_mb_gpu_device_count", "duckdb_mb_gpu_bind_numa", "duckdb_mb_gpu_ctx_create",
     "duckdb_mb_gpu_ctx_destroy", "duckdb_mb_gpu_ctx_sync", "duckdb_mb_gpu_host_alloc", "duckdb_mb_gpu_host_free",
@@ -269,6 +289,12 @@ def lib():
     L.duckdb_mb_gpu_appender_struct_field.argtypes = [vp, i32, i32, C.POINTER(vp), C.POINTER(vp)]
     L.dmb_dev_rev_enum_batch.restype = i32
     L.dmb_dev_rev_enum_batch.argtypes = [C.POINTER(RevEnumJob), i64, vp]
+    L.dmb_dev_rev_view_batch.restype = i32
+    L.dmb_dev_rev_view_batch.argtypes = [C.POINTER(RevViewJob), i64, vp]
+    L.dmb_dev_rev_dict_batch.restype = i32
+    L.dmb_dev_rev_dict_batch.argtypes = [C.POINTER(RevDictJob), i64, vp]
+    L.dmb_dev_rev_dict_mark.restype = i32
+    L.dmb_dev_rev_dict_mark.argtypes = [vp, vp, i64, vp]
     L.dmb_rev_enum_table.restype = i32
     L.dmb_rev_enum_table.argtypes = [C.POINTER(EnumDict), C.c_uint32, vp]
     L.dmb_rev_enum_lookup.restype = i64

@@ -473,6 +473,58 @@ int32_t dmb_rev_enum_table(const struct dmb_enum_dict *dict, uint32_t table_size
 /* host only: the position of `bytes` in such a table, -1 when it is not a label (the device's probe, run on the host) */
 int64_t dmb_rev_enum_lookup(const void *slots, uint32_t table_size, const struct dmb_enum_dict *dict, const uint8_t *bytes, uint32_t len);
 
+/* Arrow string views (utf8_view / binary_view) -> string_t.  A view is 16 bytes, {int32 len, 12 inline bytes} when
+ * len <= 12, else {int32 len, 4-byte prefix, int32 buffer index, int32 offset}; a string_t is the same 16 bytes inline and
+ * {len, prefix, 8-byte pointer} otherwise.  So the kernel reads no string bytes: an inline view is copied with its bytes
+ * past len zeroed, a pointer view takes its prefix from the view and points at buffers[index].host_base + offset, in
+ * place in the caller's host buffer.  A NULL row is NULL with payload 0.  A valid row with a negative len, or a pointer view
+ * whose index is >= nbuffers, whose offset is negative or whose offset + len passes that buffer's size is an error:
+ * *error takes the smallest such row (atomicMin; the caller sets it to ~0 first).  out and out_validity are written for
+ * whole 2048-row chunks (out_validity may be NULL, for a LIST child whose masks the list kernel writes). */
+typedef struct dmb_view_buffer {
+  uint64_t host_base;              /* host address of an Arrow data buffer */
+  int64_t size;                    /* its size in bytes                    */
+} dmb_view_buffer;
+
+typedef struct dmb_rev_view_job {
+  const void *in_views;            /* 16-byte views at the slice start, 16-byte aligned */
+  const uint8_t *in_validity;      /* bitmap or NULL                                    */
+  int64_t in_bit_offset;
+  const dmb_view_buffer *buffers;  /* device table of the array's data buffers          */
+  int64_t nbuffers;
+  dmb_string_t *out;               /* string_t slab: chunk k at k*2048 entries          */
+  uint64_t *out_validity;
+  unsigned long long *null_count;
+  unsigned long long *error;
+} dmb_rev_view_job;
+
+int32_t dmb_dev_rev_view_batch(const dmb_rev_view_job *job, int64_t nrows, void *stream);
+
+/* Arrow dictionary indices (1/2/4/8 bytes, signed or not) -> string_t, gathered from `table`: the dictionary's dict_len
+ * entries as string_t (converted once by dmb_dev_rev_string_batch or dmb_dev_rev_view_batch), a NULL entry marked by
+ * len DMB_DICT_ENTRY_NULL (dmb_dev_rev_dict_mark).  A NULL row, and a valid row whose entry is NULL, is NULL with
+ * payload 0.  A valid row whose index is outside [0, dict_len) is an error: *error takes the smallest such row
+ * (atomicMin; the caller sets it to ~0 first).  out and out_validity are written for whole 2048-row chunks; out_validity
+ * is required, and is a dense bitmap of the rows (bit r: row r). */
+#define DMB_DICT_ENTRY_NULL 0xFFFFFFFFu
+typedef struct dmb_rev_dict_job {
+  const void *in_indices;          /* the first index of the slice */
+  const uint8_t *in_validity;      /* bitmap or NULL               */
+  int64_t in_bit_offset;
+  const dmb_string_t *table;       /* [dict_len]                   */
+  int64_t dict_len;
+  dmb_string_t *out;
+  uint64_t *out_validity;
+  unsigned long long *null_count;
+  unsigned long long *error;
+  int32_t index_width;             /* 1 / 2 / 4 / 8                */
+  int32_t index_signed;
+} dmb_rev_dict_job;
+
+int32_t dmb_dev_rev_dict_batch(const dmb_rev_dict_job *job, int64_t nrows, void *stream);
+/* entry i of `table` whose bit i of `masks` (a dense bitmap) is 0 gets len DMB_DICT_ENTRY_NULL */
+int32_t dmb_dev_rev_dict_mark(dmb_string_t *table, const uint64_t *masks, int64_t n, void *stream);
+
 /* byte-per-row validity (MoonBit Array[Bool], src/duckdb_arrow_native.mbt:646-650) -> per-chunk
  * uint64 masks via warp ballots */
 int32_t dmb_dev_valid_bytes_to_masks(const uint8_t *valid_bytes, uint64_t *out_validity,
@@ -790,7 +842,13 @@ moonbit_bytes_t duckdb_mb_gpu_appender_error(duckdb_mb_gpu_appender *a); /* cf. 
 int32_t duckdb_mb_gpu_appender_state(duckdb_mb_gpu_appender *a);
 int64_t duckdb_mb_gpu_appender_row_count(duckdb_mb_gpu_appender *a);
 /* bulk append of one Arrow record batch (struct array, one child per column); legal in
- * Ready / Flushed, like BeginRow; returns 1/0 with the per-handle error string set */
+ * Ready / Flushed, like BeginRow; returns 1/0 with the per-handle error string set.
+ * VARCHAR / BLOB columns (and fields and LIST children of that type) take utf8 / large_utf8 (binary / large_binary), string
+ * views (vu / vz; the sizes buffer of the C data interface is required) and dictionary arrays of those (indices c C s S i I
+ * l L); the table holds what the same array cast to utf8 / binary gives.  A malformed view or an out-of-range index on a
+ * valid row fails the append before its sub-batch reaches the sink (a LIST child's element: one its own bitmap marks
+ * valid, also under a NULL list row).  A dictionary of views is converted whole: a malformed view in it fails the append
+ * whether or not a row refers to it. */
 int32_t duckdb_mb_gpu_append_arrow_batch(duckdb_mb_gpu_appender *a, const struct ArrowArray *batch,
                                          const struct ArrowSchema *schema);
 int32_t duckdb_mb_gpu_appender_flush(duckdb_mb_gpu_appender *a); /* cf. duckdb_mb_flush :1237 */
